@@ -13,8 +13,11 @@ shard with no data-path collective -> weak scaling) so the rounds compare; the s
   "post"    the other half of BASELINE's metric: distance build, PSM and point-estimate seconds (rank 0, N = 1).
 Prints ONE JSON line (see the task contract).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   torchrun ... bench.py --gpus N ...        (N > 1)
+
+--dump-outputs DIR writes what the headline run's last timed step recorded (see write_outputs) as DIR/<name>.npy:
+the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -134,8 +137,35 @@ def emit(line):
         os.write(_REAL_STDOUT, data)
 
 
-def timed_sampler(pkg, torch, dist, world, data, params, lab, chains, chain0, args, warm, steps, local_rank):
-    """`warm` untimed sweeps then `steps` timed ones (one kernel launch each) of `chains` chains on this rank.
+DUMP_BYTES = 48 << 20      # label rows written by --dump-outputs; more chains than fit are sampled (seeded)
+
+
+def write_outputs(smp, chain0, out_dir):
+    """The sample every chain recorded in the last step, as samples(c) returns it for that step: labels (float32, exact
+    below 2^24), K, r, p, loglik, logposterior (float64), and that iteration's r / split-merge acceptances (float32).
+    `chain` holds the global chain ids of the rows; when the label rows of all chains exceed DUMP_BYTES a fixed, seeded
+    subset of the chains is written."""
+    n, iters, numMH = smp.data.n, smp.options.numiters, smp.options.numMH
+    keep = np.arange(smp.nchains)
+    if smp.nchains * n * 4 > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(smp.nchains, max(DUMP_BYTES // (n * 4), 1), replace=False))
+    cols = {k: [] for k in ("labels", "K", "r", "p", "loglik", "logposterior", "r_acc", "sm_acc", "sm_split")}
+    for c in keep:
+        s = smp.samples(int(c))
+        for k in ("labels", "K", "r", "p", "loglik", "logposterior", "r_acc"):
+            cols[k].append(s[k][-1])
+        for k in ("sm_acc", "sm_split"):
+            cols[k].append(s[k].reshape(iters, numMH)[-1])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "chain.npy"), (chain0 + keep).astype(np.float64))
+    for k, v in cols.items():
+        dt = np.float64 if k in ("K", "r", "p", "loglik", "logposterior") else np.float32
+        np.save(os.path.join(out_dir, f"{k}.npy"), np.stack(v).astype(dt))
+
+
+def timed_sampler(pkg, torch, dist, world, data, params, lab, chains, chain0, args, warm, steps, local_rank, dump=None):
+    """`warm` untimed sweeps then `steps` timed ones (one kernel launch each) of `chains` chains on this rank; with `dump`
+    a directory, write_outputs() then writes what the last timed step recorded.
     Returns (device seconds max over ranks, wall seconds max over ranks, moves per chain-sweep, K of chain 0, clock summary)."""
     opts = pkg.MCMCOptionsList(numiters=warm + steps, burnin=0, thin=1, numGibbs=args.numGibbs, numMH=args.numMH)
     rp = [pkg.init_rp(params, args.seed, chain0 + c) for c in range(chains)]
@@ -170,6 +200,8 @@ def timed_sampler(pkg, torch, dist, world, data, params, lab, chains, chain0, ar
         sm = tt.clone(); dist.all_reduce(sm, op=dist.ReduceOp.SUM)
         tt = torch.stack([mx[0], mx[1], sm[2] / world])
     Kfinal = int(smp.samples(0)["K"][-1])
+    if dump:
+        write_outputs(smp, chain0, dump)
     smp.close()
     return float(tt[0]), float(tt[1]), float(tt[2]), Kfinal, clk.summary(), (labs, r0, p0)
 
@@ -254,12 +286,16 @@ def main():
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--no-post", action="store_true")
     ap.add_argument("--cpu-steps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline run's last timed step recorded as DIR/<name>.npy (rank 0's chains)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     W = max(args.warmup, 0)
-    steps = max(args.steps, 1)
+    steps = args.steps
     workload = (f"generatemixture(N={args.n}, K={args.K}; alpha={args.K}, sigma={args.sigma}, dim={args.dim}) seed {args.seed}, "
                 f"{args.chains} chains per GPU, numGibbs={args.numGibbs}, numMH={args.numMH}, every sweep recorded")
     config = {"workload": workload, "n": args.n, "chains_per_gpu": args.chains, "hyperparameters": "from true labels as prior.jl:73-110",
@@ -307,7 +343,8 @@ def main():
 
     # ---- headline: `chains` chains per GPU (weak scaling, round 1's definition) ----
     dev_s, wall_s, moves, Kfinal, clocks, (labs, r0, p0) = timed_sampler(pkg, torch, dist, world, data, params, lab, args.chains, chain0,
-                                                                        args, W, steps, local_rank)
+                                                                        args, W, steps, local_rank,
+                                                                        dump=args.dump_outputs if rank == 0 else None)
     value = world * args.chains * steps / dev_s
 
     # ---- configs[2] literally: `chains` chains in total over the N GPUs (strong scaling) ----

@@ -4,6 +4,7 @@ src/pointestimate.jl:19-26, src/utils.jl:103-108), and the oracle's numpy restat
 import ctypes
 import os
 import re
+import struct
 import numpy as np
 import pytest
 
@@ -141,9 +142,74 @@ def test_reference_utils_cases(pkg):
         assert pkg.prettytime(t) == want, (t, pkg.prettytime(t), want)
 
 
-def test_example_dataset_reader(pkg, golden):
-    """example_dataset(n) / example_datasets() (example_data.jl:33-71): the package copy, and -- where the reference's
-    own HDF5 file is present (the build container) -- the same arrays through the minimal HDF5 reader."""
+_UNDEF = 0xFFFFFFFFFFFFFFFF
+
+
+def _q(v):
+    return struct.pack("<Q", v)
+
+
+def _write_h5(path, groups):
+    """A small HDF5 file of the layout h5min.py reads (that of RedClust.jl's data/example_datasets.h5): superblock
+    version 0, an old-style root group (symbol-table B-tree + local heap) holding compact new-style groups (link
+    messages) of contiguous little-endian int64 / float64 datasets.  groups: {group: {dataset: array}}."""
+    buf = bytearray(96)                                              # superblock + root symbol-table entry, written last
+
+    def put(b):
+        buf.extend(b"\0" * (-len(buf) % 8))
+        addr = len(buf)
+        buf.extend(b)
+        return addr
+
+    def msg(mtype, payload):
+        payload += b"\0" * (-len(payload) % 8)
+        return struct.pack("<HHB3x", mtype, len(payload), 0) + payload
+
+    def ohdr(msgs):                                                  # version-1 object header
+        body = b"".join(msgs)
+        return put(struct.pack("<BBHII4x", 1, 0, len(msgs), 1, len(body)) + body)
+
+    def entry(name_off, addr, cache=0, scratch=b"\0" * 16):          # symbol-table entry
+        return _q(name_off) + _q(addr) + struct.pack("<I4x", cache) + scratch
+
+    def dataset(a):
+        a = np.ascontiguousarray(a)
+        assert a.dtype in (np.int64, np.float64)
+        data = put(a.tobytes())
+        space = struct.pack("<BBB5x", 1, a.ndim, 0) + b"".join(_q(d) for d in a.shape)
+        if a.dtype == np.int64:                                      # fixed-point, signed
+            dtype = struct.pack("<BBBBIHH", 0x10, 0x08, 0, 0, 8, 0, 64)
+        else:                                                        # IEEE binary64
+            dtype = struct.pack("<BBBBIHHBBBBI", 0x11, 0x20, 63, 0, 8, 0, 64, 52, 11, 0, 52, 1023)
+        return ohdr([msg(0x01, space), msg(0x03, dtype), msg(0x08, struct.pack("<BB", 3, 1) + _q(data) + _q(a.nbytes))])
+
+    def group(members):                                              # link info, group info, one link message per member
+        links = [msg(0x02, struct.pack("<BB", 0, 0) + _q(_UNDEF) + _q(_UNDEF)), msg(0x0A, struct.pack("<BB", 0, 0))]
+        for name, addr in members.items():
+            links.append(msg(0x06, struct.pack("<BBB", 1, 0, len(name)) + name.encode() + _q(addr)))
+        return ohdr(links)
+
+    gaddr = {g: group({k: dataset(v) for k, v in ds.items()}) for g, ds in groups.items()}
+    names = sorted(gaddr)
+    heapdata, offs = bytearray(8), {}                                # offset 0: the empty name
+    for g in names:
+        offs[g] = len(heapdata)
+        heapdata += g.encode() + b"\0" * (8 - len(g) % 8)
+    heap = put(b"HEAP" + struct.pack("<B3x", 0) + _q(len(heapdata)) + _q(_UNDEF) + _q(put(bytes(heapdata))))
+    snod = put(b"SNOD" + struct.pack("<BBH", 1, 0, len(names)) + b"".join(entry(offs[g], gaddr[g]) for g in names)
+               + bytes(40 * (8 - len(names))))                      # 2 x group leaf K (4) entries per node
+    btree = put(b"TREE" + struct.pack("<BBH", 0, 0, 1) + _q(_UNDEF) + _q(_UNDEF) + _q(0) + _q(snod) + _q(offs[names[-1]]))
+    root = ohdr([msg(0x11, _q(btree) + _q(heap))])
+    buf[:96] = (b"\x89HDF\r\n\x1a\n" + bytes([0, 0, 0, 0, 0, 8, 8, 0]) + struct.pack("<HHI", 4, 16, 0)
+                + _q(0) + _q(_UNDEF) + _q(len(buf)) + _q(_UNDEF) + entry(0, root, 1, _q(btree) + _q(heap)))
+    with open(path, "wb") as f:
+        f.write(buf)
+
+
+def test_example_dataset_reader(pkg, golden, tmp_path):
+    """example_dataset(n) / example_datasets() (example_data.jl:33-71): the package copy, and the same arrays through the
+    minimal HDF5 reader from a file of the reference's layout.  The golden arrays are RedClust.jl's own
+    data/example_datasets.h5 (tests/golden/make_golden.py); here they are written back into such a file."""
     for n in (1, 2, 3):
         d = pkg.example_dataset(n)
         assert len(d["points"]) == 100 and d["points"][0].shape == golden[n]["points"][0].shape
@@ -158,12 +224,13 @@ def test_example_dataset_reader(pkg, golden):
     assert f.keys() == ["example1", "example2", "example3"]
     assert "distance_matrix" in f["example2"].keys()
     f.close()
-    ref = "/root/reference/data/example_datasets.h5"
-    if os.path.exists(ref):
-        h = pkg.example_datasets(ref)
-        assert h.keys() == ["example1", "example2", "example3"]
-        for n in (1, 2, 3):
-            for name in golden[n]:
-                assert np.array_equal(h[f"example{n}"][name], golden[n][name]), (n, name)
-        h.close()
-        assert np.array_equal(pkg.example_dataset(3, path=ref)["distmatrix"], golden[3]["distance_matrix"])
+    ref = str(tmp_path / "example_datasets.h5")
+    _write_h5(ref, {f"example{n}": golden[n] for n in (1, 2, 3)})
+    h = pkg.example_datasets(ref)
+    assert h.keys() == ["example1", "example2", "example3"]
+    for n in (1, 2, 3):
+        assert h[f"example{n}"].keys() == sorted(golden[n])
+        for name in golden[n]:
+            assert np.array_equal(h[f"example{n}"][name], golden[n][name]), (n, name)
+    h.close()
+    assert np.array_equal(pkg.example_dataset(3, path=ref)["distmatrix"], golden[3]["distance_matrix"])

@@ -1,5 +1,6 @@
 // Dependent-issue latency of the fp64 operations the sampler's sequential paths are made of (one warp, one SM),
 // and of rc_log / rc_exp / Philox as compiled for the kernels (-fmad=false).
+// Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -fmad=false -o fp64_latency fp64_latency.cu
 #include <cstdio>
 #include <cuda_runtime.h>
 #include "../../redclust.jl_b200/csrc/rc_math.h"
