@@ -128,14 +128,15 @@ int32_t rc_init_rp(const rc_params* params, uint64_t seed, int64_t chain_id, dou
 /* Allocate `nchains` independent chains (global chain ids chain_offset .. chain_offset+nchains-1)
  * on the data's device.  init_labels: nchains x n, 1-based, any slot ids in 1..n (src/types.jl:131-137);
  * init_r / init_p: nchains values.  slot_cap: max simultaneously live clusters per chain
- * (0 = default = maximum 128) -- the reference allows up to n (SURVEY.md H4); initial labels must lie in
+ * (0 = default = 128, at most 255) -- the reference allows up to n (SURVEY.md H4); initial labels must lie in
  * 1..slot_cap (relabel with sortlabels first).             */
 int32_t rc_sampler_create(const rc_data* d, const rc_options* opt, const rc_params* par,
                           int64_t nchains, int64_t chain_offset, const int64_t* init_labels,
                           const double* init_r, const double* init_p, uint64_t seed,
                           int32_t slot_cap, rc_sampler** out);
 /* Advance every chain by `iters` iterations of the loop at src/mcmc.jl:537-555
- * (iters < 0: run to numiters).  One persistent kernel launch per call.                       */
+ * (iters < 0: run to numiters).  One persistent kernel launch per call, or one per launch group when the chains'
+ * row sums do not all fit the device (each group rebuilds them from its labels first; same results).          */
 int32_t rc_sampler_run(rc_sampler* s, int64_t iters);
 /* Seconds of device time (CUDA events) spent in rc_sampler_run so far, and iterations done:
  * MCMCResult.runtime / mean_iter_time, src/mcmc.jl:536,586-587.                                */
@@ -171,7 +172,8 @@ int32_t rc_sampler_chain_status(const rc_sampler* s, int64_t chain);
 int64_t rc_sampler_overflowed(const rc_sampler* s);
 /* Diagnostic (no reference equivalent): the sampler keeps, per chain, the sums of every row of D / log D by cluster and
  * the cluster-by-cluster block sums incrementally (exact integers).  This rebuilds both from the current labels and
- * counts the 64-bit words that differ -- 0 / 0 unless an update was lost; -1 / -1 in streaming mode.                */
+ * counts the 64-bit words that differ -- 0 / 0 unless an update was lost; -1 / -1 before the first run.  With launch
+ * groups only the chains of the group launched last still have their row sums: those are checked.                */
 int32_t rc_sampler_check_sums(const rc_sampler* s, int64_t* mismatches_S, int64_t* mismatches_W);
 /* Posterior co-clustering counts of the device-resident samples of chains [chain0, chain0+nch):
  * sum(adjacencymatrix.(clusts)) (src/mcmc.jl:560, src/utils.jl:59-63) as exact int32 counts in a

@@ -33,37 +33,37 @@ struct rc_sampler {
   rc_params par;
   int64_t nchains, chain_offset, numsamples;
   uint64_t seed;
-  int cap, tiles, npad_max, G;
-  int nsm;                     // SMs of the device
+  int cap;
   int device;                  // copied from the data handle: the sampler may be destroyed after it
   int64_t n;
-  size_t smem;
   // device
   double *LGA, *LGZ, *LOGN;
   uint8_t* labels; int* sizes; double *r, *p; int* status;
-  rc_i128 *WD, *WL, *WDbak, *WLbak; uint8_t* labbak; int* szbak; longlong2* T; unsigned short* Slist;
-  uint8_t* origM; longlong4* AB; double2* L2s; double2* NZ; double* LPR; longlong2* DG; double* terms;
-  long long* stats; unsigned* gridbar; bool coresident;
-  double2* Cc; unsigned *Vv, *epochs;   // incremental mode: cached per-slot terms, per-point / per-slot change counts that validate them
-  int tw_smem, shortcuts;
-  void* Rs;                    // row summaries of the incremental scan (nchains x n x 32 B)
+  rc_i128 *WD, *WL, *WDbak, *WLbak; uint8_t* labbak; int* szbak; unsigned short* Slist;
+  uint8_t* origM; longlong4* AB; double2* L2s; double2* NZ; longlong2* DG; double* terms;
+  long long* stats;
+  // Group state: what k_chain_inc keeps per chain that can be rebuilt from the labels at any launch, allocated for `group`
+  // chains.  group == nchains (resident): it persists across runs.  group < nchains (grouped): the chains run in launch
+  // groups of `group` that share it, each launch rebuilding S and W and starting with every cache stale.
+  longlong2* S;                // [group][cap][n] row sums by slot
+  double2* Cc; unsigned *Vv, *epochs;   // cached per-slot terms, per-point / per-slot change counts that validate them
+  void* Rs;                    // row summaries of the scan (group x n x 32 B)
   double* LLF; unsigned* LLFs; // merged-state log-likelihoods per ordered slot pair and their change counts
-  longlong2* S;                // incremental mode: [nchains][cap][n] row sums by slot (null: streaming mode)
-  bool inc;                    // incremental mode (k_chain_inc) instead of the streaming kernel (k_chain)
+  int64_t group;               // chains per launch
+  int64_t last_g0;             // first chain of the group launched last (its S is the one that exists)
+  int tw_smem, shortcuts;
   int inc_nthr;                // threads per chain (= per CTA) of k_chain_inc
   size_t inc_smem, terms_stride;
   int inc_mcap;                // split-merge members whose running sums fit the chain's shared memory
   int ovl_min_thr, rs_team;    // scan beside the restricted scans: from this many threads per chain on, with this many on the restricted scans
-  longlong2* DLp;              // copy of the data's DL with label-sorted columns (null: the data's own matrix is streamed)
-  unsigned short *colpos, *colpt;   // [n] point -> column and column -> point of DLp
   uint8_t* out_labels; int* out_K; double *out_r, *out_p, *out_ll, *out_lp;
   uint8_t *r_acc, *sm_acc, *sm_split;
   // progress
   int64_t iters_done;
   int64_t overflowed;          // chains stopped by the slot capacity so far
   double dev_seconds;
-  bool W_ready;
-  bool shared_init;            // every chain starts from the same labels: the block sums are built once and copied
+  bool W_ready;                // S and W have been built (by the first run)
+  bool shared_init;            // every chain starts from the same labels: the row sums are built once and copied
   cudaStream_t stream;
   cudaEvent_t e0, e1;
   mutable rc_host_mirror mirror;
@@ -118,88 +118,49 @@ int dalloc(T** p, size_t count) {
   return RC_OK;
 }
 
-// DLp[i][c] = DL[i][pt[c]]: the streamed matrix with its columns in label-sorted order (see rc_sampler_create)
-__global__ void k_permute_cols(const longlong2* __restrict__ DL, int64_t n, const unsigned short* __restrict__ pt, longlong2* __restrict__ out) {
-  const int64_t total = n * n;
-  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t i = t / n, c = t - i * n;
-    out[t] = DL[i * n + pt[c]];
-  }
-}
-
-// ---- block sums of ONE label vector with the whole GPU (all chains start from the same labels) -------------------
-// W[k][t] (k <= t) = sum over rows x of cluster k of the row's sums over cluster t (src/mcmc.jl:1-56 needs exactly
-// these totals).  One CTA per row: every thread walks a contiguous strip of the row keeping a running sum while the
-// label stays the same (one shared-memory atomic per label run), then the row's bins are added to the 128-bit totals
-// with a carry-propagating pair of 64-bit atomics.  Integer sums: the result does not depend on any ordering and is
-// bit-identical to what the chain kernel's own initialisation pass produces.
-__device__ __forceinline__ void atomic_add128(rc_i128* a, long long v) {
-  const unsigned long long u = (unsigned long long)v;
-  const unsigned long long old = atomicAdd(&a->lo, u);
-  const long long hi = (v < 0 ? -1LL : 0LL) + ((old + u) < old ? 1LL : 0LL);
-  if (hi) atomicAdd(reinterpret_cast<unsigned long long*>(&a->hi), (unsigned long long)hi);
-}
-__global__ void __launch_bounds__(256) k_initw_shared(const longlong2* __restrict__ DL, int n, const uint8_t* __restrict__ lab, int cap,
-                                                      rc_i128* __restrict__ WD, rc_i128* __restrict__ WL,
-                                                      const unsigned short* __restrict__ colpt) {
-  extern __shared__ unsigned long long bins[];          // [cap] D sums, [cap] L sums
-  for (int t = threadIdx.x; t < 2 * cap; t += blockDim.x) bins[t] = 0ull;
-  __syncthreads();
-  for (int x = blockIdx.x; x < n; x += gridDim.x) {
-    const longlong2* row = DL + (size_t)x * n;
-    const int w = (n + blockDim.x - 1) / blockDim.x;
-    const int j0 = threadIdx.x * w, j1 = min(n, j0 + w);
-    int cur = -1; long long d = 0, l = 0;
-    for (int j = j0; j < j1; ++j) {
-      const int lb = lab[colpt ? (int)colpt[j] : j];       // j is a column of the streamed matrix
-      if (lb != cur) {
-        if (cur >= 0) { atomicAdd(&bins[cur], (unsigned long long)d); atomicAdd(&bins[cap + cur], (unsigned long long)l); }
-        cur = lb; d = 0; l = 0;
-      }
-      const longlong2 v = row[j];
-      d += v.x; l += v.y;
-    }
-    if (cur >= 0) { atomicAdd(&bins[cur], (unsigned long long)d); atomicAdd(&bins[cap + cur], (unsigned long long)l); }
-    __syncthreads();
-    const int k = lab[x];
-    for (int t = threadIdx.x; t < cap; t += blockDim.x) {
-      const long long bd = (long long)bins[t], bl = (long long)bins[cap + t];
-      bins[t] = 0ull; bins[cap + t] = 0ull;
-      if (t >= k && (bd != 0 || bl != 0)) { atomic_add128(&WD[k * cap + t], bd); atomic_add128(&WL[k * cap + t], bl); }
-    }
-    __syncthreads();
-  }
-}
-__global__ void k_replicate_w(rc_i128* __restrict__ W, size_t per_chain, int64_t nchains) {
-  const size_t total = per_chain * (size_t)(nchains - 1);
-  for (size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x)
-    W[per_chain + t] = W[t % per_chain];
-}
-
-void fill_kparams(const rc_sampler* s, rc_kparams& kp) {
+// Kernel parameters of the launch of chains [g0, g0 + m), m = min(group, nchains - g0): every per-chain pointer starts at
+// chain g0 and chain_offset is advanced by g0 (the chains keep their Philox keys); the group state is not offset.
+void fill_kparams(const rc_sampler* s, rc_kparams& kp, int64_t g0 = 0) {
   memset(&kp, 0, sizeof(kp));
-  kp.n = (int)s->d->n; kp.cap = s->cap; kp.tiles = s->tiles; kp.npad_max = s->npad_max;
-  kp.qD = s->d->qD; kp.qL = s->d->qL; kp.DL = s->DLp ? s->DLp : s->d->DL;
+  const size_t n = (size_t)s->n, cap = (size_t)s->cap, g = (size_t)g0;
+  const size_t NS = (size_t)s->numsamples, ni = (size_t)s->opt.numiters, nm = ni * (size_t)s->opt.numMH;
+  kp.n = (int)n; kp.cap = s->cap;
+  kp.qD = s->d->qD; kp.qL = s->d->qL; kp.DL = s->d->DL;
   kp.S = s->S; kp.terms_stride = s->terms_stride; kp.inc_mcap = s->inc_mcap; kp.ovl_min_thr = s->ovl_min_thr; kp.rs_team = s->rs_team; kp.Cc = s->Cc; kp.Vv = s->Vv; kp.epochs = s->epochs; kp.tw_smem = s->tw_smem; kp.shortcuts = s->shortcuts; kp.Rs = (RowSum*)s->Rs; kp.LLF = s->LLF; kp.LLFs = s->LLFs;
-  kp.colpos = s->colpos; kp.colpt = s->colpt;
   kp.P = s->par;
   kp.abratio = s->par.alpha * rc_log(s->par.beta) - rc_lgamma(s->par.alpha);    // mcmc.jl:17,186,293
   kp.zgratio = s->par.zeta * rc_log(s->par.gamma) - rc_lgamma(s->par.zeta);     // mcmc.jl:18,187,294
   kp.lgd1 = rc_lgamma(s->par.delta1);
   kp.lgd2 = rc_lgamma(s->par.delta2);
   kp.LGA = s->LGA; kp.LGZ = s->LGZ; kp.LOGN = s->LOGN;
-  { const char* e = getenv("RCB200_L2PF"); kp.l2pf = e ? atoi(e) : 2; }   // rows of L2 lookahead (measured: 0 -> 2 rows = +2 %)
   kp.burnin = s->opt.burnin; kp.thin = s->opt.thin; kp.numGibbs = s->opt.numGibbs; kp.numMH = s->opt.numMH;
   kp.numiters = s->opt.numiters; kp.numsamples = s->numsamples;
-  kp.seed = s->seed; kp.chain_offset = s->chain_offset; kp.nchains = (int)s->nchains;
-  kp.labels = s->labels; kp.sizes = s->sizes; kp.r = s->r; kp.p = s->p; kp.status = s->status;
-  // experiment: align the scans of all CTAs (no gain measured)
-  kp.WD = s->WD; kp.WL = s->WL; kp.WDbak = s->WDbak; kp.WLbak = s->WLbak; kp.labbak = s->labbak;
-  kp.szbak = s->szbak; kp.T = s->T; kp.Slist = s->Slist; kp.origM = s->origM; kp.AB = s->AB; kp.L2s = s->L2s;
-  kp.NZ = s->NZ; kp.LPR = s->LPR; kp.DG = s->DG; kp.terms = s->terms; kp.stats = s->stats;
-  kp.gridbar = (s->coresident && getenv("RCB200_GRIDBAR")) ? s->gridbar : nullptr;
-  kp.out_labels = s->out_labels; kp.out_K = s->out_K; kp.out_r = s->out_r; kp.out_p = s->out_p;
-  kp.out_ll = s->out_ll; kp.out_lp = s->out_lp; kp.r_acc = s->r_acc; kp.sm_acc = s->sm_acc; kp.sm_split = s->sm_split;
+  kp.seed = s->seed; kp.chain_offset = s->chain_offset + g0; kp.nchains = (int)std::min<int64_t>(s->group, s->nchains - g0);
+  kp.labels = s->labels + g * n; kp.sizes = s->sizes + g * cap; kp.r = s->r + g; kp.p = s->p + g; kp.status = s->status + g;
+  kp.WD = s->WD + g * cap * cap; kp.WL = s->WL + g * cap * cap;
+  if (s->WDbak) { kp.WDbak = s->WDbak + g * cap * cap; kp.WLbak = s->WLbak + g * cap * cap; kp.labbak = s->labbak + g * n; kp.szbak = s->szbak + g * (cap + 1); }
+  kp.Slist = s->Slist + g * (n + 2); kp.origM = s->origM + g * (n + 2); kp.AB = s->AB + g * (n + 2); kp.L2s = s->L2s + g * n;
+  kp.NZ = s->NZ + g * (size_t)(s->opt.numGibbs + 1) * n;
+  kp.DG = s->DG + g * (n + 2); kp.terms = s->terms + g * s->terms_stride; kp.stats = s->stats + g * 16;
+  kp.out_labels = s->out_labels + g * NS * n; kp.out_K = s->out_K + g * NS; kp.out_r = s->out_r + g * NS; kp.out_p = s->out_p + g * NS;
+  kp.out_ll = s->out_ll + g * NS; kp.out_lp = s->out_lp + g * NS;
+  kp.r_acc = s->r_acc + g * ni; kp.sm_acc = s->sm_acc + g * nm; kp.sm_split = s->sm_split + g * nm;
+}
+
+__global__ void k_fill_u32(unsigned* __restrict__ p, size_t count, unsigned v) {
+  for (size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; t < count; t += (size_t)gridDim.x * blockDim.x) p[t] = v;
+}
+
+// Every cache of the group state stale: no point's cached terms (Vv = 0), row summary (stamp 0) or merged-state
+// log-likelihood (change count 0) is valid at the chains' change count 1 (epochs).
+int reset_caches(const rc_sampler* s) {
+  const size_t m = (size_t)s->group, n = (size_t)s->n, cap = (size_t)s->cap;
+  RC_CUDA(cudaMemsetAsync(s->Vv, 0, sizeof(unsigned) * m * n, s->stream));
+  RC_CUDA(cudaMemsetAsync(s->Rs, 0, m * n * 32, s->stream));
+  RC_CUDA(cudaMemsetAsync(s->LLFs, 0, sizeof(unsigned) * m * cap * cap, s->stream));
+  k_fill_u32<<<256, 256, 0, s->stream>>>(s->epochs, m * (cap + 1), 1u);
+  RC_CUDA(cudaGetLastError());
+  return RC_OK;
 }
 
 }  // namespace
@@ -221,19 +182,19 @@ void rc_sampler_destroy(rc_sampler* s) {
   rc_dev_free(s->LGA); rc_dev_free(s->LGZ); rc_dev_free(s->LOGN);
   rc_dev_free(s->labels); rc_dev_free(s->sizes); rc_dev_free(s->r); rc_dev_free(s->p); rc_dev_free(s->status);
   rc_dev_free(s->WD); rc_dev_free(s->WL); rc_dev_free(s->WDbak); rc_dev_free(s->WLbak); rc_dev_free(s->labbak);
-  rc_dev_free(s->szbak); rc_dev_free(s->T); rc_dev_free(s->Slist); rc_dev_free(s->origM); rc_dev_free(s->AB);
-  rc_dev_free(s->L2s); rc_dev_free(s->NZ); rc_dev_free(s->LPR); rc_dev_free(s->DG); rc_dev_free(s->terms);
-  rc_dev_free(s->stats); rc_dev_free(s->gridbar);
+  rc_dev_free(s->szbak); rc_dev_free(s->Slist); rc_dev_free(s->origM); rc_dev_free(s->AB);
+  rc_dev_free(s->L2s); rc_dev_free(s->NZ); rc_dev_free(s->DG); rc_dev_free(s->terms);
+  rc_dev_free(s->stats);
   rc_dev_free(s->out_labels); rc_dev_free(s->out_K); rc_dev_free(s->out_r); rc_dev_free(s->out_p); rc_dev_free(s->out_ll); rc_dev_free(s->out_lp);
   rc_dev_free(s->r_acc); rc_dev_free(s->sm_acc); rc_dev_free(s->sm_split);
-  rc_dev_free(s->DLp); rc_dev_free(s->colpos); rc_dev_free(s->colpt); rc_dev_free(s->S); rc_dev_free(s->Cc); rc_dev_free(s->Vv); rc_dev_free(s->epochs); rc_dev_free(s->Rs); rc_dev_free(s->LLF); rc_dev_free(s->LLFs);
+  rc_dev_free(s->S); rc_dev_free(s->Cc); rc_dev_free(s->Vv); rc_dev_free(s->epochs); rc_dev_free(s->Rs); rc_dev_free(s->LLF); rc_dev_free(s->LLFs);
   if (s->e0) cudaEventDestroy(s->e0);
   if (s->e1) cudaEventDestroy(s->e1);
   if (s->stream) cudaStreamDestroy(s->stream);
   delete s;
 }
 
-static int32_t sampler_create_impl(bool opt_loglik_only, const rc_data* d, const rc_options* opt, const rc_params* par, int64_t nchains,
+int32_t rc_sampler_create(const rc_data* d, const rc_options* opt, const rc_params* par, int64_t nchains,
                           int64_t chain_offset, const int64_t* init_labels, const double* init_r,
                           const double* init_p, uint64_t seed, int32_t slot_cap, rc_sampler** out) {
   if (!d || !opt || !par || !init_labels || !init_r || !init_p || !out || nchains < 1) {
@@ -243,52 +204,15 @@ static int32_t sampler_create_impl(bool opt_loglik_only, const rc_data* d, const
   if (st) return st;
   const int64_t n = d->n;
   if (opt->numMH > 0 && n < 2) { rc_set_error("split-merge needs at least 2 observations."); return RC_ERR_ARG; }
-  // slot capacity: 128 by default; the incremental kernel takes up to 255 (byte labels), the streaming kernel up to 128
-  const bool force_stream = getenv("RCB200_SCAN") && !strcmp(getenv("RCB200_SCAN"), "stream");
-  const int capmax = (opt_loglik_only || force_stream) ? RC_MAXCAP : RC_MAXCAP_INC;
+  // slot capacity: 128 by default, up to 255 (byte labels)
   int cap = slot_cap == 0 ? RC_MAXCAP : slot_cap;
-  if (cap < 2 || cap > capmax) { rc_set_error("slot_cap must be in 2..%d", capmax); return RC_ERR_ARG; }
+  if (cap < 2 || cap > RC_MAXCAP_INC) { rc_set_error("slot_cap must be in 2..%d", RC_MAXCAP_INC); return RC_ERR_ARG; }
   if (par->maxK < 0 || !(par->proposalsd_r > 0)) { rc_set_error("invalid hyperparameters (maxK < 0 or proposalsd_r <= 0)"); return RC_ERR_ARG; }
-  const int tiles = (int)((n + RC_W - 1) / RC_W);
-  // permutation length: every (tile, slot) run is padded by at most 7 entries.  The worst case (all slots live in
-  // every tile) is reserved when it fits; otherwise the reserve shrinks to what shared memory allows (never below
-  // 32 slots' worth per tile) and a chain whose runs need more stops with RC_ERR_SLOTS.
-  const int64_t npad_full = (((n + 7) & ~7LL) + 7LL * tiles * cap + 7) & ~7LL;
-  const int64_t npad_min = (((n + 7) & ~7LL) + 7LL * tiles * std::min(cap, 32) + 7) & ~7LL;
   if (n > 65535) { rc_set_error("n = %lld: the sampler indexes points with 16 bits (n <= 65535)", (long long)n); return RC_ERR_ARG; }
   RC_CUDA(cudaSetDevice(d->device));
   int maxsmem = 0, nsm = 0;
   RC_CUDA(cudaDeviceGetAttribute(&maxsmem, cudaDevAttrMaxSharedMemoryPerBlockOptin, d->device));
   RC_CUDA(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, d->device));
-  // chains per CTA: the chains of a CTA share every staged row tile.  Use the smallest G that lets all
-  // chains be co-resident (so they stay in rough lock step and share rows through L2 as well).
-  int G = 0, forceG = 0;
-  int64_t npad = 0;
-  if (const char* e = getenv("RCB200_CHAINS_PER_CTA")) forceG = atoi(e);   // test hook
-  // (geometry of the STREAMING kernel: labels and the column permutation of a chain live in shared memory, which bounds
-  // n at about 26 000; the incremental kernel has no such bound -- stream_ok records whether streaming is possible)
-  for (int g : {1, 2}) {
-    if (npad_min > 65528 || cap > RC_MAXCAP) break;
-    if (forceG && g != forceG) continue;
-    int64_t np = std::min<int64_t>(npad_full, 65528);
-    while (np > npad_min && rc_sampler_smem_bytes((int)n, cap, tiles, (int)np, g) > (size_t)maxsmem) np -= 64;
-    const size_t sm = rc_sampler_smem_bytes((int)n, cap, tiles, (int)np, g);
-    if (sm > (size_t)maxsmem) break;
-    G = g; npad = np;
-    const int64_t ctas = (nchains + g - 1) / g;
-    const int per_sm = std::max<int>(1, std::min<int>((int)((size_t)maxsmem / sm), 2048 / (RC_NTHR * g + 64)));
-    if (ctas <= (int64_t)nsm * per_sm) break;
-  }
-  const bool stream_ok = G != 0;
-  if (!stream_ok && (opt_loglik_only || force_stream)) {
-    rc_set_error("the streaming kernel keeps a chain's labels and column permutation in shared memory: n = %lld with slot_cap = %d does not fit "
-                 "(%d bytes available); use the incremental scan mode", (long long)n, cap, maxsmem);
-    return RC_ERR_ARG;
-  }
-  const size_t smem = stream_ok ? rc_sampler_smem_bytes((int)n, cap, tiles, (int)npad, G) : 0;
-  if (getenv("RCB200_VERBOSE") && stream_ok)
-    fprintf(stderr, "[rcb200] n=%lld cap=%d tiles=%d npad=%lld (full %lld) G=%d smem=%zu (max %d) chains=%lld\n", (long long)n, cap, tiles,
-            (long long)npad, (long long)npad_full, G, smem, maxsmem, (long long)nchains);
   const bool vb_ = getenv("RCB200_VERBOSE") != nullptr;
   auto tnow_ = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   const double tc0_ = tnow_();
@@ -321,7 +245,7 @@ static int32_t sampler_create_impl(bool opt_loglik_only, const rc_data* d, const
   s->shared_init = nchains > 1;
   for (int64_t c = 1; c < nchains && s->shared_init; ++c) s->shared_init = memcmp(lab.data(), lab.data() + c * n, (size_t)n) == 0;
   s->d = d; s->device = d->device; s->n = d->n; s->opt = *opt; s->par = *par; s->nchains = nchains; s->chain_offset = chain_offset; s->seed = seed;
-  s->nsm = nsm; s->cap = cap; s->tiles = tiles; s->npad_max = (int)npad; s->smem = smem; s->G = G;
+  s->cap = cap;
   s->numsamples = (opt->numiters - opt->burnin) / opt->thin;   // floor((numiters - burnin) / thin), types.jl:55
   const size_t NS = (size_t)std::max<int64_t>(s->numsamples, 1);
 #define TRY(x) do { st = (x); if (st) { rc_sampler_destroy(s); return st; } } while (0)
@@ -329,25 +253,22 @@ static int32_t sampler_create_impl(bool opt_loglik_only, const rc_data* d, const
   TRY(dalloc(&s->labels, (size_t)nchains * n)); TRY(dalloc(&s->sizes, (size_t)nchains * cap));
   TRY(dalloc(&s->r, nchains)); TRY(dalloc(&s->p, nchains)); TRY(dalloc(&s->status, nchains));
   TRY(dalloc(&s->WD, (size_t)nchains * cap * cap)); TRY(dalloc(&s->WL, (size_t)nchains * cap * cap));
-  // Scan mode.  Incremental (default when it fits): every chain keeps S[slot][x], the sums of row x by cluster, and a
-  // Gibbs step reads cap entries instead of a row; a move streams one row.  Streaming: the round-1 kernel that
-  // re-reduces every row against the labels (no per-chain matrix; needed when nchains * cap * n * 16 B does not fit).
+  // Group size: as many chains per launch as have their group state (S and Cc, cap x n entries each, row summaries,
+  // change counts, merged-state log-likelihoods) in 60 % of the free memory.
   {
-    const char* env = getenv("RCB200_SCAN");
-    const size_t needS = (sizeof(longlong2) + sizeof(double2)) * (size_t)nchains * cap * n;   // row sums + cached terms
+    const size_t per = (sizeof(longlong2) + sizeof(double2)) * (size_t)cap * n + (32 + sizeof(unsigned)) * (size_t)n +
+                       sizeof(unsigned) * (size_t)(cap + 1) + (sizeof(double) + sizeof(unsigned)) * (size_t)cap * cap;
     size_t freeb = 0, totalb = 0;
     cudaMemGetInfo(&freeb, &totalb);
-    bool want = !opt_loglik_only && needS <= freeb / 10 * 6;
-    if (!stream_ok && !want) {
-      rc_set_error("n = %lld, slot_cap = %d: the streaming kernel does not fit shared memory and the incremental mode's per-chain sums (%.1f GB) do not fit the device",
-                   (long long)n, cap, needS / 1e9);
+    s->group = std::min<int64_t>(nchains, (int64_t)(freeb / 10 * 6 / per));
+    if (const char* e = getenv("RCB200_CHAINS_PER_GROUP")) s->group = std::min<int64_t>(s->group, atoll(e));   // test hook
+    if (s->group < 1) {
+      rc_set_error("n = %lld, slot_cap = %d: one chain's row sums and caches (%.2f GB) do not fit 60 %% of the free device memory (%.2f GB)",
+                   (long long)n, cap, per / 1e9, freeb / 1e9);
       rc_sampler_destroy(s); return RC_ERR_ARG;
     }
-    if (cap > RC_MAXCAP && !want) { rc_set_error("slot_cap = %d > %d needs the incremental scan mode, whose per-chain sums (%.1f GB) do not fit the device", cap, RC_MAXCAP, needS / 1e9); rc_sampler_destroy(s); return RC_ERR_ARG; }
-    if (env && !strcmp(env, "stream")) want = false;
-    if (env && !strcmp(env, "inc") && !opt_loglik_only) want = true;
-    s->inc = want;
-    int nthr = nchains <= nsm ? 512 : (nchains <= 2 * nsm ? 256 : 256);
+    const int64_t L = s->group;                // chains per launch
+    int nthr = L <= nsm ? 512 : 256;
     if (const char* e = getenv("RCB200_INC_THREADS")) nthr = std::max(32, std::min(512, atoi(e) / 32 * 32));
     s->inc_nthr = nthr;
     s->shortcuts = 1;
@@ -357,32 +278,37 @@ static int32_t sampler_create_impl(bool opt_loglik_only, const rc_data* d, const
     s->ovl_min_thr = 256; s->rs_team = nthr >= 512 ? 128 : 64;
     if (const char* e = getenv("RCB200_OVERLAP_MIN_THREADS")) s->ovl_min_thr = atoi(e);
     if (const char* e = getenv("RCB200_RS_TEAM")) s->rs_team = std::max(32, atoi(e) / 32 * 32);
-    {
-      // shared memory per chain: the fixed part plus as many split-merge members (64 B each) as fit next to the other
-      // CTAs of the SM (two chains per SM when there are more chains than SMs)
-      const size_t budget = nchains <= nsm ? (size_t)maxsmem : ((size_t)maxsmem + 1024) / 2 - 1024;
-      // the per-point validity counts of the cached terms (4 B per point) go to shared memory when at least 512 split-merge
-      // members still fit beside them: the row evaluation then knows which entries are valid without a trip to memory
-      s->tw_smem = rc_sampler_inc_smem_bytes((int)n, cap, 512, 1) <= budget ? 1 : 0;
-      if (const char* e = getenv("RCB200_TW_SMEM")) s->tw_smem = atoi(e) != 0 && rc_sampler_inc_smem_bytes((int)n, cap, 0, 1) <= budget;
-      const size_t base = rc_sampler_inc_smem_bytes((int)n, cap, 0, s->tw_smem);
-      int mcap = base < budget ? (int)((budget - base) / 64) : 0;
-      mcap = std::min<int>(mcap, (int)n + 2) / 8 * 8;
-      s->inc_mcap = std::max(mcap, 0);
-      s->inc_smem = rc_sampler_inc_smem_bytes((int)n, cap, s->inc_mcap, s->tw_smem);
-      if (s->inc_smem > (size_t)maxsmem) { s->inc_mcap = 0; s->inc_smem = base; }
+    // shared memory per chain: the fixed part plus as many split-merge members (64 B each) as fit next to the other
+    // CTAs of the SM (two chains per SM when there are more chains than SMs)
+    const size_t budget = L <= nsm ? (size_t)maxsmem : ((size_t)maxsmem + 1024) / 2 - 1024;
+    // the per-point validity counts of the cached terms (4 B per point) go to shared memory when at least 512 split-merge
+    // members still fit beside them: the row evaluation then knows which entries are valid without a trip to memory
+    s->tw_smem = rc_sampler_inc_smem_bytes((int)n, cap, 512, 1) <= budget ? 1 : 0;
+    if (const char* e = getenv("RCB200_TW_SMEM")) s->tw_smem = atoi(e) != 0 && rc_sampler_inc_smem_bytes((int)n, cap, 0, 1) <= budget;
+    const size_t base = rc_sampler_inc_smem_bytes((int)n, cap, 0, s->tw_smem);
+    int mcap = base < budget ? (int)((budget - base) / 64) : 0;
+    mcap = std::min<int>(mcap, (int)n + 2) / 8 * 8;
+    s->inc_mcap = std::max(mcap, 0);
+    s->inc_smem = rc_sampler_inc_smem_bytes((int)n, cap, s->inc_mcap, s->tw_smem);
+    if (s->inc_smem > (size_t)maxsmem) { s->inc_mcap = 0; s->inc_smem = base; }
+    // (the largest case, n = 65535 and slot_cap = 255 with no member scratch and the counts in global memory, needs about
+    // 177 KB: below the 227 KB a CTA can have on sm_100)
+    if (s->inc_smem > (size_t)maxsmem) {
+      rc_set_error("n = %lld, slot_cap = %d: the chain kernel needs %zu B of shared memory per chain, the device allows %d",
+                   (long long)n, cap, s->inc_smem, maxsmem);
+      rc_sampler_destroy(s); return RC_ERR_ARG;
     }
-    if (s->inc && s->inc_smem > (size_t)maxsmem) s->inc = false;
-    if (getenv("RCB200_VERBOSE")) fprintf(stderr, "[rcb200] scan mode: %s (S needs %.2f GB, %.2f GB free), %d threads per chain, %zu B shared memory (%d split-merge members)\n", s->inc ? "incremental" : "streaming", needS / 1e9, freeb / 1e9, nthr, s->inc_smem, s->inc_mcap);
+    if (vb_) fprintf(stderr, "[rcb200] %lld of %lld chains per launch (%.2f GB of row sums and caches per chain, %.2f GB free), %d threads per chain, %zu B shared memory (%d split-merge members)\n",
+                     (long long)L, (long long)nchains, per / 1e9, freeb / 1e9, nthr, s->inc_smem, s->inc_mcap);
   }
   s->terms_stride = (size_t)std::max(cap * cap, 8192);
-  if (s->inc) {
-    TRY(dalloc(&s->S, (size_t)nchains * cap * n)); TRY(dalloc(&s->Cc, (size_t)nchains * cap * n)); TRY(dalloc(&s->Vv, (size_t)nchains * n));
-    TRY(dalloc(&s->epochs, (size_t)nchains * (cap + 1)));
-    { char* rs = nullptr; TRY(dalloc(&rs, (size_t)nchains * n * 32)); s->Rs = rs; }
-    TRY(dalloc(&s->LLF, (size_t)nchains * cap * cap)); TRY(dalloc(&s->LLFs, (size_t)nchains * cap * cap));
+  {
+    const size_t G = (size_t)s->group;
+    TRY(dalloc(&s->S, G * cap * n)); TRY(dalloc(&s->Cc, G * cap * n)); TRY(dalloc(&s->Vv, G * n));
+    TRY(dalloc(&s->epochs, G * (cap + 1)));
+    { char* rs = nullptr; TRY(dalloc(&rs, G * n * 32)); s->Rs = rs; }
+    TRY(dalloc(&s->LLF, G * cap * cap)); TRY(dalloc(&s->LLFs, G * cap * cap));
   }
-  TRY(dalloc(&s->T, (opt->numMH > 0 && !s->inc) ? (size_t)nchains * n * cap : 1));
   if (opt->numMH > 1) {
     TRY(dalloc(&s->WDbak, (size_t)nchains * cap * cap)); TRY(dalloc(&s->WLbak, (size_t)nchains * cap * cap));
     TRY(dalloc(&s->labbak, (size_t)nchains * n)); TRY(dalloc(&s->szbak, (size_t)nchains * (cap + 1)));
@@ -390,9 +316,8 @@ static int32_t sampler_create_impl(bool opt_loglik_only, const rc_data* d, const
   TRY(dalloc(&s->Slist, (size_t)nchains * (n + 2))); TRY(dalloc(&s->origM, (size_t)nchains * (n + 2)));
   TRY(dalloc(&s->AB, (size_t)nchains * (n + 2))); TRY(dalloc(&s->L2s, (size_t)nchains * n));
   TRY(dalloc(&s->NZ, opt->numMH > 0 ? (size_t)nchains * (opt->numGibbs + 1) * n : 1));
-  TRY(dalloc(&s->LPR, (size_t)nchains * (n + 2))); TRY(dalloc(&s->DG, (size_t)nchains * (n + 2)));
-  TRY(dalloc(&s->stats, (size_t)nchains * 16)); TRY(dalloc(&s->gridbar, 1));
-  s->coresident = stream_ok && rc_chain_kernel_coresident((int)nchains, smem, G, d->device); TRY(dalloc(&s->terms, (size_t)nchains * s->terms_stride));
+  TRY(dalloc(&s->DG, (size_t)nchains * (n + 2)));
+  TRY(dalloc(&s->stats, (size_t)nchains * 16)); TRY(dalloc(&s->terms, (size_t)nchains * s->terms_stride));
   TRY(dalloc(&s->out_labels, (size_t)nchains * NS * n)); TRY(dalloc(&s->out_K, (size_t)nchains * NS));
   TRY(dalloc(&s->out_r, (size_t)nchains * NS)); TRY(dalloc(&s->out_p, (size_t)nchains * NS));
   TRY(dalloc(&s->out_ll, (size_t)nchains * NS)); TRY(dalloc(&s->out_lp, (size_t)nchains * NS));
@@ -403,49 +328,10 @@ static int32_t sampler_create_impl(bool opt_loglik_only, const rc_data* d, const
 #undef TRY
 #define TRYC(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc_set_error("sampler setup: CUDA error %s at %s:%d: %s", cudaGetErrorName(e_), __FILE__, __LINE__, cudaGetErrorString(e_)); rc_sampler_destroy(s); return RC_ERR_CUDA; } } while (0)
   TRYC(cudaMemcpy(s->labels, lab.data(), lab.size(), cudaMemcpyHostToDevice));
-  // Column order of the streamed matrix.  The row reduction is fastest when the members of a cluster are contiguous
-  // columns (few (tile, label) runs, little padding, conflict-free shared-memory gathers).  When the initial labels
-  // of chain 0 are scattered over the points, the sampler streams its own copy of DL whose columns are sorted by those
-  // labels (stable).  Every sum is an exact integer, so no result changes; only direct element reads need the map.
-  {
-    int64_t changes = 0, distinct = 0;
-    std::vector<char> seen((size_t)cap, 0);
-    for (int64_t j = 0; j < n; ++j) {
-      if (j && lab[j] != lab[j - 1]) ++changes;
-      if (!seen[lab[j]]) { seen[lab[j]] = 1; ++distinct; }
-    }
-    const char* env = getenv("RCB200_COLPERM");
-    const bool want = env ? atoi(env) != 0 : changes > 4 * distinct + 8;
-    if (want && !opt_loglik_only && !s->inc) {      // (the incremental mode never reduces rows by label: no copy needed)
-      std::vector<unsigned short> pt((size_t)n), pos((size_t)n);
-      std::vector<int64_t> idx((size_t)n);
-      for (int64_t j = 0; j < n; ++j) idx[j] = j;
-      std::stable_sort(idx.begin(), idx.end(), [&](int64_t a, int64_t b) { return lab[a] < lab[b]; });
-      for (int64_t c = 0; c < n; ++c) { pt[c] = (unsigned short)idx[c]; pos[idx[c]] = (unsigned short)c; }
-      if (dalloc(&s->DLp, (size_t)n * n) == RC_OK && dalloc(&s->colpos, (size_t)n) == RC_OK && dalloc(&s->colpt, (size_t)n) == RC_OK) {
-        TRYC(cudaMemcpy(s->colpos, pos.data(), sizeof(unsigned short) * n, cudaMemcpyHostToDevice));
-        TRYC(cudaMemcpy(s->colpt, pt.data(), sizeof(unsigned short) * n, cudaMemcpyHostToDevice));
-        k_permute_cols<<<nsm * 16, 256>>>(d->DL, n, s->colpt, s->DLp);
-        TRYC(cudaGetLastError());
-        if (getenv("RCB200_VERBOSE")) fprintf(stderr, "[rcb200] columns of the streamed matrix sorted by the initial labels (%lld label changes along the points, %lld clusters)\n", (long long)changes, (long long)distinct);
-      } else {                                   // not enough memory for the copy: stream the data's own matrix
-        rc_dev_free(s->DLp); rc_dev_free(s->colpos); rc_dev_free(s->colpt);
-        s->DLp = nullptr; s->colpos = nullptr; s->colpt = nullptr;
-        (void)cudaGetLastError();
-      }
-    }
-  }
   TRYC(cudaMemcpy(s->sizes, sizes.data(), sizes.size() * sizeof(int), cudaMemcpyHostToDevice));
   TRYC(cudaMemcpy(s->r, init_r, sizeof(double) * nchains, cudaMemcpyHostToDevice));
   TRYC(cudaMemcpy(s->p, init_p, sizeof(double) * nchains, cudaMemcpyHostToDevice));
   TRYC(cudaMemset(s->status, 0, sizeof(int) * nchains));
-  if (s->inc) {
-    TRYC(cudaMemset(s->Vv, 0, sizeof(unsigned) * (size_t)nchains * n));                // no cached entry is valid
-    TRYC(cudaMemset(s->Rs, 0, (size_t)nchains * n * 32));                               // no row summary is valid (stamp 0)
-    TRYC(cudaMemset(s->LLFs, 0, sizeof(unsigned) * (size_t)nchains * cap * cap));
-    std::vector<unsigned> ones((size_t)nchains * (cap + 1), 1u);
-    TRYC(cudaMemcpy(s->epochs, ones.data(), sizeof(unsigned) * ones.size(), cudaMemcpyHostToDevice));
-  }
   TRYC(cudaMemset(s->stats, 0, sizeof(long long) * 16 * nchains));
   TRYC(cudaMemset(s->r_acc, 0, (size_t)nchains * opt->numiters));
   TRYC(cudaMemset(s->sm_acc, 0, (size_t)nchains * opt->numiters * std::max<int64_t>(opt->numMH, 1)));
@@ -453,6 +339,7 @@ static int32_t sampler_create_impl(bool opt_loglik_only, const rc_data* d, const
   TRYC(cudaStreamCreate(&s->stream));
   TRYC(cudaEventCreate(&s->e0)); TRYC(cudaEventCreate(&s->e1));
 #undef TRYC
+  if ((st = reset_caches(s))) { rc_sampler_destroy(s); return st; }
   rc_launch_tables(s->par, (int)n, s->LGA, s->LGZ, s->LOGN, s->stream);
   cudaError_t e = cudaStreamSynchronize(s->stream);
   if (e != cudaSuccess) { rc_set_error("sampler setup failed: %s", cudaGetErrorString(e)); rc_sampler_destroy(s); return RC_ERR_CUDA; }
@@ -461,41 +348,25 @@ static int32_t sampler_create_impl(bool opt_loglik_only, const rc_data* d, const
   return RC_OK;
 }
 
-int32_t rc_sampler_create(const rc_data* d, const rc_options* opt, const rc_params* par, int64_t nchains,
-                          int64_t chain_offset, const int64_t* init_labels, const double* init_r,
-                          const double* init_p, uint64_t seed, int32_t slot_cap, rc_sampler** out) {
-  return sampler_create_impl(false, d, opt, par, nchains, chain_offset, init_labels, init_r, init_p, seed, slot_cap, out);
-}
-
 int32_t rc_sampler_run(rc_sampler* s, int64_t iters) {
   if (!s) { rc_set_error("rc_sampler_run: null handle"); return RC_ERR_ARG; }
   RC_CUDA(cudaSetDevice(s->device));
   int64_t it1 = iters < 0 ? s->opt.numiters : std::min<int64_t>(s->opt.numiters, s->iters_done + iters);
   if (it1 <= s->iters_done && s->W_ready) return RC_OK;
-  rc_kparams kp;
-  fill_kparams(s, kp);
-  kp.it0 = s->iters_done; kp.it1 = it1;
-  kp.init_W = s->W_ready ? 0 : 1;
-  RC_CUDA(cudaMemsetAsync(s->gridbar, 0, sizeof(unsigned), s->stream));
+  // Resident (one group): S and W are built before the first launch and maintained from then on.  Grouped: every launch
+  // rebuilds them from its chains' labels with every cache stale; S and W are exact integers and every cache is validated
+  // by change counts, so the chains compute the same bits as resident ones.
+  const bool resident = s->group == s->nchains;
   RC_CUDA(cudaEventRecord(s->e0, s->stream));
-  if (s->inc) {
-    if (kp.init_W) {
-      if (rc_launch_inc_init(kp, s->shared_init, s->stream)) { rc_set_error("incremental-mode initialisation failed: %s", cudaGetErrorString(cudaGetLastError())); return RC_ERR_CUDA; }
-      kp.init_W = 0;
-    }
+  for (int64_t g0 = 0; g0 < s->nchains; g0 += s->group) {
+    rc_kparams kp;
+    fill_kparams(s, kp, g0);
+    kp.it0 = s->iters_done; kp.it1 = it1;
+    if (!resident) { int st = reset_caches(s); if (st) return st; }
+    if (!resident || !s->W_ready)
+      if (rc_launch_inc_init(kp, resident && s->shared_init, s->stream)) { rc_set_error("chain state initialisation failed: %s", cudaGetErrorString(cudaGetLastError())); return RC_ERR_CUDA; }
     if (kp.it1 > kp.it0) rc_launch_chain_inc(kp, s->inc_smem, s->inc_nthr, s->stream);
-  } else {
-  if (kp.init_W && s->shared_init && !getenv("RCB200_NO_SHARED_INIT")) {
-    const size_t per = (size_t)s->cap * s->cap;
-    RC_CUDA(cudaMemsetAsync(s->WD, 0, sizeof(rc_i128) * per, s->stream));
-    RC_CUDA(cudaMemsetAsync(s->WL, 0, sizeof(rc_i128) * per, s->stream));
-    k_initw_shared<<<s->nsm * 8, 256, sizeof(unsigned long long) * 2 * s->cap, s->stream>>>(s->DLp ? s->DLp : s->d->DL, (int)s->n, s->labels, s->cap, s->WD, s->WL, s->colpt);
-    k_replicate_w<<<s->nsm * 4, 256, 0, s->stream>>>(s->WD, per, s->nchains);
-    k_replicate_w<<<s->nsm * 4, 256, 0, s->stream>>>(s->WL, per, s->nchains);
-    RC_CUDA(cudaGetLastError());
-    kp.init_W = 0;
-  }
-  if (kp.init_W || kp.it1 > kp.it0) rc_launch_chain_kernel(kp, s->smem, s->G, s->stream);
+    s->last_g0 = g0;
   }
   RC_CUDA(cudaGetLastError());
   RC_CUDA(cudaEventRecord(s->e1, s->stream));
@@ -690,16 +561,17 @@ int32_t rc_sampler_copy_stats(const rc_sampler* s, int64_t* out) {
 
 int64_t rc_sampler_overflowed(const rc_sampler* s) { return s ? s->overflowed : 0; }
 
-// Invariant check of the incremental scan mode: rebuilds every chain's row sums S and block sums W from its current
-// labels and counts the 64-bit words that differ from the incrementally maintained ones (both must be 0).  In streaming
-// mode there is nothing to compare: both counts are returned as -1.
+// Invariant check of the maintained sums: rebuilds the row sums S and block sums W of the chains launched last (every
+// chain in resident mode, the last group in grouped mode: only its S still exists) from their current labels and counts
+// the 64-bit words that differ from the incrementally maintained ones (both must be 0).  Before the first run there is
+// nothing to compare: both counts are returned as -1.
 int32_t rc_sampler_check_sums(const rc_sampler* s, int64_t* mismatches_S, int64_t* mismatches_W) {
   if (!s || !mismatches_S || !mismatches_W) { rc_set_error("rc_sampler_check_sums: null pointer"); return RC_ERR_ARG; }
   *mismatches_S = -1; *mismatches_W = -1;
-  if (!s->inc || !s->W_ready) return RC_OK;
+  if (!s->W_ready) return RC_OK;
   RC_CUDA(cudaSetDevice(s->device));
   rc_kparams kp;
-  fill_kparams(s, kp);
+  fill_kparams(s, kp, s->last_g0);
   long long a = 0, b = 0;
   if (rc_inc_check(kp, &a, &b, s->stream)) { rc_set_error("rc_sampler_check_sums: rebuild failed (out of memory?)"); return RC_ERR_CUDA; }
   *mismatches_S = a; *mismatches_W = b;
@@ -714,8 +586,8 @@ int32_t rc_sampler_chain_status(const rc_sampler* s, int64_t chain) {
   return st;
 }
 
-// loglik(data, state, params) for one host label vector (src/mcmc.jl:1-56): block sums from scratch,
-// then the same evaluation the sampler uses.
+// loglik(data, state, params) for one host label vector (src/mcmc.jl:1-56): a one-chain sampler builds the block sums
+// from scratch, then the chain kernel evaluates the log-likelihood once, as the sampler does.
 int32_t rc_loglik(const rc_data* d, const rc_params* par, const int64_t* labels, double* out) {
   if (!d || !par || !labels || !out) { rc_set_error("rc_loglik: null pointer"); return RC_ERR_ARG; }
   rc_options opt = {1, 0, 1, 0, 0};
@@ -729,13 +601,15 @@ int32_t rc_loglik(const rc_data* d, const rc_params* par, const int64_t* labels,
   for (int64_t j = 0; j < n; ++j) lab[j] = (std::lower_bound(uniq.begin(), uniq.end(), labels[j]) - uniq.begin()) + 1;
   double r0 = 1.0, p0 = 0.5;
   rc_sampler* s = nullptr;
-  int st = sampler_create_impl(true, d, &opt, par, 1, 0, lab.data(), &r0, &p0, 0, 0, &s);
+  int st = rc_sampler_create(d, &opt, par, 1, 0, lab.data(), &r0, &p0, 0, 0, &s);
   if (st) return st;
   rc_kparams kp;
   fill_kparams(s, kp);
-  kp.it0 = 0; kp.it1 = 0; kp.init_W = 1; kp.loglik_only = 1;
-  rc_launch_chain_kernel(kp, s->smem, s->G, s->stream);
-  cudaError_t e = cudaStreamSynchronize(s->stream);
+  kp.loglik_only = 1;
+  if (rc_launch_inc_init(kp, false, s->stream)) { rc_set_error("rc_loglik: block sums failed: %s", cudaGetErrorString(cudaGetLastError())); rc_sampler_destroy(s); return RC_ERR_CUDA; }
+  rc_launch_chain_inc(kp, s->inc_smem, s->inc_nthr, s->stream);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s->stream);
   if (e == cudaSuccess) e = cudaMemcpy(out, s->out_ll, sizeof(double), cudaMemcpyDeviceToHost);
   rc_sampler_destroy(s);
   RC_CUDA(e);

@@ -67,15 +67,7 @@ struct rc_data {
   int qD, qL;
 };
 
-// geometry of the label-sorted column permutation the sampler reduces rows with
-#ifndef RC_LOGW
-#define RC_LOGW 10
-#endif
-#define RC_W (1 << RC_LOGW)          // columns per row tile (16 KB of DL)
-#define RC_DUMMY ((unsigned)RC_W)     // padding entry of a label run: index of the zero slot behind a staged tile
-#define RC_GROUP 8                   // columns per lane-group (runs are padded to multiples of this)
-#define RC_MAXCAP 128                // max live cluster slots per chain of the streaming kernel (k_chain)
-#define RC_NS (RC_MAXCAP / 32)
-#define RC_MAXCAP_INC 255            // ... of the incremental kernel (k_chain_inc): labels are bytes, recorded labels are 1-based bytes
+#define RC_MAXCAP 128                // default live cluster slots per chain (slot_cap = 0)
+#define RC_MAXCAP_INC 255            // largest slot_cap: labels are bytes, recorded labels are 1-based bytes
 #define RC_NSI ((RC_MAXCAP_INC + 31) / 32)
 #define RC_DETACHED 0xFF

@@ -3,16 +3,16 @@
 //
 //   sample_r!  (mcmc.jl:80-136)      -> update_r()
 //   sample_p!  (mcmc.jl:138-155)     -> update_p()
-//   sample_labels! (mcmc.jl:356-479) -> splitmerge_step() x numMH, then inc_full_scan() / full_scan()
-//   sample_labels_Gibbs! (:158-256)  -> inc_full_scan(): inc_eval_row();  full_scan(): bulk_loop() / reduce_tile() + decide_rows()
-//   sample_labels_Gibbs_restricted! (:259-354) -> restricted_scans_team() / restricted_scans()
+//   sample_labels! (mcmc.jl:356-479) -> splitmerge_step() x numMH, then inc_full_scan()
+//   sample_labels_Gibbs! (:158-256)  -> inc_full_scan(): inc_eval_row()
+//   sample_labels_Gibbs_restricted! (:259-354) -> restricted_scans_team()
 //   loglik (:1-56), logprior (:58-78), record step (:546-554), sortlabels (utils.jl:69-74)
 //
-// Two kernels share the device functions below (DESIGN.md sections 2-3).  Both work on DL[i][j] = {Dq, Lq}, the 64-bit
-// fixed-point images of D and log D: every cluster sum is an exact integer, so results do not depend on tiling, lane count,
-// reduction order -- or on whether a sum is recomputed or maintained -- and are bit-identical to the CPU oracle.
+// The kernel works on DL[i][j] = {Dq, Lq}, the 64-bit fixed-point images of D and log D (DESIGN.md section 2): every cluster
+// sum is an exact integer, so results do not depend on lane count or reduction order -- or on whether a sum is recomputed
+// or maintained -- and are bit-identical to the CPU oracle.
 //
-// k_chain_inc (default): one CTA = one chain, all iterations of a launch inside the kernel.
+// k_chain_inc: one CTA = one chain, all iterations of a launch inside the kernel.
 //   * S[slot][x] = sum of row x over the members of slot is kept in HBM; a Gibbs step reads one entry per live slot
 //     (inc_eval_row: G lanes per row, the lane's slots in registers), only a move streams a row (inc_update_S).
 //   * Rows are evaluated speculatively in batches and committed up to the first one that moves (inc_full_scan).
@@ -22,36 +22,12 @@
 //     steps resolved inside a warp (restricted_scans_team), merge proposals that cannot be accepted rejected by their bound
 //     (splitmerge_step); the scan runs dry beside the restricted scans while it is long.
 //   * W (K x K block sums, 128-bit) is maintained from the row sums of every move, so loglik() never reads D.
-//
-// k_chain<G> (round 1, RCB200_SCAN=stream or when S does not fit): the streaming kernel.
-//   * One CTA runs G chains (G x 160 threads: 4 bulk warps + 1 decision warp per chain) plus two CTA-level helper
-//     warps.  During the full Gibbs scan all chains of a CTA visit rows 0..n-1 together, so every 1024-column tile
-//     of row i of DL is staged ONCE into a 6-stage shared-memory ring by the producer warp (cp.async.bulk -> UBLKCP,
-//     mbarrier full/empty) and reduced by all G chains against their own label vectors.  The noise warp precomputes the
-//     Gumbel noise of the rows ahead of the decisions.
-//   * Row reduction: columns are kept in a (tile, label)-sorted permutation whose label runs are padded to
-//     chunks of 8; one warp reduces a tile, a lane walks its contiguous chunks keeping a running sum, a warp-shuffle
-//     segmented scan merges runs that span lanes, totals go to per-warp bins.  A move patches the permutation in place.
-//   * The decision warp does the sequential part: bins of row i -> log-weights (lane = slot) -> Gumbel arg-max ->
-//     move; it runs one row behind the bulk warps.
-//   * Split-merge: row sums of the members of ci u cj are taken once (launch state); the restricted
-//     scans then run on a single warp from running candidate sums, eight steps at a time (restricted_scans).
+// S, W and every cache can be rebuilt from the labels at any launch (k_init_S / k_initw_from_S, caches reset): chains that
+// do not all fit the device run in launch groups that share this state (rc_api.cu).
 #include <algorithm>
 #include "rc_sampler.cuh"
 
 namespace {
-
-// Tile T of the row stream lives in stage T % RC_NSTAGE and is reduced by bulk warp T % RC_BW of every chain: RC_BW
-// tiles are being reduced while one more is in flight.  A warp revisits a stage only every RC_NSTAGE * RC_BW tiles and
-// mbarrier parity waits are only unambiguous one phase ahead, so the producer publishes the tile it issues into a stage
-// (CtaShared::issued) and a consumer waits for that to reach its tile before it waits on the stage's `full` barrier.
-#ifndef RC_NSTAGE
-#define RC_NSTAGE (RC_BW + 2)
-#endif
-#define RC_PAIR 1                    // bulk warps that reduce one tile together (RC_BW / RC_PAIR tiles are reduced at a time)
-#define RC_NPAIR (RC_BW / RC_PAIR)
-// a stage holds one tile (min(n, RC_W) columns) + 8 zero slots that padding entries of the permutation read
-__host__ __device__ inline size_t stage_bytes_for(int n) { return (size_t)(n < RC_W ? ((n + 7) & ~7) : RC_W) * 16 + 128; }
 
 struct Scal {
   double r, p, logp, log1mp;
@@ -60,46 +36,18 @@ struct Scal {
   rc_i128 aaD, aaL, abD, abL, bbD, bbL;   // block sums of the proposed state (rows a, b)
   int K;
   int status;
-  int rebuild;
   int forked;                             // numMH > 1: an accepted proposal replaced the local state this iteration
   int fslotA, fslotB;                     // slots whose W rows come from the scratch rows (-1: none)
   int itmp[8];
   double llcur; unsigned llclk;           // incremental kernel: loglik of the chain's own state at change count llclk (0: none)
 };
 
-#define RC_MQ 16                     // move queue entries (moves not yet patched into the permutation)
 // cycle counters of rc_sampler_copy_stats: compile with -DRC_NO_STATS to drop the clock reads from the hot loops
 #ifdef RC_NO_STATS
 #define RC_CLOCK() 0LL
 #else
 #define RC_CLOCK() clock64()
 #endif
-#define RC_NOISE 64                  // precomputed Gumbel noise entries per row
-#define RC_NR 4                      // rows of noise the helper warp may run ahead of the decisions
-#define RC_XTHR 64                   // CTA-level helper threads: the tile producer warp and the noise warp
-struct ScanShared {                  // per chain: hand-off between the bulk warps and the decision warp
-  unsigned long long ready[2];       // the row sums of parity b are complete             (count RC_BW)
-  unsigned long long consumed[2];    // the decision warp has copied them to registers   (count 1)
-  volatile int M;                    // moves published by the decision warp
-  volatile int decided;              // rows decided
-  int rowP[2];                       // moves already patched into the permutation when the row was reduced
-  int msnap[2];                      // moves published when the decision warp released the row sums of parity b
-  int prebuilt;                      // moves contained in the permutation after a rebuild
-  int inited;
-  unsigned short mq_j[RC_MQ];
-  unsigned char mq_a[RC_MQ], mq_b[RC_MQ];
-  double noise[RC_NR][RC_NOISE];     // Gumbel noise of row i in noise[i % RC_NR] (written by the CTA's noise warp)
-  volatile int noise_ready;          // rows whose noise is complete
-};
-
-struct CtaShared {
-  unsigned long long full[RC_NSTAGE];
-  unsigned long long empty[RC_NSTAGE];
-  volatile long long issued[RC_NSTAGE];   // tile of the row stream last issued into each stage (-1: none)
-  int active[8];
-  int nact;
-  int issuer;
-};
 
 // Incremental mode (k_chain_inc): hand-off block of the chain's team.
 #define RC_INC_MAXW 16               // warps per chain, at most
@@ -139,38 +87,22 @@ struct IncShared {
 #define RC_SUM_MARGIN 41.0
 
 struct Ctx {
-  int n, cap, tiles;
+  int n, cap;
   int qD, qL;
   int ctid, cwarp, lane, barid;           // thread / warp index within the chain, named barrier of the chain
-  int nthr, nwarp;                        // threads / warps of the chain's team (RC_NTHR in k_chain, the whole CTA in k_chain_inc)
-  int bbarid;                             // named barrier of the chain's bulk warps
-  unsigned dummy;                         // permutation padding entry = byte offset of the zero slots behind a staged tile
-  size_t stage_bytes;
+  int nthr, nwarp;                        // threads / warps of the chain's team (the whole CTA, or part of it beside the restricted scans)
   const longlong2* DL;
   const rc_kparams* kp;
-  // shared memory (per chain)
+  // shared memory
   uint8_t* lab;
-  uint8_t* labL;          // the labels a split-merge step works on in place (launch state): the chain's own array, or -- incremental mode
-                          // with one proposal per iteration -- a copy, so that the scan can run beside the restricted scans
-  unsigned short* perm;
-  unsigned short* runStart;
-  unsigned char* bscratch[2];   // build_perm scratch (run counters + chunk slot masks): aliases the row-sum buffers
-  int* tileStart;
-  longlong2* partial;     // [2][RC_BW][cap] (row parity x bulk warp); aliased by rowA/rowB during loglik of a proposed state
-  ScanShared* ss;
+  uint8_t* labL;          // the labels a split-merge step works on in place (launch state): the chain's own array, or -- with one
+                          // proposal per iteration -- a copy, so that the scan can run beside the restricted scans
+  rc_i128* prows;         // [4][cap] rows A_D, A_L, B_D, B_L of the block sums of a split-merge step's proposed state
   int* sizes;
   int* szL;
   int* itmp;              // [cap]
   uint8_t* clist;         // [cap]
-  long long* red;         // [RC_NWARP * 4]
   Scal* sc;
-  // shared memory (per CTA)
-  unsigned char* stages;
-  CtaShared* cta;
-  const unsigned short* colpos;  // column of point j in the streamed matrix (null: column j), see rc_kparams::colpos
-  const unsigned short* colpt;   // point of column c (null: point c)
-  unsigned char* chain0;     // shared memory of chain slot 0; slot q starts chain_stride bytes further
-  size_t chain_stride, ss_off;
   // per-chain global memory
   rc_i128* WD;
   rc_i128* WL;
@@ -178,35 +110,29 @@ struct Ctx {
   rc_i128* WLbak;
   uint8_t* labbak;
   int* szbak;
-  longlong2* T;
-  longlong2* S;           // incremental mode (k_chain_inc): [cap][n] row sums by slot, S[k][x] = sum_{j in k} DL[x][j]; null otherwise
-  struct IncShared* inc;  // incremental mode: hand-off block of the scan
-  int mcap;               // incremental mode: members of a split-merge step whose AB / DG / L2s fit the shared-memory scratch
+  longlong2* S;           // [cap][n] row sums by slot, S[k][x] = sum_{j in k} DL[x][j]
+  struct IncShared* inc;  // hand-off block of the scan
+  int mcap;               // members of a split-merge step whose AB / DG / L2s fit the shared-memory scratch
   longlong4* mAB; longlong2* mDG; double2* mL2s;   // that scratch
-  uint8_t* live;          // incremental mode (shared memory): live slots, ascending
-  uint8_t* rank;          // incremental mode (shared memory): [cap] number of live slots below each slot
-  double* tabs;           // incremental mode (shared memory): [6][cap] lgamma(alpha + delta1 s), lgamma(zeta + delta2 s), prior term at the slot's size / at size - 1
-  int* res;               // incremental mode (shared memory): [nthr] slot chosen by each row of a batch
-  double2* Cc;            // incremental mode (global): [cap][n] cached per-slot terms, see inc_eval_row
-  RowSum* Rs;             // incremental mode (global): [n] row summaries
-  double* LLF; unsigned* LLFs;   // incremental mode (global): [cap][cap] loglik of the state with slot ci merged into cj, and the change count it was computed at (0: never)
-  unsigned* tw;           // incremental mode (shared memory when it fits, else global): [n] change count at which point x's cached entries were last made valid
-  unsigned* tchg;         // incremental mode (shared memory): [cap] change count at which each slot last gained or lost a point
+  uint8_t* live;          // (shared memory) live slots, ascending
+  uint8_t* rank;          // (shared memory) [cap] number of live slots below each slot
+  double* tabs;           // (shared memory) [6][cap] lgamma(alpha + delta1 s), lgamma(zeta + delta2 s), prior term at the slot's size / at size - 1
+  int* res;               // (shared memory) [nthr] slot chosen by each row of a batch
+  double2* Cc;            // (global) [cap][n] cached per-slot terms, see inc_eval_row
+  RowSum* Rs;             // (global) [n] row summaries
+  double* LLF; unsigned* LLFs;   // (global) [cap][cap] loglik of the state with slot ci merged into cj, and the change count it was computed at (0: never)
+  unsigned* tw;           // (shared memory when it fits, else global) [n] change count at which point x's cached entries were last made valid
+  unsigned* tchg;         // (shared memory) [cap] change count at which each slot last gained or lost a point
   unsigned short* Slist;  // members of ci u cj: S ascending, then i, then j
   uint8_t* origM;         // their labels in the chain's state
   longlong4* AB;          // [n+2] running sums of each member's row over the two candidate clusters {aD, aL, bD, bL}
   double2* L2s;           // [n]   static repulsion terms of the first two live slots, per item
   double2* NZ;            // [(numGibbs+1) * n] Gumbel noise of the free restricted scans
-  double* LPR;            // [n+2] prior term of joining a cluster of size s, for this iteration's (r, p)
   longlong2* DG;          // [n+2] DL[x][x] of the members
   double* terms;
   long long* stats;       // [16] cycle counters of this chain (see rc_sampler_copy_stats)
   unsigned long long key;
 };
-// The streamed matrix may have its COLUMNS permuted (label-sorted by the initial clustering, rc_api.cu): element (i, j)
-// of D then sits in column cpos(j) of row i.  Sums over columns do not care; direct element reads go through cpos.
-__device__ __forceinline__ int cpos(const Ctx& c, int j) { return c.colpos ? (int)__ldg(c.colpos + j) : j; }
-__device__ __forceinline__ int cpt(const Ctx& c, int col) { return c.colpt ? (int)__ldg(c.colpt + col) : col; }
 // Incremental mode: point y moved from slot a to slot b.  Every x's sums over a and b follow from row y (D is symmetric:
 // DL[x][y] == DL[y][x]); exact integers, so S stays what a from-scratch build would give.  Thread t always owns the same
 // x's for a given t0, so successive moves with the same t0 need no barrier between them (one before the sums are read again).
@@ -243,9 +169,6 @@ enum { ST_DEC_WAIT = 0, ST_DEC_WORK, ST_BULK_WAIT_CONSUMED, ST_BULK_WAIT_FULL, S
 __device__ __forceinline__ void st_add(const Ctx& c, int slot, long long v) { c.stats[slot] += v; }
 
 __device__ __forceinline__ void csync(const Ctx& c) { asm volatile("bar.sync %0, %1;" ::"r"(c.barid), "r"(c.nthr) : "memory"); }
-__device__ __forceinline__ void bsync(const Ctx& c) { asm volatile("bar.sync %0, %1;" ::"r"(c.bbarid), "r"(RC_BW * 32) : "memory"); }
-// a team is either the whole chain (RC_NTHR threads, csync) or its bulk warps (RC_BW*32 threads, bsync)
-template <bool BULK> __device__ __forceinline__ void tsync(const Ctx& c) { if (BULK) bsync(c); else csync(c); }
 
 // sum of a 128-bit value over the lanes of a warp (every lane gets the total)
 __device__ __forceinline__ rc_i128 warp_sum128(rc_i128 v) {
@@ -259,810 +182,11 @@ __device__ __forceinline__ rc_i128 warp_sum128(rc_i128 v) {
   return v;
 }
 __device__ __forceinline__ int tri(int k, int t, int cap) { return k < t ? k * cap + t : t * cap + k; }
-__device__ __forceinline__ long long shfl_up_ll(long long v, int off) { return __shfl_up_sync(0xffffffffu, v, off); }
-__device__ __forceinline__ long long shfl_xor_ll(long long v, int off) { return __shfl_xor_sync(0xffffffffu, v, off); }
-
-// ---- mbarrier / bulk-copy primitives -----------------------------------------------------------------
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-// Explicit shared-space accesses (32-bit shared addresses): the hot loops must not fall back to generic LD/ST,
-// which the compiler emits when it cannot prove that a pointer carried in Ctx points to shared memory.
-__device__ __forceinline__ longlong2 lds_ll2(unsigned a) {
-  longlong2 v;
-  asm volatile("ld.shared.v2.s64 {%0, %1}, [%2];" : "=l"(v.x), "=l"(v.y) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ void sts_ll2(unsigned a, longlong2 v) {
-  asm volatile("st.shared.v2.s64 [%0], {%1, %2};" ::"r"(a), "l"(v.x), "l"(v.y) : "memory");
-}
-__device__ __forceinline__ uint4 lds_u4(unsigned a) {
-  uint4 v;
-  asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_inval(unsigned long long* bar) {
-  asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(unsigned long long* bar) {
-  asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.shared::cta.b64 st, [%0];\n\t}" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
-  asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.expect_tx.shared::cta.b64 st, [%0], %1;\n\t}" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-// global -> shared bulk async copy (TMA engine, 1-D), completion counted in bytes on `bar`
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned bytes, unsigned long long* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-
-// ------------------------------------------------------------------------------------------------
-// (tile, label)-sorted column permutation in chunks of 8 columns: every (tile, label) run is padded to a multiple
-// of 8, so a chunk has one label (carried in the low nibbles of its entries).  A tile is reduced by ONE warp whose lane l owns the contiguous
-// chunks [l*cc, (l+1)*cc) of the tile (cc = ceil(chunks / 32)); inside a chunk the 8 entries are rotated by the
-// owning lane so that, when cluster members are contiguous columns (generatemixture sorts the labels), the 8 lanes
-// of a shared-memory wavefront hit 8 different 16-byte bank groups.
-// ------------------------------------------------------------------------------------------------
-template <bool BULK>
-__device__ void build_perm(const Ctx& c, int buf = 0) {
-  constexpr int NT = BULK ? RC_BW * 32 : RC_NTHR;
-  const uint8_t* lab = c.lab;
-  const int tid = c.ctid, E = c.tiles * c.cap;
-  unsigned int* const cnt = reinterpret_cast<unsigned int*>(c.bscratch[buf]);      // [tiles * cap] run sizes / cursors
-  unsigned char* const cmask = c.bscratch[buf] + sizeof(unsigned int) * E;          // [chunks] occupied slots
-  for (int t = tid; t < E; t += NT) cnt[t] = 0;
-  tsync<BULK>(c);
-  for (int j = tid; j < c.n; j += NT) atomicAdd(&cnt[(j >> RC_LOGW) * c.cap + lab[cpt(c, j)]], 1u);      // j: column
-  tsync<BULK>(c);
-  if (tid < 32) {
-    const int chunk = (E + 31) / 32;
-    const int b = tid * chunk, e = min(E, b + chunk);
-    unsigned s = 0;
-    for (int t = b; t < e; ++t) s += (cnt[t] + 7u) & ~7u;
-    unsigned incl = s;
-    for (int off = 1; off < 32; off <<= 1) {
-      const unsigned o = __shfl_up_sync(0xffffffffu, incl, off);
-      if (tid >= off) incl += o;
-    }
-    unsigned run = incl - s;
-    for (int t = b; t < e; ++t) { c.runStart[t] = (unsigned short)run; run += (cnt[t] + 7u) & ~7u; }
-    if (tid == 31) {
-      c.runStart[E] = (unsigned short)incl;
-      if (incl > (unsigned)c.kp->npad_max) c.sc->status = RC_ERR_SLOTS;   // padding of the (tile, label) runs exceeds the reserve
-    }
-  }
-  tsync<BULK>(c);
-  if (c.sc->status) return;
-  const int total = c.runStart[E];
-  for (int t = tid; t <= c.tiles; t += NT) c.tileStart[t] = c.runStart[t == c.tiles ? E : t * c.cap] >> 3;
-  // Every entry is a byte offset (column * 16, low 4 bits free); the chunk's label rides in the low nibbles of its
-  // entries 0 (low 4 bits of the label) and 1 (high 4 bits).  Padding entries point at the zero slots.
-  for (int t = tid; t < E; t += NT) {
-    const int g0 = c.runStart[t] >> 3, g1 = c.runStart[t + 1] >> 3;
-    const unsigned l = (unsigned)(t % c.cap);
-    for (int g = g0; g < g1; ++g) {
-      uint4 v;
-      v.x = (c.dummy | (l & 15u)) | ((c.dummy | (l >> 4)) << 16);
-      v.y = v.z = v.w = c.dummy | (c.dummy << 16);
-      reinterpret_cast<uint4*>(c.perm)[g] = v;
-      cmask[g] = 0;
-    }
-  }
-  tsync<BULK>(c);
-  for (int t = tid; t < E; t += NT) cnt[t] = 0;
-  tsync<BULK>(c);
-  for (int j = tid; j < c.n; j += NT) {
-    const int tile = j >> RC_LOGW;
-    const int e = tile * c.cap + lab[cpt(c, j)];
-    const unsigned rk = atomicAdd(&cnt[e], 1u);
-    const int g = (c.runStart[e] >> 3) + (int)(rk >> 3);                 // chunk of the run that takes the element
-    const int g0 = c.tileStart[tile], cc = (c.tileStart[tile + 1] - g0 + 32 * RC_PAIR - 1) / (32 * RC_PAIR);
-    const int owner = (g - g0) / cc;                                     // (virtual) lane that will read this chunk
-    // Slot inside the chunk: the lane reads slot s with its s-th gather; putting the column with residue r (mod 8)
-    // at slot (r - owner) mod 8 makes the 8 lanes of a shared-memory wavefront hit 8 different 16-byte bank groups.
-    // If that slot is taken (the chunk's columns are not 8 consecutive ones) any free slot will do.
-    unsigned slot = ((unsigned)j - (unsigned)owner) & 7u;
-    unsigned char* cm = &cmask[g];
-    unsigned* word = reinterpret_cast<unsigned*>(reinterpret_cast<size_t>(cm) & ~(size_t)3);
-    const unsigned sh = (unsigned)(reinterpret_cast<size_t>(cm) & 3) * 8u;
-    for (int tries = 0; tries < 8; ++tries) {
-      const unsigned bit = (1u << slot) << sh;
-      if (!(atomicOr(word, bit) & bit)) break;
-      slot = (slot + 1u) & 7u;
-    }
-    unsigned short* pe = c.perm + g * 8 + slot;
-    *pe = (unsigned short)((((unsigned)j & (RC_W - 1)) << 4) | (*pe & 15u));
-  }
-  tsync<BULK>(c);
-}
-
-// Point j (column) moved from slot a to slot b: patch the permutation in place (warp 0 of the chain).  If the
-// run of (tile, b) has no free padding entry the caller rebuilds.
-__device__ void patch_perm(const Ctx& c, int jpoint, int a, int b) {
-  const int lane = c.lane;
-  const int j = cpos(c, jpoint);                 // the point's column
-  const int tile = j >> RC_LOGW;
-  const unsigned idx = ((unsigned)j & (RC_W - 1)) << 4;
-  {
-    const int e = tile * c.cap + a;
-    const int p0 = c.runStart[e], p1 = c.runStart[e + 1];
-    for (int pb = p0; pb < p1; pb += 32) {
-      const int p = pb + lane;
-      if (p < p1 && (c.perm[p] & 0xfff0u) == idx) c.perm[p] = (unsigned short)(c.dummy | (c.perm[p] & 15u));
-    }
-  }
-  __syncwarp();
-  bool done = false;
-  {
-    const int e = tile * c.cap + b;
-    const int p0 = c.runStart[e], p1 = c.runStart[e + 1];
-    for (int pb = p0; pb < p1 && !done; pb += 32) {
-      const int p = pb + lane;
-      const unsigned m = __ballot_sync(0xffffffffu, p < p1 && (c.perm[p] & 0xfff0u) == c.dummy);
-      if (m) {
-        if (lane == __ffs(m) - 1) c.perm[p] = (unsigned short)(idx | (c.perm[p] & 15u));
-        done = true;
-      }
-    }
-  }
-  if (!done && lane == 0) c.sc->rebuild = 1;
-  __syncwarp();
-}
-
-// 8 gathers + sums of one chunk.  The permutation stores BYTE offsets (column index * 16; the low nibbles of entries
-// 0 and 1 carry the chunk's label) so a gather is one LDS.128 at [tile base + offset]; padding entries point at the
-// zero slots behind the staged tile.
-__device__ __forceinline__ void gather8_staged(unsigned tile_addr, const uint4 pk, long long& d, long long& l) {
-  const unsigned w[4] = {pk.x, pk.y, pk.z, pk.w};
-  longlong2 v[8];
-#pragma unroll
-  for (int e = 0; e < 8; ++e) {
-    const unsigned off = (e & 1) ? ((w[e >> 1] >> 16) & 0xfff0u) : (w[e >> 1] & 0xfff0u);
-    v[e] = lds_ll2(tile_addr + off);
-  }
-  d += ((v[0].x + v[1].x) + (v[2].x + v[3].x)) + ((v[4].x + v[5].x) + (v[6].x + v[7].x));
-  l += ((v[0].y + v[1].y) + (v[2].y + v[3].y)) + ((v[4].y + v[5].y) + (v[6].y + v[7].y));
-}
-__device__ __forceinline__ void gather8_global(const Ctx& c, const char* src, const uint4 pk, long long& d, long long& l) {
-  const unsigned w[4] = {pk.x, pk.y, pk.z, pk.w};
-#pragma unroll
-  for (int e = 0; e < 8; ++e) {
-    const unsigned off = (e & 1) ? ((w[e >> 1] >> 16) & 0xfff0u) : (w[e >> 1] & 0xfff0u);
-    if (off != c.dummy) {
-      const longlong2 v = __ldg(reinterpret_cast<const longlong2*>(src + off));
-      d += v.x; l += v.y;
-    }
-  }
-}
-// segmented inclusive scan of (d, l) over lanes with equal labels (labels are sorted along the lanes);
-// returns true in the last lane of each run
-__device__ __forceinline__ bool seg_scan(int lane, int lab, long long& d, long long& l) {
-  const int prev = __shfl_up_sync(0xffffffffu, lab, 1);
-  const unsigned heads = __ballot_sync(0xffffffffu, lane == 0 || prev != lab);
-  const int runstart = 31 - __clz(heads & (0xffffffffu >> (31 - lane)));
-  const int pos = lane - runstart;
-#pragma unroll
-  for (int off = 1; off < 32; off <<= 1) {
-    const long long od = shfl_up_ll(d, off), ol = shfl_up_ll(l, off);
-    if (pos >= off) { d += od; l += ol; }
-  }
-  return (lane == 31) || ((heads >> (lane + 1)) & 1u);
-}
-// One tile of one row, reduced by RC_PAIR warps (each into its own bins `part`): a lane walks its contiguous chunks keeping a
-// running sum while the label stays the same; when the label changes the finished run segment is added to its
-// bin (the run of a label ends in exactly one lane, so these read-modify-writes never collide); the open
-// segments of the 32 lanes are combined by one segmented scan at the end of the tile.
-// STAGED: `src_` is the staged tile in shared memory, otherwise the row in global memory.
-template <bool STAGED>
-__device__ __forceinline__ void reduce_tile(const Ctx& c, const longlong2* src_, int tile, longlong2* part) {
-  const int lane = c.lane;
-  const char* src = reinterpret_cast<const char*>(src_);
-  const unsigned tile_addr = STAGED ? smem_u32(src_) : 0u;
-  const unsigned part_addr = smem_u32(part), perm_addr = smem_u32(c.perm);
-  const int g0 = c.tileStart[tile], g1 = c.tileStart[tile + 1];
-  const int cc = (g1 - g0 + 32 * RC_PAIR - 1) / (32 * RC_PAIR);
-  int g = g0 + ((c.cwarp % RC_PAIR) * 32 + lane) * cc;        // the RC_PAIR warps of a tile form 32 * RC_PAIR virtual lanes
-  const int ge = min(g1, g + cc);
-  int cur = 0x100;
-  long long d = 0, l = 0;
-  uint4 pkn = make_uint4(0, 0, 0, 0);
-  if (g < ge) pkn = lds_u4(perm_addr + (unsigned)g * 16u);  // the next chunk's offsets (+ label nibbles) are loaded one step ahead
-  for (; g < ge; ++g) {
-    const uint4 pk = pkn;
-    const int lab = (int)((pk.x & 15u) | ((pk.x >> 12) & 0xf0u));
-    if (g + 1 < ge) pkn = lds_u4(perm_addr + (unsigned)(g + 1) * 16u);
-    if (lab != cur) {
-      if (cur != 0x100) {
-        longlong2 a = lds_ll2(part_addr + (unsigned)cur * 16u);
-        a.x += d; a.y += l;
-        sts_ll2(part_addr + (unsigned)cur * 16u, a);
-      }
-      cur = lab; d = 0; l = 0;
-    }
-    if (STAGED) gather8_staged(tile_addr, pk, d, l);
-    else gather8_global(c, src, pk, d, l);
-  }
-  __syncwarp();
-  const bool tail = seg_scan(lane, cur, d, l);
-  if (cur != 0x100 && tail) {
-    longlong2 a = lds_ll2(part_addr + (unsigned)cur * 16u);
-    a.x += d; a.y += l;
-    sts_ll2(part_addr + (unsigned)cur * 16u, a);
-  }
-  __syncwarp();
-}
-
-__device__ __forceinline__ void zero_partial(const Ctx& c, int buf) {   // bulk warps
-  const unsigned part = smem_u32(c.partial + (buf * RC_BW + c.cwarp) * c.cap);
-  for (int s = c.lane; s < c.cap; s += 32) sts_ll2(part + (unsigned)s * 16u, make_longlong2(0, 0));
-  __syncwarp();
-}
-
-// Row x straight from global memory / L2 (split-merge member rows, block-sum initialisation); buffer 0.
-__device__ void reduce_row_global(const Ctx& c, int x) {
-  if (c.cwarp >= RC_BW) return;
-  zero_partial(c, 0);
-  const longlong2* row = c.DL + (size_t)x * c.n;
-  longlong2* part = c.partial + c.cwarp * c.cap;
-  for (int tile = c.cwarp / RC_PAIR; tile < c.tiles; tile += RC_NPAIR) reduce_tile<false>(c, row + (size_t)tile * RC_W, tile, part);
-}
-
-__device__ __forceinline__ longlong2 bin_total(const Ctx& c, int s, int buf = 0) {
-  const unsigned p = smem_u32(c.partial + (size_t)buf * RC_BW * c.cap) + (unsigned)s * 16u;
-  longlong2 a = lds_ll2(p);
-#pragma unroll
-  for (int w = 1; w < RC_BW; ++w) {
-    const longlong2 b = lds_ll2(p + (unsigned)(w * c.cap) * 16u);
-    a.x += b.x; a.y += b.y;
-  }
-  return a;
-}
-
-// ------------------------------------------------------------------------------------------------
-// The full Gibbs scan (mcmc.jl:158-256) is a two-stage pipeline per chain:
-//   bulk warps (0..RC_BW-1): reduce row i against the label permutation into partial[i & 1] and signal
-//       ready[i & 1]; they run up to two rows ahead of the decisions.
-//   decision warp (RC_BW): for i = 0..n-1 (mcmc.jl:192-253) waits for row i's sums, corrects them for the
-//       moves the permutation did not contain yet (exact integers), evaluates the candidates (lane l owns
-//       slots l, l+32, l+64, l+96), draws by Gumbel-max, and publishes the move.
-// Moves are applied to the permutation by the bulk warps between two rows (patch in place; rebuild from
-// the labels once the decisions have caught up when a run is full).
-// ------------------------------------------------------------------------------------------------
-// NSR = rounds of 32 slots held in registers.  decide_rows<2> serves chains whose live slots (and next free slot)
-// are all below 64 -- half the register state, no spills -- and returns the row at which a slot >= 64 is needed;
-// decide_rows<NSR> continues from there.  `M` (moves published) and the counters carry over.
-// Warp-wide minimum / maximum of doubles that are not NaN (infinities allowed) with two 32-bit REDUX operations on an
-// order-preserving integer key instead of a five-round shuffle butterfly of fp64 compares (the decision warp's
-// latency chain).  -0.0 is folded onto +0.0 first; minimum and maximum are exact, so nothing else changes.
-__device__ __forceinline__ unsigned long long f64_key(double v) {
-  const unsigned long long b = (unsigned long long)__double_as_longlong(v + 0.0);
-  return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
-}
-__device__ __forceinline__ double f64_unkey(unsigned long long k) {
-  return __longlong_as_double((long long)((k >> 63) ? (k & 0x7fffffffffffffffull) : ~k));
-}
-__device__ __forceinline__ double warp_min_f64(double v) {
-  const unsigned long long k = f64_key(v);
-  const unsigned hi = (unsigned)(k >> 32), lo = (unsigned)k;
-  const unsigned hm = __reduce_min_sync(0xffffffffu, hi);
-  const unsigned lm = __reduce_min_sync(0xffffffffu, hi == hm ? lo : 0xffffffffu);
-  return f64_unkey(((unsigned long long)hm << 32) | lm);
-}
-__device__ __forceinline__ double warp_max_f64(double v) {
-  const unsigned long long k = f64_key(v);
-  const unsigned hi = (unsigned)(k >> 32), lo = (unsigned)k;
-  const unsigned hm = __reduce_max_sync(0xffffffffu, hi);
-  const unsigned lm = __reduce_max_sync(0xffffffffu, hi == hm ? lo : 0u);
-  return f64_unkey(((unsigned long long)hm << 32) | lm);
-}
-
-struct DecCarry { int M, nmoves; bool dead; long long acc_wait, acc_work, tlast; };
-template <int NSR>
-__device__ int decide_rows(const Ctx& c, unsigned it, int istart, DecCarry& cy) {
-  const int lane = c.lane;
-  const rc_kparams& kp = *c.kp;
-  const rc_params& P = kp.P;
-  const int cap = c.cap, n = c.n;
-  ScanShared* ss = c.ss;
-  const double r = c.sc->r, log1mp = c.sc->log1mp;
-  const unsigned ltmask = (1u << lane) - 1u;
-  // register-resident per-slot state: size, and the size-dependent table terms at the current size (t*) and
-  // at size - 1 (u*: used for the slot the visited point is detached from).  Tables are only touched on moves.
-  int sz[NSR];
-  double tA[NSR], tZ[NSR], tP[NSR], uA[NSR], uZ[NSR], uP[NSR];
-#pragma unroll
-  for (int w = 0; w < NSR; ++w) {
-    const int s = w * 32 + lane;
-    sz[w] = s < cap ? c.sizes[s] : 0;
-    const int s1 = sz[w] > 0 ? sz[w] : 1, s0 = sz[w] > 1 ? sz[w] - 1 : 1;
-    tA[w] = kp.LGA[sz[w]]; tZ[w] = kp.LGZ[sz[w]]; tP[w] = c.LPR[s1];
-    uA[w] = kp.LGA[sz[w] > 0 ? sz[w] - 1 : 0]; uZ[w] = kp.LGZ[sz[w] > 0 ? sz[w] - 1 : 0]; uP[w] = c.LPR[s0];
-  }
-  int M = cy.M;
-  bool dead = cy.dead;
-  long long tlast = cy.tlast, acc_wait = cy.acc_wait, acc_work = cy.acc_work;
-  int nmoves = cy.nmoves;
-  int istop = n;
-  longlong2 self1 = __ldg(c.DL + (size_t)istart * n + cpos(c, istart));              // diagonal entry of row i (prefetched two rows ahead)
-  longlong2 self2 = istart + 1 < n ? __ldg(c.DL + (size_t)(istart + 1) * n + cpos(c, istart + 1)) : make_longlong2(0, 0);
-  for (int i = istart; i < n; ++i) {
-    const int li = c.lab[i];
-    const longlong2 self = self1;
-    self1 = self2;
-    if (i + 2 < n) self2 = __ldg(c.DL + (size_t)(i + 2) * n + cpos(c, i + 2));
-    // occupancy with i detached (:193-202) -- independent of the row sums
-    unsigned occ[NSR];
-#pragma unroll
-    for (int w = 0; w < NSR; ++w) {
-      const int s = w * 32 + lane;
-      occ[w] = __ballot_sync(0xffffffffu, sz[w] - (s == li ? 1 : 0) > 0);
-    }
-    int Ki = 0, e = -1, nw = 0;
-#pragma unroll
-    for (int w = 0; w < NSR; ++w) {
-      Ki += __popc(occ[w]);
-      if (occ[w]) nw = w + 1;
-      const int lim = cap - w * 32;
-      const unsigned capmask = lim >= 32 ? 0xffffffffu : (lim <= 0 ? 0u : ((1u << lim) - 1u));
-      const unsigned emp = ~occ[w] & capmask;
-      if (e < 0 && emp) e = w * 32 + __ffs(emp) - 1;                        // findfirst(clustsizes .== 0)
-    }
-    const bool hasnew = (P.maxK == 0 || Ki < P.maxK) && Ki < n;             // :198
-    if (NSR * 32 < RC_MAXCAP && hasnew && e < 0 && cap > NSR * 32) { istop = i; break; }   // needs a slot beyond this instantiation
-    if (!dead && hasnew && e < 0) {                                         // slot capacity exhausted
-      if (lane == 0) c.sc->status = RC_ERR_SLOTS;
-      dead = true;
-    }
-    if (hasnew && e >= 0 && (e >> 5) + 1 > nw) nw = (e >> 5) + 1;           // rounds of 32 slots that hold a candidate
-    int kk[NSR];
-    bool have[NSR];
-    {
-      int base = 0;
-#pragma unroll
-      for (int w = 0; w < NSR; ++w) {
-        const int s = w * 32 + lane;
-        const bool live = (occ[w] >> lane) & 1u;
-        have[w] = live || (hasnew && s == e);
-        kk[w] = live ? base + __popc(occ[w] & ltmask) : Ki;
-        base += __popc(occ[w]);
-      }
-    }
-    // ---- row sums of row i ----
-    const long long tw0 = RC_CLOCK();
-    const int buf = i & 1;
-    mbar_wait(&ss->ready[buf], (unsigned)((i >> 1) & 1));
-    if (c.sc->status) dead = true;
-    const long long tw1 = RC_CLOCK();
-    acc_wait += tw1 - tw0; acc_work += tw0 - tlast;
-    tlast = tw1;
-    const int Prow = ss->rowP[buf];
-    if (!dead) {                                 // the noise warp runs rows ahead: this wait is normally already satisfied
-      while (ss->noise_ready <= i) __nanosleep(20);
-      __threadfence_block();
-    }
-    long long bd[NSR], bl[NSR];
-    double nzv[NSR];
-#pragma unroll
-    for (int w = 0; w < NSR; ++w) {
-      bd[w] = 0; bl[w] = 0; nzv[w] = 0.0;
-      if (w < nw) {
-        const int s = w * 32 + lane;
-        if ((occ[w] >> lane) & 1u) {
-          const longlong2 t = bin_total(c, s, buf);
-          bd[w] = t.x; bl[w] = t.y;
-        }
-        if (have[w] && kk[w] < RC_NOISE) nzv[w] = ss->noise[i & (RC_NR - 1)][kk[w]];
-      }
-    }
-    if (lane == 0) ss->msnap[buf] = M;
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&ss->consumed[buf]);
-    if (dead) { if (lane == 0) ss->decided = i + 1; continue; }
-    // moves of earlier steps that the permutation did not contain when row i was reduced
-    for (int m = Prow; m < M; ++m) {
-      const int j = ss->mq_j[m % RC_MQ], a = ss->mq_a[m % RC_MQ], b = ss->mq_b[m % RC_MQ];
-      const longlong2 ev = __ldg(c.DL + (size_t)i * n + cpos(c, j));
-#pragma unroll
-      for (int w = 0; w < NSR; ++w) {
-        const int s = w * 32 + lane;
-        const bool live = (occ[w] >> lane) & 1u;
-        if (s == a && live) { bd[w] -= ev.x; bl[w] -= ev.y; }
-        if (s == b && live) { bd[w] += ev.x; bl[w] += ev.y; }
-      }
-    }
-    // per-slot terms (:206-242)
-    double L1[NSR], L2p[NSR];
-    double acc = 0.0;
-#pragma unroll
-    for (int w = 0; w < NSR; ++w) {
-      L1[w] = 0.0; L2p[w] = 0.0;
-      if (w < nw) {
-        const int s = w * 32 + lane;
-        if ((occ[w] >> lane) & 1u) {
-          if (s == li) { bd[w] -= self.x; bl[w] -= self.y; }                // :193-194 detach i
-          const int szs = sz[w] - (s == li ? 1 : 0);
-          const double szd = (double)szs;
-          const double sD = rc_dequant(bd[w], c.qD), sL = rc_dequant(bl[w], c.qL);
-          const double a_i = P.alpha + P.delta1 * szd, b_i = P.beta + sD;
-          const double z_i = P.zeta + P.delta2 * szd, g_i = P.gamma + sD;
-          L1[w] = (s == li ? uA[w] : tA[w]) + kp.abratio - a_i * rc_log(b_i) + (P.delta1 - 1) * sL - szd * kp.lgd1;
-          L2p[w] = (s == li ? uZ[w] : tZ[w]) - z_i * rc_log(g_i) + kp.zgratio + (P.delta2 - 1) * sL - szd * kp.lgd2;
-          acc += L2p[w];                                                    // vecsum: lane-wise ascending slots
-        }
-      }
-    }
-#pragma unroll
-    for (int off = 16; off >= 1; off >>= 1) acc = acc + __shfl_xor_sync(0xffffffffu, acc, off);   // :243 canonical butterfly
-    const double L2i = acc;
-    // log-probabilities (:244-247)
-    double lp[NSR];
-    bool anynan = false;
-    double mn = RC_INF;
-#pragma unroll
-    for (int w = 0; w < NSR; ++w) {
-      lp[w] = 0.0;
-      if (w < nw) {
-        const int s = w * 32 + lane;
-        if ((occ[w] >> lane) & 1u) {
-          const double L2 = L2i - L2p[w];
-          lp[w] = (s == li ? uP[w] : tP[w]) + (L1[w] + (P.repulsion ? L2 : copysign(0.0, L2)));
-        } else if (have[w]) {                                               // :228-230 new cluster
-          const double L2 = L2i - 0.0;
-          lp[w] = (kp.LOGN[Ki + 1] + r * log1mp) + (0.0 + (P.repulsion ? L2 : copysign(0.0, L2)));
-        }
-        if (have[w]) {
-          if (rc_isnan(lp[w])) anynan = true;
-          else if (lp[w] < mn) mn = lp[w];
-        }
-      }
-    }
-    mn = warp_min_f64(mn);
-    anynan = __any_sync(0xffffffffu, anynan);
-    if (anynan) mn = RC_NAN;                                                // Julia minimum propagates NaN
-    // Gumbel-max (utils.jl:2-6): argmax of noise + shifted log-probability, first index wins ties
-    double g[NSR];
-    double gbest = -RC_INF;
-    bool gnan = false;
-#pragma unroll
-    for (int w = 0; w < NSR; ++w) {
-      g[w] = -RC_INF;
-      if (w < nw && have[w]) {
-        double nz = nzv[w];
-        if (kk[w] >= RC_NOISE) {
-          const rc_draw dr = rc_draw2(c.key, it, RC_SITE_SCAN, 0, (uint32_t)i, (uint32_t)(kk[w] >> 1));
-          nz = -rc_log(-rc_log((kk[w] & 1) ? dr.u1 : dr.u0));
-        }
-        g[w] = nz + (lp[w] - mn);
-        if (rc_isnan(g[w])) gnan = true;
-        else if (g[w] > gbest) gbest = g[w];
-      }
-    }
-    int cnew;
-    if (!__any_sync(0xffffffffu, gnan)) {
-      // fast path: maximum value, then the smallest candidate index that attains it
-      gbest = warp_max_f64(gbest);
-      int kbest = 0x7fffffff, sbest = -1;
-#pragma unroll
-      for (int w = 0; w < NSR; ++w)
-        if (w < nw && have[w] && g[w] == gbest && kk[w] < kbest) { kbest = kk[w]; sbest = w * 32 + lane; }
-      const int kmin = __reduce_min_sync(0xffffffffu, kbest);
-      const unsigned who = __ballot_sync(0xffffffffu, kbest == kmin && sbest >= 0);
-      cnew = __shfl_sync(0xffffffffu, sbest, __ffs(who) - 1);
-    } else {
-      // NaN is maximal for argmax and the first NaN wins
-      double bg = 0.0; int bk = 0x7fffffff, bs = -1; bool bnan = false;
-#pragma unroll
-      for (int w = 0; w < NSR; ++w) {
-        if (!(w < nw && have[w])) continue;
-        const bool gn = rc_isnan(g[w]);
-        bool better;
-        if (bs < 0) better = true;
-        else if (gn) better = !bnan || kk[w] < bk;
-        else if (bnan) better = false;
-        else better = g[w] > bg || (g[w] == bg && kk[w] < bk);
-        if (better) { bg = g[w]; bk = kk[w]; bs = w * 32 + lane; bnan = gn; }
-      }
-#pragma unroll
-      for (int off = 16; off >= 1; off >>= 1) {
-        const double og = __shfl_xor_sync(0xffffffffu, bg, off);
-        const int ok = __shfl_xor_sync(0xffffffffu, bk, off);
-        const int os = __shfl_xor_sync(0xffffffffu, bs, off);
-        const int on = __shfl_xor_sync(0xffffffffu, (int)bnan, off);
-        bool better;
-        if (os < 0) better = false;
-        else if (bs < 0) better = true;
-        else if (on) better = !bnan || ok < bk;
-        else if (bnan) better = false;
-        else better = og > bg || (og == bg && ok < bk);
-        if (better) { bg = og; bk = ok; bs = os; bnan = on != 0; }
-      }
-      cnew = bs;
-    }
-    if (cnew == li) {
-      if (lane == 0) ss->decided = i + 1;
-      continue;
-    }
-    // ---- the point moved (:250-252): publish, then update sizes, cached terms and the block sums ----
-    if (lane == 0) {
-      c.lab[i] = (uint8_t)cnew;
-      c.sizes[li] -= 1;
-      c.sizes[cnew] += 1;
-      ss->mq_j[M % RC_MQ] = (unsigned short)i; ss->mq_a[M % RC_MQ] = (unsigned char)li; ss->mq_b[M % RC_MQ] = (unsigned char)cnew;
-      __threadfence_block();
-      ss->M = M + 1;
-      ss->decided = i + 1;
-    }
-    M += 1; nmoves += 1;
-    const int a = li, b = cnew;
-#pragma unroll
-    for (int w = 0; w < NSR; ++w) {
-      const int s = w * 32 + lane;
-      if (s == a) {
-        sz[w] -= 1; tA[w] = uA[w]; tZ[w] = uZ[w]; tP[w] = uP[w];
-        uA[w] = kp.LGA[sz[w] > 0 ? sz[w] - 1 : 0]; uZ[w] = kp.LGZ[sz[w] > 0 ? sz[w] - 1 : 0]; uP[w] = c.LPR[sz[w] > 1 ? sz[w] - 1 : 1];
-      }
-      if (s == b) {
-        sz[w] += 1; uA[w] = tA[w]; uZ[w] = tZ[w]; uP[w] = tP[w];
-        tA[w] = kp.LGA[sz[w]]; tZ[w] = kp.LGZ[sz[w]]; tP[w] = c.LPR[sz[w]];
-      }
-    }
-#pragma unroll
-    for (int w = 0; w < NSR; ++w) {
-      const int s = w * 32 + lane;
-      if (s >= cap) continue;
-      if (s == a) {
-        const int ix = tri(a, a, cap);
-        rc_i128 x = c.WD[ix]; rc_sub128(x, rc_make128(2 * bd[w] + self.x)); c.WD[ix] = x;
-        rc_i128 y = c.WL[ix]; rc_sub128(y, rc_make128(2 * bl[w] + self.y)); c.WL[ix] = y;
-      } else if ((occ[w] >> lane) & 1u) {
-        const int ix = tri(a, s, cap);
-        rc_i128 x = c.WD[ix]; rc_sub128(x, rc_make128(bd[w])); c.WD[ix] = x;
-        rc_i128 y = c.WL[ix]; rc_sub128(y, rc_make128(bl[w])); c.WL[ix] = y;
-      }
-    }
-    __syncwarp();
-#pragma unroll
-    for (int w = 0; w < NSR; ++w) {
-      const int s = w * 32 + lane;
-      if (s >= cap) continue;
-      if (s == b) {
-        const int ix = tri(b, b, cap);
-        rc_i128 x = c.WD[ix]; rc_add128(x, rc_make128(2 * bd[w] + self.x)); c.WD[ix] = x;
-        rc_i128 y = c.WL[ix]; rc_add128(y, rc_make128(2 * bl[w] + self.y)); c.WL[ix] = y;
-      } else if ((occ[w] >> lane) & 1u) {
-        const int ix = tri(b, s, cap);
-        rc_i128 x = c.WD[ix]; rc_add128(x, rc_make128(bd[w])); c.WD[ix] = x;
-        rc_i128 y = c.WL[ix]; rc_add128(y, rc_make128(bl[w])); c.WL[ix] = y;
-      }
-    }
-    __syncwarp();
-  }
-  cy.M = M; cy.dead = dead; cy.tlast = tlast; cy.acc_wait = acc_wait; cy.acc_work = acc_work; cy.nmoves = nmoves;
-  return istop;
-}
-
-__device__ void decide_loop(const Ctx& c, unsigned it) {
-  DecCarry cy;
-  cy.M = 0; cy.nmoves = 0; cy.dead = false; cy.acc_wait = 0; cy.acc_work = 0; cy.tlast = RC_CLOCK();
-  bool low = true;                                                          // every live slot below 64?
-  for (int s = 64 + c.lane; s < c.cap; s += 32) low = low && c.sizes[s] == 0;
-  low = __all_sync(0xffffffffu, low);
-  int i = 0;
-  if (low) i = decide_rows<2>(c, it, 0, cy);
-  if (i < c.n) decide_rows<RC_NS>(c, it, i, cy);
-  if (c.lane == 0) { st_add(c, ST_DEC_WAIT, cy.acc_wait); st_add(c, ST_DEC_WORK, cy.acc_work); st_add(c, ST_MOVES, cy.nmoves); }
-}
-
-// The row tiles are staged by the CTA's producer warp (produce_rows).  Tile T = row * tiles + tile of the stream is
-// reduced by bulk warp pair T % RC_NPAIR of every chain, so up to RC_NSTAGE tiles are in flight on different warps.
-__device__ void bulk_loop(const Ctx& c, unsigned it) {
-  const int n = c.n, tiles = c.tiles, w = c.cwarp;
-  CtaShared* cs = c.cta;
-  ScanShared* ss = c.ss;
-  int Papplied = 0;
-  bool bdead = false;
-  long long a_cons = 0, a_full = 0, a_red = 0, a_rows = 0, a_patch = 0;
-  for (int i = 0; i < n; ++i) {
-    const int buf = i & 1;
-    int Msnap = 0;
-    const long long tb0 = RC_CLOCK();
-    if (i >= 2) { mbar_wait(&ss->consumed[buf], (unsigned)(((i - 2) >> 1) & 1)); Msnap = ss->msnap[buf]; }
-    const long long tb1 = RC_CLOCK();
-    a_cons += tb1 - tb0;
-    if (Msnap > Papplied) {                     // uniform over the chain's bulk warps: patch the permutation
-      bsync(c);                                 // every bulk warp is between two rows
-      if (w == 0)
-        for (int m = Papplied; m < Msnap; ++m) patch_perm(c, ss->mq_j[m % RC_MQ], ss->mq_a[m % RC_MQ], ss->mq_b[m % RC_MQ]);
-      bsync(c);
-      Papplied = Msnap;
-      if (c.sc->rebuild) {                      // a label run was full: rebuild from the labels once they are final up to row i-1
-        while (ss->decided < i) __nanosleep(64);
-        __threadfence_block();
-        bsync(c);
-        build_perm<true>(c, buf);
-        if (c.sc->status) bdead = true;         // the rebuilt permutation does not fit: the chain stops (tiles are still consumed)
-        if (c.ctid == 0) { c.sc->rebuild = 0; ss->prebuilt = ss->M; st_add(c, ST_REBUILDS, 1); }
-        bsync(c);
-        Papplied = ss->prebuilt;
-      }
-      a_patch += RC_CLOCK() - tb1;
-    }
-    zero_partial(c, buf);
-    longlong2* part = c.partial + (buf * RC_BW + w) * c.cap;
-    // tiles of this row owned by this warp's pair: T = i * tiles + tile with T % RC_NPAIR == w / RC_PAIR
-    const int first = ((w / RC_PAIR) - (int)(((unsigned)i * (unsigned)tiles) % RC_NPAIR) + RC_NPAIR) % RC_NPAIR;
-    if (first == 0 && (w % RC_PAIR) == 0 && c.lane == 0) ss->rowP[buf] = Papplied;   // this warp opens row i: patch level
-    for (int tile = first; tile < tiles; tile += RC_NPAIR) {
-      const unsigned T = (unsigned)i * (unsigned)tiles + (unsigned)tile;      // n * tiles < 2^32: 32-bit constant division
-      const int st = (int)(T % RC_NSTAGE);
-      const unsigned k = T / RC_NSTAGE;
-      const long long tf0 = RC_CLOCK();
-      while (cs->issued[st] != (long long)T) __nanosleep(20);           // the stage has moved on to tile T (see RC_NSTAGE)
-      mbar_wait(&cs->full[st], k & 1u);
-      const long long tf1 = RC_CLOCK();
-      if (!bdead) reduce_tile<true>(c, reinterpret_cast<const longlong2*>(c.stages + (size_t)st * c.stage_bytes), tile, part);
-      __syncwarp();
-      if (c.lane == 0) mbar_arrive(&cs->empty[st]);
-      a_full += tf1 - tf0; a_red += RC_CLOCK() - tf1;
-    }
-    __syncwarp();
-    if (c.lane == 0) mbar_arrive(&ss->ready[buf]);
-    a_rows += RC_CLOCK() - tb0;
-  }
-  if (c.lane == 0) {   // per-warp counters are summed over the chain's bulk warps
-    atomicAdd((unsigned long long*)&c.stats[ST_BULK_WAIT_CONSUMED], (unsigned long long)a_cons);
-    atomicAdd((unsigned long long*)&c.stats[ST_BULK_WAIT_FULL], (unsigned long long)a_full);
-    atomicAdd((unsigned long long*)&c.stats[ST_BULK_REDUCE], (unsigned long long)a_red);
-    atomicAdd((unsigned long long*)&c.stats[ST_BULK_ROWS], (unsigned long long)a_rows);
-    atomicAdd((unsigned long long*)&c.stats[ST_BULK_PATCH], (unsigned long long)a_patch);
-  }
-}
-
-// Producer warp of the CTA: stages every tile of rows 0..n-1 into the RC_NSTAGE-deep ring, one bulk async copy
-// (cp.async.bulk, completion on full[s]) per tile, as soon as all consumers released the stage (empty[s]).
-__device__ void produce_rows(const rc_kparams& kp, unsigned char* stages, size_t stage_bytes, CtaShared* cs) {
-  if ((threadIdx.x & 31) != 0) return;
-  const int n = kp.n, tiles = kp.tiles;
-  const unsigned ntile = (unsigned)n * (unsigned)tiles;
-  int row = 0, tile = 0;
-  for (unsigned t = 0; t < ntile; ++t) {
-    const int s = (int)(t % RC_NSTAGE);
-    if (t >= RC_NSTAGE) mbar_wait(&cs->empty[s], ((t / RC_NSTAGE) - 1) & 1u);
-    const int cols = min(RC_W, n - tile * RC_W);
-    const unsigned bytes = (unsigned)cols * 16u;
-    cs->issued[s] = (long long)t;
-    __threadfence_block();
-    mbar_expect_tx(&cs->full[s], bytes);
-    bulk_g2s(stages + (size_t)s * stage_bytes, kp.DL + (size_t)row * n + (size_t)tile * RC_W, bytes, &cs->full[s]);
-    if (kp.l2pf > 0 && tile == 0 && row + kp.l2pf < n) {
-      // pull a later row towards L2 while this one is consumed: the ring only keeps two tiles in flight, too little to
-      // cover a DRAM miss; whichever CTA is ahead pays the miss early, the others hit
-      const longlong2* src = kp.DL + (size_t)(row + kp.l2pf) * n;
-      asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"((unsigned)n * 16u) : "memory");
-    }
-    if (++tile == tiles) { tile = 0; ++row; }
-  }
-}
-
-__device__ __forceinline__ ScanShared* scan_shared_of(const Ctx& c, int q) {
-  return reinterpret_cast<ScanShared*>(c.chain0 + (size_t)q * c.chain_stride + c.ss_off);
-}
-// Noise warp of the CTA: the Gumbel noise -log(-log(u)) of the first RC_NOISE candidates of every row (utils.jl:2-6) for each
-// scanning chain of the CTA, up to RC_NR rows ahead of that chain's decisions.  Four dependent-chain logarithms per
-// row and chain that used to sit on the bulk warps' critical path.
-template <int G>
-__device__ void noise_rows(const rc_kparams& kp, const Ctx& c, unsigned it) {
-  const int lane = threadIdx.x & 31, n = kp.n;
-  ScanShared* ssq[G]; unsigned long long key[G]; bool act[G];
-#pragma unroll
-  for (int q = 0; q < G; ++q) {
-    act[q] = c.cta->active[q] != 0;
-    ssq[q] = scan_shared_of(c, q);
-    key[q] = rc_chain_key(kp.seed, (unsigned long long)(kp.chain_offset + (long long)blockIdx.x * G + q));
-  }
-  for (int r = 0; r < n; ++r) {
-    double a[G], b[G];
-#pragma unroll
-    for (int q = 0; q < G; ++q) {
-      if (!act[q]) continue;
-      const rc_draw dr = rc_draw2(key[q], it, RC_SITE_SCAN, 0, (uint32_t)r, (uint32_t)lane);   // utils.jl:4-5
-      a[q] = -rc_log(-rc_log(dr.u0));
-      b[q] = -rc_log(-rc_log(dr.u1));
-    }
-#pragma unroll
-    for (int q = 0; q < G; ++q) {
-      if (!act[q]) continue;
-      while (r >= ssq[q]->decided + RC_NR) __nanosleep(40);     // the slot's previous row has been decided
-      ssq[q]->noise[r & (RC_NR - 1)][2 * lane] = a[q];
-      ssq[q]->noise[r & (RC_NR - 1)][2 * lane + 1] = b[q];
-      __threadfence_block();
-      __syncwarp();
-      if (lane == 0) ssq[q]->noise_ready = r + 1;
-    }
-  }
-}
-
-// Block sums from scratch as a scan without decisions: the decision warp's place is taken by this loop, which adds the
-// row sums of row x to W[k][t], k = label of x, for the slots t >= k (every unordered pair of slots is counted once).
-__device__ void initw_loop(const Ctx& c) {
-  ScanShared* ss = c.ss;
-  const int lane = c.lane, cap = c.cap;
-  for (int i = 0; i < c.n; ++i) {
-    const int buf = i & 1;
-    const int k = c.lab[i];
-    mbar_wait(&ss->ready[buf], (unsigned)((i >> 1) & 1));
-    longlong2 b[RC_NS];
-#pragma unroll
-    for (int w = 0; w < RC_NS; ++w) {
-      const int t = w * 32 + lane;
-      b[w] = (t < cap && t >= k) ? bin_total(c, t, buf) : make_longlong2(0, 0);
-    }
-    if (lane == 0) ss->msnap[buf] = 0;
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&ss->consumed[buf]);
-#pragma unroll
-    for (int w = 0; w < RC_NS; ++w) {
-      const int t = w * 32 + lane;
-      if (b[w].x != 0 || b[w].y != 0) {
-        const int ix = k * cap + t;
-        rc_i128 a = c.WD[ix]; rc_add128(a, b[w].x); c.WD[ix] = a;
-        rc_i128 d = c.WL[ix]; rc_add128(d, b[w].y); c.WL[ix] = d;
-      }
-    }
-    __syncwarp();
-  }
-}
-
-// mode 0: the Gibbs scan; mode 1: block-sum initialisation (same row pipeline, no decisions)
-__device__ void full_scan(const Ctx& c, unsigned it, int mode = 0) {
-  ScanShared* ss = c.ss;
-  if (c.ctid == 0) {
-    if (ss->inited)
-      for (int b = 0; b < 2; ++b) { mbar_inval(&ss->ready[b]); mbar_inval(&ss->consumed[b]); }
-    for (int b = 0; b < 2; ++b) { mbar_init(&ss->ready[b], RC_BW); mbar_init(&ss->consumed[b], 1); }
-    ss->inited = 1; ss->M = 0; ss->decided = 0; ss->rowP[0] = 0; ss->rowP[1] = 0; ss->msnap[0] = 0; ss->msnap[1] = 0; ss->prebuilt = 0;
-    c.sc->rebuild = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  csync(c);
-  if (c.cwarp < RC_BW) bulk_loop(c, it);
-  else if (mode == 0) decide_loop(c, it);
-  else initw_loop(c);
-  csync(c);
-  // moves published after the last patch pass are not in the permutation: the next user rebuilds it
-  if (c.cwarp == 0) {                                                       // :254
-    int K = 0;
-    for (int s = c.lane; s < c.cap; s += 32) K += c.sizes[s] > 0;
-    for (int off = 16; off; off >>= 1) K += __shfl_xor_sync(0xffffffffu, K, off);
-    if (c.lane == 0) c.sc->K = K;
-  }
-  csync(c);
-}
-
-// Block sums from scratch: W[k][t] = sum_{x in k, y in t} DL[x][y].  Zeroed here, accumulated by a scan pass in mode 1.
-__device__ void zero_W(const Ctx& c) {
-  for (int t = c.ctid; t < c.cap * c.cap; t += c.nthr) {
-    rc_i128 z; z.lo = 0; z.hi = 0;
-    c.WD[t] = z; c.WL[t] = z;
-  }
-  csync(c);
-}
 
 // ------------------------------------------------------------------------------------------------
 // loglik (mcmc.jl:1-56) from the block sums.  `sz` are the cluster sizes of the evaluated state; rows of
-// slots fslotA / fslotB (proposed state of a split-merge step) come from the scratch rows aliased on
-// c.partial, everything else from the chain's W.
+// slots fslotA / fslotB (proposed state of a split-merge step) come from the scratch rows c.prows,
+// everything else from the chain's W.
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ rc_i128 getW(const Ctx& c, bool logm, int k, int t) {
   const Scal& s = *c.sc;
@@ -1071,7 +195,7 @@ __device__ __forceinline__ rc_i128 getW(const Ctx& c, bool logm, int k, int t) {
     if (A >= 0 && B >= 0 && ((k == A && t == B) || (k == B && t == A))) return logm ? s.abL : s.abD;
     if (k == A && t == A) return logm ? s.aaL : s.aaD;
     if (k == B && t == B) return logm ? s.bbL : s.bbD;
-    const rc_i128* rows = reinterpret_cast<const rc_i128*>(c.partial);    // [rowA_D | rowA_L | rowB_D | rowB_L] x cap
+    const rc_i128* rows = c.prows;    // [rowA_D | rowA_L | rowB_D | rowB_L] x cap
     const bool isA = (k == A || t == A);
     const int other = isA ? (k == A ? t : k) : (k == B ? t : k);
     return rows[((isA ? 0 : 2) + (logm ? 1 : 0)) * c.cap + other];
@@ -1140,15 +264,13 @@ __device__ double loglik_eval(const Ctx& c, const int* sz) {
   return c.sc->dtmp[0];
 }
 
-// loglik of the chain's own state (fslotA / fslotB must be -1).  Incremental kernel: the value only changes when the state does,
-// so it is kept with the chain's change count -- a stationary chain evaluates it once, not twice per iteration.
+// loglik of the chain's own state (fslotA / fslotB must be -1).  The value only changes when the state does, so it is kept
+// with the chain's change count -- a stationary chain evaluates it once, not twice per iteration.
 __device__ double loglik_cur(const Ctx& c) {
-  if (c.inc && c.sc->llclk == c.inc->clk) return c.sc->llcur;               // (uniform: both were written before the last barrier)
+  if (c.sc->llclk == c.inc->clk) return c.sc->llcur;                        // (uniform: both were written before the last barrier)
   const double v = loglik_eval(c, c.sizes);
-  if (c.inc) {
-    if (c.ctid == 0) { c.sc->llcur = v; c.sc->llclk = c.inc->clk; }
-    csync(c);
-  }
+  if (c.ctid == 0) { c.sc->llcur = v; c.sc->llclk = c.inc->clk; }
+  csync(c);
   return v;
 }
 
@@ -1245,222 +367,15 @@ __device__ void update_p(const Ctx& c, unsigned it) {
 
 // ------------------------------------------------------------------------------------------------
 // Prior term of joining an existing cluster of size s (mcmc.jl:226, 324) for this iteration's (r, p):
-// LPR[s] = log(s+1) + log p + log(s-1+r) - log(s), evaluated in the reference's order.
+// log(s+1) + log p + log(s-1+r) - log(s), evaluated in the reference's order, on demand (only a few sizes are ever needed
+// per iteration, so no table is built).
 // ------------------------------------------------------------------------------------------------
-// ... and the same value on demand (incremental kernel: only a few sizes are ever needed per iteration, so no table is built)
 __device__ __forceinline__ double lpr_at(const Ctx& c, int s) {
   return c.kp->LOGN[s + 1] + c.sc->logp + rc_log((double)(s - 1) + c.sc->r) - c.kp->LOGN[s];
 }
-__device__ void build_lpr(const Ctx& c) {
-  const rc_kparams& kp = *c.kp;
-  const double r = c.sc->r, logp = c.sc->logp;
-  for (int s = 1 + c.ctid; s <= c.n; s += c.nthr)
-    c.LPR[s] = kp.LOGN[s + 1] + logp + rc_log((double)(s - 1) + r) - kp.LOGN[s];
-  csync(c);
-}
 
 // ------------------------------------------------------------------------------------------------
-// All restricted Gibbs scans of one split-merge step (mcmc.jl:259-354, called at :411-414, :419, :454)
-// over the items Slist[0..nS) on the launch state, which lives IN PLACE in c.lab / c.szL (the chain's own
-// labels of the members are kept in origM and restored by the caller).  Runs on warp 0 of the chain.
-//   * AB[q] holds the sums of member q's row over the current members of the two candidate clusters; a
-//     move of item y updates all of them from row y (exact integers), so a step that does not move reads
-//     nothing but its own entry.
-//   * the Gumbel noise and the repulsion terms of non-candidate slots do not depend on the evolving state
-//     and are precomputed (NZ, L2s).
-//   * the transition probability (:347-351) is only evaluated in the last scan -- the reference discards
-//     the return value of the intermediate scans (:411-414).
-// Returns the log transition probability of the last scan in c.sc->ltp.
-// ------------------------------------------------------------------------------------------------
-#define RC_RS_NU 16
-// Eight consecutive steps are evaluated at once (lane = 4 * step + role, one logarithm per lane) on the assumption that
-// none of the earlier ones moves its item; the steps up to and including the first move are exact and are committed,
-// the rest is evaluated again after the move has been applied.  Every committed step sees exactly the inputs of the
-// sequential scan, so the results are the same bits.
-#define RC_RS_B 8
-#ifndef RC_RS_PF
-#define RC_RS_PF 4      // steps of a short batch whose rows the idle warps pull towards L2
-#endif
-__device__ void restricted_scans(const Ctx& c, int nS, int ca, int cb, int c1, int c2, bool split) {
-  const rc_kparams& kp = *c.kp;
-  const rc_params& P = kp.P;
-  const int lane = c.lane;
-  const int mt = nS + 2;
-  const int numGibbs = (int)kp.numGibbs;
-  if (nS == 0) { if (lane == 0) c.sc->ltp = 0.0; __syncwarp(); return; }
-  int xs[RC_RS_NU];
-#pragma unroll
-  for (int u = 0; u < RC_RS_NU; ++u) { const int q = u * 32 + lane; xs[u] = q < mt ? cpos(c, (int)c.Slist[q]) : -1; }   // member columns
-  const bool c1dyn = (c1 == ca || c1 == cb), c2dyn = (c2 == ca || c2 == cb);
-  const int st = lane >> 2, role = lane & 3, quad = lane & ~3;
-  const bool isA = (role & 1) == 0;
-  double ltp = 0.0;
-  for (int g = 0; g <= numGibbs; ++g) {
-    const bool last = g == numGibbs;
-    const bool forced = last && !split;
-    int pos0 = 0;
-    while (pos0 < nS) {
-      const int nb = min(RC_RS_B, nS - pos0);
-      const int pos = pos0 + st;
-      const bool on = st < nb;
-      int y = 0, cur = 0, cnew = 0, k = 0;
-      double lt = 0.0;
-      if (on) {
-        y = c.Slist[pos];
-        const longlong2 self = c.DG[pos];
-        const longlong4 ab = c.AB[pos];
-        const double2 l2s = c.L2s[pos];
-        const double2 nz = forced ? make_double2(0.0, 0.0) : c.NZ[(size_t)g * nS + pos];
-        cur = c.labL[y];
-        // sums over the candidates with y detached (:303-304)
-        const long long sAd = ab.x - (cur == ca ? self.x : 0), sAl = ab.y - (cur == ca ? self.y : 0);
-        const long long sBd = ab.z - (cur == cb ? self.x : 0), sBl = ab.w - (cur == cb ? self.y : 0);
-        const int szA = c.szL[ca] - (cur == ca ? 1 : 0), szB = c.szL[cb] - (cur == cb ? 1 : 0);
-        // roles 0..3: {L2'(ca), L2'(cb), L1(ca), L1(cb)} -- one logarithm each
-        double X;
-        {
-          const int szs = isA ? szA : szB;
-          const double szd = (double)szs;
-          const double sD = rc_dequant(isA ? sAd : sBd, c.qD), sL = rc_dequant(isA ? sAl : sBl, c.qL);
-          if ((role & 2) == 0) {                                                                    // :313-319, 327-330
-            const double z_i = P.zeta + P.delta2 * szd, g_i = P.gamma + sD;
-            X = kp.LGZ[szs] - z_i * rc_log(g_i) + kp.zgratio + (P.delta2 - 1) * sL - szd * kp.lgd2;
-          } else {                                                                                  // :307-312, 321-326
-            const double a_i = P.alpha + P.delta1 * szd, b_i = P.beta + sD;
-            X = kp.LGA[szs] + kp.abratio - a_i * rc_log(b_i) + (P.delta1 - 1) * sL - szd * kp.lgd1;
-          }
-        }
-        const unsigned qm = 0xfu << quad;
-        const double L2pA = __shfl_sync(qm, X, quad), L2pB = __shfl_sync(qm, X, quad + 1);
-        const double L1A = __shfl_sync(qm, X, quad + 2), L1B = __shfl_sync(qm, X, quad + 3);
-        const double L2p1 = c1dyn ? (c1 == ca ? L2pA : L2pB) : l2s.x;
-        const double L2p2 = c2dyn ? (c2 == ca ? L2pA : L2pB) : l2s.y;
-        const double L2i = L2p1 + L2p2;                                                             // :331 (quirk Q2)
-        const double L2a = L2i - L2pA, L2b = L2i - L2pB;                                            // :332-334
-        double lp0 = c.LPR[szA] + (L1A + (P.repulsion ? L2a : copysign(0.0, L2a)));                 // :335
-        double lp1 = c.LPR[szB] + (L1B + (P.repulsion ? L2b : copysign(0.0, L2b)));
-        if (!forced) {                                                                              // :336-338
-          double mn = lp0;
-          if (!rc_isnan(mn)) { if (rc_isnan(lp1) || lp1 < mn) mn = lp1; }
-          lp0 -= mn; lp1 -= mn;
-          const double g0 = nz.x + lp0, g1 = nz.y + lp1;
-          k = 0;
-          if (!rc_isnan(g0)) { if (rc_isnan(g1) || g1 > g0) k = 1; }
-          cnew = k == 0 ? ca : cb;
-        } else {                                                                                    // :339-342
-          cnew = c.origM[pos];
-          k = (ca == cnew) ? 0 : 1;
-        }
-        if (last) {                                                                                 // :347-351
-          double mn = lp0;                                                                          // quirk Q3
-          if (!rc_isnan(mn)) { if (rc_isnan(lp1) || lp1 < mn) mn = lp1; }
-          lp0 += mn; lp1 += mn;
-          double p0 = rc_exp(lp0), p1 = rc_exp(lp1);
-          const double den = p0 + p1;
-          p0 /= den; p1 /= den;
-          lt = rc_log(k == 0 ? p0 : p1);
-        }
-      }
-      __syncwarp();
-      // the first step of the batch that moves its item: it and everything before it stand
-      const unsigned mv = __ballot_sync(0xffffffffu, on && role == 0 && cnew != cur);
-      const int sfirst = mv ? (__ffs(mv) - 1) >> 2 : -1;
-      const int nvalid = sfirst >= 0 ? sfirst + 1 : nb;
-      if (last)
-        for (int q = 0; q < nvalid; ++q) ltp += __shfl_sync(0xffffffffu, lt, 4 * q);               // in step order, as the scan adds them
-      if (sfirst >= 0) {                                                                            // :344-345
-        const int ym = __shfl_sync(0xffffffffu, y, 4 * sfirst);
-        const int curm = __shfl_sync(0xffffffffu, cur, 4 * sfirst), newm = __shfl_sync(0xffffffffu, cnew, 4 * sfirst);
-        if (lane == 0) { c.labL[ym] = (uint8_t)newm; c.szL[curm] -= 1; c.szL[newm] += 1; }
-        // every member's candidate sums follow the move (D is symmetric: DL[q][y] == DL[y][q])
-        const longlong2* row = c.DL + (size_t)ym * c.n;
-        const bool a2b = curm == ca;
-        longlong2 ev[RC_RS_NU];                                 // row y at the member columns (only read when y moves)
-#pragma unroll
-        for (int u = 0; u < RC_RS_NU; ++u) ev[u] = xs[u] >= 0 ? __ldg(row + xs[u]) : make_longlong2(0, 0);
-#pragma unroll
-        for (int u = 0; u < RC_RS_NU; ++u) {
-          const int q = u * 32 + lane;
-          if (q < mt) {
-            longlong4 t = c.AB[q];
-            if (a2b) { t.x -= ev[u].x; t.y -= ev[u].y; t.z += ev[u].x; t.w += ev[u].y; }
-            else { t.x += ev[u].x; t.y += ev[u].y; t.z -= ev[u].x; t.w -= ev[u].y; }
-            c.AB[q] = t;
-          }
-        }
-        for (int q = RC_RS_NU * 32 + lane; q < mt; q += 32) {   // members beyond the register window
-          const longlong2 e = __ldg(row + cpos(c, c.Slist[q]));
-          longlong4 t = c.AB[q];
-          if (a2b) { t.x -= e.x; t.y -= e.y; t.z += e.x; t.w += e.y; }
-          else { t.x += e.x; t.y += e.y; t.z -= e.x; t.w -= e.y; }
-          c.AB[q] = t;
-        }
-      }
-      __syncwarp();
-      pos0 += nvalid;
-    }
-  }
-  if (lane == 0) c.sc->ltp = ltp;
-  __syncwarp();
-}
-
-// Split-merge setup for a MERGE proposal: the restricted scans need, for every member x of ci u cj, only the
-// sums of its row over the members by launch label (AB) and -- when they are not candidates -- over the
-// first two live slots (L2s).  One warp per member row gathers exactly those entries instead of reducing the
-// whole row.  CL1 / CL2 hold the members of the first two live slots (n1, n2 entries).
-__device__ void member_sums_gather(const Ctx& c, int nS, int ca, int cb, int c1, int c2, const unsigned short* CL1, int n1,
-                                   const unsigned short* CL2, int n2) {
-  const rc_kparams& kp = *c.kp;
-  const rc_params& P = kp.P;
-  const int lane = c.lane, mt = nS + 2;
-  for (int q = c.cwarp; q < mt; q += c.nwarp) {
-    const int x = c.Slist[q];
-    const longlong2* row = c.DL + (size_t)x * c.n;
-    long long v[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // aD aL bD bL c1D c1L c2D c2L
-    for (int q2 = lane; q2 < mt; q2 += 32) {
-      const int y = c.Slist[q2];
-      const longlong2 e = __ldg(row + cpos(c, y));
-      const int l = c.labL[y];
-      if (l == ca) { v[0] += e.x; v[1] += e.y; } else if (l == cb) { v[2] += e.x; v[3] += e.y; }
-    }
-    if (c.S) {                                    // incremental mode: the sums over an untouched cluster are already in S
-      if (q < nS && lane < 2) {
-        const int t = lane == 0 ? c1 : c2;
-        if (t != ca && t != cb) { const longlong2 e = c.S[(size_t)t * c.n + x]; v[lane == 0 ? 4 : 6] = e.x; v[lane == 0 ? 5 : 7] = e.y; }
-      }
-    } else {
-      for (int t = lane; t < n1; t += 32) { const longlong2 e = __ldg(row + cpos(c, CL1[t])); v[4] += e.x; v[5] += e.y; }
-      for (int t = lane; t < n2; t += 32) { const longlong2 e = __ldg(row + cpos(c, CL2[t])); v[6] += e.x; v[7] += e.y; }
-    }
-#pragma unroll
-    for (int h = 0; h < 8; ++h)
-      for (int off = 16; off; off >>= 1) v[h] += shfl_xor_ll(v[h], off);   // (incremental mode: lanes 0 / 1 hold the only non-zero v[4..7])
-    if (lane == 0) {
-      longlong4 ab; ab.x = v[0]; ab.y = v[1]; ab.z = v[2]; ab.w = v[3];
-      c.AB[q] = ab;
-      c.DG[q] = __ldg(row + cpos(c, x));
-    }
-    if (q < nS) {
-      double val = 0.0;
-      if (lane < 2) {
-        const int t = lane == 0 ? c1 : c2;
-        if (t != ca && t != cb) {
-          const int szs = c.szL[t];
-          const double szd = (double)szs;
-          const double sD = rc_dequant(lane == 0 ? v[4] : v[6], c.qD), sL = rc_dequant(lane == 0 ? v[5] : v[7], c.qL);
-          const double z_i = P.zeta + P.delta2 * szd, g_i = P.gamma + sD;
-          val = kp.LGZ[szs] - z_i * rc_log(g_i) + kp.zgratio + (P.delta2 - 1) * sL - szd * kp.lgd2;
-        }
-      }
-      const double other = __shfl_sync(0xffffffffu, val, 1);
-      if (lane == 0) c.L2s[q] = make_double2(val, other);
-    }
-    __syncwarp();
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Incremental mode versions of the two functions above, run by the whole team of the chain.
+// Split-merge setup and restricted Gibbs scans (mcmc.jl:259-354), run by the whole team of the chain.
 // member_sums_inc: thread t owns the members q = t, t + nthr, ...; it walks ALL members y and adds DL[y][x_q]
 // (= DL[x_q][y], D is symmetric; reading row y makes the threads of a warp hit neighbouring columns) to the sum of
 // y's launch label.  No reductions; the sums over the first two live slots, clusters the launch did not touch, are
@@ -1520,13 +435,27 @@ __device__ void member_sums_inc(const Ctx& c, int nS, int ca, int cb, int c1, in
   }
 }
 
-// restricted_scans for the whole team: every warp evaluates eight consecutive steps (a quad of lanes per step, as
-// restricted_scans does) and resolves them among themselves -- each quad holds the matrix entries between its item and
-// the items of the warp's earlier steps, so when an earlier step moves its item the later quads correct their sums in
-// registers and decide again, in step order.  A warp's eight steps are therefore final given the state at the start of
-// the batch.  A batch covers 8 * nwact steps: the warps up to and including the first one with a move are committed, that
-// warp's moves (up to eight) are applied to the running candidate sums of all members by all threads with one round of
-// gathers, and the scan continues behind them.
+// ------------------------------------------------------------------------------------------------
+// All restricted Gibbs scans of one split-merge step (mcmc.jl:259-354, called at :411-414, :419, :454) over the items
+// Slist[0..nS) on the launch state, which lives IN PLACE in c.labL / c.szL (the chain's own labels of the members are kept
+// in origM and restored by the caller).
+//   * AB[q] holds the sums of member q's row over the current members of the two candidate clusters; a move of item y
+//     updates all of them from row y (exact integers), so a step that does not move reads nothing but its own entry.
+//   * the Gumbel noise and the repulsion terms of non-candidate slots do not depend on the evolving state and are
+//     precomputed (NZ, L2s).
+//   * the transition probability (:347-351) is only evaluated in the last scan -- the reference discards the return value
+//     of the intermediate scans (:411-414).
+// Every warp evaluates eight consecutive steps (a quad of lanes per step, one logarithm per lane) and resolves them among
+// themselves -- each quad holds the matrix entries between its item and the items of the warp's earlier steps, so when an
+// earlier step moves its item the later quads correct their sums in registers and decide again, in step order.  A warp's
+// eight steps are therefore final given the state at the start of the batch.  A batch covers 8 * nwact steps: the warps up
+// to and including the first one with a move are committed, that warp's moves (up to eight) are applied to the running
+// candidate sums of all members by all threads with one round of gathers, and the scan continues behind them.  Every
+// committed step sees exactly the inputs of the sequential scan, so the results are the same bits.
+// Returns the log transition probability of the last scan in c.sc->ltp.
+// ------------------------------------------------------------------------------------------------
+#define RC_RS_B 8       // steps per warp
+#define RC_RS_PF 4      // steps of a short batch whose rows the idle warps pull towards L2
 __device__ void restricted_scans_team(const Ctx& c, int nS, int ca, int cb, int c1, int c2, bool split) {
   const rc_kparams& kp = *c.kp;
   const rc_params& P = kp.P;
@@ -1767,7 +696,7 @@ __device__ void splitmerge_step(Ctx& c, unsigned it, unsigned mh, bool commit) {
   csync(c);
   if (tid == 0) { c.sc->itmp[1] = 0; c.sc->itmp[2] = 0; }
   if (P.maxK > 0 && ci == cj && K >= P.maxK) { csync(c); return; }          // :384-386
-  if (ci != cj && c.S && kp.shortcuts) {
+  if (ci != cj && kp.shortcuts) {
     // Merge proposals that cannot be accepted.  The acceptance ratio of a merge (:435-468) is
     //   prior ratio + likelihood ratio - log proposal ratio,   log proposal ratio = -(sum of the final scan's log transition
     // probabilities) >= 0,
@@ -1783,7 +712,7 @@ __device__ void splitmerge_step(Ctx& c, unsigned it, unsigned mh, bool commit) {
     double ll_fin;
     if (have) ll_fin = c.LLF[pidx];
     else {
-      rc_i128* rows = reinterpret_cast<rc_i128*>(c.partial);
+      rc_i128* rows = c.prows;
       for (int t = tid; t < cap; t += c.nthr) {                             // row cj of the merged state
         rc_i128 bD = c.WD[tri(ci, t, cap)], bL = c.WL[tri(ci, t, cap)];
         rc_add128(bD, c.WD[tri(cj, t, cap)]); rc_add128(bL, c.WL[tri(cj, t, cap)]);
@@ -1840,10 +769,10 @@ __device__ void splitmerge_step(Ctx& c, unsigned it, unsigned mh, bool commit) {
     csync(c);
   }
   const int nS = c.sc->itmp[3];
-  // incremental mode: the per-member running sums live in shared memory when the members fit (the restricted scans
-  // are a chain of dependent reads and writes of exactly these arrays)
+  // the per-member running sums live in shared memory when the members fit (the restricted scans are a chain of dependent
+  // reads and writes of exactly these arrays)
   longlong4* const gAB = c.AB; longlong2* const gDG = c.DG; double2* const gL2s = c.L2s;
-  if (c.S && nS + 2 <= c.mcap) { c.AB = c.mAB; c.DG = c.mDG; c.L2s = c.mL2s; }
+  if (nS + 2 <= c.mcap) { c.AB = c.mAB; c.DG = c.mDG; c.L2s = c.mL2s; }
   auto unswap = [&]() { c.AB = gAB; c.DG = gDG; c.L2s = gL2s; };
   if (tid == 0) { c.Slist[nS] = (unsigned short)pi; c.origM[nS] = (uint8_t)ci; c.Slist[nS + 1] = (unsigned short)pj; c.origM[nS + 1] = (uint8_t)cj; }
   // launch state (:393-408), in place in c.labL / c.szL
@@ -1893,65 +822,9 @@ __device__ void splitmerge_step(Ctx& c, unsigned it, unsigned mh, bool commit) {
     csync(c);
   }
   const int c1 = c.sc->itmp[5], c2 = c.sc->itmp[6];
-  if (split && !c.S) {
-    // row sums by slot of every member of S u {i, j} under the launch labels (all slots are needed for the
-    // block sums of the proposed state)
-    build_perm<false>(c);
-    if (c.sc->status) {                                      // does not fit: undo the in-place launch labels and stop the chain
-      for (int q = tid; q < nS + 2; q += c.nthr) c.labL[c.Slist[q]] = c.origM[q];
-      csync(c);
-      unswap();
-      return;
-    }
-    for (int pos = 0; pos < nS + 2; ++pos) {
-      reduce_row_global(c, c.Slist[pos]);
-      csync(c);
-      for (int s = tid; s < cap; s += c.nthr) c.T[(size_t)pos * cap + s] = bin_total(c, s);
-      csync(c);
-    }
-    // state-independent inputs of the restricted scans: candidate sums under the launch labels, diagonal
-    // entries, repulsion terms of the first two live slots when they are not candidates
-    for (int q = tid; q < nS + 2; q += c.nthr) {
-      const longlong2 ta = c.T[(size_t)q * cap + ca], tb = c.T[(size_t)q * cap + cb];
-      longlong4 ab; ab.x = ta.x; ab.y = ta.y; ab.z = tb.x; ab.w = tb.y;
-      c.AB[q] = ab;
-      const int x = c.Slist[q];
-      c.DG[q] = __ldg(c.DL + (size_t)x * n + cpos(c, x));
-    }
-    for (int pos = tid; pos < nS; pos += c.nthr) {
-      double v[2] = {0.0, 0.0};
-      for (int h = 0; h < 2; ++h) {
-        const int t = h == 0 ? c1 : c2;
-        if (t == ca || t == cb) continue;
-        const longlong2 tt = c.T[(size_t)pos * cap + t];
-        const int szs = c.szL[t];
-        const double szd = (double)szs;
-        const double sD = rc_dequant(tt.x, c.qD), sL = rc_dequant(tt.y, c.qL);
-        const double z_i = P.zeta + P.delta2 * szd, g_i = P.gamma + sD;
-        v[h] = kp.LGZ[szs] - z_i * rc_log(g_i) + kp.zgratio + (P.delta2 - 1) * sL - szd * kp.lgd2;
-      }
-      c.L2s[pos] = make_double2(v[0], v[1]);
-    }
-  } else if (c.S) {
-    // incremental mode (split or merge): member x member entries by launch label; the sums over the first two live
-    // slots, when they are not candidates, are clusters the launch did not touch and come straight from S
-    member_sums_inc(c, nS, ca, cb, c1, c2);
-  } else {
-    // merge: only member-restricted sums are needed; T's memory serves as scratch for the member lists of the
-    // first two live slots (unordered: integer sums do not depend on the order)
-    unsigned short* CL1 = reinterpret_cast<unsigned short*>(c.T);
-    unsigned short* CL2 = CL1 + n;
-    if (tid == 0) { c.itmp[8] = 0; c.itmp[9] = 0; }
-    csync(c);
-    const bool need1 = c1 != ca && c1 != cb, need2 = c2 != ca && c2 != cb;
-    for (int k = tid; k < n; k += c.nthr) {
-      const int l = c.labL[k];
-      if (need1 && l == c1) CL1[atomicAdd(&c.itmp[8], 1)] = (unsigned short)k;
-      else if (need2 && l == c2) CL2[atomicAdd(&c.itmp[9], 1)] = (unsigned short)k;
-    }
-    csync(c);
-    member_sums_gather(c, nS, ca, cb, c1, c2, CL1, c.itmp[8], CL2, c.itmp[9]);
-  }
+  // member x member entries by launch label; the sums over the first two live slots, when they are not candidates, are
+  // clusters the launch did not touch and come straight from S
+  member_sums_inc(c, nS, ca, cb, c1, c2);
   {
     const int nfree = (int)kp.numGibbs + (split ? 1 : 0);
     for (int e = tid; e < nfree * nS; e += c.nthr) {
@@ -1962,7 +835,7 @@ __device__ void splitmerge_step(Ctx& c, unsigned it, unsigned mh, bool commit) {
   }
   csync(c);
   const long long tm1 = RC_CLOCK();
-  if (c.S && c.labL != c.lab && nS + 2 <= 1024 && !c.inc->scanfast) {   // (large member sets need every thread; a scan decided by its row summaries is too short to matter)
+  if (c.labL != c.lab && nS + 2 <= 1024 && !c.inc->scanfast) {   // (large member sets need every thread; a scan decided by its row summaries is too short to matter)
     // The restricted scans are a chain of dependent steps that keeps one or two warps busy.  With one proposal per
     // iteration the full scan that follows does not depend on them unless the proposal is accepted (quirk Q1: then the
     // scan is discarded), so the rest of the CTA runs it now, DRY: it commits nothing and stops at the first row that
@@ -1980,8 +853,7 @@ __device__ void splitmerge_step(Ctx& c, unsigned it, unsigned mh, bool commit) {
       cB.ctid = tid - TA; cB.cwarp = cB.ctid >> 5; cB.nthr = c.nthr - TA; cB.nwarp = cB.nthr / 32; cB.barid = 3;
       inc_full_scan(cB, it, 0, true);
     }
-  } else if (c.S) restricted_scans_team(c, nS, ca, cb, c1, c2, split);
-  else if (warp == 0) restricted_scans(c, nS, ca, cb, c1, c2, split);
+  } else restricted_scans_team(c, nS, ca, cb, c1, c2, split);
   csync(c);
   const long long tm2 = RC_CLOCK();
   if (tid == 0) { st_add(c, ST_MH_SETUP, tm1 - tm0); st_add(c, ST_MH_RSCAN, tm2 - tm1); }
@@ -1996,28 +868,19 @@ __device__ void splitmerge_step(Ctx& c, unsigned it, unsigned mh, bool commit) {
       log_proposal_ratio = c.sc->ltp;
     }
     // block sums of the proposed state: rows a (= new slot ca) and b (= cb)
-    rc_i128* rows = reinterpret_cast<rc_i128*>(c.partial);   // [rowA_D | rowA_L | rowB_D | rowB_L] x cap
-    if (c.S) {
-      // the slots other than ca / cb are untouched clusters: their sums over the members that ended in ca are entries of S.
-      // A warp per slot, the members over its lanes.
-      for (int t = warp; t < cap; t += c.nwarp) {
-        rc_i128 sd, sl; sd.lo = 0; sd.hi = 0; sl.lo = 0; sl.hi = 0;
-        if (t != ca && t != cb && c.sizes[t] > 0) {
-          for (int q = lane; q < nS + 2; q += 32) {
-            const int x = c.Slist[q];
-            if (c.labL[x] == ca) { const longlong2 v = c.S[(size_t)t * n + x]; rc_add128(sd, v.x); rc_add128(sl, v.y); }
-          }
-          sd = warp_sum128(sd); sl = warp_sum128(sl);
+    rc_i128* rows = c.prows;   // [rowA_D | rowA_L | rowB_D | rowB_L] x cap
+    // the slots other than ca / cb are untouched clusters: their sums over the members that ended in ca are entries of S.
+    // A warp per slot, the members over its lanes.
+    for (int t = warp; t < cap; t += c.nwarp) {
+      rc_i128 sd, sl; sd.lo = 0; sd.hi = 0; sl.lo = 0; sl.hi = 0;
+      if (t != ca && t != cb && c.sizes[t] > 0) {
+        for (int q = lane; q < nS + 2; q += 32) {
+          const int x = c.Slist[q];
+          if (c.labL[x] == ca) { const longlong2 v = c.S[(size_t)t * n + x]; rc_add128(sd, v.x); rc_add128(sl, v.y); }
         }
-        if (lane == 0) { rows[0 * cap + t] = sd; rows[1 * cap + t] = sl; }
+        sd = warp_sum128(sd); sl = warp_sum128(sl);
       }
-    } else {
-      for (int t = tid; t < cap; t += c.nthr) {
-        rc_i128 sd, sl; sd.lo = 0; sd.hi = 0; sl.lo = 0; sl.hi = 0;
-        for (int q = 0; q < nS + 2; ++q)
-          if (c.labL[c.Slist[q]] == ca) { const longlong2 v = c.T[(size_t)q * cap + t]; rc_add128(sd, v.x); rc_add128(sl, v.y); }
-        rows[0 * cap + t] = sd; rows[1 * cap + t] = sl;
-      }
+      if (lane == 0) { rows[0 * cap + t] = sd; rows[1 * cap + t] = sl; }
     }
     // within / cross sums from the running candidate sums of the final state:
     //   aa = sum_{x in a_F} sum_{y in a_F} DL[x][y],  ab = sum_{x in a_F} sum_{y in b_F} DL[x][y]
@@ -2062,7 +925,7 @@ __device__ void splitmerge_step(Ctx& c, unsigned it, unsigned mh, bool commit) {
                           rc_log((double)c.sizes[ci]) + rc_log((double)c.sizes[cj]));
       log_proposal_ratio = -c.sc->ltp;
     }
-    rc_i128* rows = reinterpret_cast<rc_i128*>(c.partial);
+    rc_i128* rows = c.prows;
     for (int t = tid; t < cap; t += c.nthr) {                               // row cj of the merged state
       rc_i128 bD = c.WD[tri(ci, t, cap)], bL = c.WL[tri(ci, t, cap)];
       rc_add128(bD, c.WD[tri(cj, t, cap)]); rc_add128(bL, c.WL[tri(cj, t, cap)]);
@@ -2099,7 +962,7 @@ __device__ void splitmerge_step(Ctx& c, unsigned it, unsigned mh, bool commit) {
       csync(c);
       if (tid == 0) c.sc->forked = 1;
     }
-    const rc_i128* rows = reinterpret_cast<const rc_i128*>(c.partial);   // [rowA_D | rowA_L | rowB_D | rowB_L] x cap
+    const rc_i128* rows = c.prows;   // [rowA_D | rowA_L | rowB_D | rowB_L] x cap
     const int A = split ? ca : ci, B = split ? cb : cj;
     for (int t = tid; t < cap; t += c.nthr) {
       if (t != A && t != B) {
@@ -2116,17 +979,15 @@ __device__ void splitmerge_step(Ctx& c, unsigned it, unsigned mh, bool commit) {
     if (!split)
       for (int q = tid; q < nS + 2; q += c.nthr) c.labL[c.Slist[q]] = (uint8_t)cj;     // :436-445 (split: labels are final in place)
     for (int s = tid; s < cap; s += c.nthr) c.sizes[s] = c.szL[s];
-    if (c.S) {                                  // incremental mode: the row sums follow the members that changed slot
-      csync(c);
-      for (int q = 0; q < nS + 2; ++q) {
-        const int y = c.Slist[q], from = c.origM[q], to = c.labL[y];
-        if (from != to) inc_update_S(c, y, from, to);
-      }
-      const unsigned m = c.inc->clk + 1;                                    // cached per-slot terms: all stale
-      csync(c);
-      for (int s2 = tid; s2 < cap; s2 += c.nthr) c.tchg[s2] = m;
-      if (tid == 0) c.inc->clk = m;
+    csync(c);                                   // the row sums follow the members that changed slot
+    for (int q = 0; q < nS + 2; ++q) {
+      const int y = c.Slist[q], from = c.origM[q], to = c.labL[y];
+      if (from != to) inc_update_S(c, y, from, to);
     }
+    const unsigned m = c.inc->clk + 1;                                      // cached per-slot terms: all stale
+    csync(c);
+    for (int s2 = tid; s2 < cap; s2 += c.nthr) c.tchg[s2] = m;
+    if (tid == 0) c.inc->clk = m;
   } else {
     // restore the labels of the members (the proposal lived in place)
     for (int q = tid; q < nS + 2; q += c.nthr) c.labL[c.Slist[q]] = c.origM[q];
@@ -2155,14 +1016,14 @@ __device__ void record_labels(const Ctx& c, uint8_t* out) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// Incremental mode (k_chain_inc): the full Gibbs scan (mcmc.jl:158-256) WITHOUT streaming the matrix.
+// The full Gibbs scan (mcmc.jl:158-256) WITHOUT streaming the matrix.
 //   S[k][x] = sum_{j in k} DL[x][j] is kept per chain in global memory ([cap][n], exact integers).  Row x's candidate
 //   sums are then cap 16-byte loads instead of a 16 n-byte row; a move of point i from a to b streams row i once and
 //   updates S[a][.] and S[b][.] (inc_update_S).  The threads of the chain evaluate consecutive rows at once (one row per
 //   thread) on the assumption that none of the earlier ones moves its point; the rows up to and including the first one
 //   that moves are exactly what the sequential scan computes and are committed, the rest is evaluated again after the
 //   move has been applied.  Every committed row sees the inputs of the sequential scan, so the results are the same bits as the
-//   streaming kernel's and the oracle's.
+//   oracle's.
 // ------------------------------------------------------------------------------------------------
 
 // One row of the scan is evaluated by a GROUP of G adjacent lanes (G = 4: 8 rows per warp, slots < 64; G = 8: 4 rows per
@@ -2642,15 +1503,14 @@ __device__ void inc_full_scan(const Ctx& c, unsigned it, int istart, bool dry) {
   csync(c);
 }
 
-struct IncLayout { size_t partial, sc, inc, red, sizes, szL, itmp, clist, lab, labL, live, rank, tabs, res, ep, tw, mAB, mDG, mL2s, total; };
+struct IncLayout { size_t prows, sc, inc, sizes, szL, itmp, clist, lab, labL, live, rank, tabs, res, ep, tw, mAB, mDG, mL2s, total; };
 __host__ __device__ inline IncLayout inc_layout(int n, int cap, int mcap, int tw_smem) {
   IncLayout L;
   size_t o = 0;
   auto take = [&](size_t bytes) { size_t p = o; o += (bytes + 15) & ~(size_t)15; return p; };
-  L.partial = take(sizeof(rc_i128) * 4 * cap);      // rows of the proposed state during a split-merge step
+  L.prows = take(sizeof(rc_i128) * 4 * cap);        // rows of the proposed state during a split-merge step
   L.sc = take(sizeof(Scal));
   L.inc = take(sizeof(IncShared));
-  L.red = take(sizeof(long long) * 16 * 4);
   L.sizes = take(sizeof(int) * cap);
   L.szL = take(sizeof(int) * cap);
   L.itmp = take(sizeof(int) * (cap > 64 ? cap : 64));
@@ -2677,12 +1537,9 @@ __global__ void __launch_bounds__(512, 1) k_chain_inc(const __grid_constant__ rc
   const int chain = blockIdx.x;
   const int n = kp.n, cap = kp.cap;
   Ctx c;
-  c.n = n; c.cap = cap; c.tiles = kp.tiles; c.qD = kp.qD; c.qL = kp.qL; c.DL = kp.DL; c.kp = &kp;
-  c.colpos = nullptr; c.colpt = nullptr;
-  c.ctid = threadIdx.x; c.cwarp = c.ctid >> 5; c.lane = c.ctid & 31; c.barid = 1; c.bbarid = 2;
+  c.n = n; c.cap = cap; c.qD = kp.qD; c.qL = kp.qL; c.DL = kp.DL; c.kp = &kp;
+  c.ctid = threadIdx.x; c.cwarp = c.ctid >> 5; c.lane = c.ctid & 31; c.barid = 1;
   c.nthr = blockDim.x; c.nwarp = blockDim.x >> 5;
-  c.dummy = 0; c.stage_bytes = 0; c.stages = nullptr; c.cta = nullptr; c.chain0 = nullptr; c.chain_stride = 0; c.ss_off = 0;
-  c.perm = nullptr; c.runStart = nullptr; c.bscratch[0] = nullptr; c.bscratch[1] = nullptr; c.tileStart = nullptr; c.ss = nullptr;
   {
     const IncLayout L = inc_layout(n, cap, kp.inc_mcap, kp.tw_smem);
     c.mcap = kp.inc_mcap;
@@ -2697,10 +1554,9 @@ __global__ void __launch_bounds__(512, 1) k_chain_inc(const __grid_constant__ rc
     c.tw = kp.tw_smem ? reinterpret_cast<unsigned*>(smem + L.tw) : kp.Vv + (size_t)chain * n;
     c.Rs = kp.Rs + (size_t)chain * n;
     c.LLF = kp.LLF + (size_t)chain * cap * cap; c.LLFs = kp.LLFs + (size_t)chain * cap * cap;
-    c.partial = reinterpret_cast<longlong2*>(smem + L.partial);
+    c.prows = reinterpret_cast<rc_i128*>(smem + L.prows);
     c.sc = reinterpret_cast<Scal*>(smem + L.sc);
     c.inc = reinterpret_cast<IncShared*>(smem + L.inc);
-    c.red = reinterpret_cast<long long*>(smem + L.red);
     c.sizes = reinterpret_cast<int*>(smem + L.sizes);
     c.szL = reinterpret_cast<int*>(smem + L.szL);
     c.itmp = reinterpret_cast<int*>(smem + L.itmp);
@@ -2711,7 +1567,6 @@ __global__ void __launch_bounds__(512, 1) k_chain_inc(const __grid_constant__ rc
   const int ch = chain;
   c.WD = kp.WD + (size_t)ch * cap * cap;
   c.WL = kp.WL + (size_t)ch * cap * cap;
-  c.T = nullptr;
   c.S = kp.S + (size_t)ch * cap * n;
   c.Cc = kp.Cc + (size_t)ch * cap * n;
   c.WDbak = kp.WDbak ? kp.WDbak + (size_t)ch * cap * cap : nullptr;
@@ -2723,7 +1578,6 @@ __global__ void __launch_bounds__(512, 1) k_chain_inc(const __grid_constant__ rc
   c.AB = kp.AB + (size_t)ch * (n + 2);
   c.L2s = kp.L2s + (size_t)ch * n;
   c.NZ = kp.NZ + (size_t)ch * (kp.numGibbs + 1) * n;
-  c.LPR = kp.LPR + (size_t)ch * (n + 2);
   c.DG = kp.DG + (size_t)ch * (n + 2);
   c.stats = kp.stats + (size_t)ch * 16;
   c.terms = kp.terms + (size_t)ch * kp.terms_stride;
@@ -2738,13 +1592,18 @@ __global__ void __launch_bounds__(512, 1) k_chain_inc(const __grid_constant__ rc
     Scal& s = *c.sc;
     s.r = kp.r[chain]; s.p = kp.p[chain];
     s.logp = rc_log(s.p); s.log1mp = rc_log(1 - s.p);
-    s.status = kp.status[chain]; s.rebuild = 0; s.fslotA = -1; s.fslotB = -1; s.ltp = 0.0; s.forked = 0;
+    s.status = kp.status[chain]; s.fslotA = -1; s.fslotB = -1; s.ltp = 0.0; s.forked = 0;
     c.inc->hint = 0;
     int K = 0;
     for (int q = 0; q < cap; ++q) K += kp.sizes[(size_t)chain * cap + q] > 0;
     s.K = K;
   }
   csync(c);
+  if (kp.loglik_only) {                                                      // rc_loglik: the loaded state's log-likelihood only
+    const double ll = loglik_cur(c);
+    if (tid == 0) kp.out_ll[chain] = ll;
+    return;
+  }
 
   for (long long iter = kp.it0 + 1; iter <= kp.it1; ++iter) {
     const unsigned it = (unsigned)iter;
@@ -2780,7 +1639,10 @@ __global__ void __launch_bounds__(512, 1) k_chain_inc(const __grid_constant__ rc
         kp.sm_split[((size_t)chain * kp.numiters + (iter - 1)) * kp.numMH + mh] = (uint8_t)spl;
       }
       csync(c);
-      if (acc) do_scan = false;                              // quirk Q1, see k_chain
+      // Quirk Q1 (SURVEY.md A.6): an accepted proposal rebinds sample_labels!'s LOCAL state; the remaining
+      // proposals and the final scan (:477) run on that local object and the caller's labels are untouched this
+      // iteration.  The scan's draws are independent of everything kept (structured stream), so it is skipped.
+      if (acc) do_scan = false;
     }
     if (multi && c.sc->status == 0) {                        // back to the chain's own state
       if (c.sc->forked) {
@@ -2905,270 +1767,6 @@ __global__ void __launch_bounds__(256) k_initw_from_S(const longlong2* __restric
   if (cur >= 0 && cur <= t) { atomic_add128g(&wd[cur * cap + t], d); atomic_add128g(&wl[cur * cap + t], l); }
 }
 
-struct ChainLayout {
-  size_t partial, sc, ss, red, perm, runStart, bscratch, tileStart, sizes, szL, itmp, clist, lab, total;
-  int scratch_aliased;
-};
-__host__ __device__ inline ChainLayout chain_layout(int n, int cap, int tiles, int npad_max) {
-  ChainLayout L;
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t p = o; o += (bytes + 15) & ~(size_t)15; return p; };
-  L.partial = take(sizeof(longlong2) * 2 * RC_BW * cap);
-  L.sc = take(sizeof(Scal));
-  L.ss = take(sizeof(ScanShared));
-  L.red = take(sizeof(long long) * RC_NWARP * 4);
-  L.perm = take(sizeof(unsigned short) * npad_max);
-  L.runStart = take(sizeof(unsigned short) * (tiles * cap + 1));
-  {
-    const size_t need = sizeof(unsigned int) * tiles * cap + npad_max / 8 + 8;
-    L.scratch_aliased = need <= sizeof(longlong2) * RC_BW * cap;
-    L.bscratch = L.scratch_aliased ? L.partial : take(need);
-  }
-  L.tileStart = take(sizeof(int) * (tiles + 1));
-  L.sizes = take(sizeof(int) * cap);
-  L.szL = take(sizeof(int) * cap);
-  L.itmp = take(sizeof(int) * (cap > 16 ? cap : 16));
-  L.clist = take(cap);
-  L.lab = take(n);
-  L.total = (o + 127) & ~(size_t)127;
-  return L;
-}
-__host__ __device__ inline size_t cta_header_bytes() { return (sizeof(CtaShared) + 127) & ~(size_t)127; }
-
-template <int G>
-__global__ void __launch_bounds__(RC_NTHR * G + RC_XTHR, 1) k_chain(const __grid_constant__ rc_kparams kp) {
-  extern __shared__ __align__(128) unsigned char smem[];
-  const bool is_helper = threadIdx.x >= RC_NTHR * G;       // the two last warps serve the whole CTA:
-  const bool is_producer = is_helper && threadIdx.x < RC_NTHR * G + 32;   // stages the row tiles during the scans
-  const bool is_noise = is_helper && !is_producer;         // precomputes the Gumbel noise of the scans
-  const int cl = is_helper ? 0 : threadIdx.x / RC_NTHR;    // chain slot within the CTA
-  const int chain = blockIdx.x * G + cl;
-  const bool valid = !is_helper && chain < kp.nchains;
-  const int n = kp.n, cap = kp.cap, tiles = kp.tiles;
-  Ctx c;
-  c.n = n; c.cap = cap; c.tiles = tiles; c.qD = kp.qD; c.qL = kp.qL; c.DL = kp.DL; c.kp = &kp;
-  c.colpos = kp.colpos; c.colpt = kp.colpt;
-  c.ctid = threadIdx.x % RC_NTHR; c.cwarp = c.ctid >> 5; c.lane = c.ctid & 31; c.barid = 1 + cl; c.bbarid = 1 + G + cl;
-  c.nthr = RC_NTHR; c.nwarp = RC_NWARP; c.S = nullptr; c.inc = nullptr; c.mcap = 0; c.mAB = nullptr; c.mDG = nullptr; c.mL2s = nullptr; c.live = nullptr; c.rank = nullptr; c.tabs = nullptr; c.res = nullptr; c.Cc = nullptr; c.tw = nullptr; c.tchg = nullptr; c.Rs = nullptr; c.LLF = nullptr; c.LLFs = nullptr;
-  {
-    const ChainLayout L = chain_layout(n, cap, tiles, kp.npad_max);
-    c.stage_bytes = stage_bytes_for(n);
-    c.dummy = (unsigned)(c.stage_bytes - 128);   // byte offset of the zero slots
-    c.cta = reinterpret_cast<CtaShared*>(smem);
-    c.stages = smem + cta_header_bytes();
-    c.chain0 = c.stages + (size_t)RC_NSTAGE * c.stage_bytes; c.chain_stride = L.total; c.ss_off = L.ss;
-    unsigned char* base = c.chain0 + (size_t)cl * L.total;
-    c.partial = reinterpret_cast<longlong2*>(base + L.partial);
-    c.sc = reinterpret_cast<Scal*>(base + L.sc);
-    c.ss = reinterpret_cast<ScanShared*>(base + L.ss);
-    c.red = reinterpret_cast<long long*>(base + L.red);
-    c.perm = reinterpret_cast<unsigned short*>(base + L.perm);
-    c.runStart = reinterpret_cast<unsigned short*>(base + L.runStart);
-    c.bscratch[0] = base + L.bscratch;
-    c.bscratch[1] = base + L.bscratch + (L.scratch_aliased ? sizeof(longlong2) * RC_BW * cap : 0);
-    c.tileStart = reinterpret_cast<int*>(base + L.tileStart);
-    c.sizes = reinterpret_cast<int*>(base + L.sizes);
-    c.szL = reinterpret_cast<int*>(base + L.szL);
-    c.itmp = reinterpret_cast<int*>(base + L.itmp);
-    c.clist = base + L.clist;
-    c.lab = base + L.lab;
-    c.labL = c.lab;
-  }
-  const int ch = valid ? chain : 0;
-  c.WD = kp.WD + (size_t)ch * cap * cap;
-  c.WL = kp.WL + (size_t)ch * cap * cap;
-  c.T = kp.T + (size_t)ch * n * cap;
-  c.WDbak = kp.WDbak ? kp.WDbak + (size_t)ch * cap * cap : nullptr;
-  c.WLbak = kp.WLbak ? kp.WLbak + (size_t)ch * cap * cap : nullptr;
-  c.labbak = kp.labbak ? kp.labbak + (size_t)ch * n : nullptr;
-  c.szbak = kp.szbak ? kp.szbak + (size_t)ch * (cap + 1) : nullptr;
-  c.Slist = kp.Slist + (size_t)ch * (n + 2);
-  c.origM = kp.origM + (size_t)ch * (n + 2);
-  c.AB = kp.AB + (size_t)ch * (n + 2);
-  c.L2s = kp.L2s + (size_t)ch * n;
-  c.NZ = kp.NZ + (size_t)ch * (kp.numGibbs + 1) * n;
-  c.LPR = kp.LPR + (size_t)ch * (n + 2);
-  c.DG = kp.DG + (size_t)ch * (n + 2);
-  c.stats = kp.stats + (size_t)ch * 16;
-  c.terms = kp.terms + (size_t)ch * kp.terms_stride;
-  c.key = rc_chain_key(kp.seed, (unsigned long long)(kp.chain_offset + ch));
-  const int tid = c.ctid;
-
-  // zero slots behind every stage (padding entries of the permutation point there)
-  if (is_producer) {   // mirrors the CTA-level barrier sequence of the chain warps below
-    for (int t = threadIdx.x & 31; t < RC_NSTAGE * 8; t += 32)
-      reinterpret_cast<longlong2*>(c.stages + (size_t)(t / 8) * c.stage_bytes + (size_t)c.dummy)[t % 8] = make_longlong2(0, 0);
-    __syncthreads();
-    auto mirror = [&](bool grid) {
-      __syncthreads();
-      __syncthreads();
-      if (grid) __syncthreads();
-      if (c.cta->nact > 0) produce_rows(kp, c.stages, c.stage_bytes, c.cta);
-      __syncthreads();
-    };
-    if (kp.init_W) mirror(false);
-    if (kp.loglik_only) return;
-    for (long long iter = kp.it0 + 1; iter <= kp.it1; ++iter) mirror(kp.gridbar != nullptr);
-    return;
-  }
-  if (is_noise) {      // same barrier sequence as the producer warp
-    __syncthreads();
-    auto mirror = [&](bool grid, bool scan, unsigned it) {
-      __syncthreads();
-      __syncthreads();
-      if (grid) __syncthreads();
-      if (scan && c.cta->nact > 0) noise_rows<G>(kp, c, it);
-      __syncthreads();
-    };
-    if (kp.init_W) mirror(false, false, 0u);
-    if (kp.loglik_only) return;
-    for (long long iter = kp.it0 + 1; iter <= kp.it1; ++iter) mirror(kp.gridbar != nullptr, true, (unsigned)iter);
-    return;
-  }
-  if (valid) {   // load the chain's state
-    for (int j = tid; j < n; j += RC_NTHR) c.lab[j] = kp.labels[(size_t)chain * n + j];
-    for (int s = tid; s < cap; s += RC_NTHR) c.sizes[s] = kp.sizes[(size_t)chain * cap + s];
-    if (tid == 0) {
-      Scal& s = *c.sc;
-      s.r = kp.r[chain]; s.p = kp.p[chain];
-      s.logp = rc_log(s.p); s.log1mp = rc_log(1 - s.p);
-      s.status = kp.status[chain]; s.rebuild = 0; c.ss->inited = 0; s.fslotA = -1; s.fslotB = -1; s.ltp = 0.0;
-      int K = 0;
-      for (int q = 0; q < cap; ++q) K += kp.sizes[(size_t)chain * cap + q] > 0;
-      s.K = K;
-    }
-    csync(c);
-    build_perm<false>(c);
-    if (kp.init_W && c.sc->status == 0) zero_W(c);
-  }
-  __syncthreads();
-  // ---- CTA level: agree on the chains that scan, (re)arm the tile ring, run the row pipeline ----
-  bool rings_used = false;
-  auto cta_scan = [&](bool do_scan, unsigned it, int mode, unsigned epoch) {
-    if (tid == 0) c.cta->active[cl] = do_scan ? 1 : 0;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      int nact = 0;
-      for (int q = 0; q < G; ++q) {
-        nact += c.cta->active[q] ? 1 : 0;
-        ScanShared* sq = scan_shared_of(c, q);               // the noise warp starts as soon as the next barrier opens
-        sq->noise_ready = 0; sq->decided = 0;
-      }
-      c.cta->nact = nact;
-      if (rings_used)
-        for (int s = 0; s < RC_NSTAGE; ++s) { mbar_inval(&c.cta->full[s]); mbar_inval(&c.cta->empty[s]); }
-      for (int s = 0; s < RC_NSTAGE; ++s) { mbar_init(&c.cta->full[s], 1); mbar_init(&c.cta->empty[s], (unsigned)max(nact, 1) * RC_PAIR); c.cta->issued[s] = -1; }
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    rings_used = true;
-    __syncthreads();
-    // experiment (RCB200_GRIDBAR): all CTAs start the scan together
-    if (kp.gridbar && mode == 0) {
-      if (threadIdx.x == 0) {
-        __threadfence();
-        atomicAdd(kp.gridbar, 1u);
-        const unsigned target = gridDim.x * epoch;
-        while (*(volatile unsigned*)kp.gridbar < target) __nanosleep(200);
-      }
-      __syncthreads();
-    }
-    if (do_scan) full_scan(c, it, mode);
-    __syncthreads();
-  };
-  if (kp.init_W) cta_scan(valid && c.sc->status == 0, 0u, 1, 0u);
-  if (kp.loglik_only) {
-    if (valid) {
-      const double ll = loglik_eval(c, c.sizes);
-      if (tid == 0) kp.out_ll[chain] = ll;
-    }
-    return;
-  }
-
-  for (long long iter = kp.it0 + 1; iter <= kp.it1; ++iter) {
-    const unsigned it = (unsigned)iter;
-    const long long ti0 = RC_CLOCK();
-    bool alive = valid;
-    if (alive) { csync(c); alive = c.sc->status == 0; }
-    bool do_scan = alive;
-    if (alive) {
-      if (c.cwarp == 0) {
-        const bool ra = update_r(c, it);                                     // mcmc.jl:538
-        if (tid == 0) {
-          kp.r_acc[(size_t)chain * kp.numiters + (iter - 1)] = ra ? 1 : 0;
-          update_p(c, it);                                                   // :539
-        }
-      }
-      csync(c);
-      build_lpr(c);
-      if (tid == 0) st_add(c, ST_RP, RC_CLOCK() - ti0);
-      // sample_labels! (:540)
-      const bool multi = kp.numMH > 1;
-      if (multi) {                                           // the chain's own state, in case a proposal is accepted and committed
-        for (int j = tid; j < n; j += RC_NTHR) c.labbak[j] = c.lab[j];
-        for (int s = tid; s < cap; s += RC_NTHR) c.szbak[s] = c.sizes[s];
-        if (tid == 0) { c.szbak[cap] = c.sc->K; c.sc->forked = 0; }
-        csync(c);
-      }
-      for (unsigned mh = 0; mh < (unsigned)kp.numMH; ++mh) {
-        splitmerge_step(c, it, mh, mh + 1 < (unsigned)kp.numMH);
-        if (c.sc->status) { do_scan = false; break; }
-        const int acc = c.sc->itmp[1], spl = c.sc->itmp[2];
-        if (tid == 0) {
-          kp.sm_acc[((size_t)chain * kp.numiters + (iter - 1)) * kp.numMH + mh] = (uint8_t)acc;
-          kp.sm_split[((size_t)chain * kp.numiters + (iter - 1)) * kp.numMH + mh] = (uint8_t)spl;
-        }
-        csync(c);
-        // Quirk Q1 (SURVEY.md A.6): an accepted proposal rebinds sample_labels!'s LOCAL state; the remaining
-        // proposals and the final scan (:477) run on that local object and the caller's labels are untouched this
-        // iteration.  The scan's draws are independent of everything kept (structured stream), so it is skipped.
-        if (acc) do_scan = false;
-      }
-      if (multi && c.sc->status == 0) {                      // back to the chain's own state
-        if (c.sc->forked) {
-          for (int t = tid; t < cap * cap; t += RC_NTHR) { c.WD[t] = c.WDbak[t]; c.WL[t] = c.WLbak[t]; }
-          for (int j = tid; j < n; j += RC_NTHR) c.lab[j] = c.labbak[j];
-          for (int s = tid; s < cap; s += RC_NTHR) c.sizes[s] = c.szbak[s];
-          if (tid == 0) c.sc->K = c.szbak[cap];
-        }
-        csync(c);
-      }
-      if (do_scan) {
-        build_perm<false>(c);              // the scan's last moves / the proposal's launch labels are not in it
-        if (c.sc->status) do_scan = false;
-      }
-    }
-    const long long ts0 = RC_CLOCK();
-    cta_scan(do_scan, it, 0, (unsigned)(iter - kp.it0));
-    const long long ts1 = RC_CLOCK();
-    if (valid && tid == 0) st_add(c, ST_SCAN_TOTAL, ts1 - ts0);
-    if (alive) alive = c.sc->status == 0;
-    if (alive && iter > kp.burnin && (iter - kp.burnin) % kp.thin == 0) {    // :546-554
-      const long long j = (iter - kp.burnin) / kp.thin - 1;
-      if (j < kp.numsamples) {
-        record_labels(c, kp.out_labels + ((size_t)chain * kp.numsamples + j) * n);
-        const double ll = loglik_eval(c, c.sizes);
-        if (c.cwarp == 0) {
-          const double lpv = logprior_eval(c);
-          if (tid == 0) {
-            const size_t o = (size_t)chain * kp.numsamples + j;
-            kp.out_K[o] = c.sc->K; kp.out_r[o] = c.sc->r; kp.out_p[o] = c.sc->p;
-            kp.out_ll[o] = ll; kp.out_lp[o] = ll + lpv;
-          }
-        }
-        csync(c);
-      }
-    }
-    if (valid && tid == 0) { st_add(c, ST_RECORD, RC_CLOCK() - ts1); st_add(c, ST_ITER_TOTAL, RC_CLOCK() - ti0); }
-  }
-  if (valid) {   // store the chain's state
-    csync(c);
-    for (int j = tid; j < n; j += RC_NTHR) kp.labels[(size_t)chain * n + j] = c.lab[j];
-    for (int s = tid; s < cap; s += RC_NTHR) kp.sizes[(size_t)chain * cap + s] = c.sizes[s];
-    if (tid == 0) { kp.r[chain] = c.sc->r; kp.p[chain] = c.sc->p; kp.status[chain] = c.sc->status; }
-  }
-}
-
 // sample_rp (mcmc.jl:592-636): the (r, p)-only chain fitprior runs on the cluster sizes of its notional clustering
 // (prior.jl:80).  One warp; update_r / update_p are the sampler's own (mcmc.jl:80-155); the initial r is drawn with
 // SCALE sigma (mcmc.jl:617: rand(Gamma(eta, sigma)), where runsampler uses 1/sigma -- reproduced as written).
@@ -3209,34 +1807,6 @@ __global__ void k_tables(rc_params P, int n, double* LGA, double* LGZ, double* L
 }
 
 }  // namespace
-
-size_t rc_sampler_smem_bytes(int n, int cap, int tiles, int npad_max, int G) {
-  return cta_header_bytes() + (size_t)RC_NSTAGE * stage_bytes_for(n) + (size_t)G * chain_layout(n, cap, tiles, npad_max).total;
-}
-
-bool rc_chain_kernel_coresident(int nchains, size_t smem, int G, int device) {
-  int nsm = 0, per = 0;
-  cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device);
-  if (G == 2) {
-    cudaFuncSetAttribute(k_chain<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, k_chain<2>, RC_NTHR * 2 + RC_XTHR, smem);
-  } else {
-    cudaFuncSetAttribute(k_chain<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, k_chain<1>, RC_NTHR + RC_XTHR, smem);
-  }
-  return (nchains + G - 1) / G <= nsm * per;
-}
-
-void rc_launch_chain_kernel(const rc_kparams& kp, size_t smem, int G, cudaStream_t st) {
-  const int grid = (kp.nchains + G - 1) / G;
-  if (G == 2) {
-    cudaFuncSetAttribute(k_chain<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    k_chain<2><<<grid, RC_NTHR * 2 + RC_XTHR, smem, st>>>(kp);
-  } else {
-    cudaFuncSetAttribute(k_chain<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    k_chain<1><<<grid, RC_NTHR + RC_XTHR, smem, st>>>(kp);
-  }
-}
 
 size_t rc_sampler_inc_smem_bytes(int n, int cap, int mcap, int tw_smem) { return inc_layout(n, cap, mcap, tw_smem).total; }
 

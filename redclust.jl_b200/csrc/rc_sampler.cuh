@@ -2,19 +2,11 @@
 #pragma once
 #include "rc_common.cuh"
 
-#ifndef RC_BW
-#define RC_BW 4                      // bulk (row-reduction) warps per chain
-#endif
-#define RC_NWARP (RC_BW + 1)         // + one decision warp
-#define RC_NTHR (RC_NWARP * 32)      // threads per chain
-
 struct RowSum { double cT, c2, L2i; int T; unsigned stamp; };   // row summary of the incremental scan, see rc_sampler.cu
 struct rc_kparams {
-  int n, cap, tiles, npad_max;
+  int n, cap;
   int qD, qL;
-  const longlong2* DL;  // the streamed matrix: rc_data::DL, or the sampler's copy with label-sorted columns
-  const unsigned short* colpos;   // [n] column of point j in DL (null: identity)
-  const unsigned short* colpt;    // [n] point of column c in DL (null: identity)
+  const longlong2* DL;  // rc_data::DL
   rc_params P;
   double abratio, zgratio, lgd1, lgd2;
   const double* LGA;    // lgamma(alpha + delta1 * s), s = 0..n+1
@@ -25,7 +17,6 @@ struct rc_kparams {
   unsigned long long seed;
   long long chain_offset;
   int nchains;
-  int init_W;           // 1: (re)build the block-sum matrices from the labels before iterating
   // per-chain state (global memory)
   uint8_t* labels;      // [nchains][n]   0-based slot ids
   int* sizes;           // [nchains][cap]
@@ -37,25 +28,23 @@ struct rc_kparams {
   rc_i128 *WDbak, *WLbak; // [nchains][cap*cap]  numMH > 1 only: the chain's own block sums while a proposal is committed
   uint8_t* labbak;      // [nchains][n]
   int* szbak;           // [nchains][cap+1]
-  longlong2* T;         // [nchains][n][cap]   split-merge scratch: row sums by slot of the members of ci u cj (streaming mode)
-  longlong2* S;         // [nchains][cap][n]   incremental mode: row sums by slot of EVERY point, S[k][x] = sum_{j in k} DL[x][j]
+  longlong2* S;         // [nchains][cap][n]   row sums by slot of EVERY point, S[k][x] = sum_{j in k} DL[x][j]
   unsigned short* Slist;// [nchains][n+2]  members of ci u cj of the current split-merge step
   uint8_t* origM;       // [nchains][n+2]  their labels in the chain's state
   longlong4* AB;        // [nchains][n+2]  running candidate sums of the members (restricted scans)
   double2* L2s;         // [nchains][n]    static repulsion terms per item
   double2* NZ;          // [nchains][(numGibbs+1)*n] Gumbel noise of the free restricted scans
-  double* LPR;          // [nchains][n+2]  prior term by cluster size for the current (r, p)
   longlong2* DG;        // [nchains][n+2]  diagonal entries DL[x][x] of the split-merge members
   double* terms;        // [nchains][terms_stride]  log-likelihood terms / reduction scratch
   size_t terms_stride;  // max(cap*cap, 8192) doubles
-  double2* Cc;          // [nchains][cap][n]  incremental mode: cached per-slot terms (L1, L2') of every (slot, point)
+  double2* Cc;          // [nchains][cap][n]  cached per-slot terms (L1, L2') of every (slot, point)
   unsigned* Vv;         // [nchains][n]       change count at which each point's cached entries were last all valid (0: never)
   unsigned* epochs;     // [nchains][cap + 1] change count at which each slot last changed (>= 1), then the chain's change count
   int tw_smem;          // the per-point counts of a chain live in shared memory during a launch
   int shortcuts;        // 1: rows decided by their summaries and merge proposals rejected by their bound skip the work (same results; RCB200_SHORTCUTS=0 turns both off)
   double* LLF; unsigned* LLFs;   // [nchains][cap][cap] merged-state log-likelihoods per ordered slot pair and their change counts
   RowSum* Rs;           // [nchains][n]       row summaries of the incremental scan (32 B each, see rc_sampler.cu)
-  int inc_mcap;         // incremental mode: split-merge members that fit the shared-memory scratch (64 B each)
+  int inc_mcap;         // split-merge members that fit the shared-memory scratch (64 B each)
   int ovl_min_thr;      // the scan runs beside the restricted scans when the chain has at least this many threads (0: never)
   int rs_team;          // ... and this many of them run the restricted scans
   // outputs
@@ -64,15 +53,10 @@ struct rc_kparams {
   double *out_r, *out_p, *out_ll, *out_lp;
   uint8_t *r_acc, *sm_acc, *sm_split;
   long long* stats;     // [nchains][16] cycle counters (debug / profiling aid)
-  unsigned* gridbar;    // grid-wide arrival counter (zeroed before every launch) or null when the CTAs are not co-resident
   // standalone log-likelihood mode (rc_loglik): skip iterations, write loglik to out_ll[chain]
   int loglik_only;
-  int l2pf;             // rows of lookahead of the producer's L2 prefetch (0: off)
 };
 
-size_t rc_sampler_smem_bytes(int n, int cap, int tiles, int npad_max, int G);
-void rc_launch_chain_kernel(const rc_kparams& kp, size_t smem, int G, cudaStream_t st);
-bool rc_chain_kernel_coresident(int nchains, size_t smem, int G, int device);
 size_t rc_sampler_inc_smem_bytes(int n, int cap, int mcap, int tw_smem);
 int rc_launch_inc_init(const rc_kparams& kp, bool shared_labels, cudaStream_t st);
 int rc_inc_check(const rc_kparams& kp, long long* mismatches_S, long long* mismatches_W, cudaStream_t st);

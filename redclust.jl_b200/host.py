@@ -262,7 +262,8 @@ class Sampler:
 
     def check_sums(self):
         """(mismatching words of the row sums, of the block sums) after rebuilding both from the labels: (0, 0) when the
-        incremental scan mode kept them exact, (-1, -1) in streaming mode."""
+        incremental updates kept them exact, (-1, -1) before the first run.  With launch groups (chains whose row sums do
+        not all fit the device) the chains of the group launched last are checked."""
         a, b = C.c_int64(), C.c_int64()
         check(lib().rc_sampler_check_sums(self._h, C.byref(a), C.byref(b)))
         return a.value, b.value

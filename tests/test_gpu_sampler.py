@@ -18,7 +18,7 @@ def run_both(pkg, orc, D, labels, params, numiters, burnin, thin, numGibbs, numM
     rp = [pkg.init_rp(params, seed, c) for c in range(nchains)]
     smp = pkg.Sampler(data, opts, params, labs, [x[0] for x in rp], [x[1] for x in rp], seed=seed, slot_cap=slot_cap)
     smp.run(-1)
-    assert smp.check_sums() in ((0, 0), (-1, -1))            # incrementally maintained sums == a rebuild from the labels
+    assert smp.check_sums() == (0, 0)                        # incrementally maintained sums == a rebuild from the labels
     out = []
     for c in range(nchains):
         got = smp.samples(c)
@@ -119,7 +119,7 @@ def test_multichain_n1000(pkg, orc):
 
 
 def test_multitile_n2500_resume(pkg, orc):
-    X, lab = mixture(2500, 12, 20, 0.2, 8)     # two row tiles (RC_W = 2048)
+    X, lab = mixture(2500, 12, 20, 0.2, 8)
     data = pkg.MCMCData.from_points(X)
     D = data.D
     params = pkg.params_from_labels(D, lab)
@@ -168,26 +168,34 @@ def test_slot_overflow_stops_only_the_chain_that_overflowed(pkg, orc, golden):
     pytest.skip("no slot capacity in 11..18 stopped some but not all of the chains")
 
 
-@pytest.mark.parametrize("G", [1, 2])
-def test_chains_per_cta_share_rows(pkg, orc, golden, monkeypatch, G):
-    """G chains of a CTA consume the same staged row tiles; 3 chains leave a ragged last CTA for G = 2."""
-    monkeypatch.setenv("RCB200_CHAINS_PER_CTA", str(G))
+@pytest.mark.parametrize("m", [1, 2])
+def test_launch_groups_are_bit_identical(pkg, orc, golden, monkeypatch, m):
+    """Chains run in launch groups of m (the mode of chains whose row sums do not all fit the device): every launch rebuilds
+    the row sums from the labels with every cache stale, and the results do not change a bit; 3 chains leave a ragged last
+    group for m = 2.  check_sums covers the last group."""
+    monkeypatch.setenv("RCB200_CHAINS_PER_GROUP", str(m))
     D, lab = golden[1]["distance_matrix"], golden[1]["cluster_labels"]
     params = pkg.params_from_labels(D, lab)
-    res, _ = run_both(pkg, orc, D, lab, params, 60, 0, 2, 5, 1, seed=31 + G, nchains=3)
+    res, _ = run_both(pkg, orc, D, lab, params, 60, 0, 2, 5, 1, seed=31 + m, nchains=3)
     for got, ref, st in res:
         assert_same(got, ref, st)
 
 
-def test_multitile_two_chains_per_cta(pkg, orc, monkeypatch):
-    monkeypatch.setenv("RCB200_CHAINS_PER_CTA", "2")
+def test_launch_groups_resume_n2500(pkg, orc, monkeypatch):
+    """One chain per launch group at n = 2500, resumed: every call rebuilds each group's state, and three calls equal one run."""
+    monkeypatch.setenv("RCB200_CHAINS_PER_GROUP", "1")
     X, lab = mixture(2500, 12, 20, 0.2, 8)
     data = pkg.MCMCData.from_points(X)
     D = data.D
     params = pkg.params_from_labels(D, lab)
-    res, _ = run_both(pkg, orc, D, lab, params, 4, 0, 1, 5, 1, seed=2, nchains=2)
-    for got, ref, st in res:
-        assert_same(got, ref, st)
+    opts = pkg.MCMCOptionsList(numiters=4, burnin=0, thin=1)
+    rp = [pkg.init_rp(params, 2, c) for c in range(2)]
+    smp = pkg.Sampler(data, opts, params, np.tile(lab, (2, 1)), [x[0] for x in rp], [x[1] for x in rp], seed=2)
+    smp.run(2); smp.run(1); smp.run(-1)
+    assert smp.check_sums() == (0, 0)
+    for c in range(2):
+        ref = orc.run_chain(D, orc.Options(4, 0, 1, 5, 1), oparams(orc, params), lab, rp[c][0], rp[c][1], seed=2, chain=c)
+        assert_same(smp.samples(c), ref, smp.state(c))
 
 
 def test_several_proposals_per_iteration(pkg, orc, golden):
@@ -207,7 +215,8 @@ def test_several_proposals_per_iteration(pkg, orc, golden):
 
 def test_tiny_problems_and_many_slots(pkg, orc):
     """n = 2 ... 65 with weak priors: chains wander between 1 and n clusters, i.e. through the empty-slot allocation, the
-    64-slot -> 128-slot switch of the decision warp, singleton split / merge proposals and numMH in {0, 1, 3}."""
+    switch from 4 to 8 lanes per row of the scan once a slot beyond 63 is live, singleton split / merge proposals and
+    numMH in {0, 1, 3}."""
     rng = np.random.default_rng(0)
     params = pkg.PriorHyperparamsList(delta1=2.0, alpha=5.0, beta=3.0, delta2=2.5, zeta=6.0, gamma=4.0, eta=4.0, sigma=2.0,
                                       u=2.0, v=10.0, K_initial=2)
@@ -231,8 +240,8 @@ def test_tiny_problems_and_many_slots(pkg, orc):
 
 
 def test_points_in_random_order(pkg, orc):
-    """Cluster members scattered over the columns (every row tile holds every label: many short (tile, label) runs,
-    frequent bin flushes, random shared-memory banks) and a start that is 4 % off: three tiles, two chains per CTA."""
+    """Cluster members scattered over the points (no cluster is a contiguous run of rows) and a start that is 4 % off:
+    three chains."""
     X, lab = mixture(3000, 25, 30, 0.15, 21)
     perm = np.random.default_rng(4).permutation(lab.size)
     X, lab = X[perm], orc.sortlabels(lab[perm])
@@ -256,12 +265,11 @@ def test_points_in_random_order(pkg, orc):
     dict(RCB200_INC_THREADS="64", RCB200_OVERLAP_MIN_THREADS="64", RCB200_RS_TEAM="32"),
 ])
 def test_team_shapes_are_bit_identical(pkg, orc, monkeypatch, env):
-    """The incremental kernel's team shapes (threads per chain, threads on the restricted scans, scan beside or after them,
+    """The chain kernel's team shapes (threads per chain, threads on the restricted scans, scan beside or after them,
     where the cached terms' validity counts live) change the schedule, never a bit: a chain that moves points, splits and
     merges (loose mixture, wrong initial labels), three chains, against the oracle; the maintained sums equal a rebuild."""
     for k, v in env.items():
         monkeypatch.setenv(k, v)
-    monkeypatch.setenv("RCB200_SCAN", "inc")
     X, lab = mixture(700, 9, 12, 0.45, 21)
     g = np.random.default_rng(3)
     init = lab.copy()
@@ -287,7 +295,6 @@ def test_shortcuts_fire_and_change_nothing(pkg, orc, monkeypatch, shortcuts):
     rejects hopeless merge proposals without their restricted scans: on a well separated mixture most rows and most merge
     proposals take the shortcut, and every output still equals the oracle's -- as it does with RCB200_SHORTCUTS=0."""
     monkeypatch.setenv("RCB200_SHORTCUTS", shortcuts)
-    monkeypatch.setenv("RCB200_SCAN", "inc")
     X, lab = mixture(600, 6, 10, 0.12, 4)
     data = pkg.MCMCData.from_points(X)
     D = data.D

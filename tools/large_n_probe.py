@@ -1,5 +1,4 @@
-"""The sampler beyond the streaming kernel's n of about 26 000 (its labels and column permutation live in shared memory):
-incremental mode at n = 30 000 by default, a few sweeps of a few chains, checked by the sums invariant (the maintained
+"""The sampler at large n (30 000 by default; up to 65 535, the 16-bit point indices): a few sweeps of a few chains, checked by the sums invariant (the maintained
 row / block sums against a rebuild from the labels) and by the log-likelihood of the final state recomputed through
 rc_loglik-free means (block sums rebuilt).  usage: python tools/large_n_probe.py [n] [chains] [sweeps]"""
 import os, sys, time

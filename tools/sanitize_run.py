@@ -1,6 +1,6 @@
-"""Small sampler runs for compute-sanitizer (racecheck / synccheck / memcheck): both scan modes on the reference's n = 100
-fixture (split-merge, several proposals per iteration, two chains) and a two-tile n = 2500 problem, each checked
-against the oracle.  usage: compute-sanitizer --tool racecheck python tools/sanitize_run.py [small|large]"""
+"""Small sampler runs for compute-sanitizer (racecheck / synccheck / memcheck): all chains in one launch and one chain per
+launch group, on the reference's n = 100 fixture (split-merge, several proposals per iteration, two chains) and an
+n = 2500 problem, each checked against the oracle.  usage: compute-sanitizer --tool racecheck python tools/sanitize_run.py [small|large]"""
 import os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -13,7 +13,10 @@ pkg, orc = g.load_package(), g.load_oracle()
 
 
 def run(D, lab, iters, numMH, nch, mode, seed):
-    os.environ["RCB200_SCAN"] = mode
+    if mode == "grouped":
+        os.environ["RCB200_CHAINS_PER_GROUP"] = "1"
+    else:
+        os.environ.pop("RCB200_CHAINS_PER_GROUP", None)
     params = pkg.params_from_labels(D, lab)
     opts = pkg.MCMCOptionsList(numiters=iters, burnin=0, thin=1, numGibbs=3, numMH=numMH)
     rp = [pkg.init_rp(params, seed, c) for c in range(nch)]
@@ -28,11 +31,11 @@ def run(D, lab, iters, numMH, nch, mode, seed):
 if which == "small":
     gd = np.load(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden", "example1.npz"))
     D, lab = gd["distance_matrix"], gd["cluster_labels"]
-    for mode in ("inc", "stream"):
+    for mode in ("resident", "grouped"):
         run(D, lab, 12, 1, 2, mode, 3)
         run(D, np.ones(100, np.int64), 8, 2, 1, mode, 4)
 else:
     X, lab = mixture(2500, 12, 20, 0.2, 8)
     D = orc.distm(X)
-    for mode in ("inc", "stream"):
+    for mode in ("resident", "grouped"):
         run(D, lab, 2, 1, 2, mode, 5)
