@@ -49,6 +49,7 @@ struct rc_sampler {
   double2* Cc; unsigned *Vv, *epochs;   // cached per-slot terms, per-point / per-slot change counts that validate them
   void* Rs;                    // row summaries of the scan (group x n x 32 B)
   double* LLF; unsigned* LLFs; // merged-state log-likelihoods per ordered slot pair and their change counts
+  double4* Cm; unsigned* Cms;  // per-slot margins of the row summaries, the change count they were built at and whether the build succeeded
   int64_t group;               // chains per launch
   int64_t last_g0;             // first chain of the group launched last (its S is the one that exists)
   int tw_smem, shortcuts;
@@ -126,7 +127,7 @@ void fill_kparams(const rc_sampler* s, rc_kparams& kp, int64_t g0 = 0) {
   const size_t NS = (size_t)s->numsamples, ni = (size_t)s->opt.numiters, nm = ni * (size_t)s->opt.numMH;
   kp.n = (int)n; kp.cap = s->cap;
   kp.qD = s->d->qD; kp.qL = s->d->qL; kp.DL = s->d->DL;
-  kp.S = s->S; kp.terms_stride = s->terms_stride; kp.inc_mcap = s->inc_mcap; kp.ovl_min_thr = s->ovl_min_thr; kp.rs_team = s->rs_team; kp.Cc = s->Cc; kp.Vv = s->Vv; kp.epochs = s->epochs; kp.tw_smem = s->tw_smem; kp.shortcuts = s->shortcuts; kp.Rs = (RowSum*)s->Rs; kp.LLF = s->LLF; kp.LLFs = s->LLFs;
+  kp.S = s->S; kp.terms_stride = s->terms_stride; kp.inc_mcap = s->inc_mcap; kp.ovl_min_thr = s->ovl_min_thr; kp.rs_team = s->rs_team; kp.Cc = s->Cc; kp.Vv = s->Vv; kp.epochs = s->epochs; kp.tw_smem = s->tw_smem; kp.shortcuts = s->shortcuts; kp.Rs = (RowSum*)s->Rs; kp.LLF = s->LLF; kp.LLFs = s->LLFs; kp.Cm = s->Cm; kp.Cms = s->Cms;
   kp.P = s->par;
   kp.abratio = s->par.alpha * rc_log(s->par.beta) - rc_lgamma(s->par.alpha);    // mcmc.jl:17,186,293
   kp.zgratio = s->par.zeta * rc_log(s->par.gamma) - rc_lgamma(s->par.zeta);     // mcmc.jl:18,187,294
@@ -151,13 +152,14 @@ __global__ void k_fill_u32(unsigned* __restrict__ p, size_t count, unsigned v) {
   for (size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; t < count; t += (size_t)gridDim.x * blockDim.x) p[t] = v;
 }
 
-// Every cache of the group state stale: no point's cached terms (Vv = 0), row summary (stamp 0) or merged-state
-// log-likelihood (change count 0) is valid at the chains' change count 1 (epochs).
+// Every cache of the group state stale: no point's cached terms (Vv = 0), row summary (stamp 0), per-slot margin (change
+// count 0) or merged-state log-likelihood (change count 0) is valid at the chains' change count 1 (epochs).
 int reset_caches(const rc_sampler* s) {
   const size_t m = (size_t)s->group, n = (size_t)s->n, cap = (size_t)s->cap;
   RC_CUDA(cudaMemsetAsync(s->Vv, 0, sizeof(unsigned) * m * n, s->stream));
   RC_CUDA(cudaMemsetAsync(s->Rs, 0, m * n * 32, s->stream));
   RC_CUDA(cudaMemsetAsync(s->LLFs, 0, sizeof(unsigned) * m * cap * cap, s->stream));
+  RC_CUDA(cudaMemsetAsync(s->Cms, 0, sizeof(unsigned) * m * 2, s->stream));
   k_fill_u32<<<256, 256, 0, s->stream>>>(s->epochs, m * (cap + 1), 1u);
   RC_CUDA(cudaGetLastError());
   return RC_OK;
@@ -187,7 +189,7 @@ void rc_sampler_destroy(rc_sampler* s) {
   rc_dev_free(s->stats);
   rc_dev_free(s->out_labels); rc_dev_free(s->out_K); rc_dev_free(s->out_r); rc_dev_free(s->out_p); rc_dev_free(s->out_ll); rc_dev_free(s->out_lp);
   rc_dev_free(s->r_acc); rc_dev_free(s->sm_acc); rc_dev_free(s->sm_split);
-  rc_dev_free(s->S); rc_dev_free(s->Cc); rc_dev_free(s->Vv); rc_dev_free(s->epochs); rc_dev_free(s->Rs); rc_dev_free(s->LLF); rc_dev_free(s->LLFs);
+  rc_dev_free(s->S); rc_dev_free(s->Cc); rc_dev_free(s->Vv); rc_dev_free(s->epochs); rc_dev_free(s->Rs); rc_dev_free(s->LLF); rc_dev_free(s->LLFs); rc_dev_free(s->Cm); rc_dev_free(s->Cms);
   if (s->e0) cudaEventDestroy(s->e0);
   if (s->e1) cudaEventDestroy(s->e1);
   if (s->stream) cudaStreamDestroy(s->stream);
@@ -254,10 +256,11 @@ int32_t rc_sampler_create(const rc_data* d, const rc_options* opt, const rc_para
   TRY(dalloc(&s->r, nchains)); TRY(dalloc(&s->p, nchains)); TRY(dalloc(&s->status, nchains));
   TRY(dalloc(&s->WD, (size_t)nchains * cap * cap)); TRY(dalloc(&s->WL, (size_t)nchains * cap * cap));
   // Group size: as many chains per launch as have their group state (S and Cc, cap x n entries each, row summaries,
-  // change counts, merged-state log-likelihoods) in 60 % of the free memory.
+  // change counts, merged-state log-likelihoods, per-slot margins) in 60 % of the free memory.
   {
     const size_t per = (sizeof(longlong2) + sizeof(double2)) * (size_t)cap * n + (32 + sizeof(unsigned)) * (size_t)n +
-                       sizeof(unsigned) * (size_t)(cap + 1) + (sizeof(double) + sizeof(unsigned)) * (size_t)cap * cap;
+                       sizeof(unsigned) * (size_t)(cap + 1) + (sizeof(double) + sizeof(unsigned)) * (size_t)cap * cap +
+                       sizeof(double4) * (size_t)cap + sizeof(unsigned) * 2;
     size_t freeb = 0, totalb = 0;
     cudaMemGetInfo(&freeb, &totalb);
     s->group = std::min<int64_t>(nchains, (int64_t)(freeb / 10 * 6 / per));
@@ -308,6 +311,7 @@ int32_t rc_sampler_create(const rc_data* d, const rc_options* opt, const rc_para
     TRY(dalloc(&s->epochs, G * (cap + 1)));
     { char* rs = nullptr; TRY(dalloc(&rs, G * n * 32)); s->Rs = rs; }
     TRY(dalloc(&s->LLF, G * cap * cap)); TRY(dalloc(&s->LLFs, G * cap * cap));
+    TRY(dalloc(&s->Cm, G * cap)); TRY(dalloc(&s->Cms, G * 2));
   }
   if (opt->numMH > 1) {
     TRY(dalloc(&s->WDbak, (size_t)nchains * cap * cap)); TRY(dalloc(&s->WLbak, (size_t)nchains * cap * cap));

@@ -69,6 +69,8 @@ struct IncShared {
   int scanfast;      // at least half the rows of the last complete pass were: the scan is short, nothing is gained by running it beside the restricted scans
   int tabs_ok;       // every live slot's size-dependent prior term is finite ...
   double maxtab;     // ... and this is their maximum (at the slot's size and at size - 1)
+  unsigned cm_clk;   // change count the per-slot margins (Cm) were built at (0: never) ...
+  int cm_ok;         // ... and whether that build succeeded (see inc_margins_build)
   int rs_mv[RC_INC_MAXW][8];            // restricted scans: per warp the moves of its eight steps, in step order: item << 1 | (1: ca -> cb)
   int rs_nm[RC_INC_MAXW];               // ... and how many
   double rs_win[RC_RS_MAXW][6][16];     // ... per evaluating warp: LGA / LGZ / LPR at the sixteen sizes its steps can see ({A, B} x 3 tables)
@@ -120,6 +122,7 @@ struct Ctx {
   int* res;               // (shared memory) [nthr] slot chosen by each row of a batch
   double2* Cc;            // (global) [cap][n] cached per-slot terms, see inc_eval_row
   RowSum* Rs;             // (global) [n] row summaries
+  double4* Cm; unsigned* Cms;    // (global) [cap] per-slot margins of the row summaries, [2] their change count and build result
   double* LLF; unsigned* LLFs;   // (global) [cap][cap] loglik of the state with slot ci merged into cj, and the change count it was computed at (0: never)
   unsigned* tw;           // (shared memory when it fits, else global) [n] change count at which point x's cached entries were last made valid
   unsigned* tchg;         // (shared memory) [cap] change count at which each slot last gained or lost a point
@@ -163,7 +166,9 @@ __device__ __forceinline__ void inc_update_S(const Ctx& c, int y, int a, int b, 
     Sa[x] = sa; Sb[x] = sb;
   }
 }
-// stats slots
+// stats slots (in the default library, -DRC_NO_STATS, the timing slots stay 0 and a few count events instead: dec_wait the
+// merge proposals rejected by their bound, bulk_rows the rows decided by their summaries, bulk_reduce the scans decided by
+// the per-slot margins)
 enum { ST_DEC_WAIT = 0, ST_DEC_WORK, ST_BULK_WAIT_CONSUMED, ST_BULK_WAIT_FULL, ST_BULK_ROWS, ST_BULK_PATCH, ST_MOVES, ST_REBUILDS,
        ST_MH_SETUP, ST_MH_RSCAN, ST_MH_LOGLIK, ST_SCAN_TOTAL, ST_RECORD, ST_ITER_TOTAL, ST_RP, ST_BULK_REDUCE };
 __device__ __forceinline__ void st_add(const Ctx& c, int slot, long long v) { c.stats[slot] += v; }
@@ -1332,6 +1337,107 @@ __device__ void inc_build_tables(const Ctx& c, int only_a = -1, int only_b = -1)
   __syncwarp();
 }
 
+// bar.red.or over the team: true when v holds in any thread (a barrier like csync)
+__device__ __forceinline__ bool team_any(int barid, int nthr, bool v) {
+  int r;
+  asm volatile("{\n .reg .pred p, q;\n setp.ne.s32 p, %1, 0;\n bar.red.or.pred q, %2, %3, p;\n selp.s32 %0, 1, 0, q;\n}"
+               : "=r"(r) : "r"((int)v), "r"(barid), "r"(nthr) : "memory");
+  return r != 0;
+}
+// doubles <-> 64-bit integers of the same order (finite values), for min / max by integer atomics
+__device__ __forceinline__ long long ord_key(double x) { const long long b = __double_as_longlong(x); return b >= 0 ? b : b ^ 0x7fffffffffffffffLL; }
+__device__ __forceinline__ double ord_val(long long k) { return __longlong_as_double(k >= 0 ? k : k ^ 0x7fffffffffffffffLL); }
+#define RC_CM_BIG 0x1p1000       // magnitudes below this: no sum of four such values overflows
+
+// Per-slot margins of the row summaries.  Of the row-summary test (RowSum) only tab_T, maxtab and the new-cluster base
+// A = LOGN[Ki + 1] + r log(1 - p) depend on (r, p); everything per row is fixed while the chain's state is.  So when every
+// row's summary is current, its leader is its own slot T and that slot keeps at least two points, slot T stores over its rows
+//   Cm[T].x = min fl(cT - c2),   Cm[T].y = min fl(cT - L2i) (repulsion) / min cT (none),   Cm[T].z = max(|cT|, |c2|, |L2i|)
+// and a scan tests O(K) slots instead of n summaries (inc_scan_by_margins).  Min and max are exact, so the order in which
+// rows are reduced does not matter.  Built after a committed scan that moved no point; a failed build is not retried until
+// the state changes (Cms = {change count, ok}).  red: [3][cap] shared-memory scratch.  Whole team.
+__device__ __noinline__ void inc_margins_build(const RowCtx rc, IncShared* sh, double4* Cm, unsigned* Cms, long long* red,
+                                               int tid, int NT, int barid) {
+  const int n = rc.n, cap = rc.cap;
+  const unsigned clk = sh->clk;
+  const bool rep = rc.kp->P.repulsion;
+  for (int s = tid; s < cap; s += NT) { red[s] = LLONG_MAX; red[cap + s] = LLONG_MAX; red[2 * cap + s] = 0; }
+  asm volatile("bar.sync %0, %1;" ::"r"(barid), "r"(NT) : "memory");
+  bool ok = true;
+  int cs = -1;                                                              // the thread's current slot and its running values
+  double ma = 0.0, mb = 0.0, mg = 0.0;
+  auto flush = [&]() {
+    if (cs < 0) return;
+    atomicMin(red + cs, ord_key(ma)); atomicMin(red + cap + cs, ord_key(mb));
+    atomicMax(red + 2 * cap + cs, __double_as_longlong(mg));              // (mg >= 0: its bits order like the value)
+  };
+  for (int i = tid; i < n; i += NT) {
+    const RowSum rs = rc.Rs[i];
+    const int T = rs.T;
+    // (comparisons are false for NaN: a NaN term fails like an infinite one)
+    if (rs.stamp != clk || T != (int)rc.lab[i] || rc.sizes[T] < 2 ||
+        !(fabs(rs.cT) < RC_CM_BIG && fabs(rs.c2) < RC_CM_BIG && fabs(rs.L2i) < RC_CM_BIG)) { ok = false; break; }
+    const double a = rs.cT - rs.c2, b = rep ? rs.cT - rs.L2i : rs.cT;
+    const double m = fmax(fabs(rs.cT), fmax(fabs(rs.c2), fabs(rs.L2i)));
+    if (T != cs) { flush(); cs = T; ma = a; mb = b; mg = m; }
+    else { ma = fmin(ma, a); mb = fmin(mb, b); mg = fmax(mg, m); }
+  }
+  if (ok) flush();
+  ok = !team_any(barid, NT, !ok);
+  if (ok)
+    for (int s = tid; s < cap; s += NT) Cm[s] = make_double4(ord_val(red[s]), ord_val(red[cap + s]), __longlong_as_double(red[2 * cap + s]), 0.0);
+  if (tid == 0) { Cms[0] = clk; Cms[1] = ok ? 1u : 0u; sh->cm_clk = clk; sh->cm_ok = ok ? 1 : 0; }
+  asm volatile("bar.sync %0, %1;" ::"r"(barid), "r"(NT) : "memory");
+}
+
+// A whole scan decided by the per-slot margins: true when every row would be decided by its summary and stays where it is.
+// Every warp tests every live slot T (t5 = tab_T at size - 1, the point detached) against
+//   (1)  fl(fl(t5 - maxtab) + Cm[T].x) > 41 + eps1,   eps1 = 2^-46 (E1 + 64),  E1 = Cm[T].z + |t5| + |maxtab|
+//   (2)  fl(fl(t5 - A)      + Cm[T].y) > 41 + eps2,   eps2 = 2^-46 (E2 + 64),  E2 = Cm[T].z + |t5| + |A|   (new cluster possible)
+// and then every row's leader uniform is drawn and checked to be > 0, as the row-summary path does.
+// Proof that (1) implies the row test tab_T + cT - (maxtab + c2) > 41, i.e. fl(fl(t5 + cT) - fl(maxtab + c2)) > 41, for every
+// row of T (for (2) replace maxtab by A and c2 by L2i, or by +-0 without repulsion, where lpnew = A exactly; A is computed
+// by the same operations as in the row test).  u = 2^-53, M = Cm[T].z, all magnitudes below 2^1000 (checked, so nothing
+// overflows and every term is finite):  with d = fl(cT - c2) >= Cm[T].x (the minimum is exact)
+//   fl(t5 + cT) - fl(maxtab + c2) >= t5 - maxtab + cT - c2 - u(|t5| + |cT| + |maxtab| + |c2|)
+//   cT - c2 >= d - u(|cT| + |c2|) >= Cm[T].x - 2uM
+//   t5 - maxtab + Cm[T].x >= w - u(|t5| + |maxtab|) - u(1 + u)(|t5| + |maxtab| + 2M(1 + u))   (w: the left side of (1))
+// so the row's exact difference is >= w - u(3|t5| + 3|maxtab| + 6M)(1 + 2u) > w - 2^-50 E1 > 41 + 2^-46 E1 + 2^-40 - 2^-50 E1
+// (computing eps and its sum with 41 loses less than 2^-96 E1 + 2^-47), hence > 41 + 2^-41, and its rounding stays above
+// 41 (ulp(41) = 2^-47).  Rows of T pass the row test, so the new path decides a subset of what the row summaries decide,
+// with the same outcome (no move), and no output changes.  Whole team; one barrier.
+__device__ __noinline__ bool inc_scan_by_margins(const RowCtx rc, const double4* Cm, unsigned it, int tid, int NT, int barid) {
+  const rc_params& P = rc.kp->P;
+  const IncShared* sh = rc.inc;
+  const int n = rc.n, cap = rc.cap;
+  const int Ki = sh->nlive;
+  const bool hasnew = (P.maxK == 0 || Ki < P.maxK) && Ki < n;               // :198 (every point's own cluster survives)
+  const double maxtab = sh->maxtab;
+  if (hasnew && sh->e0 < 0) return false;                                   // (the row evaluation reports the missing slot)
+  const double A = rc.kp->LOGN[Ki + 1] + rc.sc->r * rc.sc->log1mp;          // (as in the row test)
+  bool fail = false;
+  for (int s = tid & 31; s < cap; s += 32)
+    if (rc.sizes[s] > 0) {
+      const double4 m = Cm[s];
+      const double t5 = rc.tabs[5 * cap + s];
+      const double e1 = m.z + fabs(t5) + fabs(maxtab);
+      bool pass = e1 < RC_CM_BIG && (t5 - maxtab) + m.x > RC_SUM_MARGIN + 0x1p-46 * (e1 + 64.0);
+      if (hasnew) {
+        const double e2 = m.z + fabs(t5) + fabs(A);
+        pass = pass && e2 < RC_CM_BIG && (t5 - A) + m.y > RC_SUM_MARGIN + 0x1p-46 * (e2 + 64.0);
+      }
+      if (!pass) fail = true;
+    }
+  fail = __any_sync(0xffffffffu, fail);
+  if (!fail)
+    for (int i = tid; i < n; i += NT) {                                     // the leader's own uniform must be > 0 (else its noise is -Inf)
+      const int kk = (int)rc.rank[rc.lab[i]];
+      const rc_draw dr = rc_draw2(rc.key, it, RC_SITE_SCAN, 0, (uint32_t)i, (uint32_t)(kk >> 1));
+      if (!(((kk & 1) ? dr.u1 : dr.u0) > 0.0)) fail = true;
+    }
+  return !team_any(barid, NT, fail);
+}
+
 // The full scan (mcmc.jl:192-253) from row istart in batches of up to nthr / G consecutive rows (G lanes per row), by the
 // team described by c (the whole CTA, or the warps that have nothing to do during the restricted scans).
 // dry: nothing is committed -- the scan stops at the first row that would move its point (or overflow) and leaves that
@@ -1354,6 +1460,14 @@ __device__ void inc_full_scan(const Ctx& c, unsigned it, int istart, bool dry) {
   int nrows = sh->hint > 0 ? sh->hint : NT, streak = 0;
   int skipA = 0;                                                            // batches to go before the summaries are tried again
   long long nfast = 0;
+  // a committed scan whose per-slot margins are current: decided as a whole when they prove that no row moves
+  if (!dry && istart == 0 && sh->mksum && sh->tabs_ok && sh->cm_ok && sh->cm_clk == sh->clk &&
+      inc_scan_by_margins(rc, c.Cm, it, tid, NT, c.barid)) {
+    i0 = n; nfast = n;
+#ifdef RC_NO_STATS
+    if (tid == 0) st_add(c, ST_BULK_REDUCE, 1);                             // (default library: scans decided by the margins)
+#endif
+  }
   while (i0 < n) {
     const int slot3 = batch % 3;
     if (tid == 0) { const int nx = (batch + 1) % 3; sh->sfirst[nx] = RC_INC_NONE; sh->fa[nx] = RC_INC_NONE; sh->fm[nx] = RC_INC_NONE; }
@@ -1501,6 +1615,10 @@ __device__ void inc_full_scan(const Ctx& c, unsigned it, int istart, bool dry) {
     if (lane == 0) { c.sc->K = K; st_add(c, ST_MOVES, sh->nmoves); sh->hint = nrows; sh->mksum = (sh->nmoves <= 2 && c.kp->shortcuts) ? 1 : 0; }
   }
   csync(c);
+  // nothing moved and the margins are not current: build them (in the split-merge member scratch, dead here) while every
+  // row's summary is fresh
+  if (sh->nmoves == 0 && sh->mksum && sh->cm_clk != sh->clk && 4 * c.mcap >= 3 * cap)
+    inc_margins_build(rc, sh, c.Cm, c.Cms, reinterpret_cast<long long*>(c.mAB), tid, NT, c.barid);
 }
 
 struct IncLayout { size_t prows, sc, inc, sizes, szL, itmp, clist, lab, labL, live, rank, tabs, res, ep, tw, mAB, mDG, mL2s, total; };
@@ -1554,6 +1672,7 @@ __global__ void __launch_bounds__(512, 1) k_chain_inc(const __grid_constant__ rc
     c.tw = kp.tw_smem ? reinterpret_cast<unsigned*>(smem + L.tw) : kp.Vv + (size_t)chain * n;
     c.Rs = kp.Rs + (size_t)chain * n;
     c.LLF = kp.LLF + (size_t)chain * cap * cap; c.LLFs = kp.LLFs + (size_t)chain * cap * cap;
+    c.Cm = kp.Cm + (size_t)chain * cap; c.Cms = kp.Cms + (size_t)chain * 2;
     c.prows = reinterpret_cast<rc_i128*>(smem + L.prows);
     c.sc = reinterpret_cast<Scal*>(smem + L.sc);
     c.inc = reinterpret_cast<IncShared*>(smem + L.inc);
@@ -1587,7 +1706,7 @@ __global__ void __launch_bounds__(512, 1) k_chain_inc(const __grid_constant__ rc
   for (int j = tid; j < n; j += nt) c.lab[j] = kp.labels[(size_t)chain * n + j];
   for (int s = tid; s < cap; s += nt) { c.sizes[s] = kp.sizes[(size_t)chain * cap + s]; c.tchg[s] = kp.epochs[(size_t)chain * (cap + 1) + s]; }
   if (kp.tw_smem) for (int j = tid; j < n; j += nt) c.tw[j] = kp.Vv[(size_t)chain * n + j];
-  if (tid == 0) { c.inc->clk = kp.epochs[(size_t)chain * (cap + 1) + cap]; c.inc->mksum = kp.shortcuts ? 1 : 0; c.inc->tabs_ok = 0; c.inc->maxtab = 0.0; c.inc->nfast_dry = 0; c.inc->scanfast = 0; c.sc->llclk = 0u; c.sc->llcur = 0.0; }
+  if (tid == 0) { c.inc->clk = kp.epochs[(size_t)chain * (cap + 1) + cap]; c.inc->mksum = kp.shortcuts ? 1 : 0; c.inc->tabs_ok = 0; c.inc->maxtab = 0.0; c.inc->nfast_dry = 0; c.inc->scanfast = 0; c.sc->llclk = 0u; c.sc->llcur = 0.0; c.inc->cm_clk = c.Cms[0]; c.inc->cm_ok = (int)c.Cms[1]; }
   if (tid == 0) {
     Scal& s = *c.sc;
     s.r = kp.r[chain]; s.p = kp.p[chain];

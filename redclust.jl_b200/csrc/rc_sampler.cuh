@@ -44,6 +44,8 @@ struct rc_kparams {
   int shortcuts;        // 1: rows decided by their summaries and merge proposals rejected by their bound skip the work (same results; RCB200_SHORTCUTS=0 turns both off)
   double* LLF; unsigned* LLFs;   // [nchains][cap][cap] merged-state log-likelihoods per ordered slot pair and their change counts
   RowSum* Rs;           // [nchains][n]       row summaries of the incremental scan (32 B each, see rc_sampler.cu)
+  double4* Cm;          // [nchains][cap]     per-slot margins of the row summaries (see inc_margins_build)
+  unsigned* Cms;        // [nchains][2]       the change count they were built at (0: never) and whether that build succeeded
   int inc_mcap;         // split-merge members that fit the shared-memory scratch (64 B each)
   int ovl_min_thr;      // the scan runs beside the restricted scans when the chain has at least this many threads (0: never)
   int rs_team;          // ... and this many of them run the restricted scans

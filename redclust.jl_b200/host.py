@@ -307,6 +307,9 @@ class Sampler:
         check(lib().rc_sampler_copy_state(self._h, chain, ptr(lab), C.byref(r), C.byref(p)))
         return MCMCState(lab, r.value, p.value)
 
+    # Cycle counters in librcb200_stats.so.  In the default library the timing slots stay 0 and three slots count events:
+    # dec_wait the merge proposals rejected by their bound, bulk_rows the rows decided by their summaries, bulk_reduce the
+    # scans decided as a whole by the per-slot margins.
     STAT_NAMES = ("dec_wait", "dec_work", "bulk_wait_consumed", "bulk_wait_full", "bulk_rows", "bulk_patch", "moves", "rebuilds",
                   "mh_setup", "mh_rscan", "mh_loglik", "scan_total", "record", "iter_total", "rp", "bulk_reduce")
 
