@@ -184,6 +184,26 @@ int32_t rc_sampler_psm_counts_dev(const rc_sampler* s, int64_t chain0, int64_t n
 int32_t rc_sampler_psm(const rc_sampler* s, int64_t chain0, int64_t nch, double* psm_out);
 void rc_sampler_destroy(rc_sampler* s);
 
+/* ---- posterior predictive allocation of new observations (no reference equivalent) -------------------------------------
+ * For new point x (row x of Dnew, m x n: dissimilarities to the training points in data order, finite and > 0) and sample s,
+ * P_s(x, k) is the full Gibbs scan's conditional for x as point n + 1 of the augmented data in state (labels_s, r_s, p_s)
+ * (src/mcmc.jl:193-247) normalised as sample_logweights draws from it (src/utils.jl:2-6): candidates are the slots 1..K_s
+ * of sortlabels(labels_s) and, when maxK == 0 or K_s < maxK, the new slot K_s + 1.  Outputs (host):
+ *   cocl_out[x][j] = (1/S) sum_s P_s(x, c_s(j))   (m x n),   newcl_out[x] = (1/S) sum_s P_s(x, K_s + 1)   (m)
+ * summed in ascending sample order; S = 0 gives NaN.  lp_out (NULL or S x m x 256) receives the un-normalised
+ * log-probabilities of the candidates, slot k at index k - 1, NaN beyond the last candidate.  More than 255 clusters in a
+ * sample: RC_ERR_SLOTS; r <= 0 or p outside (0, 1): RC_ERR_ARG; a bad entry of Dnew: RC_ERR_DOMAIN.                     */
+int32_t rc_predict(const rc_data* d, const rc_params* par, const double* Dnew, int64_t m, const int64_t* labels, const double* r,
+                   const double* p, int64_t S, double* cocl_out, double* newcl_out, double* lp_out);
+/* The same over the device-resident recorded samples of chains [chain0, chain0 + nch) (chain-major, sample-minor) with the
+ * sampler's hyperparameters (src/mcmc.jl:193-247, src/utils.jl:2-6).  Needs a run to numiters (RC_ERR_STATE before: the
+ * samples are not all recorded) and chains that did not stop at the slot capacity (RC_ERR_SLOTS).                        */
+int32_t rc_sampler_predict(const rc_sampler* s, const double* Dnew, int64_t m, int64_t chain0, int64_t nch, double* cocl_out,
+                           double* newcl_out);
+/* Dissimilarities of new points Y (m x dim) to training points X (n x dim), both row-major host fp64, into out (m x n):
+ * bit-equal to rows n.., columns ..n of rc_data_from_points on the stacked points (the rows of rc_distm_rows_dev). */
+int32_t rc_crossdist(const double* X, int64_t n, const double* Y, int64_t m, int64_t dim, int32_t device, double* out);
+
 /* ---- stand-alone pieces ------------------------------------------------------------------ */
 /* loglik(data, state, params) and logprior(state, params) for one host label vector:
  * src/mcmc.jl:1-78.                                                                            */

@@ -72,6 +72,9 @@ SIGNATURES = {
     "rc_sampler_psm_counts_dev": (C.c_int32, [_vp, C.c_int64, C.c_int64, _vp]),
     "rc_sampler_psm": (C.c_int32, [_vp, C.c_int64, C.c_int64, _vp]),
     "rc_sampler_destroy": (None, [_vp]),
+    "rc_predict": (C.c_int32, [_vp, _P(rc_params), _vp, C.c_int64, _vp, _vp, _vp, C.c_int64, _vp, _vp, _vp]),
+    "rc_sampler_predict": (C.c_int32, [_vp, _vp, C.c_int64, C.c_int64, C.c_int64, _vp, _vp]),
+    "rc_crossdist": (C.c_int32, [_vp, C.c_int64, _vp, C.c_int64, C.c_int64, C.c_int32, _vp]),
     "rc_loglik": (C.c_int32, [_vp, _P(rc_params), _vp, _P(C.c_double)]),
     "rc_psm": (C.c_int32, [_vp, C.c_int64, C.c_int64, C.c_int32, _vp]),
     "rc_psm_counts_dev": (C.c_int32, [_vp, C.c_int64, C.c_int64, C.c_int32, _vp]),

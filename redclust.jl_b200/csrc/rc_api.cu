@@ -129,8 +129,8 @@ void fill_kparams(const rc_sampler* s, rc_kparams& kp, int64_t g0 = 0) {
   kp.qD = s->d->qD; kp.qL = s->d->qL; kp.DL = s->d->DL;
   kp.S = s->S; kp.terms_stride = s->terms_stride; kp.inc_mcap = s->inc_mcap; kp.ovl_min_thr = s->ovl_min_thr; kp.rs_team = s->rs_team; kp.Cc = s->Cc; kp.Vv = s->Vv; kp.epochs = s->epochs; kp.tw_smem = s->tw_smem; kp.shortcuts = s->shortcuts; kp.Rs = (RowSum*)s->Rs; kp.LLF = s->LLF; kp.LLFs = s->LLFs; kp.Cm = s->Cm; kp.Cms = s->Cms;
   kp.P = s->par;
-  kp.abratio = s->par.alpha * rc_log(s->par.beta) - rc_lgamma(s->par.alpha);    // mcmc.jl:17,186,293
-  kp.zgratio = s->par.zeta * rc_log(s->par.gamma) - rc_lgamma(s->par.zeta);     // mcmc.jl:18,187,294
+  kp.abratio = rc_gamma_lognorm(s->par.alpha, s->par.beta);    // mcmc.jl:17,186,293
+  kp.zgratio = rc_gamma_lognorm(s->par.zeta, s->par.gamma);     // mcmc.jl:18,187,294
   kp.lgd1 = rc_lgamma(s->par.delta1);
   kp.lgd2 = rc_lgamma(s->par.delta2);
   kp.LGA = s->LGA; kp.LGZ = s->LGZ; kp.LOGN = s->LOGN;
@@ -669,6 +669,13 @@ const uint8_t* rc_sampler_dev_labels(const rc_sampler* s, int64_t* S, int64_t* n
   if (nchains) *nchains = s->nchains;
   if (device) *device = s->device;
   return s->out_labels;
+}
+
+// internal accessor used by rc_predict.cu: the data, hyperparameters, progress and recorded K / r / p traces of the sampler
+const rc_data* rc_sampler_dev_traces(const rc_sampler* s, rc_params* par, int64_t* iters_done, int64_t* numiters, const int** K,
+                                     const double** r, const double** p) {
+  *par = s->par; *iters_done = s->iters_done; *numiters = s->opt.numiters; *K = s->out_K; *r = s->out_r; *p = s->out_p;
+  return s->d;
 }
 
 }  // extern "C"

@@ -10,6 +10,7 @@
 
 // ---- error plumbing ----------------------------------------------------------------------------
 void rc_set_error(const char* fmt, ...);
+int rc_select_device(int32_t device);   // rc_data.cu
 // Device memory of the long-lived handles comes from the device's stream-ordered pool with a bounded release
 // threshold (32 GB, RCB200_POOL_KEEP_GB): a destroyed handle's gigabytes are reused by the next one instead of going back
 // to the driver (RCB200_NO_POOL=1: plain cudaMalloc / cudaFree).
@@ -65,7 +66,14 @@ struct rc_data {
   double* D;
   longlong2* DL;
   int qD, qL;
+  double mD, mL;        // max |D| over every entry and max |log D| (the diagonal's log is 0): qD, qL are chosen from them
 };
+
+// the domain error of MCMCData(D) and of new-point dissimilarities (their log must be finite for the fixed-point image)
+#define RC_DOMAIN_MSG                                                                                                  \
+  "D must have finite entries and strictly positive off-diagonal dissimilarities: log D must be finite for the "      \
+  "fixed-point image the sampler streams (the reference accepts a zero and carries log D = -Inf, src/types.jl:155). " \
+  "Remove duplicate observations or add a small jitter to them."
 
 #define RC_MAXCAP 128                // default live cluster slots per chain (slot_cap = 0)
 #define RC_MAXCAP_INC 255            // largest slot_cap: labels are bytes, recorded labels are 1-based bytes

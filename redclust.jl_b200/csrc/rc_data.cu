@@ -182,13 +182,12 @@ int finish_data(rc_data* d) {
   rc_dev_free(flags); rc_dev_free(maxbits);
   if (hflags[0]) { rc_set_error("D must be symmetric."); return RC_ERR_NOTSYM; }
   if (hflags[1]) {
-    rc_set_error("D must have finite entries and strictly positive off-diagonal dissimilarities: log D must be finite for the "
-                 "fixed-point image the sampler streams (the reference accepts a zero and carries log D = -Inf, src/types.jl:155). "
-                 "Remove duplicate observations or add a small jitter to them.");
+    rc_set_error(RC_DOMAIN_MSG);
     return RC_ERR_DOMAIN;
   }
   double mD, mL;
   memcpy(&mD, &hbits[0], 8); memcpy(&mL, &hbits[1], 8);
+  d->mD = mD; d->mL = mL;
   d->qD = rc_choose_q(mD, n);
   d->qL = rc_choose_q(mL, n);
   if (d->qD < 0 || d->qL < 0) { rc_set_error("dissimilarities too large for the fixed-point image."); return RC_ERR_DOMAIN; }
@@ -235,7 +234,10 @@ __global__ void __launch_bounds__(256) k_distm_rows(const double* __restrict__ X
   }
 }
 
-int select_device(int32_t device) {
+}  // namespace
+
+// the device of an entry point: fails with RC_ERR_CUDA without one and RC_ERR_ARG out of range
+int rc_select_device(int32_t device) {
   int cnt = 0;
   if (cudaGetDeviceCount(&cnt) != cudaSuccess || cnt == 0) {
     rc_set_error("no CUDA device available (librcb200 has no CPU fallback)");
@@ -245,8 +247,6 @@ int select_device(int32_t device) {
   RC_CUDA(cudaSetDevice(device));
   return RC_OK;
 }
-
-}  // namespace
 
 extern "C" {
 
@@ -258,7 +258,7 @@ int32_t rc_device_count(void) {
 
 int32_t rc_data_from_dist(const double* D, int64_t n, int32_t device, rc_data** out) {
   if (!D || !out || n < 1) { rc_set_error("rc_data_from_dist: null pointer or n < 1"); return RC_ERR_ARG; }
-  int st = select_device(device);
+  int st = rc_select_device(device);
   if (st) return st;
   rc_data* d = new rc_data();
   d->n = n; d->device = device; d->D = nullptr; d->DL = nullptr;
@@ -282,7 +282,7 @@ int32_t rc_data_from_dist(const double* D, int64_t n, int32_t device, rc_data** 
 
 int32_t rc_data_from_points(const double* X, int64_t dim, int64_t n, int32_t device, rc_data** out) {
   if (!X || !out || n < 1 || dim < 1) { rc_set_error("rc_data_from_points: null pointer or empty input"); return RC_ERR_ARG; }
-  int st = select_device(device);
+  int st = rc_select_device(device);
   if (st) return st;
   rc_data* d = new rc_data();
   d->n = n; d->device = device; d->D = nullptr; d->DL = nullptr;
@@ -314,7 +314,7 @@ int32_t rc_data_from_points(const double* X, int64_t dim, int64_t n, int32_t dev
 // caller all-gathers the blocks and hands the complete matrix to rc_data_from_dist_dev.
 int32_t rc_distm_rows_dev(const double* X, int64_t dim, int64_t n, int64_t row0, int64_t nrows, int32_t device, void* D_rows_dev) {
   if (!X || !D_rows_dev || n < 1 || dim < 1 || row0 < 0 || nrows < 0 || row0 + nrows > n) { rc_set_error("rc_distm_rows_dev: bad arguments"); return RC_ERR_ARG; }
-  int st = select_device(device);
+  int st = rc_select_device(device);
   if (st) return st;
   if (nrows == 0) return RC_OK;
   double *dX = nullptr, *sq = nullptr;
@@ -336,7 +336,7 @@ int32_t rc_distm_rows_dev(const double* X, int64_t dim, int64_t n, int64_t row0,
 // MCMCData(D) from a matrix that already lives on the device (same checks and images as rc_data_from_dist).
 int32_t rc_data_from_dist_dev(const void* D_dev, int64_t n, int32_t device, rc_data** out) {
   if (!D_dev || !out || n < 1) { rc_set_error("rc_data_from_dist_dev: null pointer or n < 1"); return RC_ERR_ARG; }
-  int st = select_device(device);
+  int st = rc_select_device(device);
   if (st) return st;
   rc_data* d = new rc_data();
   d->n = n; d->device = device; d->D = nullptr; d->DL = nullptr;

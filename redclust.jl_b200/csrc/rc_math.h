@@ -215,6 +215,10 @@ RC_HD double rc_min0(double x) {
   return x < 0.0 ? x : 0.0;
 }
 
+// shape * log(rate) - lgamma(shape): the log normalising constant of the Gamma(shape, rate) priors of the within- and
+// between-cluster dissimilarities, abratio = (alpha, beta) and zgratio = (zeta, gamma) at /root/reference/src/mcmc.jl:17-18,186-187,293-294.
+RC_HD double rc_gamma_lognorm(double shape, double rate) { return shape * rc_log(rate) - rc_lgamma(shape); }
+
 // ---- fixed-point images of D and log D ------------------------------------------------------
 // Row/cluster sums of D and log D are accumulated as exact 64-bit integers of q-bit fixed-point
 // images (order-independent => identical on CPU and GPU for any tiling).  Block totals for the

@@ -338,6 +338,16 @@ class Sampler:
         check(lib().rc_comm_sampler_psm(comm._h, self._h, ptr(out), None))
         return out
 
+    def predict(self, newdist, chain0=0, nch=None):
+        """predictivecoclustering over the recorded samples of chains chain0 .. chain0 + nch - 1 (chain-major, as
+        samples_all()) without copying them to the host: dict(coclustering = m x n, newcluster = m)."""
+        nch = self.nchains - chain0 if nch is None else nch
+        Dn = _newdist(self.data.n, newdist)
+        m = Dn.shape[0]
+        out = dict(coclustering=np.empty((m, self.data.n)), newcluster=np.empty(m))
+        check(lib().rc_sampler_predict(self._h, ptr(Dn), m, chain0, nch, ptr(out["coclustering"]), ptr(out["newcluster"])))
+        return out
+
     def close(self):
         L = getattr(_lib, "_lib", None)
         if getattr(self, "_h", None) and L is not None:
@@ -480,6 +490,86 @@ def psm(labels, device=0):
     out = np.zeros((L.shape[1], L.shape[1]))
     check(lib().rc_psm(ptr(L), L.shape[0], L.shape[1], device, ptr(out)))
     return out
+
+
+# ---- posterior predictive allocation of new observations (no reference equivalent; the conditional of the full Gibbs
+# scan, mcmc.jl:193-247, for a point that is not in the data, normalised as sample_logweights draws from it, utils.jl:2-6)
+def _newdist(n, newdist):
+    Dn = np.asarray(newdist, dtype=np.float64)
+    if Dn.ndim == 1:
+        Dn = Dn[None, :]
+    if Dn.ndim != 2 or Dn.shape[0] < 1 or Dn.shape[1] != n:
+        raise ArgumentError(f"newdist must be an m × {n} matrix: one row per new point, one column per training point.")
+    return np.ascontiguousarray(Dn)
+
+
+def crossdistances(points, newpoints, device=0):
+    """Euclidean distances of m new points to the n training points (m x n), bit-equal to the rows of the new points in
+    MCMCData.from_points(vstack(points, newpoints)).D -- the `newdist` argument of the predictive calls."""
+    X = np.ascontiguousarray(np.asarray(points, dtype=np.float64))
+    Y = np.ascontiguousarray(np.asarray(newpoints, dtype=np.float64))
+    if Y.ndim == 1:
+        Y = Y[None, :]
+    if X.ndim != 2 or Y.ndim != 2 or X.shape[1] != Y.shape[1] or X.shape[0] < 1 or Y.shape[0] < 1:
+        raise ArgumentError("points and newpoints must be n × dim and m × dim with the same dim.")
+    out = np.empty((Y.shape[0], X.shape[0]))
+    check(lib().rc_crossdist(ptr(X), X.shape[0], ptr(Y), Y.shape[0], X.shape[1], device, ptr(out)))
+    return out
+
+
+def predictive_from_labels(data, newdist, labels, r, p, params, logprobs=False):
+    """The predictive of S label vectors (S x n, any positive labels; each is relabelled by sortlabels) with their r and
+    p: dict(coclustering = m x n, newcluster = m), and with logprobs=True the S x m x 256 un-normalised log-probabilities
+    of the candidate slots (slot k at index k - 1, NaN beyond the last candidate)."""
+    Dn = _newdist(data.n, newdist)
+    L = np.ascontiguousarray(np.asarray(labels, dtype=np.int64).reshape(-1, data.n))
+    S, m = L.shape[0], Dn.shape[0]
+    rr = np.ascontiguousarray(np.asarray(r, dtype=np.float64).reshape(-1))
+    pp = np.ascontiguousarray(np.asarray(p, dtype=np.float64).reshape(-1))
+    if rr.size != S or pp.size != S:
+        raise ArgumentError("r and p must hold one value per sample.")
+    out = dict(coclustering=np.empty((m, data.n)), newcluster=np.empty(m))
+    lp = np.empty((S, m, 256)) if logprobs else None
+    q = params._c()
+    check(lib().rc_predict(data._h, C.byref(q), ptr(Dn), m, ptr(L), ptr(rr), ptr(pp), S, ptr(out["coclustering"]),
+                           ptr(out["newcluster"]), ptr(lp)))
+    if logprobs:
+        out["logprobs"] = lp
+    return out
+
+
+def predictivecoclustering(samples, data, newdist):
+    """Posterior predictive allocation of new observations: for each new point x (row of newdist, m x n dissimilarities to
+    the training points of `data`) coclustering[x, j] is the posterior probability that x joins the cluster of training
+    point j, newcluster[x] that it opens a cluster of its own -- the scan step's conditional (mcmc.jl:193-247) averaged
+    over the samples.  `samples` is an MCMCResult or a list of them (pooled in list order, sampled with the same
+    hyperparameters).  Returns dict(coclustering = m x n, newcluster = m)."""
+    res = list(samples) if isinstance(samples, (list, tuple)) else [samples]
+    if not res:
+        raise ArgumentError("samples must hold at least one MCMCResult.")
+    params = res[0].params
+    for x in res[1:]:
+        if bytes(x.params._c()) != bytes(params._c()):
+            raise ArgumentError("the results to pool were sampled with different hyperparameters.")
+    labs = [np.asarray(c, dtype=np.int64) for x in res for c in x.clusts]
+    if any(c.shape != (data.n,) for c in labs):
+        raise ArgumentError(f"the samples must label the {data.n} points of data.")
+    L = np.stack(labs) if labs else np.zeros((0, data.n), np.int64)
+    r = np.concatenate([np.asarray(x.r, dtype=np.float64) for x in res])
+    p = np.concatenate([np.asarray(x.p, dtype=np.float64) for x in res])
+    return predictive_from_labels(data, newdist, L, r, p, params)
+
+
+def allocationprobabilities(data, newdist, clusts, r, p, params):
+    """Allocation probabilities of new points for one partition `clusts` (such as a point estimate) with its r and p:
+    m x (K + 1), column k for the k-th distinct label in ascending order, the last column for a new cluster (0 when maxK
+    leaves no room for one).  These are the kernel's probabilities of the one-sample predictive."""
+    c = np.asarray(clusts, dtype=np.int64)
+    if c.shape != (data.n,):
+        raise ArgumentError(f"clusts must label the {data.n} points of data.")
+    out = predictive_from_labels(data, newdist, c[None, :], [r], [p], params)
+    _, first = np.unique(c, return_index=True)
+    return np.column_stack([out["coclustering"][:, first], out["newcluster"]])
 
 
 _LOSS = {"binder": 0, "omARI": 1, "VI": 2, "ID": 3}

@@ -248,6 +248,58 @@ function sample_rp(clustsizes::Vector{Int}, options::MCMCOptionsList = MCMCOptio
     return (r = r, p = p)
 end
 
+# ---- posterior predictive allocation of new observations (no reference equivalent): the conditional of the full Gibbs
+# scan (src/mcmc.jl:193-247) for a point that is not in the data, normalised as sample_logweights draws from it
+# (src/utils.jl:2-6), averaged over the samples.  newdist is m x n (a row per new point); the C side is row-major.
+
+"Euclidean distances (m x n) of new points to the training points, bit-equal to the stacked MCMCData(points) rows."
+function crossdistances(pnts::AbstractVector{<:AbstractVector{<:Float64}}, newpnts::AbstractVector{<:AbstractVector{<:Float64}}; device::Integer = 0)
+    dim = length(pnts[1])
+    all(length(v) == dim for v in newpnts) || throw(ArgumentError("points and newpoints must have the same dimension."))
+    X = [pnts[i][j] for j in 1:dim, i in 1:length(pnts)]          # dim x n column-major = n x dim row-major
+    Y = [newpnts[i][j] for j in 1:dim, i in 1:length(newpnts)]
+    out = Matrix{Float64}(undef, length(pnts), length(newpnts))   # n x m column-major = m x n row-major
+    GC.@preserve X Y check(ccall((:rc_crossdist, LIB[]), Int32, (Ptr{Float64}, Int64, Ptr{Float64}, Int64, Int64, Int32, Ptr{Float64}),
+                                 X, length(pnts), Y, length(newpnts), dim, device, out))
+    return permutedims(out)
+end
+
+function _predict(data::MCMCData, newdist::AbstractMatrix{Float64}, clusts::Vector{<:AbstractVector{<:Integer}},
+                  r::Vector{Float64}, p::Vector{Float64}, params::PriorHyperparamsList)
+    n = getfield(data, :n); m = size(newdist, 1); S = length(clusts)
+    size(newdist, 2) == n || throw(ArgumentError("newdist must be an m × $n matrix: one row per new point, one column per training point."))
+    all(length(c) == n for c in clusts) || throw(ArgumentError("the samples must label the $n points of data."))
+    Dt = Matrix{Float64}(permutedims(newdist))                     # n x m column-major = m x n row-major
+    L = Matrix{Int64}(undef, n, S)
+    for s in 1:S; L[:, s] .= clusts[s]; end
+    cocl = Matrix{Float64}(undef, n, m); newcl = Vector{Float64}(undef, m)
+    GC.@preserve Dt L r p check(ccall((:rc_predict, LIB[]), Int32,
+        (Ptr{Cvoid}, Ref{rc_params}, Ptr{Float64}, Int64, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+        getfield(data, :handle), rc_params(params), Dt, m, L, r, p, S, cocl, newcl, C_NULL))
+    return (coclustering = permutedims(cocl), newcluster = newcl)
+end
+
+"""
+    predictivecoclustering(samples, data, newdist) -> (coclustering = m x n, newcluster = m)
+
+coclustering[x, j]: posterior probability that new point x joins the cluster of training point j; newcluster[x]: that
+it opens a cluster of its own.  `samples` is an MCMCResult or a vector of them sampled with the same hyperparameters.
+"""
+function predictivecoclustering(samples::Union{MCMCResult,Vector{MCMCResult}}, data::MCMCData, newdist::AbstractMatrix{Float64})
+    res = samples isa MCMCResult ? [samples] : samples
+    isempty(res) && throw(ArgumentError("samples must hold at least one MCMCResult."))
+    all(x.params == res[1].params for x in res) || throw(ArgumentError("the results to pool were sampled with different hyperparameters."))
+    return _predict(data, newdist, [c for x in res for c in x.clusts], vcat([x.r for x in res]...), vcat([x.p for x in res]...), res[1].params)
+end
+
+"Allocation probabilities (m x (K + 1)) of new points for one partition: column k for the k-th distinct label in ascending order, the last for a new cluster."
+function allocationprobabilities(data::MCMCData, newdist::AbstractMatrix{Float64}, clusts::AbstractVector{<:Integer}, r::Float64, p::Float64,
+                                 params::PriorHyperparamsList)
+    out = _predict(data, newdist, [clusts], [r], [p], params)
+    first = [findfirst(==(u), clusts) for u in sort(unique(clusts))]
+    return hcat(out.coclustering[:, first], out.newcluster)
+end
+
 function getpointestimate(samples::MCMCResult; method::String = "MAP", loss::Union{String,Function} = "VI")
     if method == "MPEL" && loss isa String && loss ∉ ["binder", "omARI", "VI", "ID"]
         throw(ArgumentError("Invalid loss function specifier."))
