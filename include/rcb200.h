@@ -224,6 +224,16 @@ int32_t rc_mpel(const int64_t* labels, int64_t S, int64_t n, int32_t loss, int32
 int32_t rc_mpel_rows_dev(const int64_t* labels, int64_t S, int64_t n, int32_t loss, int32_t device, int64_t row_first,
                          int64_t row_stride, int64_t nrows, void* M_rows_dev);
 int32_t rc_mpel_finish_dev(const void* M_upper_dev, int64_t S, int32_t device, double* loss_sums, int64_t* best);
+/* MPEL with the Binder loss over pooled samples, from the co-clustering counts N alone (src/pointestimate.jl:34-59,68-76,
+ * counts of src/mcmc.jl:560): with P_s = sum_k C(n_k, 2) and W_s = sum_{a<b} N_ab [c_s(a) == c_s(b)], the disagreeing pairs
+ * of sample s summed over every sample t are T_s = S P_s + sum_t P_t - 2 W_s, an exact integer.  loss_sums[s] = T_s / C(n, 2)
+ * (rc_mpel's binder column sums up to its fp64 rounding), *best = first argmin of T (0-based), totals[s] = T_s.  O(S n^2)
+ * work and no S x S matrix.  Needs 1 <= S < 2^31 and n <= 65 535.  loss_sums, best and totals may each be NULL.       */
+int32_t rc_binder_mpel(const int64_t* labels, int64_t S, int64_t n, int32_t device, double* loss_sums, int64_t* best, int64_t* totals);
+/* The same over the device-resident samples of chains [chain0, chain0 + nch) (chain-major, sample-minor: *best indexes
+ * them in that order); nothing is copied to the host.  RC_ERR_STATE before a run to numiters, RC_ERR_SLOTS when a chain
+ * of the range stopped at the slot capacity, RC_ERR_ARG for a bad range.                                                */
+int32_t rc_sampler_binder_mpel(const rc_sampler* s, int64_t chain0, int64_t nch, double* loss_sums, int64_t* best, int64_t* totals);
 
 /* ---- multi-GPU exchange steps (SURVEY.md 8e) -------------------------------------------------------
  * One process per GPU.  The sampler needs no collective (independent chains: chain_offset above).  The three steps
@@ -234,6 +244,9 @@ int32_t rc_mpel_finish_dev(const void* M_upper_dev, int64_t S, int32_t device, d
  *   rc_comm_sampler_psm       src/mcmc.jl:560 over the chains of every rank: int32 counts + ONE all-reduce + divide
  *   rc_comm_psm               the same for host label vectors sharded over the ranks (S_local of them on this rank)
  *   rc_comm_mpel              src/pointestimate.jl:49-57 with the candidate rows dealt cyclically + all-gather
+ *   rc_comm_sampler_binder_mpel  src/pointestimate.jl:34-59,68-76 over the chains of every rank (src/mcmc.jl:560): the
+ *                             all-reduced counts, per-rank int64 W and P, ONE all-gather; every rank gets T over all
+ *                             samples in rank order (= global chain order; *best indexes that concatenation)
  * psm_out (host, n x n fp64) and counts_dev_out (device, n x n int32) may each be NULL.  Results are bit-equal to the
  * single-GPU entry points.                                                                              */
 typedef struct rc_comm rc_comm;
@@ -246,6 +259,7 @@ int32_t rc_comm_data_from_points(rc_comm* c, const double* X, int64_t dim, int64
 int32_t rc_comm_sampler_psm(rc_comm* c, const rc_sampler* s, double* psm_out, void* counts_dev_out);
 int32_t rc_comm_psm(rc_comm* c, const int64_t* labels, int64_t S_local, int64_t n, double* psm_out, void* counts_dev_out);
 int32_t rc_comm_mpel(rc_comm* c, const int64_t* labels, int64_t S, int64_t n, int32_t loss, double* loss_sums, int64_t* best);
+int32_t rc_comm_sampler_binder_mpel(rc_comm* c, const rc_sampler* s, double* loss_sums, int64_t* best, int64_t* totals);
 
 #ifdef __cplusplus
 }

@@ -81,6 +81,8 @@ SIGNATURES = {
     "rc_mpel": (C.c_int32, [_vp, C.c_int64, C.c_int64, C.c_int32, C.c_int32, _vp, _P(C.c_int64)]),
     "rc_mpel_rows_dev": (C.c_int32, [_vp, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int64, _vp]),
     "rc_mpel_finish_dev": (C.c_int32, [_vp, C.c_int64, C.c_int32, _vp, _P(C.c_int64)]),
+    "rc_binder_mpel": (C.c_int32, [_vp, C.c_int64, C.c_int64, C.c_int32, _vp, _P(C.c_int64), _vp]),
+    "rc_sampler_binder_mpel": (C.c_int32, [_vp, C.c_int64, C.c_int64, _vp, _P(C.c_int64), _vp]),
     "rc_comm_unique_id": (C.c_int32, [_vp]),
     "rc_comm_init": (C.c_int32, [_vp, C.c_int32, C.c_int32, C.c_int32, _P(_vp)]),
     "rc_comm_info": (C.c_int32, [_vp, _P(C.c_int32), _P(C.c_int32)]),
@@ -90,6 +92,7 @@ SIGNATURES = {
     "rc_comm_sampler_psm": (C.c_int32, [_vp, _vp, _vp, _vp]),
     "rc_comm_psm": (C.c_int32, [_vp, _vp, C.c_int64, C.c_int64, _vp, _vp]),
     "rc_comm_mpel": (C.c_int32, [_vp, _vp, C.c_int64, C.c_int64, C.c_int32, _vp, _P(C.c_int64)]),
+    "rc_comm_sampler_binder_mpel": (C.c_int32, [_vp, _vp, _vp, _P(C.c_int64), _vp]),
 }
 
 

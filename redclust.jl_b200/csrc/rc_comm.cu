@@ -227,6 +227,63 @@ int32_t rc_comm_psm(rc_comm* c, const int64_t* labels, int64_t S_local, int64_t 
   return st;
 }
 
+// Binder MPEL over the samples of every rank (src/pointestimate.jl:34-59,68-76 with the counts of src/mcmc.jl:560): the
+// all-reduced counts of rc_comm_sampler_psm, W and P of this rank's samples, ONE all-gather of the per-rank int64 vectors
+// (padded to the largest rank), and the totals over all samples in rank order.  Integers throughout: identical to one
+// GPU over the same chains.  Every rank first learns whether any rank refuses, so none is left waiting in a collective.
+int32_t rc_comm_sampler_binder_mpel(rc_comm* c, const rc_sampler* s, double* loss_sums, int64_t* best, int64_t* totals) {
+  if (!c || !s) { rc_set_error("rc_comm_sampler_binder_mpel: null handle"); return RC_ERR_ARG; }
+  RC_CUDA(cudaSetDevice(c->device));
+  const int64_t n = rc_sampler_n(s), nch = rc_sampler_nchains(s), R = nch * rc_sampler_numsamples(s);
+  const int local = rc_sampler_binder_check(s, 0, nch, "rc_comm_sampler_binder_mpel");
+  const std::string why = local ? rc_last_error() : "";
+  long long* info = nullptr;                                   // per rank: {status, samples}
+  RC_CUDA(cudaMalloc(&info, sizeof(long long) * 2 * (c->world + 1)));
+  const long long mine[2] = {local, (long long)R};
+  std::vector<long long> all(2 * (size_t)c->world);
+  cudaError_t e = cudaMemcpy(info, mine, sizeof(mine), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess && nccl()->AllGather(info, info + 2, 2, ncclInt64, c->comm, c->stream) != ncclSuccess) e = cudaErrorUnknown;
+  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+  if (e == cudaSuccess) e = cudaMemcpy(all.data(), info + 2, sizeof(long long) * 2 * c->world, cudaMemcpyDeviceToHost);
+  cudaFree(info);
+  if (e != cudaSuccess) { rc_set_error("rc_comm_sampler_binder_mpel: exchange of the sample counts failed"); return RC_ERR_CUDA; }
+  int64_t total = 0, per = 0;
+  for (int r = 0; r < c->world; ++r) {
+    if (all[2 * r] != 0) {
+      if (local) { rc_set_error("%s", why.c_str()); return local; }
+      rc_set_error("rc_comm_sampler_binder_mpel: rank %d refused (status %lld)", r, all[2 * r]);
+      return (int32_t)all[2 * r];
+    }
+    total += all[2 * r + 1];
+    per = std::max<int64_t>(per, all[2 * r + 1]);
+  }
+  if (total >= ((int64_t)1 << 31)) { rc_set_error("rc_comm_sampler_binder_mpel: %lld samples in all; needs < 2^31", (long long)total); return RC_ERR_ARG; }
+  int* counts = nullptr;
+  unsigned long long* buf = nullptr;                           // [world + 1][2 per]: this rank's {W, P}, then the gathered ranks
+  RC_CUDA(cudaMalloc(&counts, sizeof(int) * (size_t)n * n));
+  if (cudaMalloc(&buf, sizeof(unsigned long long) * 2 * (size_t)per * (c->world + 1)) != cudaSuccess) {
+    cudaFree(counts); rc_set_error("rc_comm_sampler_binder_mpel: out of device memory"); return RC_ERR_CUDA;
+  }
+  std::vector<unsigned long long> wp(2 * (size_t)per, 0ull), gathered(2 * (size_t)per * c->world);
+  int st = rc_comm_sampler_psm(c, s, nullptr, counts);
+  if (!st) st = rc_sampler_binder_wp(s, 0, nch, counts, total, wp.data(), wp.data() + per);
+  if (!st && cudaMemcpy(buf, wp.data(), sizeof(unsigned long long) * 2 * per, cudaMemcpyHostToDevice) != cudaSuccess) st = RC_ERR_CUDA;
+  if (!st && (nccl()->AllGather(buf, buf + 2 * per, 2 * (size_t)per, ncclInt64, c->comm, c->stream) != ncclSuccess ||
+              cudaStreamSynchronize(c->stream) != cudaSuccess ||
+              cudaMemcpy(gathered.data(), buf + 2 * per, sizeof(unsigned long long) * gathered.size(), cudaMemcpyDeviceToHost) != cudaSuccess)) {
+    rc_set_error("rc_comm_sampler_binder_mpel: all-gather of the per-rank totals failed"); st = RC_ERR_CUDA;
+  }
+  cudaFree(counts); cudaFree(buf);
+  if (st) return st;
+  std::vector<unsigned long long> W, P;                        // rank order = global chain order
+  for (int r = 0; r < c->world; ++r) {
+    const unsigned long long* g = gathered.data() + 2 * (size_t)per * r;
+    W.insert(W.end(), g, g + all[2 * r + 1]);
+    P.insert(P.end(), g + per, g + per + all[2 * r + 1]);
+  }
+  return rc_binder_finish(W.data(), P.data(), total, n, loss_sums, best, totals);
+}
+
 // MPEL search with the candidate samples dealt cyclically over the ranks (src/pointestimate.jl:49-57): every rank holds
 // all S label vectors, evaluates rows rank, rank + world, ... of the upper triangle of the loss matrix, one all-gather
 // assembles it, the column sums run in ascending row order -- bit-equal to rc_mpel on one GPU.

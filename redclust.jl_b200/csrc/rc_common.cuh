@@ -30,6 +30,13 @@ void rc_dev_free(void* p);
 int rc_distm_dmma(const double* X_dev, int64_t dim, int64_t n, int64_t row0, int64_t nrows, double* D_dev);
 // int32 co-clustering counts on the device -> host fp64 counts / denom (rc_post.cu)
 int rc_counts_to_host_psm(const int* counts, size_t total, double denom, double* out);
+// posterior expected Binder loss from the counts (rc_post.cu): the sampler-range checks, W and P of a chain range against
+// counts of at most nmax samples, and the exact totals T_s = S P_s + sum_t P_t - 2 W_s with their first argmin
+int rc_sampler_binder_check(const rc_sampler* s, int64_t chain0, int64_t nch, const char* who);
+int rc_sampler_binder_wp(const rc_sampler* s, int64_t chain0, int64_t nch, const int* counts, int64_t nmax, unsigned long long* W,
+                         unsigned long long* P);
+int rc_binder_finish(const unsigned long long* W, const unsigned long long* P, int64_t S, int64_t n, double* loss_sums,
+                     int64_t* best, int64_t* totals);
 
 // ---- 128-bit two's complement accumulators (block totals of the fixed-point images) ------------
 struct rc_i128 {

@@ -3,6 +3,8 @@
 //   MPEL  lossmatrix[i,j] = lossfn(c_i, c_j), argmin of column sums   /root/reference/src/pointestimate.jl:34-59
 //         binder = randindex[3] (Mirkin), omARI = 1 - randindex[1], VI = varinfo, ID = max(H) - I
 //         (Clustering.jl randindex / varinfo / mutualinfo, restated from their contingency-table definitions)
+//   Binder MPEL over pooled samples   the same argmin for binderloss (pointestimate.jl:68-76) from the counts alone:
+//         O(S n^2) compares, no S x S matrix (k_binder_w, k_binder_pairs, rc_binder_finish)
 // The reference materialises S dense n x n Bool matrices; here the label matrix is transposed once
 // (point-major, samples contiguous) and co-clustering counts are byte-compare popcounts -- exact integers.
 #include <vector>
@@ -20,6 +22,8 @@ int rc_psm_counts_tc(const uint8_t* Lt, int64_t n, int64_t Rpad, int64_t R, int 
 double rc_psm_tc_macs(int64_t n, int64_t R, int kmax);
 
 extern "C" const uint8_t* rc_sampler_dev_labels(const rc_sampler* s, int64_t* S, int64_t* n, int64_t* nchains, int* device);
+extern "C" const rc_data* rc_sampler_dev_traces(const rc_sampler* s, rc_params* par, int64_t* iters_done, int64_t* numiters, const int** K,
+                                                const double** r, const double** p);
 
 namespace {
 
@@ -108,9 +112,109 @@ __global__ void k_maxlabel(const uint8_t* __restrict__ L, size_t total, int* __r
   if ((threadIdx.x & 31) == 0 && m) atomicMax(out, (int)m);
 }
 
+// ---- Binder MPEL over pooled samples ---------------------------------------------------------------
+// W_s = sum_{a<b} N_ab [c_s(a) == c_s(b)] for every sample s, N the co-clustering counts.  One CTA per 64 x 64 tile
+// (i, j >= i) of point pairs stages its N tile in shared memory (zero where a pair is not counted: a >= b, or outside n),
+// then walks 128-sample chunks of the transposed labels: lane l holds the 32-bit word of samples 4l..4l+3, warp g the
+// tile's points a = 8g..8g+7 against every b.  A byte-equality mask of the a- and b-words selects which of the four
+// per-sample accumulators N_ab goes to.
+//
+// Exactness: every N_ab <= nmax (the samples behind the counts).  Per chunk a thread adds at most 8 x 64 = 512 values
+// into each accumulator, so Acc = uint32 is exact for nmax < 2^23 (512 * nmax < 2^32); beyond that Acc = uint64
+// (512 * 2^31 = 2^40).  A CTA's sum over its 8 warps is at most 4096 * nmax < 2^43 and is added once per (CTA, chunk,
+// sample) into the uint64 W_s, which never exceeds C(n, 2) * nmax < 2^31 * 2^31 = 2^62 for n <= 65 535 and nmax < 2^31.
+// Integer adds commute, so W does not depend on the tiling, the grid or the order of the atomics.
+#define BT 64   // points per tile side
+#define BW 32   // label words (128 samples) per chunk, one per lane
+
+__device__ __forceinline__ unsigned eq_mask(unsigned a, unsigned b) {   // 0x80 in every byte where a and b agree
+  const unsigned x = a ^ b;
+  return ~(((x & 0x7f7f7f7fu) + 0x7f7f7f7fu) | x) & 0x80808080u;
+}
+
+template <typename Acc>
+__global__ void __launch_bounds__(256) k_binder_w(const uint8_t* __restrict__ Lt, int64_t n, int64_t Rpad, int64_t R,
+                                                  const int* __restrict__ counts, unsigned long long* __restrict__ W) {
+  const int bi = blockIdx.y, bj = blockIdx.x;
+  if (bj < bi) return;
+  __shared__ __align__(16) int Ns[BT][BT];                 // Ns[b][a] = N(i0 + a, j0 + b) or 0
+  __shared__ unsigned A[BT][BW], B[BT][BW];
+  __shared__ unsigned long long red[8][4 * BW];
+  const int lane = threadIdx.x & 31, g = threadIdx.x >> 5;
+  const int64_t i0 = (int64_t)bi * BT, j0 = (int64_t)bj * BT;
+  for (int q = threadIdx.x; q < BT * BT; q += 256) {
+    const int b = q / BT, a = q % BT;
+    const int64_t i = i0 + a, j = j0 + b;
+    Ns[b][a] = (i < j && j < n) ? counts[j * n + i] : 0;
+  }
+  const int64_t words = Rpad / 4, nchunk = (words + BW - 1) / BW;
+  const unsigned* Lw = reinterpret_cast<const unsigned*>(Lt);
+  for (int64_t c = blockIdx.z; c < nchunk; c += gridDim.z) {
+    const int64_t w0 = c * BW;
+    __syncthreads();                                       // Ns written; the previous chunk is done with A, B, red
+    for (int q = threadIdx.x; q < BT * BW; q += 256) {
+      const int row = q / BW, w = q % BW;
+      const bool okw = w0 + w < words;
+      A[row][w] = (okw && i0 + row < n) ? Lw[(i0 + row) * words + w0 + w] : 0u;
+      B[row][w] = (okw && j0 + row < n) ? Lw[(j0 + row) * words + w0 + w] : 0u;
+    }
+    __syncthreads();
+    unsigned la[8];
+#pragma unroll
+    for (int q = 0; q < 8; ++q) la[q] = A[8 * g + q][lane];
+    Acc acc[4] = {0, 0, 0, 0};
+#pragma unroll 2
+    for (int b = 0; b < BT; ++b) {
+      const unsigned lb = B[b][lane];
+      const int4 n0 = *reinterpret_cast<const int4*>(&Ns[b][8 * g]), n1 = *reinterpret_cast<const int4*>(&Ns[b][8 * g + 4]);
+      const unsigned nv[8] = {(unsigned)n0.x, (unsigned)n0.y, (unsigned)n0.z, (unsigned)n0.w,
+                              (unsigned)n1.x, (unsigned)n1.y, (unsigned)n1.z, (unsigned)n1.w};
+#pragma unroll
+      for (int q = 0; q < 8; ++q) {
+        const unsigned m = eq_mask(la[q], lb) >> 7;        // 1 in every byte where the labels agree
+#pragma unroll
+        for (int k = 0; k < 4; ++k) acc[k] += (Acc)nv[q] * __byte_perm(m, 0u, 0x4440u + k);   // byte k of m, as 0 or 1
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) red[g][4 * lane + k] = acc[k];
+    __syncthreads();
+    if (threadIdx.x < 4 * BW) {
+      const int64_t s = 4 * w0 + threadIdx.x;              // byte k of word w holds sample 4w + k
+      unsigned long long v = 0;
+#pragma unroll
+      for (int q = 0; q < 8; ++q) v += red[q][threadIdx.x];
+      if (s < R && v) atomicAdd(&W[s], v);
+    }
+  }
+}
+
+// P_s = sum_k C(n_k, 2) from the label histogram of sample s (L sample-major, any byte labels); one CTA per sample.
+__global__ void __launch_bounds__(256) k_binder_pairs(const uint8_t* __restrict__ L, int64_t n, unsigned long long* __restrict__ P) {
+  __shared__ unsigned h[256];
+  __shared__ unsigned long long part[8];
+  const uint8_t* l = L + (int64_t)blockIdx.x * n;
+  h[threadIdx.x] = 0;
+  __syncthreads();
+  for (int64_t x = threadIdx.x; x < n; x += 256) atomicAdd(&h[l[x]], 1u);
+  __syncthreads();
+  const unsigned long long c = h[threadIdx.x];
+  unsigned long long v = c ? c * (c - 1) / 2 : 0;
+  for (int off = 16; off; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = v;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned long long t = 0;
+    for (int q = 0; q < 8; ++q) t += part[q];
+    P[blockIdx.x] = t;
+  }
+}
+
 // Co-clustering counts of R label vectors (device, sample-major).  Default: the tensor-core kernel of
 // rc_psm_tc.cu (labels up to 128); RCB200_PSM=compare or more labels: the byte-compare kernel.  Both are exact.
-int psm_counts_device(const uint8_t* L, int64_t R, int64_t n, int* counts) {
+// Lt_keep (may be NULL) receives the transposed labels (n x Rpad, Rpad = R rounded up to 64, filler 0), which the
+// caller then frees.
+int psm_counts_device(const uint8_t* L, int64_t R, int64_t n, int* counts, uint8_t** Lt_keep = nullptr) {
   const int64_t Rpad = (R + 63) & ~63LL;
   uint8_t* Lt = nullptr; int* dmax = nullptr;
   RC_CUDA(cudaMalloc(&Lt, (size_t)n * Rpad));
@@ -143,8 +247,50 @@ int psm_counts_device(const uint8_t* L, int64_t R, int64_t n, int* counts) {
             (long long)n, (long long)R, kmax, tc ? "tcgen05-i8" : "byte-compare", ms, (double)n * n * R / (ms * 1e-3), 2 * macs / (ms * 1e-3) * 1e-12);
     cudaEventDestroy(e0); cudaEventDestroy(e1);
   }
-  cudaFree(Lt);
+  if (Lt_keep && !st && e == cudaSuccess) *Lt_keep = Lt;
+  else cudaFree(Lt);
   if (st) return st;
+  RC_CUDA(e);
+  return RC_OK;
+}
+
+// Binder totals of R device label vectors (sample-major L, transposed Lt as psm_counts_device keeps it, or NULL to
+// transpose here) against co-clustering counts of at most nmax samples: W (uint64 per sample) and P (C(n_k, 2) summed
+// per sample) to the host.  w_ms (may be NULL): the W kernel's time, CUDA events.
+static int binder_wp(const uint8_t* L, const uint8_t* Lt, int64_t R, int64_t n, const int* counts, int64_t nmax,
+                     unsigned long long* W_out, unsigned long long* P_out, float* w_ms) {
+  const int64_t Rpad = (R + 63) & ~63LL;
+  uint8_t* own = nullptr;
+  unsigned long long *W = nullptr, *P = nullptr;
+  if (!Lt) {
+    RC_CUDA(cudaMalloc(&own, (size_t)n * Rpad));
+    dim3 tb(32, 8), tg((unsigned)((n + 31) / 32), (unsigned)((Rpad + 31) / 32));
+    k_transpose<<<tg, tb>>>(L, R, n, Rpad, own);
+    Lt = own;
+  }
+  cudaError_t e = cudaMalloc(&W, sizeof(unsigned long long) * (size_t)R);
+  if (e == cudaSuccess) e = cudaMalloc(&P, sizeof(unsigned long long) * (size_t)R);
+  if (e == cudaSuccess) e = cudaMemset(W, 0, sizeof(unsigned long long) * (size_t)R);
+  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  if (e == cudaSuccess && w_ms) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, 0); }
+  if (e == cudaSuccess) {
+    const unsigned nb = (unsigned)((n + BT - 1) / BT);
+    const int64_t tiles = (int64_t)nb * (nb + 1) / 2, nchunk = (Rpad / 4 + BW - 1) / BW;
+    // enough CTAs to fill the device several times; beyond that a CTA walks more chunks and reuses its N tile
+    const unsigned gz = (unsigned)std::min<int64_t>({nchunk, 65535, std::max<int64_t>(1, (148 * 16 + tiles - 1) / tiles)});
+    const dim3 grid(nb, nb, gz);
+    if (nmax < ((int64_t)1 << 23)) k_binder_w<unsigned><<<grid, 256>>>(Lt, n, Rpad, R, counts, W);
+    else k_binder_w<unsigned long long><<<grid, 256>>>(Lt, n, Rpad, R, counts, W);
+    if (w_ms) cudaEventRecord(e1, 0);
+    k_binder_pairs<<<(unsigned)R, 256>>>(L, n, P);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaDeviceSynchronize();
+  if (e == cudaSuccess && w_ms) cudaEventElapsedTime(w_ms, e0, e1);
+  if (e0) { cudaEventDestroy(e0); cudaEventDestroy(e1); }
+  if (e == cudaSuccess) e = cudaMemcpy(W_out, W, sizeof(unsigned long long) * (size_t)R, cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess) e = cudaMemcpy(P_out, P, sizeof(unsigned long long) * (size_t)R, cudaMemcpyDeviceToHost);
+  cudaFree(W); cudaFree(P); cudaFree(own);
   RC_CUDA(e);
   return RC_OK;
 }
@@ -368,6 +514,121 @@ int32_t rc_psm(const int64_t* labels, int64_t S, int64_t n, int32_t device, doub
   cudaFree(dL); cudaFree(counts);
   if (verbose) fprintf(stderr, "[rcb200] rc_psm: relabel %.3f s, upload + counts %.3f s, download + divide %.3f s\n", t1 - t0, t2 - t1, now() - t2);
   return st;
+}
+
+}  // extern "C"
+
+// ---- posterior expected Binder loss of every sample from the co-clustering counts -------------------------------------
+// The reference's MPEL (src/pointestimate.jl:34-59) with binderloss (:68-76, the Mirkin count of disagreeing pairs over
+// C(n, 2)) sums, for candidate s, the disagreeing pairs of s and every sample t.  With P_s = sum_k C(n_k, 2) and
+// W_s = sum_{a<b} N_ab [c_s(a) == c_s(b)] (N the counts of src/mcmc.jl:560), that sum is exactly
+//   T_s = S * P_s + sum_t P_t - 2 W_s
+// (a pair together in s and apart in t, or apart in s and together in t).  Everything is an integer: T_s < 2^63 for
+// S < 2^31 and n <= 65 535.  loss_sums[s] = T_s / C(n, 2) (one rounding), best = first argmin of T.
+
+int rc_binder_finish(const unsigned long long* W, const unsigned long long* P, int64_t S, int64_t n, double* loss_sums,
+                     int64_t* best, int64_t* totals) {
+  unsigned long long sumP = 0;
+  for (int64_t s = 0; s < S; ++s) sumP += P[s];
+  const double pairs = (double)(n * (n - 1) / 2);
+  int64_t b = 0;
+  unsigned long long tb = 0;
+  for (int64_t s = 0; s < S; ++s) {
+    const unsigned long long t = (unsigned long long)S * P[s] + sumP - 2 * W[s];
+    if (s == 0 || t < tb) { tb = t; b = s; }
+    if (loss_sums) loss_sums[s] = (double)t / pairs;
+    if (totals) totals[s] = (int64_t)t;
+  }
+  if (best) *best = b;
+  return RC_OK;
+}
+
+int rc_binder_check_args(int64_t S, int64_t n, const char* who) {
+  if (S < 1 || S >= ((int64_t)1 << 31) || n < 1 || n > 65535) {
+    rc_set_error("%s: needs 1 <= samples < 2^31 and 1 <= n <= 65535 (S = %lld, n = %lld)", who, (long long)S, (long long)n);
+    return RC_ERR_ARG;
+  }
+  return RC_OK;
+}
+
+// The sampler's samples of chains [chain0, chain0 + nch) exist only after a run to numiters, and not for a chain that
+// stopped at the slot capacity (the rules of rc_sampler_predict).
+int rc_sampler_binder_check(const rc_sampler* s, int64_t chain0, int64_t nch, const char* who) {
+  int64_t S, n, nchains; int device;
+  rc_sampler_dev_labels(s, &S, &n, &nchains, &device);
+  if (chain0 < 0 || nch < 1 || chain0 + nch > nchains) { rc_set_error("%s: bad chain range", who); return RC_ERR_ARG; }
+  rc_params par; const int* K; const double *r, *p; int64_t done, numiters;
+  rc_sampler_dev_traces(s, &par, &done, &numiters, &K, &r, &p);
+  if (done < numiters) {
+    rc_set_error("%s: the sampler ran %lld of %lld iterations; its samples are recorded only by a complete run", who, (long long)done,
+                 (long long)numiters);
+    return RC_ERR_STATE;
+  }
+  for (int64_t c = chain0; c < chain0 + nch; ++c)
+    if (rc_sampler_chain_status(s, c) != 0) {
+      rc_set_error("%s: chain %lld stopped at the slot capacity; its samples are incomplete", who, (long long)c);
+      return RC_ERR_SLOTS;
+    }
+  return rc_binder_check_args(nch * S, n, who);
+}
+
+// W and P of the device-resident samples of chains [chain0, chain0 + nch) against counts of at most nmax samples.
+int rc_sampler_binder_wp(const rc_sampler* s, int64_t chain0, int64_t nch, const int* counts, int64_t nmax, unsigned long long* W,
+                         unsigned long long* P) {
+  int64_t S, n, nchains; int device;
+  const uint8_t* L = rc_sampler_dev_labels(s, &S, &n, &nchains, &device);
+  RC_CUDA(cudaSetDevice(device));
+  return binder_wp(L + (size_t)chain0 * S * n, nullptr, nch * S, n, counts, nmax, W, P, nullptr);
+}
+
+// counts, W, P and the totals of R device label vectors (sample-major, bytes)
+static int binder_device(const uint8_t* L, int64_t R, int64_t n, double* loss_sums, int64_t* best, int64_t* totals) {
+  int* counts = nullptr; uint8_t* Lt = nullptr;
+  RC_CUDA(cudaMalloc(&counts, sizeof(int) * (size_t)n * n));
+  const bool verbose = getenv("RCB200_VERBOSE") != nullptr;
+  auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+  const double t0 = now();
+  int st = psm_counts_device(L, R, n, counts, &Lt);
+  const double t1 = now();
+  std::vector<unsigned long long> W((size_t)R), P((size_t)R);
+  float w_ms = 0;
+  if (!st) st = binder_wp(L, Lt, R, n, counts, R, W.data(), P.data(), &w_ms);
+  cudaFree(Lt); cudaFree(counts);
+  if (st) return st;
+  if (verbose)
+    fprintf(stderr, "[rcb200] binder mpel: n=%lld samples=%lld counts %.3f ms, W kernel %.3f ms (CUDA events), %.3e pair-samples/s\n",
+            (long long)n, (long long)R, (t1 - t0) * 1e3, w_ms, 0.5 * (double)n * (double)(n - 1) * (double)R / (w_ms * 1e-3));
+  return rc_binder_finish(W.data(), P.data(), R, n, loss_sums, best, totals);
+}
+
+extern "C" {
+
+int32_t rc_binder_mpel(const int64_t* labels, int64_t S, int64_t n, int32_t device, double* loss_sums, int64_t* best, int64_t* totals) {
+  if (!labels) { rc_set_error("rc_binder_mpel: null pointer"); return RC_ERR_ARG; }
+  int st = rc_binder_check_args(S, n, "rc_binder_mpel");
+  if (st) return st;
+  st = rc_select_device(device);
+  if (st) return st;
+  std::vector<uint8_t> L; std::vector<int> K;
+  st = compact_labels(labels, S, n, L, K);
+  if (st) return st;
+  uint8_t* dL = nullptr;
+  RC_CUDA(cudaMalloc(&dL, L.size()));
+  cudaError_t e = cudaMemcpy(dL, L.data(), L.size(), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) st = binder_device(dL, S, n, loss_sums, best, totals);
+  cudaFree(dL);
+  RC_CUDA(e);
+  return st;
+}
+
+int32_t rc_sampler_binder_mpel(const rc_sampler* s, int64_t chain0, int64_t nch, double* loss_sums, int64_t* best, int64_t* totals) {
+  if (!s) { rc_set_error("rc_sampler_binder_mpel: null handle"); return RC_ERR_ARG; }
+  int st = rc_sampler_binder_check(s, chain0, nch, "rc_sampler_binder_mpel");
+  if (st) return st;
+  int64_t S, n, nchains; int device;
+  const uint8_t* L = rc_sampler_dev_labels(s, &S, &n, &nchains, &device);
+  RC_CUDA(cudaSetDevice(device));
+  return binder_device(L + (size_t)chain0 * S * n, nch * S, n, loss_sums, best, totals);   // chain-major, sample-minor
 }
 
 }  // extern "C"

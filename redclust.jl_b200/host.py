@@ -348,6 +348,43 @@ class Sampler:
         check(lib().rc_sampler_predict(self._h, ptr(Dn), m, chain0, nch, ptr(out["coclustering"]), ptr(out["newcluster"])))
         return out
 
+    def binder_pointestimate(self, chain0=0, nch=None):
+        """getpointestimate(method="MPEL", loss="binder") over the pooled recorded samples of chains chain0 .. chain0 + nch
+        - 1, from their co-clustering counts on the device (rc_sampler_binder_mpel): dict(clust = the winning partition,
+        chain, index = its sample within that chain, sums = expected Binder loss sums of every sample (chain-major),
+        totals = the same as exact integer counts of disagreeing pairs)."""
+        nch = self.nchains - chain0 if nch is None else nch
+        S = int(lib().rc_sampler_numsamples(self._h))
+        total = max(nch, 0) * S
+        sums, totals, best = np.empty(total), np.empty(total, np.int64), C.c_int64()
+        check(lib().rc_sampler_binder_mpel(self._h, chain0, nch, ptr(sums), C.byref(best), ptr(totals)))
+        chain, index = chain0 + best.value // S, best.value % S
+        return dict(clust=self.samples(chain)["labels"][index], chain=chain, index=index, sums=sums, totals=totals)
+
+    def binder_pointestimate_allreduce(self, group=None, device=None, comm=None):
+        """binder_pointestimate over the chains of every rank (rc_comm_sampler_binder_mpel): the all-reduced counts, one
+        ncclAllGather of the per-rank totals; equal to one GPU over the same chains.  dict(best = index into the samples
+        of all ranks in rank order, sums, totals, and clust / chain / index of the winner on the rank that holds it, None
+        on the others)."""
+        comm = comm or Comm.from_torch(group, self.data.device if device is None else device)
+        S = int(lib().rc_sampler_numsamples(self._h))
+        mine = self.nchains * S
+        if comm.world > 1:
+            import torch.distributed as dist
+            sizes = [None] * comm.world
+            dist.all_gather_object(sizes, mine, group=group)
+        else:
+            sizes = [mine]
+        total = sum(sizes)
+        sums, totals, best = np.empty(total), np.empty(total, np.int64), C.c_int64()
+        check(lib().rc_comm_sampler_binder_mpel(comm._h, self._h, ptr(sums), C.byref(best), ptr(totals)))
+        out = dict(best=best.value, sums=sums, totals=totals, clust=None, chain=None, index=None)
+        local = best.value - sum(sizes[:comm.rank])
+        if 0 <= local < mine:
+            out.update(chain=local // S, index=local % S)
+            out["clust"] = self.samples(out["chain"])["labels"][out["index"]]
+        return out
+
     def close(self):
         L = getattr(_lib, "_lib", None)
         if getattr(self, "_h", None) and L is not None:
@@ -627,12 +664,58 @@ def mpel_loss_sums_sharded(labels, loss, group=None, device=None, comm=None):
     return sums, int(best.value)
 
 
+def binder_loss_sums(labels, device=0):
+    """Expected Binder loss of every sample against all of them (S x n host labels), from their co-clustering counts on
+    the device (rc_binder_mpel): (sums, best, totals) with sums[s] = totals[s] / C(n, 2), totals the exact integer counts
+    of disagreeing pairs summed over the samples, best their first argmin.  O(S n^2) work and no S x S matrix, so it
+    takes pooled chains; sums agree with mpel_loss_sums(labels, "binder") up to that call's fp64 rounding."""
+    L = np.ascontiguousarray(np.asarray(labels, dtype=np.int64))
+    if L.ndim != 2:
+        raise ArgumentError("labels must be an S × n matrix.")
+    sums, totals, best = np.empty(L.shape[0]), np.empty(L.shape[0], np.int64), C.c_int64()
+    check(lib().rc_binder_mpel(ptr(L), L.shape[0], L.shape[1], device, ptr(sums), C.byref(best), ptr(totals)))
+    return sums, int(best.value), totals
+
+
+_PAIRWISE_BYTES = 64 << 30          # the S x S fp64 loss matrix of the pairwise MPEL path must stay below this
+
+
+def _pooled_pointestimate(results, method, loss, device):
+    """getpointestimate over a list of MCMCResult (runsampler with nchains > 1), pooled in list order."""
+    if not results:
+        raise ArgumentError("samples must hold at least one MCMCResult.")
+    if any(r is None for r in results):
+        raise ArgumentError("a chain stopped at the slot capacity (its result is None); drop it before pooling.")
+    clusts = [c for r in results for c in r.clusts]
+    if len({np.asarray(c).shape for c in clusts}) > 1:
+        raise ArgumentError("the results to pool label different numbers of points.")
+    if method == "MAP":
+        i = int(np.argmax(np.concatenate([np.asarray(r.logposterior) for r in results])))
+    elif method == "MLE":
+        i = int(np.argmax(np.concatenate([np.asarray(r.loglik) for r in results])))
+    elif isinstance(loss, str) and loss == "binder":
+        _, i, _ = binder_loss_sums(np.stack(clusts), device)
+    else:
+        S = len(clusts)
+        if 8 * S * S > _PAIRWISE_BYTES:
+            raise ArgumentError(f"{S} pooled samples need a {8 * S * S / 2**30:.0f} GiB pairwise loss matrix for loss={loss!r}; "
+                                'loss="binder" takes pooled samples without one.')
+        pooled = MCMCResult()
+        pooled.clusts = clusts
+        return getpointestimate(pooled, method, loss, device)
+    return clusts[i], i
+
+
 def getpointestimate(samples, method="MAP", loss="VI", device=0):
-    """getpointestimate(samples; method, loss) -> (clust, i)   (pointestimate.jl:17-60); i is 0-based here."""
+    """getpointestimate(samples; method, loss) -> (clust, i)   (pointestimate.jl:17-60); i is 0-based here.  `samples` is
+    an MCMCResult or a list of them (runsampler with nchains > 1), pooled in list order with i indexing the
+    concatenation; MPEL with loss="binder" over a list runs from the pooled co-clustering counts (binder_loss_sums)."""
     if method == "MPEL" and isinstance(loss, str) and loss not in _LOSS:
         raise ArgumentError("Invalid loss function specifier.")
     if method not in ("MAP", "MLE", "MPEL"):
         raise ArgumentError("Invalid method specifier.")
+    if isinstance(samples, (list, tuple)):
+        return _pooled_pointestimate(list(samples), method, loss, device)
     if method == "MAP":
         i = int(np.argmax(samples.logposterior))
     elif method == "MLE":

@@ -317,4 +317,61 @@ function getpointestimate(samples::MCMCResult; method::String = "MAP", loss::Uni
     return (samples.clusts[i], i)
 end
 
+"""
+    binder_loss_sums(clusts) -> (sums, best, totals)
+
+Expected Binder loss of every sample against all of them (src/pointestimate.jl:34-59,68-76) from their co-clustering
+counts on the GPU (rc_binder_mpel): totals are the exact integer counts of disagreeing pairs summed over the samples,
+sums = totals / binomial(n, 2), best the first argmin (1-based).  No S x S matrix, so it takes pooled chains.  (The
+sampler-resident entry points rc_sampler_binder_mpel / rc_comm_sampler_binder_mpel need the sampler handle, which this
+runsampler releases before it returns.)
+"""
+function binder_loss_sums(clusts::Vector{<:AbstractVector{<:Integer}}; device::Integer = 0)
+    S = length(clusts); n = length(clusts[1])
+    all(length(c) == n for c in clusts) || throw(ArgumentError("the samples to pool label different numbers of points."))
+    L = Matrix{Int64}(undef, n, S)
+    for j in 1:S; L[:, j] .= clusts[j]; end
+    sums = Vector{Float64}(undef, S); totals = Vector{Int64}(undef, S); best = Ref{Int64}(0)
+    GC.@preserve L check(ccall((:rc_binder_mpel, LIB[]), Int32, (Ptr{Int64}, Int64, Int64, Int32, Ptr{Float64}, Ref{Int64}, Ptr{Int64}),
+                               L, S, n, device, sums, best, totals))
+    return sums, best[] + 1, totals
+end
+
+"""
+    getpointestimate(results::Vector{MCMCResult}; method, loss) -> (clust, i)
+
+The samples of several chains (runsampler with nchains > 1) pooled in vector order; i indexes the concatenation.  MPEL
+with loss = "binder" runs from the pooled co-clustering counts (binder_loss_sums); the other losses build the pairwise
+S x S loss matrix, refused beyond 64 GiB.
+"""
+function getpointestimate(results::Vector{MCMCResult}; method::String = "MAP", loss::Union{String,Function} = "VI")
+    if method == "MPEL" && loss isa String && loss ∉ ["binder", "omARI", "VI", "ID"]
+        throw(ArgumentError("Invalid loss function specifier."))
+    end
+    method ∉ ["MAP", "MLE", "MPEL"] && throw(ArgumentError("Invalid method specifier."))
+    isempty(results) && throw(ArgumentError("samples must hold at least one MCMCResult."))
+    clusts = [c for r in results for c in r.clusts]
+    all(length(c) == length(clusts[1]) for c in clusts) || throw(ArgumentError("the results to pool label different numbers of points."))
+    if method == "MAP"
+        i = argmax(vcat([r.logposterior for r in results]...))
+    elseif method == "MLE"
+        i = argmax(vcat([r.loglik for r in results]...))
+    elseif loss == "binder"
+        _, i, _ = binder_loss_sums(clusts)
+    else
+        S = length(clusts)
+        8 * S^2 > 64 * 2^30 && throw(ArgumentError("$S pooled samples need a pairwise loss matrix above 64 GiB for loss = $loss; loss = \"binder\" takes pooled samples without one."))
+        if loss isa String
+            _, i = mpel(clusts, loss)
+        else                                                # user-supplied loss: host loop, as the reference
+            M = zeros(S, S)
+            for a in 1:S, b in (a + 1):S
+                M[a, b] = M[b, a] = loss(clusts[a], clusts[b])
+            end
+            i = argmin(vec(sum(M, dims = 1)))
+        end
+    end
+    return (clusts[i], i)
+end
+
 end # module

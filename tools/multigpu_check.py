@@ -49,6 +49,19 @@ if rank == 0:
     print(f"world={world} n={n} chains={cpr * world} samples/chain={iters}: psm_allreduce {dt * 1e3:.1f} ms; "
           f"equal to the single-process PSM of the same chains: {np.array_equal(psm, ref)}", flush=True)
     assert np.array_equal(psm, ref)
+# Binder MPEL over the chains of every rank: all-reduced counts, per-rank W and P, one all_gather of the int64 totals
+torch.cuda.synchronize(); dist.barrier()
+t = time.perf_counter()
+bp = smp.binder_pointestimate_allreduce()
+torch.cuda.synchronize(); dist.barrier()
+dt = time.perf_counter() - t
+if rank == 0:
+    one = make(0, cpr * world, data).binder_pointestimate()
+    okb = (np.array_equal(bp["totals"], one["totals"]) and np.array_equal(bp["sums"], one["sums"])
+           and bp["best"] == one["chain"] * opts.numsamples + one["index"])
+    print(f"world={world} n={n} chains={cpr * world}: binder_pointestimate_allreduce over {bp['totals'].size} samples {dt * 1e3:.1f} ms; "
+          f"equal to one process over the same chains: {okb}", flush=True)
+    assert okb
 # one common set of label vectors on every rank: rank 0's samples, broadcast, then 5 % of the labels reshuffled with a
 # fixed seed so that the samples differ from each other
 S = np.ascontiguousarray(smp.samples(0)["labels"])
