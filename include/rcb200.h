@@ -178,9 +178,10 @@ int32_t rc_sampler_check_sums(const rc_sampler* s, int64_t* mismatches_S, int64_
 /* Posterior co-clustering counts of the device-resident samples of chains [chain0, chain0+nch):
  * sum(adjacencymatrix.(clusts)) (src/mcmc.jl:560, src/utils.jl:59-63) as exact int32 counts in a
  * DEVICE buffer of n*n int32 (e.g. a torch tensor's data_ptr, so the caller can all-reduce it
- * over NCCL before dividing).                                                                  */
+ * over NCCL before dividing).  RC_ERR_STATE before a run to numiters (the samples are not all recorded),
+ * RC_ERR_SLOTS when a chain of the range stopped at the slot capacity, RC_ERR_ARG for a bad range.    */
 int32_t rc_sampler_psm_counts_dev(const rc_sampler* s, int64_t chain0, int64_t nch, void* counts_dev);
-/* Same, divided by the number of samples, into a host n x n fp64 matrix.                       */
+/* Same, divided by the number of samples, into a host n x n fp64 matrix; the same refusals.     */
 int32_t rc_sampler_psm(const rc_sampler* s, int64_t chain0, int64_t nch, double* psm_out);
 void rc_sampler_destroy(rc_sampler* s);
 
@@ -241,7 +242,8 @@ int32_t rc_sampler_binder_mpel(const rc_sampler* s, int64_t chain0, int64_t nch,
  * launcher (torch.distributed, MPI, Julia Distributed, ...) hands the 128 bytes to every rank, every rank calls
  * rc_comm_init.  NCCL is resolved at run time (libnccl.so.2), so the library loads without it.
  *   rc_comm_data_from_points  MCMCData(points), src/types.jl:159-162: row blocks of pairwise(Euclidean()) + all-gather
- *   rc_comm_sampler_psm       src/mcmc.jl:560 over the chains of every rank: int32 counts + ONE all-reduce + divide
+ *   rc_comm_sampler_psm       src/mcmc.jl:560 over the chains of every rank: int32 counts + ONE all-reduce + divide;
+ *                             refuses as rc_sampler_psm does on any rank (every rank returns the error)
  *   rc_comm_psm               the same for host label vectors sharded over the ranks (S_local of them on this rank)
  *   rc_comm_mpel              src/pointestimate.jl:49-57 with the candidate rows dealt cyclically + all-gather
  *   rc_comm_sampler_binder_mpel  src/pointestimate.jl:34-59,68-76 over the chains of every rank (src/mcmc.jl:560): the

@@ -630,9 +630,8 @@ int32_t rc_sample_rp(const int64_t* clustsizes, int64_t nsizes, const rc_options
   int st = validate_options(opt);
   if (st) return st;
   if (!(par->proposalsd_r > 0)) { rc_set_error("invalid hyperparameters (proposalsd_r <= 0)"); return RC_ERR_ARG; }
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) { (void)cudaGetLastError(); rc_set_error("no CUDA device available (librcb200 has no CPU fallback)"); return RC_ERR_CUDA; }
-  RC_CUDA(cudaSetDevice(device));
+  st = rc_select_device(device);
+  if (st) return st;
   std::vector<int> C;                                  // C = clustsizes[findall(clustsizes .> 0)]  (:613)
   long long n = 0;
   for (int64_t k = 0; k < nsizes; ++k) if (clustsizes[k] > 0) { C.push_back((int)clustsizes[k]); n += clustsizes[k]; }
@@ -662,20 +661,27 @@ int32_t rc_sample_rp(const int64_t* clustsizes, int64_t nsizes, const rc_options
   return RC_OK;
 }
 
-// internal accessors used by rc_post.cu
-const uint8_t* rc_sampler_dev_labels(const rc_sampler* s, int64_t* S, int64_t* n, int64_t* nchains, int* device) {
-  if (S) *S = s->numsamples;
-  if (n) *n = s->n;
-  if (nchains) *nchains = s->nchains;
-  if (device) *device = s->device;
-  return s->out_labels;
-}
-
-// internal accessor used by rc_predict.cu: the data, hyperparameters, progress and recorded K / r / p traces of the sampler
-const rc_data* rc_sampler_dev_traces(const rc_sampler* s, rc_params* par, int64_t* iters_done, int64_t* numiters, const int** K,
-                                     const double** r, const double** p) {
-  *par = s->par; *iters_done = s->iters_done; *numiters = s->opt.numiters; *K = s->out_K; *r = s->out_r; *p = s->out_p;
-  return s->d;
-}
-
 }  // extern "C"
+
+// The samples of a chain range for the post-processing entry points: only a run to numiters has recorded every sample,
+// and a chain stopped by the slot capacity has not (its out_labels were never written).
+int rc_sampler_range(const rc_sampler* s, int64_t chain0, int64_t nch, const char* who, rc_sample_range& v) {
+  if (chain0 < 0 || nch < 1 || chain0 + nch > s->nchains) { rc_set_error("%s: bad chain range", who); return RC_ERR_ARG; }
+  if (s->iters_done < s->opt.numiters) {
+    rc_set_error("%s: the sampler ran %lld of %lld iterations; its samples are recorded only by a complete run", who,
+                 (long long)s->iters_done, (long long)s->opt.numiters);
+    return RC_ERR_STATE;
+  }
+  TRYP(rc_select_device(s->device));
+  std::vector<int> status((size_t)nch);
+  RC_CUDA(cudaMemcpy(status.data(), s->status + chain0, sizeof(int) * (size_t)nch, cudaMemcpyDeviceToHost));
+  for (int64_t c = 0; c < nch; ++c)
+    if (status[c] != 0) {
+      rc_set_error("%s: chain %lld stopped at the slot capacity; its samples are incomplete", who, (long long)(chain0 + c));
+      return RC_ERR_SLOTS;
+    }
+  const size_t first = (size_t)chain0 * s->numsamples;
+  v.d = s->d; v.par = s->par; v.n = s->n; v.R = nch * s->numsamples;
+  v.labels = s->out_labels + first * s->n; v.K = s->out_K + first; v.r = s->out_r + first; v.p = s->out_p + first;
+  return RC_OK;
+}

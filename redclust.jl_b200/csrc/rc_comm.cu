@@ -99,7 +99,7 @@ int32_t rc_comm_init(const uint8_t* id128, int32_t rank, int32_t world, int32_t 
   if (!id128 || !out || world < 1 || rank < 0 || rank >= world) { rc_set_error("rc_comm_init: bad arguments"); return RC_ERR_ARG; }
   NcclApi* a = nccl();
   if (!a) { rc_set_error("NCCL is not available (libnccl.so.2 could not be loaded)"); return RC_ERR_CUDA; }
-  RC_CUDA(cudaSetDevice(device));
+  TRYP(rc_select_device(device));
   ncclUniqueId id;
   memcpy(id.internal, id128, 128);
   rc_comm* c = new rc_comm();
@@ -110,13 +110,13 @@ int32_t rc_comm_init(const uint8_t* id128, int32_t rank, int32_t world, int32_t 
   // NCCL connects its channels lazily on the first collective (tens of milliseconds): pay that here, not in the first
   // PSM exchange (round 1 timed a 64 MB all-reduce at 118 ms because it was the communicator's first)
   {
-    int* w = nullptr;
-    if (cudaMalloc(&w, 256 * sizeof(int)) == cudaSuccess) {
+    Bufs B;
+    int* w;
+    if (B.get(&w, 256) == RC_OK) {
       cudaMemset(w, 0, 256 * sizeof(int));
       a->AllReduce(w, w, 256, ncclInt32, ncclSum, c->comm, c->stream);
       a->AllGather(w, w, 256 / world, ncclInt32, c->comm, c->stream);
       cudaStreamSynchronize(c->stream);
-      cudaFree(w);
     }
   }
   *out = c;
@@ -155,8 +155,9 @@ int32_t rc_comm_data_from_points(rc_comm* c, const double* X, int64_t dim, int64
   if (!c || !X || !out || n < 1 || dim < 1) { rc_set_error("rc_comm_data_from_points: bad arguments"); return RC_ERR_ARG; }
   RC_CUDA(cudaSetDevice(c->device));
   const int64_t per = (n + c->world - 1) / c->world;                  // equal blocks, the last one padded
-  double* full = nullptr;
-  RC_CUDA(cudaMalloc(&full, sizeof(double) * (size_t)per * c->world * n));
+  Bufs B;
+  double* full;
+  TRYP(B.get(&full, (size_t)per * c->world * n));
   const int64_t row0 = std::min<int64_t>((int64_t)c->rank * per, n), nrows = std::min<int64_t>(per, n - row0);
   double* mine = full + (size_t)c->rank * per * n;
   int st = RC_OK;
@@ -167,7 +168,6 @@ int32_t rc_comm_data_from_points(rc_comm* c, const double* X, int64_t dim, int64
     if (r != ncclSuccess || cudaStreamSynchronize(c->stream) != cudaSuccess) { rc_set_error("all-gather of the distance rows failed"); st = RC_ERR_CUDA; }
   }
   if (!st) st = rc_data_from_dist_dev(full, n, c->device, out);
-  cudaFree(full);
   return st;
 }
 
@@ -175,106 +175,122 @@ int32_t rc_comm_data_from_points(rc_comm* c, const double* X, int64_t dim, int64
 // of the n x n matrix, one divide by the global number of samples.  psm_out (host n x n fp64) may be NULL when only
 // counts_dev_out (device n x n int32, may be NULL too) is wanted.
 static int32_t finish_psm(rc_comm* c, int* counts, int64_t n, long long local_samples, double* psm_out) {
-  long long* tot = nullptr;
-  RC_CUDA(cudaMalloc(&tot, sizeof(long long)));
+  Bufs B;
+  long long* tot;
+  TRYP(B.get(&tot, 1));
   RC_CUDA(cudaMemcpy(tot, &local_samples, sizeof(long long), cudaMemcpyHostToDevice));
   RC_CUDA(cudaDeviceSynchronize());
   if (c->world > 1) {
     cudaEvent_t e0, e1;
     cudaEventCreate(&e0); cudaEventCreate(&e1);
     cudaEventRecord(e0, c->stream);
-    RC_NCCL(nccl()->AllReduce(counts, counts, (size_t)n * n, ncclInt32, ncclSum, c->comm, c->stream));
+    ncclResult_t r = nccl()->AllReduce(counts, counts, (size_t)n * n, ncclInt32, ncclSum, c->comm, c->stream);
     cudaEventRecord(e1, c->stream);
-    RC_NCCL(nccl()->AllReduce(tot, tot, 1, ncclInt64, ncclSum, c->comm, c->stream));
-    RC_CUDA(cudaStreamSynchronize(c->stream));
-    if (getenv("RCB200_VERBOSE")) {
+    if (r == ncclSuccess) r = nccl()->AllReduce(tot, tot, 1, ncclInt64, ncclSum, c->comm, c->stream);
+    const cudaError_t e = r == ncclSuccess ? cudaStreamSynchronize(c->stream) : cudaSuccess;
+    if (r == ncclSuccess && e == cudaSuccess && getenv("RCB200_VERBOSE")) {
       float ms = 0; cudaEventElapsedTime(&ms, e0, e1);
       const double bytes = 4.0 * (double)n * (double)n;
       fprintf(stderr, "[rcb200] rank %d: ncclAllReduce of the %lld x %lld int32 counts (%.2f GB): %.2f ms, algorithm bandwidth %.1f GB/s, bus bandwidth %.1f GB/s\n",
               c->rank, (long long)n, (long long)n, bytes / 1e9, ms, bytes / ms / 1e6, bytes / ms / 1e6 * 2.0 * (c->world - 1) / c->world);
     }
     cudaEventDestroy(e0); cudaEventDestroy(e1);
+    RC_NCCL(r);
+    RC_CUDA(e);
   }
   long long total = 0;
   RC_CUDA(cudaMemcpy(&total, tot, sizeof(long long), cudaMemcpyDeviceToHost));
-  cudaFree(tot);
   if (psm_out) return rc_counts_to_host_psm(counts, (size_t)n * n, (double)total, psm_out);
+  return RC_OK;
+}
+
+// The {status, samples} of every rank, exchanged before the collectives of a call that a rank may refuse: a refusing rank
+// returns its own error and the others "rank r refused", instead of leaving them waiting in the next collective.
+// all (out): world x {status, samples}.
+static int agree(rc_comm* c, int local, int64_t samples, const char* who, std::vector<long long>& all) {
+  const std::string why = local ? rc_last_error() : "";
+  Bufs B;
+  long long* info;                                             // this rank's pair, then the gathered ranks
+  TRYP(B.get(&info, 2 * (size_t)(c->world + 1)));
+  const long long mine[2] = {local, (long long)samples};
+  all.assign(2 * (size_t)c->world, 0);
+  cudaError_t e = cudaMemcpy(info, mine, sizeof(mine), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess && nccl()->AllGather(info, info + 2, 2, ncclInt64, c->comm, c->stream) != ncclSuccess) e = cudaErrorUnknown;
+  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+  if (e == cudaSuccess) e = cudaMemcpy(all.data(), info + 2, sizeof(long long) * 2 * c->world, cudaMemcpyDeviceToHost);
+  if (e != cudaSuccess) { rc_set_error("%s: exchange of the sample counts failed", who); return RC_ERR_CUDA; }
+  for (int r = 0; r < c->world; ++r)
+    if (all[2 * r] != 0) {
+      if (local) { rc_set_error("%s", why.c_str()); return local; }
+      rc_set_error("%s: rank %d refused (status %lld)", who, r, all[2 * r]);
+      return (int32_t)all[2 * r];
+    }
   return RC_OK;
 }
 
 int32_t rc_comm_sampler_psm(rc_comm* c, const rc_sampler* s, double* psm_out, void* counts_dev_out) {
   if (!c || !s) { rc_set_error("rc_comm_sampler_psm: null handle"); return RC_ERR_ARG; }
   RC_CUDA(cudaSetDevice(c->device));
-  const int64_t n = rc_sampler_n(s), nch = rc_sampler_nchains(s), S = rc_sampler_numsamples(s);
+  rc_sample_range v;
+  const int local = rc_sampler_range(s, 0, rc_sampler_nchains(s), "rc_comm_sampler_psm", v);
+  std::vector<long long> all;
+  TRYP(agree(c, local, local ? 0 : v.R, "rc_comm_sampler_psm", all));
+  Bufs B;
   int* counts = (int*)counts_dev_out;
-  if (!counts) RC_CUDA(cudaMalloc(&counts, sizeof(int) * (size_t)n * n));
-  int st = rc_sampler_psm_counts_dev(s, 0, nch, counts);
-  if (!st) st = finish_psm(c, counts, n, (long long)(nch * S), psm_out);
-  if (!counts_dev_out) cudaFree(counts);
-  return st;
+  if (!counts) TRYP(B.get(&counts, (size_t)v.n * v.n));
+  TRYP(psm_counts_device(v.labels, v.R, v.n, counts, B));
+  return finish_psm(c, counts, v.n, (long long)v.R, psm_out);
 }
 
 int32_t rc_comm_psm(rc_comm* c, const int64_t* labels, int64_t S_local, int64_t n, double* psm_out, void* counts_dev_out) {
   if (!c || (!labels && S_local > 0) || n < 1 || S_local < 0) { rc_set_error("rc_comm_psm: bad arguments"); return RC_ERR_ARG; }
   RC_CUDA(cudaSetDevice(c->device));
+  Bufs B;
   int* counts = (int*)counts_dev_out;
-  if (!counts) RC_CUDA(cudaMalloc(&counts, sizeof(int) * (size_t)n * n));
+  if (!counts) TRYP(B.get(&counts, (size_t)n * n));
   int st = RC_OK;
   if (S_local > 0) st = rc_psm_counts_dev(labels, S_local, n, c->device, counts);
   else st = cudaMemset(counts, 0, sizeof(int) * (size_t)n * n) == cudaSuccess ? RC_OK : RC_ERR_CUDA;
   if (!st) st = finish_psm(c, counts, n, (long long)S_local, psm_out);
-  if (!counts_dev_out) cudaFree(counts);
   return st;
 }
 
-// Binder MPEL over the samples of every rank (src/pointestimate.jl:34-59,68-76 with the counts of src/mcmc.jl:560): the
-// all-reduced counts of rc_comm_sampler_psm, W and P of this rank's samples, ONE all-gather of the per-rank int64 vectors
-// (padded to the largest rank), and the totals over all samples in rank order.  Integers throughout: identical to one
-// GPU over the same chains.  Every rank first learns whether any rank refuses, so none is left waiting in a collective.
+// Binder MPEL over the samples of every rank (src/pointestimate.jl:34-59,68-76 with the counts of src/mcmc.jl:560): this
+// rank's counts, all-reduced as rc_comm_sampler_psm does, W and P of this rank's samples against them (from the transposed
+// labels the counts were built from), ONE all-gather of the per-rank int64 vectors (padded to the largest rank), and the
+// totals over all samples in rank order.  Integers throughout: identical to one GPU over the same chains.
 int32_t rc_comm_sampler_binder_mpel(rc_comm* c, const rc_sampler* s, double* loss_sums, int64_t* best, int64_t* totals) {
   if (!c || !s) { rc_set_error("rc_comm_sampler_binder_mpel: null handle"); return RC_ERR_ARG; }
   RC_CUDA(cudaSetDevice(c->device));
-  const int64_t n = rc_sampler_n(s), nch = rc_sampler_nchains(s), R = nch * rc_sampler_numsamples(s);
-  const int local = rc_sampler_binder_check(s, 0, nch, "rc_comm_sampler_binder_mpel");
-  const std::string why = local ? rc_last_error() : "";
-  long long* info = nullptr;                                   // per rank: {status, samples}
-  RC_CUDA(cudaMalloc(&info, sizeof(long long) * 2 * (c->world + 1)));
-  const long long mine[2] = {local, (long long)R};
-  std::vector<long long> all(2 * (size_t)c->world);
-  cudaError_t e = cudaMemcpy(info, mine, sizeof(mine), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess && nccl()->AllGather(info, info + 2, 2, ncclInt64, c->comm, c->stream) != ncclSuccess) e = cudaErrorUnknown;
-  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-  if (e == cudaSuccess) e = cudaMemcpy(all.data(), info + 2, sizeof(long long) * 2 * c->world, cudaMemcpyDeviceToHost);
-  cudaFree(info);
-  if (e != cudaSuccess) { rc_set_error("rc_comm_sampler_binder_mpel: exchange of the sample counts failed"); return RC_ERR_CUDA; }
+  const char* who = "rc_comm_sampler_binder_mpel";
+  rc_sample_range v;
+  int local = rc_sampler_range(s, 0, rc_sampler_nchains(s), who, v);
+  if (!local) local = rc_binder_check_args(v.R, v.n, who);
+  std::vector<long long> all;
+  TRYP(agree(c, local, local ? 0 : v.R, who, all));
+  const int64_t n = v.n;
   int64_t total = 0, per = 0;
   for (int r = 0; r < c->world; ++r) {
-    if (all[2 * r] != 0) {
-      if (local) { rc_set_error("%s", why.c_str()); return local; }
-      rc_set_error("rc_comm_sampler_binder_mpel: rank %d refused (status %lld)", r, all[2 * r]);
-      return (int32_t)all[2 * r];
-    }
     total += all[2 * r + 1];
     per = std::max<int64_t>(per, all[2 * r + 1]);
   }
-  if (total >= ((int64_t)1 << 31)) { rc_set_error("rc_comm_sampler_binder_mpel: %lld samples in all; needs < 2^31", (long long)total); return RC_ERR_ARG; }
-  int* counts = nullptr;
-  unsigned long long* buf = nullptr;                           // [world + 1][2 per]: this rank's {W, P}, then the gathered ranks
-  RC_CUDA(cudaMalloc(&counts, sizeof(int) * (size_t)n * n));
-  if (cudaMalloc(&buf, sizeof(unsigned long long) * 2 * (size_t)per * (c->world + 1)) != cudaSuccess) {
-    cudaFree(counts); rc_set_error("rc_comm_sampler_binder_mpel: out of device memory"); return RC_ERR_CUDA;
-  }
+  if (total >= ((int64_t)1 << 31)) { rc_set_error("%s: %lld samples in all; needs < 2^31", who, (long long)total); return RC_ERR_ARG; }
+  Bufs B;
+  int* counts;
+  unsigned long long* buf;                                     // [world + 1][2 per]: this rank's {W, P}, then the gathered ranks
+  const uint8_t* Lt;
+  TRYP(B.get(&counts, (size_t)n * n));
+  TRYP(B.get(&buf, 2 * (size_t)per * (c->world + 1)));
   std::vector<unsigned long long> wp(2 * (size_t)per, 0ull), gathered(2 * (size_t)per * c->world);
-  int st = rc_comm_sampler_psm(c, s, nullptr, counts);
-  if (!st) st = rc_sampler_binder_wp(s, 0, nch, counts, total, wp.data(), wp.data() + per);
-  if (!st && cudaMemcpy(buf, wp.data(), sizeof(unsigned long long) * 2 * per, cudaMemcpyHostToDevice) != cudaSuccess) st = RC_ERR_CUDA;
-  if (!st && (nccl()->AllGather(buf, buf + 2 * per, 2 * (size_t)per, ncclInt64, c->comm, c->stream) != ncclSuccess ||
-              cudaStreamSynchronize(c->stream) != cudaSuccess ||
-              cudaMemcpy(gathered.data(), buf + 2 * per, sizeof(unsigned long long) * gathered.size(), cudaMemcpyDeviceToHost) != cudaSuccess)) {
-    rc_set_error("rc_comm_sampler_binder_mpel: all-gather of the per-rank totals failed"); st = RC_ERR_CUDA;
+  TRYP(psm_counts_device(v.labels, v.R, n, counts, B, &Lt));
+  TRYP(finish_psm(c, counts, n, (long long)v.R, nullptr));
+  TRYP(binder_wp(v.labels, Lt, v.R, n, counts, total, wp.data(), wp.data() + per, nullptr));
+  RC_CUDA(cudaMemcpy(buf, wp.data(), sizeof(unsigned long long) * 2 * per, cudaMemcpyHostToDevice));
+  if (nccl()->AllGather(buf, buf + 2 * per, 2 * (size_t)per, ncclInt64, c->comm, c->stream) != ncclSuccess ||
+      cudaStreamSynchronize(c->stream) != cudaSuccess ||
+      cudaMemcpy(gathered.data(), buf + 2 * per, sizeof(unsigned long long) * gathered.size(), cudaMemcpyDeviceToHost) != cudaSuccess) {
+    rc_set_error("%s: all-gather of the per-rank totals failed", who); return RC_ERR_CUDA;
   }
-  cudaFree(counts); cudaFree(buf);
-  if (st) return st;
   std::vector<unsigned long long> W, P;                        // rank order = global chain order
   for (int r = 0; r < c->world; ++r) {
     const unsigned long long* g = gathered.data() + 2 * (size_t)per * r;
@@ -292,9 +308,9 @@ int32_t rc_comm_mpel(rc_comm* c, const int64_t* labels, int64_t S, int64_t n, in
   RC_CUDA(cudaSetDevice(c->device));
   if (c->world == 1) return rc_mpel(labels, S, n, loss, c->device, loss_sums, best);
   const int64_t per = (S + c->world - 1) / c->world;
-  double *flat = nullptr, *upper = nullptr;
-  RC_CUDA(cudaMalloc(&flat, sizeof(double) * (size_t)per * c->world * S));
-  if (cudaMalloc(&upper, sizeof(double) * (size_t)S * S) != cudaSuccess) { cudaFree(flat); rc_set_error("out of device memory for the loss matrix"); return RC_ERR_CUDA; }
+  Bufs B;
+  double *flat, *upper;
+  TRYP(B.get(&flat, (size_t)per * c->world * S)); TRYP(B.get(&upper, (size_t)S * S));
   double* mine = flat + (size_t)c->rank * per * S;
   int st = cudaMemset(mine, 0, sizeof(double) * (size_t)per * S) == cudaSuccess ? RC_OK : RC_ERR_CUDA;
   if (!st) st = rc_mpel_rows_dev(labels, S, n, loss, c->device, c->rank, c->world, per, mine);
@@ -308,7 +324,6 @@ int32_t rc_comm_mpel(rc_comm* c, const int64_t* labels, int64_t S, int64_t n, in
     if (cudaStreamSynchronize(c->stream) != cudaSuccess) { rc_set_error("assembling the loss matrix failed"); st = RC_ERR_CUDA; }
   }
   if (!st) st = rc_mpel_finish_dev(upper, S, c->device, loss_sums, best);
-  cudaFree(flat); cudaFree(upper);
   return st;
 }
 

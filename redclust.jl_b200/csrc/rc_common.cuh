@@ -4,6 +4,8 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <string>
+#include <vector>
+#include <algorithm>
 #include "../../include/rcb200.h"
 #include "rc_math.h"
 #include "rc_rng.h"
@@ -26,15 +28,48 @@ void rc_dev_free(void* p);
     }                                                                                          \
   } while (0)
 
+#define TRYP(x) do { int st_ = (x); if (st_) return st_; } while (0)
+
+// Device buffers of one call, released on every return path.
+struct Bufs {
+  std::vector<void*> p;
+  template <class T> int get(T** out, size_t count) {
+    *out = nullptr;
+    cudaError_t e = cudaMalloc((void**)out, sizeof(T) * std::max<size_t>(count, 1));
+    if (e != cudaSuccess) { (void)cudaGetLastError(); rc_set_error("out of device memory (%zu bytes)", sizeof(T) * count); return RC_ERR_CUDA; }
+    p.push_back(*out);
+    return RC_OK;
+  }
+  ~Bufs() { for (void* q : p) cudaFree(q); }
+};
+
+// The recorded samples of chains [chain0, chain0 + nch) of a sampler, on its device (rc_api.cu): R = nch * numsamples
+// label vectors of n bytes (1..K, chain-major, sample-minor) and their K, r, p, with the sampler's data and hyperparameters.
+struct rc_sample_range {
+  const rc_data* d;
+  rc_params par;
+  const uint8_t* labels;
+  const int* K;
+  const double *r, *p;
+  int64_t R, n;
+};
+// Selects the sampler's device and fills v.  A range outside the chains: RC_ERR_ARG; a run that has not reached numiters
+// (the samples are not all recorded): RC_ERR_STATE; a chain of the range that stopped at the slot capacity: RC_ERR_SLOTS.
+int rc_sampler_range(const rc_sampler* s, int64_t chain0, int64_t nch, const char* who, rc_sample_range& v);
+
 // pairwise Euclidean distances on the FP64 tensor cores (rc_gram.cu): X_dev n x dim row-major -> rows [row0, row0 + nrows) in D_dev (nrows x n)
 int rc_distm_dmma(const double* X_dev, int64_t dim, int64_t n, int64_t row0, int64_t nrows, double* D_dev);
 // int32 co-clustering counts on the device -> host fp64 counts / denom (rc_post.cu)
 int rc_counts_to_host_psm(const int* counts, size_t total, double denom, double* out);
-// posterior expected Binder loss from the counts (rc_post.cu): the sampler-range checks, W and P of a chain range against
-// counts of at most nmax samples, and the exact totals T_s = S P_s + sum_t P_t - 2 W_s with their first argmin
-int rc_sampler_binder_check(const rc_sampler* s, int64_t chain0, int64_t nch, const char* who);
-int rc_sampler_binder_wp(const rc_sampler* s, int64_t chain0, int64_t nch, const int* counts, int64_t nmax, unsigned long long* W,
-                         unsigned long long* P);
+// co-clustering counts of R device label vectors (sample-major) into counts (n x n int32), rc_post.cu.  The transposed
+// labels live in B; Lt (may be NULL) receives them for binder_wp.
+int psm_counts_device(const uint8_t* L, int64_t R, int64_t n, int* counts, Bufs& B, const uint8_t** Lt = nullptr);
+// posterior expected Binder loss from the counts (rc_post.cu): the sample and size limits, W and P of R label vectors (L and
+// its transpose Lt from psm_counts_device) against counts of at most nmax samples, and the exact totals
+// T_s = S P_s + sum_t P_t - 2 W_s with their first argmin
+int rc_binder_check_args(int64_t S, int64_t n, const char* who);
+int binder_wp(const uint8_t* L, const uint8_t* Lt, int64_t R, int64_t n, const int* counts, int64_t nmax, unsigned long long* W_out,
+              unsigned long long* P_out, float* w_ms);
 int rc_binder_finish(const unsigned long long* W, const unsigned long long* P, int64_t S, int64_t n, double* loss_sums,
                      int64_t* best, int64_t* totals);
 

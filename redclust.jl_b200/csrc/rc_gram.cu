@@ -268,9 +268,8 @@ int32_t rc_oracle_coclustering(const double* X, int64_t dim, int64_t n, int64_t 
   if (!X || !W || !out || n < 1 || dim < 1 || K < 1 || K > dim || numiters < 1 || !(sigma > 0)) {
     rc_set_error("rc_oracle_coclustering: bad arguments"); return RC_ERR_ARG;
   }
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) { (void)cudaGetLastError(); rc_set_error("no CUDA device available (librcb200 has no CPU fallback)"); return RC_ERR_CUDA; }
-  RC_CUDA(cudaSetDevice(device));
+  const int st = rc_select_device(device);
+  if (st) return st;
   // draws per chunk: the stacked posterior rows of a chunk are one n x (B K) operand of at most ~1 GB
   int64_t B = std::max<int64_t>(1, std::min<int64_t>(numiters, ((int64_t)1 << 27) / std::max<int64_t>(1, n * K)));
   const int64_t Kd = (B * K + GK - 1) / GK * GK;

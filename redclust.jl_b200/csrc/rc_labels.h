@@ -1,4 +1,4 @@
-// rc_labels.h -- host relabelling of label vectors shared by rc_post.cu and rc_predict.cu (internal).
+// rc_labels.h -- host relabelling and upload of label vectors shared by rc_post.cu and rc_predict.cu (internal).
 #pragma once
 #include <vector>
 #include <thread>
@@ -54,5 +54,15 @@ static int compact_labels(const int64_t* labels, int64_t S, int64_t n, std::vect
   body(0);
   for (auto& t : pool) t.join();
   if (bad.load() >= 0) { rc_set_error("more than 255 clusters in sample %lld", (long long)bad.load()); return RC_ERR_SLOTS; }
+  return RC_OK;
+}
+
+// The device labels of the entry points that take host label vectors: compact_labels, then the S x n bytes uploaded to
+// *dL, a buffer of B.  K: every sample's number of clusters (host).
+static int upload_labels(const int64_t* labels, int64_t S, int64_t n, Bufs& B, uint8_t** dL, std::vector<int>& K) {
+  std::vector<uint8_t> L;
+  TRYP(compact_labels(labels, S, n, L, K));
+  TRYP(B.get(dL, L.size()));
+  RC_CUDA(cudaMemcpy(*dL, L.data(), L.size(), cudaMemcpyHostToDevice));
   return RC_OK;
 }

@@ -21,10 +21,6 @@
 int rc_psm_counts_tc(const uint8_t* Lt, int64_t n, int64_t Rpad, int64_t R, int kmax, int* counts, cudaStream_t st);
 double rc_psm_tc_macs(int64_t n, int64_t R, int kmax);
 
-extern "C" const uint8_t* rc_sampler_dev_labels(const rc_sampler* s, int64_t* S, int64_t* n, int64_t* nchains, int* device);
-extern "C" const rc_data* rc_sampler_dev_traces(const rc_sampler* s, rc_params* par, int64_t* iters_done, int64_t* numiters, const int** K,
-                                                const double** r, const double** p);
-
 namespace {
 
 // Lt[i][r] = L[r][i]; rows r >= R are filled with 0 (every pair then "matches" Rpad - R extra times,
@@ -210,23 +206,23 @@ __global__ void __launch_bounds__(256) k_binder_pairs(const uint8_t* __restrict_
   }
 }
 
+}  // namespace
+
 // Co-clustering counts of R label vectors (device, sample-major).  Default: the tensor-core kernel of
 // rc_psm_tc.cu (labels up to 128); RCB200_PSM=compare or more labels: the byte-compare kernel.  Both are exact.
-// Lt_keep (may be NULL) receives the transposed labels (n x Rpad, Rpad = R rounded up to 64, filler 0), which the
-// caller then frees.
-int psm_counts_device(const uint8_t* L, int64_t R, int64_t n, int* counts, uint8_t** Lt_keep = nullptr) {
+// No label vectors (a sampler without samples): zero counts.  The transposed labels (n x Rpad, Rpad = R rounded up to 64,
+// filler 0) are a buffer of B; Lt_keep (may be NULL) receives them.
+int psm_counts_device(const uint8_t* L, int64_t R, int64_t n, int* counts, Bufs& B, const uint8_t** Lt_keep) {
+  if (R == 0) { RC_CUDA(cudaMemset(counts, 0, sizeof(int) * (size_t)n * n)); return RC_OK; }
   const int64_t Rpad = (R + 63) & ~63LL;
-  uint8_t* Lt = nullptr; int* dmax = nullptr;
-  RC_CUDA(cudaMalloc(&Lt, (size_t)n * Rpad));
-  if (cudaMalloc(&dmax, sizeof(int)) != cudaSuccess) { cudaFree(Lt); rc_set_error("out of device memory"); return RC_ERR_CUDA; }
+  uint8_t* Lt; int* dmax;
+  TRYP(B.get(&Lt, (size_t)n * Rpad)); TRYP(B.get(&dmax, 1));
   cudaMemset(dmax, 0, sizeof(int));
   dim3 tb(32, 8), tg((unsigned)((n + 31) / 32), (unsigned)((Rpad + 31) / 32));
   k_transpose<<<tg, tb>>>(L, R, n, Rpad, Lt);
   k_maxlabel<<<148 * 4, 256>>>(Lt, (size_t)n * Rpad, dmax);     // n * Rpad is a multiple of 64
   int kmax = 0;
-  cudaError_t e = cudaMemcpy(&kmax, dmax, sizeof(int), cudaMemcpyDeviceToHost);
-  cudaFree(dmax);
-  if (e != cudaSuccess) { cudaFree(Lt); RC_CUDA(e); }
+  RC_CUDA(cudaMemcpy(&kmax, dmax, sizeof(int), cudaMemcpyDeviceToHost));
   const char* mode = getenv("RCB200_PSM");
   const bool tc = kmax <= 128 && !(mode && !strcmp(mode, "compare"));
   cudaEvent_t e0 = nullptr, e1 = nullptr;
@@ -239,7 +235,7 @@ int psm_counts_device(const uint8_t* L, int64_t R, int64_t n, int* counts, uint8
     k_psm_counts<<<dim3(nb, nb), 256>>>(Lt, n, Rpad, R, counts);
   }
   if (verbose) cudaEventRecord(e1, 0);
-  e = cudaDeviceSynchronize();
+  const cudaError_t e = cudaDeviceSynchronize();
   if (verbose) {
     float ms = 0; cudaEventElapsedTime(&ms, e0, e1);
     const double macs = tc ? rc_psm_tc_macs(n, R, kmax) : 0.0;
@@ -247,30 +243,22 @@ int psm_counts_device(const uint8_t* L, int64_t R, int64_t n, int* counts, uint8
             (long long)n, (long long)R, kmax, tc ? "tcgen05-i8" : "byte-compare", ms, (double)n * n * R / (ms * 1e-3), 2 * macs / (ms * 1e-3) * 1e-12);
     cudaEventDestroy(e0); cudaEventDestroy(e1);
   }
-  if (Lt_keep && !st && e == cudaSuccess) *Lt_keep = Lt;
-  else cudaFree(Lt);
   if (st) return st;
   RC_CUDA(e);
+  if (Lt_keep) *Lt_keep = Lt;
   return RC_OK;
 }
 
-// Binder totals of R device label vectors (sample-major L, transposed Lt as psm_counts_device keeps it, or NULL to
-// transpose here) against co-clustering counts of at most nmax samples: W (uint64 per sample) and P (C(n_k, 2) summed
-// per sample) to the host.  w_ms (may be NULL): the W kernel's time, CUDA events.
-static int binder_wp(const uint8_t* L, const uint8_t* Lt, int64_t R, int64_t n, const int* counts, int64_t nmax,
-                     unsigned long long* W_out, unsigned long long* P_out, float* w_ms) {
+// Binder totals of R device label vectors (sample-major L and its transpose Lt from psm_counts_device) against
+// co-clustering counts of at most nmax samples: W (uint64 per sample) and P (C(n_k, 2) summed per sample) to the host.
+// w_ms (may be NULL): the W kernel's time, CUDA events.
+int binder_wp(const uint8_t* L, const uint8_t* Lt, int64_t R, int64_t n, const int* counts, int64_t nmax,
+              unsigned long long* W_out, unsigned long long* P_out, float* w_ms) {
   const int64_t Rpad = (R + 63) & ~63LL;
-  uint8_t* own = nullptr;
-  unsigned long long *W = nullptr, *P = nullptr;
-  if (!Lt) {
-    RC_CUDA(cudaMalloc(&own, (size_t)n * Rpad));
-    dim3 tb(32, 8), tg((unsigned)((n + 31) / 32), (unsigned)((Rpad + 31) / 32));
-    k_transpose<<<tg, tb>>>(L, R, n, Rpad, own);
-    Lt = own;
-  }
-  cudaError_t e = cudaMalloc(&W, sizeof(unsigned long long) * (size_t)R);
-  if (e == cudaSuccess) e = cudaMalloc(&P, sizeof(unsigned long long) * (size_t)R);
-  if (e == cudaSuccess) e = cudaMemset(W, 0, sizeof(unsigned long long) * (size_t)R);
+  Bufs B;
+  unsigned long long *W, *P;
+  TRYP(B.get(&W, (size_t)R)); TRYP(B.get(&P, (size_t)R));
+  cudaError_t e = cudaMemset(W, 0, sizeof(unsigned long long) * (size_t)R);
   cudaEvent_t e0 = nullptr, e1 = nullptr;
   if (e == cudaSuccess && w_ms) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, 0); }
   if (e == cudaSuccess) {
@@ -290,10 +278,11 @@ static int binder_wp(const uint8_t* L, const uint8_t* Lt, int64_t R, int64_t n, 
   if (e0) { cudaEventDestroy(e0); cudaEventDestroy(e1); }
   if (e == cudaSuccess) e = cudaMemcpy(W_out, W, sizeof(unsigned long long) * (size_t)R, cudaMemcpyDeviceToHost);
   if (e == cudaSuccess) e = cudaMemcpy(P_out, P, sizeof(unsigned long long) * (size_t)R, cudaMemcpyDeviceToHost);
-  cudaFree(W); cudaFree(P); cudaFree(own);
   RC_CUDA(e);
   return RC_OK;
 }
+
+namespace {
 
 // ---- MPEL ----------------------------------------------------------------------------------------
 // One CTA per (i, block of PJ columns j > i): sample i's labels are staged once, then for every j the
@@ -451,68 +440,50 @@ extern "C" {
 
 int32_t rc_sampler_psm_counts_dev(const rc_sampler* s, int64_t chain0, int64_t nch, void* counts_dev) {
   if (!s || !counts_dev) { rc_set_error("rc_sampler_psm_counts_dev: null pointer"); return RC_ERR_ARG; }
-  int64_t S, n, nchains; int device;
-  const uint8_t* L = rc_sampler_dev_labels(s, &S, &n, &nchains, &device);
-  if (chain0 < 0 || nch < 1 || chain0 + nch > nchains) { rc_set_error("rc_sampler_psm_counts_dev: bad chain range"); return RC_ERR_ARG; }
-  RC_CUDA(cudaSetDevice(device));
-  if (S == 0) { RC_CUDA(cudaMemset(counts_dev, 0, sizeof(int) * (size_t)n * n)); return RC_OK; }
-  return psm_counts_device(L + (size_t)chain0 * S * n, nch * S, n, (int*)counts_dev);
+  rc_sample_range v;
+  TRYP(rc_sampler_range(s, chain0, nch, "rc_sampler_psm_counts_dev", v));
+  Bufs B;
+  return psm_counts_device(v.labels, v.R, v.n, (int*)counts_dev, B);
 }
 
 int32_t rc_sampler_psm(const rc_sampler* s, int64_t chain0, int64_t nch, double* psm_out) {
   if (!s || !psm_out) { rc_set_error("rc_sampler_psm: null pointer"); return RC_ERR_ARG; }
-  int64_t S, n, nchains; int device;
-  rc_sampler_dev_labels(s, &S, &n, &nchains, &device);
-  RC_CUDA(cudaSetDevice(device));
-  int* counts = nullptr;
-  RC_CUDA(cudaMalloc(&counts, sizeof(int) * (size_t)n * n));
-  int st = rc_sampler_psm_counts_dev(s, chain0, nch, counts);
-  if (!st) st = rc_counts_to_host_psm(counts, (size_t)n * n, (double)(nch * S), psm_out);   // ./ numsamples (0/0 = NaN if no samples)
-  cudaFree(counts);
-  return st;
+  rc_sample_range v;
+  TRYP(rc_sampler_range(s, chain0, nch, "rc_sampler_psm", v));
+  Bufs B;
+  int* counts;
+  TRYP(B.get(&counts, (size_t)v.n * v.n));
+  TRYP(psm_counts_device(v.labels, v.R, v.n, counts, B));
+  return rc_counts_to_host_psm(counts, (size_t)v.n * v.n, (double)v.R, psm_out);   // ./ numsamples (0/0 = NaN if no samples)
 }
 
 // Exact co-clustering counts of S host label vectors into a caller DEVICE buffer (n x n int32): the per-rank half of
 // a PSM whose samples are sharded over GPUs (the caller all-reduces the counts and divides by the global S).
 int32_t rc_psm_counts_dev(const int64_t* labels, int64_t S, int64_t n, int32_t device, void* counts_dev) {
   if (!labels || !counts_dev || S < 0 || n < 1) { rc_set_error("rc_psm_counts_dev: bad arguments"); return RC_ERR_ARG; }
-  int cnt = 0;
-  if (cudaGetDeviceCount(&cnt) != cudaSuccess || cnt == 0) { rc_set_error("no CUDA device available (librcb200 has no CPU fallback)"); return RC_ERR_CUDA; }
-  RC_CUDA(cudaSetDevice(device));
+  TRYP(rc_select_device(device));
   if (S == 0) { RC_CUDA(cudaMemset(counts_dev, 0, sizeof(int) * (size_t)n * n)); return RC_OK; }
-  std::vector<uint8_t> L; std::vector<int> K;
-  int st = compact_labels(labels, S, n, L, K);
-  if (st) return st;
-  uint8_t* dL = nullptr;
-  RC_CUDA(cudaMalloc(&dL, L.size()));
-  cudaError_t e = cudaMemcpy(dL, L.data(), L.size(), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) st = psm_counts_device(dL, S, n, (int*)counts_dev);
-  cudaFree(dL);
-  RC_CUDA(e);
-  return st;
+  Bufs B;
+  uint8_t* dL; std::vector<int> K;
+  TRYP(upload_labels(labels, S, n, B, &dL, K));
+  return psm_counts_device(dL, S, n, (int*)counts_dev, B);
 }
 
 int32_t rc_psm(const int64_t* labels, int64_t S, int64_t n, int32_t device, double* psm_out) {
   if (!labels || !psm_out || S < 1 || n < 1) { rc_set_error("rc_psm: null pointer or empty input"); return RC_ERR_ARG; }
-  int cnt = 0;
-  if (cudaGetDeviceCount(&cnt) != cudaSuccess || cnt == 0) { rc_set_error("no CUDA device available (librcb200 has no CPU fallback)"); return RC_ERR_CUDA; }
-  RC_CUDA(cudaSetDevice(device));
+  TRYP(rc_select_device(device));
   const bool verbose = getenv("RCB200_VERBOSE") != nullptr;
   auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   const double t0 = now();
-  std::vector<uint8_t> L; std::vector<int> K;
-  int st = compact_labels(labels, S, n, L, K);
-  if (st) return st;
+  Bufs B;
+  uint8_t* dL; int* counts; std::vector<int> K;
+  TRYP(upload_labels(labels, S, n, B, &dL, K));
   const double t1 = now();
-  uint8_t* dL = nullptr; int* counts = nullptr;
-  RC_CUDA(cudaMalloc(&dL, L.size()));
-  RC_CUDA(cudaMemcpy(dL, L.data(), L.size(), cudaMemcpyHostToDevice));
-  if (cudaMalloc(&counts, sizeof(int) * (size_t)n * n) != cudaSuccess) { cudaFree(dL); rc_set_error("out of device memory"); return RC_ERR_CUDA; }
-  st = psm_counts_device(dL, S, n, counts);
+  TRYP(B.get(&counts, (size_t)n * n));
+  int st = psm_counts_device(dL, S, n, counts, B);
   const double t2 = now();
   if (!st) st = rc_counts_to_host_psm(counts, (size_t)n * n, (double)S, psm_out);
-  cudaFree(dL); cudaFree(counts);
-  if (verbose) fprintf(stderr, "[rcb200] rc_psm: relabel %.3f s, upload + counts %.3f s, download + divide %.3f s\n", t1 - t0, t2 - t1, now() - t2);
+  if (verbose) fprintf(stderr, "[rcb200] rc_psm: relabel + upload %.3f s, counts %.3f s, download + divide %.3f s\n", t1 - t0, t2 - t1, now() - t2);
   return st;
 }
 
@@ -551,50 +522,19 @@ int rc_binder_check_args(int64_t S, int64_t n, const char* who) {
   return RC_OK;
 }
 
-// The sampler's samples of chains [chain0, chain0 + nch) exist only after a run to numiters, and not for a chain that
-// stopped at the slot capacity (the rules of rc_sampler_predict).
-int rc_sampler_binder_check(const rc_sampler* s, int64_t chain0, int64_t nch, const char* who) {
-  int64_t S, n, nchains; int device;
-  rc_sampler_dev_labels(s, &S, &n, &nchains, &device);
-  if (chain0 < 0 || nch < 1 || chain0 + nch > nchains) { rc_set_error("%s: bad chain range", who); return RC_ERR_ARG; }
-  rc_params par; const int* K; const double *r, *p; int64_t done, numiters;
-  rc_sampler_dev_traces(s, &par, &done, &numiters, &K, &r, &p);
-  if (done < numiters) {
-    rc_set_error("%s: the sampler ran %lld of %lld iterations; its samples are recorded only by a complete run", who, (long long)done,
-                 (long long)numiters);
-    return RC_ERR_STATE;
-  }
-  for (int64_t c = chain0; c < chain0 + nch; ++c)
-    if (rc_sampler_chain_status(s, c) != 0) {
-      rc_set_error("%s: chain %lld stopped at the slot capacity; its samples are incomplete", who, (long long)c);
-      return RC_ERR_SLOTS;
-    }
-  return rc_binder_check_args(nch * S, n, who);
-}
-
-// W and P of the device-resident samples of chains [chain0, chain0 + nch) against counts of at most nmax samples.
-int rc_sampler_binder_wp(const rc_sampler* s, int64_t chain0, int64_t nch, const int* counts, int64_t nmax, unsigned long long* W,
-                         unsigned long long* P) {
-  int64_t S, n, nchains; int device;
-  const uint8_t* L = rc_sampler_dev_labels(s, &S, &n, &nchains, &device);
-  RC_CUDA(cudaSetDevice(device));
-  return binder_wp(L + (size_t)chain0 * S * n, nullptr, nch * S, n, counts, nmax, W, P, nullptr);
-}
-
 // counts, W, P and the totals of R device label vectors (sample-major, bytes)
 static int binder_device(const uint8_t* L, int64_t R, int64_t n, double* loss_sums, int64_t* best, int64_t* totals) {
-  int* counts = nullptr; uint8_t* Lt = nullptr;
-  RC_CUDA(cudaMalloc(&counts, sizeof(int) * (size_t)n * n));
+  Bufs B;
+  int* counts; const uint8_t* Lt;
+  TRYP(B.get(&counts, (size_t)n * n));
   const bool verbose = getenv("RCB200_VERBOSE") != nullptr;
   auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   const double t0 = now();
-  int st = psm_counts_device(L, R, n, counts, &Lt);
+  TRYP(psm_counts_device(L, R, n, counts, B, &Lt));
   const double t1 = now();
   std::vector<unsigned long long> W((size_t)R), P((size_t)R);
   float w_ms = 0;
-  if (!st) st = binder_wp(L, Lt, R, n, counts, R, W.data(), P.data(), &w_ms);
-  cudaFree(Lt); cudaFree(counts);
-  if (st) return st;
+  TRYP(binder_wp(L, Lt, R, n, counts, R, W.data(), P.data(), &w_ms));
   if (verbose)
     fprintf(stderr, "[rcb200] binder mpel: n=%lld samples=%lld counts %.3f ms, W kernel %.3f ms (CUDA events), %.3e pair-samples/s\n",
             (long long)n, (long long)R, (t1 - t0) * 1e3, w_ms, 0.5 * (double)n * (double)(n - 1) * (double)R / (w_ms * 1e-3));
@@ -605,53 +545,31 @@ extern "C" {
 
 int32_t rc_binder_mpel(const int64_t* labels, int64_t S, int64_t n, int32_t device, double* loss_sums, int64_t* best, int64_t* totals) {
   if (!labels) { rc_set_error("rc_binder_mpel: null pointer"); return RC_ERR_ARG; }
-  int st = rc_binder_check_args(S, n, "rc_binder_mpel");
-  if (st) return st;
-  st = rc_select_device(device);
-  if (st) return st;
-  std::vector<uint8_t> L; std::vector<int> K;
-  st = compact_labels(labels, S, n, L, K);
-  if (st) return st;
-  uint8_t* dL = nullptr;
-  RC_CUDA(cudaMalloc(&dL, L.size()));
-  cudaError_t e = cudaMemcpy(dL, L.data(), L.size(), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) st = binder_device(dL, S, n, loss_sums, best, totals);
-  cudaFree(dL);
-  RC_CUDA(e);
-  return st;
+  TRYP(rc_binder_check_args(S, n, "rc_binder_mpel"));
+  TRYP(rc_select_device(device));
+  Bufs B;
+  uint8_t* dL; std::vector<int> K;
+  TRYP(upload_labels(labels, S, n, B, &dL, K));
+  return binder_device(dL, S, n, loss_sums, best, totals);
 }
 
 int32_t rc_sampler_binder_mpel(const rc_sampler* s, int64_t chain0, int64_t nch, double* loss_sums, int64_t* best, int64_t* totals) {
   if (!s) { rc_set_error("rc_sampler_binder_mpel: null handle"); return RC_ERR_ARG; }
-  int st = rc_sampler_binder_check(s, chain0, nch, "rc_sampler_binder_mpel");
-  if (st) return st;
-  int64_t S, n, nchains; int device;
-  const uint8_t* L = rc_sampler_dev_labels(s, &S, &n, &nchains, &device);
-  RC_CUDA(cudaSetDevice(device));
-  return binder_device(L + (size_t)chain0 * S * n, nch * S, n, loss_sums, best, totals);   // chain-major, sample-minor
+  rc_sample_range v;
+  TRYP(rc_sampler_range(s, chain0, nch, "rc_sampler_binder_mpel", v));
+  TRYP(rc_binder_check_args(v.R, v.n, "rc_sampler_binder_mpel"));
+  return binder_device(v.labels, v.R, v.n, loss_sums, best, totals);   // chain-major, sample-minor
 }
 
 }  // extern "C"
-
-// Device buffers that are released when the call returns, whatever the path.
-struct DevScratch {
-  std::vector<void*> p;
-  ~DevScratch() { for (void* q : p) cudaFree(q); }
-  template <class T> cudaError_t get(T** out, size_t count) {
-    cudaError_t e = cudaMalloc((void**)out, sizeof(T) * (count ? count : 1));
-    if (e == cudaSuccess) p.push_back(*out);
-    return e;
-  }
-};
 
 // Shared front end of the MPEL entry points: relabel, upload, size the contingency table, and launch the pair-loss
 // kernel for the rows row_first, row_first + row_stride, ... (nrows of them).  mirror = 1 writes the full symmetric
 // S x S matrix M; mirror = 0 writes the rows' strict upper triangle into an nrows x S block.
 static int mpel_pairs(const int64_t* labels, int64_t S, int64_t n, int32_t loss, int64_t row_first, int64_t row_stride,
-                      int64_t nrows, int mirror, double* M, DevScratch& scr, int* kmax_out) {
-  std::vector<uint8_t> L; std::vector<int> K;
-  int st = compact_labels(labels, S, n, L, K);
-  if (st) return st;
+                      int64_t nrows, int mirror, double* M, Bufs& B, int* kmax_out) {
+  uint8_t* dL; std::vector<int> K;
+  TRYP(upload_labels(labels, S, n, B, &dL, K));
   int kmax = 0;
   for (int k : K) kmax = std::max(kmax, k);
   if (kmax_out) *kmax_out = kmax;
@@ -661,9 +579,8 @@ static int mpel_pairs(const int64_t* labels, int64_t S, int64_t n, int32_t loss,
   if (smem > 220 * 1024) { rc_set_error("rc_mpel: n = %lld with %d x %d clusters does not fit shared memory", (long long)n, kmax, kmax); return RC_ERR_SLOTS; }
   int stride = (int)((n + 31) / 32);
   while ((stride & 3) || !((stride >> 2) & 1)) ++stride;      // multiple of 4 with an odd quotient: lane segments start in different banks
-  uint8_t* dL = nullptr; int* dK = nullptr; double* nlogn = nullptr;
-  if (scr.get(&dL, L.size()) || scr.get(&dK, (size_t)S) || scr.get(&nlogn, (size_t)(n + 1))) { rc_set_error("rc_mpel: out of device memory"); return RC_ERR_CUDA; }
-  RC_CUDA(cudaMemcpy(dL, L.data(), L.size(), cudaMemcpyHostToDevice));
+  int* dK; double* nlogn;
+  TRYP(B.get(&dK, (size_t)S)); TRYP(B.get(&nlogn, (size_t)(n + 1)));
   RC_CUDA(cudaMemcpy(dK, K.data(), sizeof(int) * S, cudaMemcpyHostToDevice));
   k_nlogn<<<(unsigned)((n + 256) / 256), 256>>>(n, nlogn);
   RC_CUDA(cudaFuncSetAttribute(k_pair_loss, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -684,13 +601,6 @@ static int mpel_argmin(const double* sums_dev, int64_t S, double* loss_sums, int
   return RC_OK;
 }
 
-static int mpel_device_ready(int32_t device) {
-  int cnt = 0;
-  if (cudaGetDeviceCount(&cnt) != cudaSuccess || cnt == 0) { rc_set_error("no CUDA device available (librcb200 has no CPU fallback)"); return RC_ERR_CUDA; }
-  RC_CUDA(cudaSetDevice(device));
-  return RC_OK;
-}
-
 extern "C" {
 
 // Multi-GPU MPEL (SURVEY 8e): the candidate rows row_first, row_first + row_stride, ... (nrows of them) of the strict
@@ -702,43 +612,38 @@ int32_t rc_mpel_rows_dev(const int64_t* labels, int64_t S, int64_t n, int32_t lo
   if (!labels || !M_rows_dev || S < 1 || n < 1 || loss < 0 || loss > 3 || row_first < 0 || row_stride < 1 || nrows < 0) {
     rc_set_error("rc_mpel_rows_dev: bad arguments"); return RC_ERR_ARG;
   }
-  int st = mpel_device_ready(device);
-  if (st) return st;
-  DevScratch scr;
+  TRYP(rc_select_device(device));
+  Bufs B;
   RC_CUDA(cudaMemset(M_rows_dev, 0, sizeof(double) * (size_t)nrows * S));
-  st = mpel_pairs(labels, S, n, loss, row_first, row_stride, nrows, 0, (double*)M_rows_dev, scr, nullptr);
-  if (st) return st;
+  TRYP(mpel_pairs(labels, S, n, loss, row_first, row_stride, nrows, 0, (double*)M_rows_dev, B, nullptr));
   RC_CUDA(cudaDeviceSynchronize());
   return RC_OK;
 }
 
 int32_t rc_mpel_finish_dev(const void* M_upper_dev, int64_t S, int32_t device, double* loss_sums, int64_t* best) {
   if (!M_upper_dev || S < 1) { rc_set_error("rc_mpel_finish_dev: bad arguments"); return RC_ERR_ARG; }
-  int st = mpel_device_ready(device);
-  if (st) return st;
-  DevScratch scr;
-  double* sums = nullptr;
-  if (scr.get(&sums, (size_t)S)) { rc_set_error("rc_mpel: out of device memory"); return RC_ERR_CUDA; }
+  TRYP(rc_select_device(device));
+  Bufs B;
+  double* sums;
+  TRYP(B.get(&sums, (size_t)S));
   k_colsum_upper<<<(unsigned)((S + 127) / 128), 128>>>((const double*)M_upper_dev, S, sums);
   return mpel_argmin(sums, S, loss_sums, best);
 }
 
 int32_t rc_mpel(const int64_t* labels, int64_t S, int64_t n, int32_t loss, int32_t device, double* loss_sums, int64_t* best) {
   if (!labels || S < 1 || n < 1 || loss < 0 || loss > 3) { rc_set_error("rc_mpel: bad arguments"); return RC_ERR_ARG; }
-  int st = mpel_device_ready(device);
-  if (st) return st;
-  DevScratch scr;
-  double *M = nullptr, *sums = nullptr;
-  if (scr.get(&M, (size_t)S * S) || scr.get(&sums, (size_t)S)) { rc_set_error("rc_mpel: out of device memory"); return RC_ERR_CUDA; }
+  TRYP(rc_select_device(device));
+  Bufs B;
+  double *M, *sums;
+  TRYP(B.get(&M, (size_t)S * S)); TRYP(B.get(&sums, (size_t)S));
   RC_CUDA(cudaMemset(M, 0, sizeof(double) * (size_t)S * S));
   const bool verbose = getenv("RCB200_VERBOSE") != nullptr;
   auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   int kmax = 0;
-  st = mpel_pairs(labels, S, n, loss, 0, 1, S, 1, M, scr, &kmax);
-  if (st) return st;
+  TRYP(mpel_pairs(labels, S, n, loss, 0, 1, S, 1, M, B, &kmax));
   const double tk = now();
   k_colsum<<<(unsigned)((S + 127) / 128), 128>>>(M, S, sums);
-  st = mpel_argmin(sums, S, loss_sums, best);
+  const int st = mpel_argmin(sums, S, loss_sums, best);
   if (verbose) {
     const double dt = now() - tk;
     fprintf(stderr, "[rcb200] rc_mpel: S=%lld n=%lld kmax=%d loss=%d pair kernel + column sums %.3f s (%.3e pairs/s)\n", (long long)S, (long long)n, kmax,

@@ -25,10 +25,6 @@
 #include "rc_common.cuh"
 #include "rc_labels.h"
 
-extern "C" const uint8_t* rc_sampler_dev_labels(const rc_sampler* s, int64_t* S, int64_t* n, int64_t* nchains, int* device);
-extern "C" const rc_data* rc_sampler_dev_traces(const rc_sampler* s, rc_params* par, int64_t* iters_done, int64_t* numiters, const int** K,
-                                                const double** r, const double** p);
-
 namespace {
 
 #define PX 4                          // new points per CTA of k_pred_sums and k_pred_cocl
@@ -335,20 +331,6 @@ struct PTimer {
   ~PTimer() { for (cudaEvent_t e : ev) cudaEventDestroy(e); }
 };
 
-// Device buffers of one call, released on every return path.
-struct Bufs {
-  std::vector<void*> p;
-  template <class T> int get(T** out, size_t count) {
-    *out = nullptr;
-    cudaError_t e = cudaMalloc((void**)out, sizeof(T) * std::max<size_t>(count, 1));
-    if (e != cudaSuccess) { (void)cudaGetLastError(); rc_set_error("out of device memory (%zu bytes)", sizeof(T) * count); return RC_ERR_CUDA; }
-    p.push_back(*out);
-    return RC_OK;
-  }
-  ~Bufs() { for (void* q : p) cudaFree(q); }
-};
-#define TRYP(x) do { int st_ = (x); if (st_) return st_; } while (0)
-
 // Validate Dnew (m x n host) and build its fixed-point image at each row's augmented-data scales.
 int new_image(const rc_data* d, const double* Dnew, int64_t m, Bufs& B, longlong2** img, int2** qdev, PTimer& tm) {
   const int64_t n = d->n;
@@ -461,17 +443,16 @@ int32_t rc_predict(const rc_data* d, const rc_params* par, const double* Dnew, i
     rc_set_error("rc_predict: null pointer or bad size"); return RC_ERR_ARG;
   }
   TRYP(check_rp(r, p, S));
-  std::vector<uint8_t> L; std::vector<int> K;
-  if (S > 0) TRYP(compact_labels(labels, S, d->n, L, K));
   TRYP(rc_select_device(d->device));
   Bufs B;
+  uint8_t* dl = nullptr; std::vector<int> K;
+  if (S > 0) TRYP(upload_labels(labels, S, d->n, B, &dl, K));
   PTimer tm;
   longlong2* img; int2* q;
   TRYP(new_image(d, Dnew, m, B, &img, &q, tm));
-  uint8_t* dl = nullptr; double *dr = nullptr, *dp = nullptr;
-  TRYP(B.get(&dl, L.size())); TRYP(B.get(&dr, (size_t)S)); TRYP(B.get(&dp, (size_t)S));
+  double *dr, *dp;
+  TRYP(B.get(&dr, (size_t)S)); TRYP(B.get(&dp, (size_t)S));
   if (S > 0) {
-    RC_CUDA(cudaMemcpy(dl, L.data(), L.size(), cudaMemcpyHostToDevice));
     RC_CUDA(cudaMemcpy(dr, r, sizeof(double) * (size_t)S, cudaMemcpyHostToDevice));
     RC_CUDA(cudaMemcpy(dp, p, sizeof(double) * (size_t)S, cudaMemcpyHostToDevice));
   }
@@ -482,33 +463,17 @@ int32_t rc_predict(const rc_data* d, const rc_params* par, const double* Dnew, i
 int32_t rc_sampler_predict(const rc_sampler* s, const double* Dnew, int64_t m, int64_t chain0, int64_t nch, double* cocl_out,
                            double* newcl_out) {
   if (!s || !Dnew || !cocl_out || !newcl_out || m < 1) { rc_set_error("rc_sampler_predict: null pointer or bad size"); return RC_ERR_ARG; }
-  int64_t S, n, nchains; int device;
-  const uint8_t* lab = rc_sampler_dev_labels(s, &S, &n, &nchains, &device);
-  if (chain0 < 0 || nch < 1 || chain0 + nch > nchains) { rc_set_error("rc_sampler_predict: bad chain range"); return RC_ERR_ARG; }
-  rc_params P; const int* Kd; const double *r, *p; int64_t done, numiters;
-  const rc_data* d = rc_sampler_dev_traces(s, &P, &done, &numiters, &Kd, &r, &p);
-  // only a run to numiters has recorded every sample, and a chain stopped by the slot capacity has not
-  if (done < numiters) {
-    rc_set_error("rc_sampler_predict: the sampler ran %lld of %lld iterations; its samples are recorded only by a complete run",
-                 (long long)done, (long long)numiters);
-    return RC_ERR_STATE;
-  }
-  for (int64_t c = chain0; c < chain0 + nch; ++c)
-    if (rc_sampler_chain_status(s, c) != 0) {
-      rc_set_error("rc_sampler_predict: chain %lld stopped at the slot capacity; its samples are incomplete", (long long)c);
-      return RC_ERR_SLOTS;
-    }
-  TRYP(rc_select_device(device));
+  rc_sample_range v;
+  TRYP(rc_sampler_range(s, chain0, nch, "rc_sampler_predict", v));
   Bufs B;
   PTimer tm;
   longlong2* img; int2* q;
-  TRYP(new_image(d, Dnew, m, B, &img, &q, tm));
-  const int64_t total = nch * S, first = chain0 * S;     // chain-major, sample-minor, as the recorded traces
-  std::vector<int> K((size_t)total);
-  if (total > 0) RC_CUDA(cudaMemcpy(K.data(), Kd + first, sizeof(int) * (size_t)total, cudaMemcpyDeviceToHost));
+  TRYP(new_image(v.d, Dnew, m, B, &img, &q, tm));
+  std::vector<int> K((size_t)v.R);
+  if (v.R > 0) RC_CUDA(cudaMemcpy(K.data(), v.K, sizeof(int) * (size_t)v.R, cudaMemcpyDeviceToHost));
   const int Kmax = K.empty() ? 1 : *std::max_element(K.begin(), K.end());
   if (Kmax > RC_MAXCAP_INC) { rc_set_error("rc_sampler_predict: recorded K = %d exceeds %d", Kmax, RC_MAXCAP_INC); return RC_ERR_STATE; }
-  return predict_core(d, P, img, q, m, lab + (size_t)first * n, r + first, p + first, total, Kmax, cocl_out, newcl_out, nullptr, B, tm);
+  return predict_core(v.d, v.par, img, q, m, v.labels, v.r, v.p, v.R, Kmax, cocl_out, newcl_out, nullptr, B, tm);
 }
 
 int32_t rc_crossdist(const double* X, int64_t n, const double* Y, int64_t m, int64_t dim, int32_t device, double* out) {

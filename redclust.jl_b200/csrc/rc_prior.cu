@@ -380,12 +380,11 @@ int32_t rc_kmeans(const double* X, int64_t n, int64_t dim, int64_t k, const int6
   if (!X || !assignments || n < 1 || dim < 1 || k < 1 || k > n || maxiter < 0 || (!init_idx && !u01) || n > 0x7fffff00LL || k > 0x7fffffLL) {
     rc_set_error("rc_kmeans: bad arguments (need 1 <= k <= n, dim >= 1 and either init_idx or u01)"); return RC_ERR_ARG;
   }
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) { rc_set_error("rc_kmeans: no CUDA device (librcb200 has no CPU path)"); return RC_ERR_CUDA; }
+  const int st = rc_select_device(device);
+  if (st) return st;
   if (init_idx)
     for (int64_t c = 0; c < k; ++c)
       if (init_idx[c] < 0 || init_idx[c] >= n) { rc_set_error("rc_kmeans: initial centre index out of range"); return RC_ERR_ARG; }
-  RC_CUDA(cudaSetDevice(device));
   const int nb = (int)((n + 127) / 128), nba = (int)((n + 31) / 32);          // blocks of the seeding / of the assignment
   int P = (int)(592 / k); if (P < 1) P = 1; if (P > 64) P = 64;
   while (P > 1 && (n + P - 1) / P < 64) --P;
