@@ -236,6 +236,25 @@ int32_t rc_binder_mpel(const int64_t* labels, int64_t S, int64_t n, int32_t devi
  * of the range stopped at the slot capacity, RC_ERR_ARG for a bad range.                                                */
 int32_t rc_sampler_binder_mpel(const rc_sampler* s, int64_t chain0, int64_t nch, double* loss_sums, int64_t* best, int64_t* totals);
 
+/* ---- convergence across chains (no reference equivalent; the reference's diagnostics are per chain, src/mcmc.jl:564-573) --
+ * Split-R-hat (BDA3 11.4) of every point pair's co-clustering indicator [c(a) = c(b)], which does not depend on the labels,
+ * over C chains of S recorded samples: L = floor(S / 2), chain c gives group 2c = its samples [0, L) and group 2c + 1 = its
+ * samples [S - L, S) (the middle sample of an odd S is dropped), m = 2C.  With N_g the samples of group g in which a and b
+ * share a label, N = sum N_g, Q = sum N_g^2, Wn = L N - Q, Bn = m Q - N^2 (exact int64):
+ *   R = sqrt((L-1)/L + ((L-1) Bn) / ((m-1) L Wn)) for Wn > 0, 1 for Wn = Bn = 0, +Inf for Wn = 0 < Bn.
+ * sum: the largest R over a < b, its pair (0-based, first in row-major order on ties) and the number of pairs with R > 1.01
+ * (Vehtari et al. 2021).  rhat_out: NULL or the n x n matrix (symmetric, unit diagonal).  meandev / maxdev: NULL or one value
+ * per chain, the mean and largest |p_c - pbar| over the pairs, p_c chain c's co-clustering frequency over its 2L samples and
+ * pbar the pooled one.  labels: nchains x S x n (chain-major, any positive labels).  Needs S >= 4, 2 <= n <= 65 535 and
+ * m L < 2^31 (RC_ERR_ARG); buffers that do not fit the free device memory are refused with their sizes (RC_ERR_CUDA).  */
+typedef struct rc_rhat_summary { double max; int64_t a, b, above; } rc_rhat_summary;
+int32_t rc_cocl_rhat(const int64_t* labels, int64_t nchains, int64_t S, int64_t n, int32_t device, rc_rhat_summary* sum,
+                     double* rhat_out, double* meandev, double* maxdev);
+/* The same over the device-resident samples of chains [chain0, chain0 + nch) of a sampler.  RC_ERR_STATE before a run to
+ * numiters, RC_ERR_SLOTS when a chain of the range stopped at the slot capacity, RC_ERR_ARG for a bad range.            */
+int32_t rc_sampler_cocl_rhat(const rc_sampler* s, int64_t chain0, int64_t nch, rc_rhat_summary* sum, double* rhat_out,
+                             double* meandev, double* maxdev);
+
 /* ---- multi-GPU exchange steps (SURVEY.md 8e) -------------------------------------------------------
  * One process per GPU.  The sampler needs no collective (independent chains: chain_offset above).  The three steps
  * that exchange data run over an NCCL communicator owned by an rc_comm handle: rank 0 calls rc_comm_unique_id, the
@@ -249,6 +268,9 @@ int32_t rc_sampler_binder_mpel(const rc_sampler* s, int64_t chain0, int64_t nch,
  *   rc_comm_sampler_binder_mpel  src/pointestimate.jl:34-59,68-76 over the chains of every rank (src/mcmc.jl:560): the
  *                             all-reduced counts, per-rank int64 W and P, ONE all-gather; every rank gets T over all
  *                             samples in rank order (= global chain order; *best indexes that concatenation)
+ *   rc_comm_sampler_cocl_rhat  rc_sampler_cocl_rhat over the chains of every rank: the all-reduced counts N, each rank's Q
+ *                             of its own chains, ONE all-reduce of Q and ONE all-gather of the chains' deviations;
+ *                             meandev / maxdev hold every rank's chains in rank order
  * psm_out (host, n x n fp64) and counts_dev_out (device, n x n int32) may each be NULL.  Results are bit-equal to the
  * single-GPU entry points.                                                                              */
 typedef struct rc_comm rc_comm;
@@ -262,6 +284,8 @@ int32_t rc_comm_sampler_psm(rc_comm* c, const rc_sampler* s, double* psm_out, vo
 int32_t rc_comm_psm(rc_comm* c, const int64_t* labels, int64_t S_local, int64_t n, double* psm_out, void* counts_dev_out);
 int32_t rc_comm_mpel(rc_comm* c, const int64_t* labels, int64_t S, int64_t n, int32_t loss, double* loss_sums, int64_t* best);
 int32_t rc_comm_sampler_binder_mpel(rc_comm* c, const rc_sampler* s, double* loss_sums, int64_t* best, int64_t* totals);
+int32_t rc_comm_sampler_cocl_rhat(rc_comm* c, const rc_sampler* s, rc_rhat_summary* sum, double* rhat_out, double* meandev,
+                                  double* maxdev);
 
 #ifdef __cplusplus
 }

@@ -13,6 +13,7 @@ The directory name contains a dot, so it is loaded under the module name `redclu
 from .host import (Comm, MCMCOptionsList, PriorHyperparamsList, MCMCData, MCMCState, MCMCResult, Sampler, runsampler,
                    getpointestimate, binderloss, infodist, adjacencymatrix, sortlabels, makematrix, uppertriangle,
                    generatemixture, example_dataset, example_datasets, prettytime, prettynumber, evaluateclustering, summarise, params_from_labels, pair_stats, psm, psm_counts_dev, psm_sharded, mpel_loss_sums, binder_loss_sums, mpel_loss_sums_sharded, cyclic_rows, assemble_cyclic_rows, init_rp, ArgumentError,
-                   crossdistances, predictivecoclustering, allocationprobabilities, predictive_from_labels)
+                   crossdistances, predictivecoclustering, allocationprobabilities, predictive_from_labels,
+                   convergencediagnostics, cocl_rhat)
 from ._lib import RCError, LIB_PATH
 from .prior import fitprior, fitprior2, sampledist, sampleK, kmedoids, kmedoids_device, kmeans

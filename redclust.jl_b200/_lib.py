@@ -20,6 +20,10 @@ class rc_params(C.Structure):
         ("K_initial", C.c_int64), ("maxK", C.c_int64), ("repulsion", C.c_int32), ("_pad", C.c_int32)]
 
 
+class rc_rhat_summary(C.Structure):
+    _fields_ = [("max", C.c_double), ("a", C.c_int64), ("b", C.c_int64), ("above", C.c_int64)]
+
+
 class RCError(RuntimeError):
     """ErrorException of the Julia API (error(...) in src/types.jl)."""
 
@@ -83,6 +87,8 @@ SIGNATURES = {
     "rc_mpel_finish_dev": (C.c_int32, [_vp, C.c_int64, C.c_int32, _vp, _P(C.c_int64)]),
     "rc_binder_mpel": (C.c_int32, [_vp, C.c_int64, C.c_int64, C.c_int32, _vp, _P(C.c_int64), _vp]),
     "rc_sampler_binder_mpel": (C.c_int32, [_vp, C.c_int64, C.c_int64, _vp, _P(C.c_int64), _vp]),
+    "rc_cocl_rhat": (C.c_int32, [_vp, C.c_int64, C.c_int64, C.c_int64, C.c_int32, _P(rc_rhat_summary), _vp, _vp, _vp]),
+    "rc_sampler_cocl_rhat": (C.c_int32, [_vp, C.c_int64, C.c_int64, _P(rc_rhat_summary), _vp, _vp, _vp]),
     "rc_comm_unique_id": (C.c_int32, [_vp]),
     "rc_comm_init": (C.c_int32, [_vp, C.c_int32, C.c_int32, C.c_int32, _P(_vp)]),
     "rc_comm_info": (C.c_int32, [_vp, _P(C.c_int32), _P(C.c_int32)]),
@@ -93,6 +99,7 @@ SIGNATURES = {
     "rc_comm_psm": (C.c_int32, [_vp, _vp, C.c_int64, C.c_int64, _vp, _vp]),
     "rc_comm_mpel": (C.c_int32, [_vp, _vp, C.c_int64, C.c_int64, C.c_int32, _vp, _P(C.c_int64)]),
     "rc_comm_sampler_binder_mpel": (C.c_int32, [_vp, _vp, _vp, _P(C.c_int64), _vp]),
+    "rc_comm_sampler_cocl_rhat": (C.c_int32, [_vp, _vp, _P(rc_rhat_summary), _vp, _vp, _vp]),
 }
 
 

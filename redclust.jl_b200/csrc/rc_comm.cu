@@ -300,6 +300,61 @@ int32_t rc_comm_sampler_binder_mpel(rc_comm* c, const rc_sampler* s, double* los
   return rc_binder_finish(W.data(), P.data(), total, n, loss_sums, best, totals);
 }
 
+// Split-R-hat of the co-clustering indicators over the chains of every rank (rc_rhat.cu): this rank's pooled counts,
+// all-reduced as rc_comm_sampler_psm does; pass 2 over the rank's own chains against them with m = 2 x all chains; ONE
+// all-reduce of Q (int64) and ONE all-gather of the chains' {sum d, max d} padded to the largest rank; every rank then
+// finishes.  Integers throughout: identical to one GPU over the same chains.  The buffers are sized before the status
+// exchange, so a rank that cannot hold them refuses with the others.
+int32_t rc_comm_sampler_cocl_rhat(rc_comm* c, const rc_sampler* s, rc_rhat_summary* sum, double* rhat_out, double* meandev,
+                                  double* maxdev) {
+  if (!c || !s) { rc_set_error("rc_comm_sampler_cocl_rhat: null handle"); return RC_ERR_ARG; }
+  RC_CUDA(cudaSetDevice(c->device));
+  const char* who = "rc_comm_sampler_cocl_rhat";
+  const int64_t Cl = rc_sampler_nchains(s), S = rc_sampler_numsamples(s);
+  rc_sample_range v;
+  Bufs B;
+  RhatDev d;
+  RhatTimes t;
+  int local = rc_sampler_range(s, 0, Cl, who, v);
+  if (!local) local = rhat_check_args(Cl, S, v.n, who);
+  if (!local) local = rhat_alloc(Cl, S, v.n, rhat_out != nullptr, B, d, who);
+  std::vector<long long> all;
+  TRYP(agree(c, local, local ? 0 : Cl, who, all));
+  const int64_t n = v.n;
+  int64_t C = 0, per = 0;
+  for (int r = 0; r < c->world; ++r) {
+    C += all[2 * r + 1];
+    per = std::max<int64_t>(per, all[2 * r + 1]);
+  }
+  TRYP(rhat_check_args(C, S, n, who));                          // the same on every rank
+  unsigned long long* buf;                                     // [world + 1][2 per]: this rank's chains, then the gathered ranks
+  TRYP(B.get(&buf, 2 * (size_t)per * (c->world + 1)));
+  RC_CUDA(cudaMemset(buf, 0, sizeof(unsigned long long) * 2 * (size_t)per));
+  TRYP(rhat_pass1(v.labels, Cl, S, n, d, t));
+  TRYP(finish_psm(c, d.N, n, (long long)(Cl * S), nullptr));
+  TRYP(rhat_pass2(v.labels, Cl, S, n, 2 * C, d, t));
+  RC_CUDA(cudaMemcpy(buf, d.dev, sizeof(unsigned long long) * 2 * (size_t)Cl, cudaMemcpyDeviceToDevice));
+  if (c->world > 1) {
+    if (nccl()->AllReduce(d.Q, d.Q, (size_t)(n * n), ncclInt64, ncclSum, c->comm, c->stream) != ncclSuccess ||
+        nccl()->AllGather(buf, buf + 2 * per, 2 * (size_t)per, ncclInt64, c->comm, c->stream) != ncclSuccess ||
+        cudaStreamSynchronize(c->stream) != cudaSuccess) {
+      rc_set_error("%s: all-reduce of Q or all-gather of the chain deviations failed", who); return RC_ERR_CUDA;
+    }
+  } else {
+    RC_CUDA(cudaMemcpy(buf + 2 * per, buf, sizeof(unsigned long long) * 2 * (size_t)per, cudaMemcpyDeviceToDevice));
+  }
+  std::vector<unsigned long long> gathered(2 * (size_t)per * c->world), dev;   // rank order = global chain order
+  RC_CUDA(cudaMemcpy(gathered.data(), buf + 2 * per, sizeof(unsigned long long) * gathered.size(), cudaMemcpyDeviceToHost));
+  for (int r = 0; r < c->world; ++r) {
+    const unsigned long long* g = gathered.data() + 2 * (size_t)per * r;
+    dev.insert(dev.end(), g, g + 2 * all[2 * r + 1]);
+  }
+  TRYP(rhat_finish(d, S, n, 2 * C, sum, rhat_out, t));
+  rhat_deviations(dev.data(), C, S, n, 2 * C, meandev, maxdev);
+  rhat_report(t, Cl, S, n);
+  return RC_OK;
+}
+
 // MPEL search with the candidate samples dealt cyclically over the ranks (src/pointestimate.jl:49-57): every rank holds
 // all S label vectors, evaluates rows rank, rank + world, ... of the upper triangle of the loss matrix, one all-gather
 // assembles it, the column sums run in ascending row order -- bit-equal to rc_mpel on one GPU.

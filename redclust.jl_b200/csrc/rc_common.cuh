@@ -73,6 +73,25 @@ int binder_wp(const uint8_t* L, const uint8_t* Lt, int64_t R, int64_t n, const i
 int rc_binder_finish(const unsigned long long* W, const unsigned long long* P, int64_t S, int64_t n, double* loss_sums,
                      int64_t* best, int64_t* totals);
 
+// split-R-hat of the co-clustering indicators (rc_rhat.cu).  The limits on chains, samples per chain and n; the device
+// buffers of one call (N the pooled counts, Q = sum of squared group counts, Na / Nb one chain's halves, dev = {sum d,
+// max d} per local chain, R the matrix or NULL); pass 1 (N), pass 2 (Q and dev against the N of m groups in all), the
+// finish (summary, matrix) and the deviations from the host copy of dev.  RhatTimes: CUDA-event times with RCB200_VERBOSE.
+struct RhatDev {
+  int *N, *Na, *Nb;
+  long long* Q;
+  unsigned long long* dev;
+  double* R;
+};
+struct RhatTimes { float pass1_ms = 0, pass2_counts_ms = 0, acc_ms = 0, finish_ms = 0; };
+int rhat_check_args(int64_t C, int64_t S, int64_t n, const char* who);
+int rhat_alloc(int64_t Cl, int64_t S, int64_t n, bool matrix, Bufs& B, RhatDev& d, const char* who);
+int rhat_pass1(const uint8_t* L, int64_t Cl, int64_t S, int64_t n, RhatDev& d, RhatTimes& t);
+int rhat_pass2(const uint8_t* L, int64_t Cl, int64_t S, int64_t n, int64_t m, RhatDev& d, RhatTimes& t);
+int rhat_finish(const RhatDev& d, int64_t S, int64_t n, int64_t m, rc_rhat_summary* sum, double* rhat_out, RhatTimes& t);
+void rhat_deviations(const unsigned long long* dev, int64_t C, int64_t S, int64_t n, int64_t m, double* meandev, double* maxdev);
+void rhat_report(const RhatTimes& t, int64_t C, int64_t S, int64_t n);
+
 // ---- 128-bit two's complement accumulators (block totals of the fixed-point images) ------------
 struct rc_i128 {
   unsigned long long lo;

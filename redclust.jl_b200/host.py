@@ -24,7 +24,7 @@ import os
 import numpy as np
 
 from . import _lib
-from ._lib import RCError, rc_options, rc_params, check, ptr, lib
+from ._lib import RCError, rc_options, rc_params, rc_rhat_summary, check, ptr, lib
 
 
 class ArgumentError(ValueError):
@@ -385,6 +385,52 @@ class Sampler:
             out["clust"] = self.samples(out["chain"])["labels"][out["index"]]
         return out
 
+    def _traces(self, chain0, nch):
+        """K, r, p, loglik and logposterior of chains chain0 .. chain0 + nch - 1 as nch x numsamples arrays."""
+        S = int(lib().rc_sampler_numsamples(self._h))
+        out = {k: np.empty((nch, S)) for k in _TRACES}
+        K = np.empty(S, np.int64)
+        for i, c in enumerate(range(chain0, chain0 + nch)):
+            check(lib().rc_sampler_copy_samples(self._h, c, None, ptr(K), *(ptr(out[k][i]) for k in _TRACES[1:])))
+            out["K"][i] = K
+        return out
+
+    def convergencediagnostics(self, chain0=0, nch=None, matrix=False):
+        """Convergence across chains chain0 .. chain0 + nch - 1 (rc_sampler_cocl_rhat): the split-R-hat of every point pair's
+        co-clustering indicator, computed from the device-resident samples, and each chain's distance from the pooled PSM,
+        with the split-R-hat of the traces K, r, p, loglik and logposterior.  Returns dict(rhat_max, rhat_pair = (a, b)
+        0-based, pairs_above = pairs with R-hat > 1.01, chain_meandev / chain_maxdev = mean and largest |p_c - pbar| over
+        the pairs per chain, rhat = the n x n matrix when matrix=True else None, traces = {name: split-R-hat})."""
+        nch = self.nchains - chain0 if nch is None else nch
+        n, k = self.data.n, max(nch, 0)
+        sm, md, xd = rc_rhat_summary(), np.empty(k), np.empty(k)
+        R = np.empty((n, n)) if matrix else None
+        check(lib().rc_sampler_cocl_rhat(self._h, chain0, nch, C.byref(sm), ptr(R), ptr(md), ptr(xd)))
+        tr = self._traces(chain0, nch)
+        return _rhat_dict(sm, R, md, xd, {name: _split_rhat(x) for name, x in tr.items()})
+
+    def convergencediagnostics_allreduce(self, group=None, device=None, comm=None, matrix=False):
+        """convergencediagnostics over the chains of every rank (rc_comm_sampler_cocl_rhat): the all-reduced co-clustering
+        counts, one ncclAllReduce of the squared group counts and one ncclAllGather of the chain deviations; equal to one
+        GPU over the same chains.  chain_meandev / chain_maxdev and the traces cover every rank's chains in rank order."""
+        comm = comm or Comm.from_torch(group, self.data.device if device is None else device)
+        if comm.world > 1:
+            import torch.distributed as dist
+            sizes = [None] * comm.world
+            dist.all_gather_object(sizes, self.nchains, group=group)
+        else:
+            sizes = [self.nchains]
+        n, total = self.data.n, sum(sizes)
+        sm, md, xd = rc_rhat_summary(), np.empty(total), np.empty(total)
+        R = np.empty((n, n)) if matrix else None
+        check(lib().rc_comm_sampler_cocl_rhat(comm._h, self._h, C.byref(sm), ptr(R), ptr(md), ptr(xd)))
+        tr = self._traces(0, self.nchains)
+        if comm.world > 1:
+            parts = [None] * comm.world
+            dist.all_gather_object(parts, tr, group=group)
+            tr = {k: np.concatenate([p[k] for p in parts]) for k in _TRACES}
+        return _rhat_dict(sm, R, md, xd, {name: _split_rhat(x) for name, x in tr.items()})
+
     def close(self):
         L = getattr(_lib, "_lib", None)
         if getattr(self, "_h", None) and L is not None:
@@ -675,6 +721,68 @@ def binder_loss_sums(labels, device=0):
     sums, totals, best = np.empty(L.shape[0]), np.empty(L.shape[0], np.int64), C.c_int64()
     check(lib().rc_binder_mpel(ptr(L), L.shape[0], L.shape[1], device, ptr(sums), C.byref(best), ptr(totals)))
     return sums, int(best.value), totals
+
+
+# ---- convergence across chains (no reference equivalent: the reference's diagnostics are per chain, mcmc.jl:564-573) ----
+_TRACES = ("K", "r", "p", "loglik", "logposterior")
+
+
+def _split_rhat(x):
+    """Split-R-hat (BDA3 11.4) of a C x S trace: the first and last floor(S / 2) samples of every chain are the 2C groups
+    (the middle sample of an odd S is dropped); sqrt(var+ / W) with W the mean within-group sample variance (ddof = 1) and
+    B / L the sample variance of the group means.  W = 0 means every group is constant, decided by comparing the values:
+    1 when they all hold the same value, +Inf otherwise."""
+    x = np.asarray(x, dtype=np.float64)
+    S = x.shape[1]
+    if S < 4:
+        raise ArgumentError("split-R-hat needs at least 4 samples per chain.")
+    L = S // 2
+    g = np.concatenate([x[:, :L], x[:, S - L:]])
+    if np.all(g == g[:, :1]):
+        return 1.0 if np.all(g == g[0, 0]) else math.inf
+    W = float(np.mean(np.var(g, axis=1, ddof=1)))
+    B = L * float(np.var(np.mean(g, axis=1), ddof=1))
+    return math.sqrt(((L - 1) / L * W + B / L) / W)
+
+
+def _rhat_dict(sm, R, meandev, maxdev, traces):
+    return dict(rhat_max=float(sm.max), rhat_pair=(int(sm.a), int(sm.b)), pairs_above=int(sm.above), chain_meandev=meandev,
+                chain_maxdev=maxdev, rhat=R, traces=traces)
+
+
+def cocl_rhat(labels, device=0, matrix=False):
+    """The co-clustering part of convergencediagnostics for host label vectors, labels = C chains x S samples x n points
+    (any positive labels; rc_cocl_rhat): dict(rhat_max, rhat_pair, pairs_above, chain_meandev, chain_maxdev, rhat)."""
+    L = np.ascontiguousarray(np.asarray(labels, dtype=np.int64))
+    if L.ndim != 3:
+        raise ArgumentError("labels must be a chains × samples × n array.")
+    Cn, S, n = L.shape
+    sm, md, xd = rc_rhat_summary(), np.empty(Cn), np.empty(Cn)
+    R = np.empty((n, n)) if matrix else None
+    check(lib().rc_cocl_rhat(ptr(L), Cn, S, n, device, C.byref(sm), ptr(R), ptr(md), ptr(xd)))
+    out = _rhat_dict(sm, R, md, xd, None)
+    del out["traces"]
+    return out
+
+
+def convergencediagnostics(results, device=0, matrix=False):
+    """Convergence across the chains of a list of MCMCResult (runsampler with nchains > 1): the split-R-hat of every point
+    pair's co-clustering indicator (labels switch between chains, these indicators do not) and each chain's distance from
+    the pooled PSM, on the device, with the split-R-hat of the traces K, r, p, loglik and logposterior on the host.  Returns
+    the dict of Sampler.convergencediagnostics.  Chains that sample another mode of the partition show as pairs with
+    R-hat above 1.01 and as a chain whose chain_meandev stands out."""
+    res = list(results) if isinstance(results, (list, tuple)) else [results]
+    if not res:
+        raise ArgumentError("results must hold at least one MCMCResult.")
+    if any(r is None for r in res):
+        raise ArgumentError("a chain stopped at the slot capacity (its result is None); drop it before the diagnostics.")
+    if len({len(r.clusts) for r in res}) > 1:
+        raise ArgumentError("the results hold different numbers of samples.")
+    if len({np.asarray(c).shape for r in res for c in r.clusts}) > 1:
+        raise ArgumentError("the results label different numbers of points.")
+    out = cocl_rhat(np.stack([np.stack(r.clusts) for r in res]), device, matrix)
+    out["traces"] = {k: _split_rhat(np.stack([np.asarray(getattr(r, k)) for r in res])) for k in _TRACES}
+    return out
 
 
 _PAIRWISE_BYTES = 64 << 30          # the S x S fp64 loss matrix of the pairwise MPEL path must stay below this

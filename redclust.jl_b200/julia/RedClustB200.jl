@@ -15,7 +15,7 @@ import RedClust
 import Clustering
 using RedClust: MCMCOptionsList, PriorHyperparamsList, MCMCResult, MCMCState, ClustLabelVector, fitprior
 using RedClust: iac_ess_acf, sortlabels
-using StatsBase: mean_and_var, mean
+using StatsBase: mean_and_var, mean, var
 import Libdl
 
 const LIB = Ref{String}(get(ENV, "RCB200_LIB", joinpath(@__DIR__, "..", "librcb200.so")))
@@ -372,6 +372,75 @@ function getpointestimate(results::Vector{MCMCResult}; method::String = "MAP", l
         end
     end
     return (clusts[i], i)
+end
+
+# ---- convergence across chains (no reference equivalent: the reference's diagnostics are per chain, src/mcmc.jl:564-573)
+struct rc_rhat_summary
+    max::Float64; a::Int64; b::Int64; above::Int64
+end
+
+"""
+    splitrhat(x::Matrix{Float64}) -> Float64
+
+Split-R-hat (BDA3 11.4) of a trace with one chain per ROW: the first and last floor(S / 2) samples of every chain are the
+groups (the middle sample of an odd S is dropped), sample variances with ddof = 1.  When every group is constant (W = 0,
+decided by comparing the values) it is 1 if they all hold the same value and Inf otherwise.
+"""
+function splitrhat(x::AbstractMatrix{<:Real})
+    S = size(x, 2)
+    S >= 4 || throw(ArgumentError("split-R-hat needs at least 4 samples per chain."))
+    h = S ÷ 2
+    g = vcat(Float64.(x[:, 1:h]), Float64.(x[:, (S - h + 1):S]))
+    if all(g .== g[:, 1:1])
+        return all(g .== g[1, 1]) ? 1.0 : Inf
+    end
+    W = mean([var(g[j, :]) for j in 1:size(g, 1)])
+    B = h * var([mean(g[j, :]) for j in 1:size(g, 1)])
+    return sqrt(((h - 1) / h * W + B / h) / W)
+end
+
+"""
+    cocl_rhat(labels::Array{Int,3}; device = 0, matrix = false)
+
+The co-clustering part of `convergencediagnostics` for labels of size n x S x C (point, sample, chain; the C side's
+chains x samples x n row-major): split-R-hat of every point pair's co-clustering indicator (rc_cocl_rhat) and each chain's
+distance from the pooled PSM.  Pairs are 1-based here.
+"""
+function cocl_rhat(labels::Array{Int,3}; device::Integer = 0, matrix::Bool = false)
+    n, S, C = size(labels)
+    sm = Ref(rc_rhat_summary(0.0, 0, 0, 0))
+    md = Vector{Float64}(undef, C); xd = Vector{Float64}(undef, C)
+    R = matrix ? Matrix{Float64}(undef, n, n) : nothing
+    L = Array{Int64}(labels)
+    GC.@preserve L R check(ccall((:rc_cocl_rhat, LIB[]), Int32,
+        (Ptr{Int64}, Int64, Int64, Int64, Int32, Ref{rc_rhat_summary}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+        L, C, S, n, device, sm, isnothing(R) ? C_NULL : R, md, xd))
+    s = sm[]
+    return (rhat_max = s.max, rhat_pair = (s.a + 1, s.b + 1), pairs_above = s.above, chain_meandev = md, chain_maxdev = xd, rhat = R)
+end
+
+"""
+    convergencediagnostics(results::Vector{MCMCResult}; device = 0, matrix = false)
+
+Convergence across chains: `cocl_rhat` over the results' samples (on the GPU) and `splitrhat` of their traces K, r, p,
+loglik and logposterior.  Chains that sample another mode of the partition show as pairs with R-hat above 1.01 and as a
+chain whose chain_meandev stands out.  (The sampler-resident entry points rc_sampler_cocl_rhat / rc_comm_sampler_cocl_rhat
+need the sampler handle, which this runsampler releases before it returns.)
+"""
+function convergencediagnostics(results::Vector{MCMCResult}; device::Integer = 0, matrix::Bool = false)
+    isempty(results) && throw(ArgumentError("results must hold at least one MCMCResult."))
+    S = length(results[1].clusts)
+    all(length(r.clusts) == S for r in results) || throw(ArgumentError("the results hold different numbers of samples."))
+    n = length(results[1].clusts[1])
+    all(length(c) == n for r in results for c in r.clusts) || throw(ArgumentError("the results label different numbers of points."))
+    L = Array{Int64}(undef, n, S, length(results))
+    for (c, r) in enumerate(results), s in 1:S
+        L[:, s, c] .= r.clusts[s]
+    end
+    out = cocl_rhat(L; device = device, matrix = matrix)
+    traces = Dict(k => splitrhat(permutedims(hcat([Float64.(getfield(r, k)) for r in results]...)))
+                  for k in (:K, :r, :p, :loglik, :logposterior))
+    return merge(out, (traces = traces,))
 end
 
 end # module

@@ -1,5 +1,6 @@
 """N-rank check of the sharded paths of SURVEY 8e over NCCL: distance build by row blocks + all_gather, chains sharded
-across GPUs with per-rank int32 PSM counts + one all_reduce of the n x n matrix, MPEL candidates sharded + all_gather.
+across GPUs with per-rank int32 PSM counts + one all_reduce of the n x n matrix, MPEL candidates sharded + all_gather,
+and the convergence diagnostics over the chains of every rank.
 torchrun --nproc-per-node N tools/multigpu_check.py [n] [chains_per_rank] [iters]
 Rank 0 compares each with the single-process result (all three are bit-equal) and prints timings."""
 import os, sys, time
@@ -62,6 +63,20 @@ if rank == 0:
     print(f"world={world} n={n} chains={cpr * world}: binder_pointestimate_allreduce over {bp['totals'].size} samples {dt * 1e3:.1f} ms; "
           f"equal to one process over the same chains: {okb}", flush=True)
     assert okb
+# convergence across the chains of every rank: all-reduced counts N, one all_reduce of Q, one all_gather of the deviations
+torch.cuda.synchronize(); dist.barrier()
+t = time.perf_counter()
+cd = smp.convergencediagnostics_allreduce(matrix=True)
+torch.cuda.synchronize(); dist.barrier()
+dt = time.perf_counter() - t
+if rank == 0:
+    one = make(0, cpr * world, data).convergencediagnostics(matrix=True)
+    okc = (np.array_equal(cd["rhat"], one["rhat"]) and cd["rhat_max"] == one["rhat_max"] and cd["rhat_pair"] == one["rhat_pair"]
+           and cd["pairs_above"] == one["pairs_above"] and np.array_equal(cd["chain_meandev"], one["chain_meandev"])
+           and np.array_equal(cd["chain_maxdev"], one["chain_maxdev"]) and cd["traces"] == one["traces"])
+    print(f"world={world} n={n} chains={cpr * world}: convergencediagnostics_allreduce {dt * 1e3:.1f} ms; "
+          f"equal to one process over the same chains: {okc}", flush=True)
+    assert okc
 # one common set of label vectors on every rank: rank 0's samples, broadcast, then 5 % of the labels reshuffled with a
 # fixed seed so that the samples differ from each other
 S = np.ascontiguousarray(smp.samples(0)["labels"])
