@@ -255,6 +255,21 @@ int32_t rc_cocl_rhat(const int64_t* labels, int64_t nchains, int64_t S, int64_t 
 int32_t rc_sampler_cocl_rhat(const rc_sampler* s, int64_t chain0, int64_t nch, rc_rhat_summary* sum, double* rhat_out,
                              double* meandev, double* maxdev);
 
+/* ---- distances from given partitions to the samples (no reference call; Wade & Ghahramani 2018, section 4) -------------
+ * Distances from nref reference partitions (host, nref x n, any positive labels, <= 255 clusters each) to S samples, with
+ * the losses of rc_mpel (0 binder, 1 omARI, 2 VI, 3 ID).  dist_out: nref x S fp64; pairs_out (NULL or nref x S int64): exact
+ * Binder disagreement counts; K_out (NULL or S int32): clusters per sample.  dist_out[r][t] is bit-equal to M[0][t + 1] of
+ * rc_mpel's matrix on the stacked label set [ref_r; samples].  One contingency table per (reference, sample): O(nref S n)
+ * work and no S x S matrix, so it takes the pooled samples of many chains.  nref < 1, a bad loss code or a NULL dist_out:
+ * RC_ERR_ARG; more than 255 clusters in a reference or a table that does not fit shared memory: RC_ERR_SLOTS.           */
+int32_t rc_partition_dists(const int64_t* refs, int64_t nref, const int64_t* labels, int64_t S, int64_t n, int32_t loss,
+                           int32_t device, double* dist_out, int64_t* pairs_out, int32_t* K_out);
+/* The same over the device-resident samples of chains [chain0, chain0 + nch) (chain-major, sample-minor); no sample is
+ * copied to the host.  RC_ERR_STATE before a run to numiters, RC_ERR_SLOTS when a chain of the range stopped at the slot
+ * capacity, RC_ERR_ARG for a bad range.                                                                                */
+int32_t rc_sampler_partition_dists(const rc_sampler* s, const int64_t* refs, int64_t nref, int64_t chain0, int64_t nch,
+                                   int32_t loss, double* dist_out, int64_t* pairs_out, int32_t* K_out);
+
 /* ---- multi-GPU exchange steps (SURVEY.md 8e) -------------------------------------------------------
  * One process per GPU.  The sampler needs no collective (independent chains: chain_offset above).  The three steps
  * that exchange data run over an NCCL communicator owned by an rc_comm handle: rank 0 calls rc_comm_unique_id, the
@@ -271,6 +286,9 @@ int32_t rc_sampler_cocl_rhat(const rc_sampler* s, int64_t chain0, int64_t nch, r
  *   rc_comm_sampler_cocl_rhat  rc_sampler_cocl_rhat over the chains of every rank: the all-reduced counts N, each rank's Q
  *                             of its own chains, ONE all-reduce of Q and ONE all-gather of the chains' deviations;
  *                             meandev / maxdev hold every rank's chains in rank order
+ *   rc_comm_sampler_partition_dists  rc_sampler_partition_dists over the chains of every rank: the references on every
+ *                             rank, ONE all-gather of the per-rank {dist, pairs, K}; the outputs cover every rank's samples
+ *                             in rank order (dist_out nref x all samples)
  * psm_out (host, n x n fp64) and counts_dev_out (device, n x n int32) may each be NULL.  Results are bit-equal to the
  * single-GPU entry points.                                                                              */
 typedef struct rc_comm rc_comm;
@@ -286,6 +304,8 @@ int32_t rc_comm_mpel(rc_comm* c, const int64_t* labels, int64_t S, int64_t n, in
 int32_t rc_comm_sampler_binder_mpel(rc_comm* c, const rc_sampler* s, double* loss_sums, int64_t* best, int64_t* totals);
 int32_t rc_comm_sampler_cocl_rhat(rc_comm* c, const rc_sampler* s, rc_rhat_summary* sum, double* rhat_out, double* meandev,
                                   double* maxdev);
+int32_t rc_comm_sampler_partition_dists(rc_comm* c, const rc_sampler* s, const int64_t* refs, int64_t nref, int32_t loss,
+                                        double* dist_out, int64_t* pairs_out, int32_t* K_out);
 
 #ifdef __cplusplus
 }

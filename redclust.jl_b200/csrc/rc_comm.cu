@@ -204,28 +204,34 @@ static int32_t finish_psm(rc_comm* c, int* counts, int64_t n, long long local_sa
   return RC_OK;
 }
 
-// The {status, samples} of every rank, exchanged before the collectives of a call that a rank may refuse: a refusing rank
+// The {status, vals...} of every rank, exchanged before the collectives of a call that a rank may refuse: a refusing rank
 // returns its own error and the others "rank r refused", instead of leaving them waiting in the next collective.
-// all (out): world x {status, samples}.
-static int agree(rc_comm* c, int local, int64_t samples, const char* who, std::vector<long long>& all) {
+// all (out): world x {status, vals...}.
+static int agree_vals(rc_comm* c, int local, const std::vector<long long>& vals, const char* who, std::vector<long long>& all) {
   const std::string why = local ? rc_last_error() : "";
+  const size_t w = 1 + vals.size();
   Bufs B;
-  long long* info;                                             // this rank's pair, then the gathered ranks
-  TRYP(B.get(&info, 2 * (size_t)(c->world + 1)));
-  const long long mine[2] = {local, (long long)samples};
-  all.assign(2 * (size_t)c->world, 0);
-  cudaError_t e = cudaMemcpy(info, mine, sizeof(mine), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess && nccl()->AllGather(info, info + 2, 2, ncclInt64, c->comm, c->stream) != ncclSuccess) e = cudaErrorUnknown;
+  long long* info;                                             // this rank's values, then the gathered ranks
+  TRYP(B.get(&info, w * (size_t)(c->world + 1)));
+  std::vector<long long> mine(1, (long long)local);
+  mine.insert(mine.end(), vals.begin(), vals.end());
+  all.assign(w * (size_t)c->world, 0);
+  cudaError_t e = cudaMemcpy(info, mine.data(), sizeof(long long) * w, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess && nccl()->AllGather(info, info + w, w, ncclInt64, c->comm, c->stream) != ncclSuccess) e = cudaErrorUnknown;
   if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-  if (e == cudaSuccess) e = cudaMemcpy(all.data(), info + 2, sizeof(long long) * 2 * c->world, cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess) e = cudaMemcpy(all.data(), info + w, sizeof(long long) * w * c->world, cudaMemcpyDeviceToHost);
   if (e != cudaSuccess) { rc_set_error("%s: exchange of the sample counts failed", who); return RC_ERR_CUDA; }
   for (int r = 0; r < c->world; ++r)
-    if (all[2 * r] != 0) {
+    if (all[w * r] != 0) {
       if (local) { rc_set_error("%s", why.c_str()); return local; }
-      rc_set_error("%s: rank %d refused (status %lld)", who, r, all[2 * r]);
-      return (int32_t)all[2 * r];
+      rc_set_error("%s: rank %d refused (status %lld)", who, r, all[w * r]);
+      return (int32_t)all[w * r];
     }
   return RC_OK;
+}
+// the {status, samples} form: all = world x {status, samples}
+static int agree(rc_comm* c, int local, int64_t samples, const char* who, std::vector<long long>& all) {
+  return agree_vals(c, local, {(long long)samples}, who, all);
 }
 
 int32_t rc_comm_sampler_psm(rc_comm* c, const rc_sampler* s, double* psm_out, void* counts_dev_out) {
@@ -352,6 +358,85 @@ int32_t rc_comm_sampler_cocl_rhat(rc_comm* c, const rc_sampler* s, rc_rhat_summa
   TRYP(rhat_finish(d, S, n, 2 * C, sum, rhat_out, t));
   rhat_deviations(dev.data(), C, S, n, 2 * C, meandev, maxdev);
   rhat_report(t, Cl, S, n);
+  return RC_OK;
+}
+
+// Distances from reference partitions to the samples of every rank (rc_sampler_partition_dists over chains sharded over
+// GPUs): every rank holds the references and computes its own samples; ONE all-gather of the per-rank {dist, pairs, K}
+// blocks (8-byte words, padded to the largest rank) gives every rank all samples in rank order (= global chain order).
+// Each distance comes from the same kernel and the same table as on one GPU: identical to one GPU over the same chains.
+// Nothing a rank can refuse happens after a collective it might leave the others waiting in.  The first exchange carries
+// {samples, their largest K, nref, a hash of the references, pairs wanted}: every rank then applies the same checks to the
+// same values (equal nref, references and pairs on every rank; the table of the references against the largest K of ALL
+// samples fits the shared memory, so the call refuses exactly when one GPU over the same chains would).  The buffers are
+// allocated before a second exchange of the status.
+int32_t rc_comm_sampler_partition_dists(rc_comm* c, const rc_sampler* s, const int64_t* refs, int64_t nref, int32_t loss,
+                                        double* dist_out, int64_t* pairs_out, int32_t* K_out) {
+  if (!c || !s) { rc_set_error("rc_comm_sampler_partition_dists: null handle"); return RC_ERR_ARG; }
+  RC_CUDA(cudaSetDevice(c->device));
+  const char* who = "rc_comm_sampler_partition_dists";
+  rc_sample_range v;
+  Bufs B;
+  PartitionRefs r;
+  std::vector<int> Kh;
+  int kmax = 0;
+  int local = rc_sampler_range(s, 0, rc_sampler_nchains(s), who, v);
+  if (!local) local = partition_refs(refs, nref, v.n, loss, dist_out, who, B, r);
+  if (!local) local = sample_K(v.K, v.R, Kh, &kmax);
+  const long long want_pairs = pairs_out != nullptr;
+  unsigned long long h = 14695981039346656037ull;             // FNV-1a of the references as given
+  if (!local)
+    for (int64_t t = 0; t < nref * v.n; ++t) h = (h ^ (unsigned long long)refs[t]) * 1099511628211ull;
+  std::vector<long long> all, ok;
+  TRYP(agree_vals(c, local, {local ? 0 : (long long)v.R, kmax, (long long)nref, (long long)h, want_pairs}, who, all));
+  int64_t total = 0, per = 0;
+  int kall = 0;
+  for (int q = 0; q < c->world; ++q) {
+    const long long* a = all.data() + 6 * q;
+    total += a[1];
+    per = std::max<int64_t>(per, a[1]);
+    kall = std::max<int>(kall, (int)a[2]);
+    if (a[3] != nref || a[4] != (long long)h || a[5] != want_pairs) {
+      rc_set_error("%s: rank %d holds other references or another pairs_out (nref %lld, pairs %lld)", who, q, a[3], a[5]);
+      return RC_ERR_ARG;
+    }
+  }
+  if (total < 1) { rc_set_error("%s: no samples on any rank", who); return RC_ERR_ARG; }
+  PairLaunch p;
+  TRYP(pair_geometry(v.n, r.kmax, kall, who, p));
+  // one rank's block: dist (nref x R_rank fp64 bits), then from word nref * per the pairs (nref x R_rank) when wanted, then K
+  const int64_t kw = (want_pairs ? 2 : 1) * nref * per, words = kw + per;
+  long long* buf = nullptr;                                    // [world + 1][words]: this rank's block, then the gathered ranks
+  local = B.get(&buf, (size_t)words * (c->world + 1));
+  if (!local) local = pair_nlogn(v.n, B, p);
+  TRYP(agree(c, local, 0, who, ok));
+  RC_CUDA(cudaMemset(buf, 0, sizeof(long long) * words));
+  if (v.R > 0) {
+    TRYP(partition_dists_run(r, p, v.labels, v.K, v.R, v.n, (double*)buf, want_pairs ? buf + nref * per : nullptr));
+    const std::vector<long long> K64(Kh.begin(), Kh.end());
+    RC_CUDA(cudaMemcpy(buf + kw, K64.data(), sizeof(long long) * v.R, cudaMemcpyHostToDevice));
+  }
+  const long long* gathered = buf;
+  if (c->world > 1) {
+    if (nccl()->AllGather(buf, buf + words, (size_t)words, ncclInt64, c->comm, c->stream) != ncclSuccess ||
+        cudaStreamSynchronize(c->stream) != cudaSuccess) {
+      rc_set_error("%s: all-gather of the per-rank distances failed", who); return RC_ERR_CUDA;
+    }
+    gathered = buf + words;
+  }
+  std::vector<long long> hv((size_t)words * c->world);
+  RC_CUDA(cudaMemcpy(hv.data(), gathered, sizeof(long long) * hv.size(), cudaMemcpyDeviceToHost));
+  int64_t off = 0;                                             // rank order = global chain order
+  for (int q = 0; q < c->world; ++q) {
+    const int64_t Rq = all[6 * q + 1];
+    const long long* g = hv.data() + (size_t)words * q;
+    for (int64_t k = 0; k < nref; ++k) {
+      memcpy(dist_out + k * total + off, g + k * Rq, sizeof(double) * Rq);
+      if (pairs_out) memcpy(pairs_out + k * total + off, g + nref * per + k * Rq, sizeof(int64_t) * Rq);
+    }
+    if (K_out) for (int64_t t = 0; t < Rq; ++t) K_out[off + t] = (int32_t)g[kw + t];
+    off += Rq;
+  }
   return RC_OK;
 }
 

@@ -73,6 +73,32 @@ int binder_wp(const uint8_t* L, const uint8_t* Lt, int64_t R, int64_t n, const i
 int rc_binder_finish(const unsigned long long* W, const unsigned long long* P, int64_t S, int64_t n, double* loss_sums,
                      int64_t* best, int64_t* totals);
 
+// distances from reference partitions to samples (rc_post.cu).  PartitionRefs: the references relabelled and uploaded
+// (bytes nref x n, their K, the largest K) with the loss code, after the argument checks of the entry points.  PairLaunch:
+// the launch geometry of k_pair_loss; pair_geometry checks that a krow x kcol table fits the shared memory (RC_ERR_SLOTS,
+// no device work), pair_nlogn fills its N log N table.  sample_K: the K of S device samples on the host and their largest.
+// partition_dists_run: dist (nref x S fp64) and pairs (NULL or nref x S int64, exact Binder counts) of the references
+// against S device samples (bytes 1..K, device K) into device buffers.
+struct PartitionRefs {
+  uint8_t* L;
+  int* K;
+  int kmax;
+  int64_t nref;
+  int loss;
+};
+struct PairLaunch {
+  int wide, tabwords, stride;
+  size_t smem;
+  double* nlogn;
+};
+int partition_refs(const int64_t* refs, int64_t nref, int64_t n, int32_t loss, const void* dist_out, const char* who, Bufs& B,
+                   PartitionRefs& r);
+int pair_geometry(int64_t n, int krow, int kcol, const char* who, PairLaunch& p);
+int pair_nlogn(int64_t n, Bufs& B, PairLaunch& p);
+int sample_K(const int* Kd, int64_t S, std::vector<int>& Kh, int* kmax);
+int partition_dists_run(const PartitionRefs& r, const PairLaunch& p, const uint8_t* L, const int* Kd, int64_t S, int64_t n, double* dist,
+                        long long* pairs);
+
 // split-R-hat of the co-clustering indicators (rc_rhat.cu).  The limits on chains, samples per chain and n; the device
 // buffers of one call (N the pooled counts, Q = sum of squared group counts, Na / Nb one chain's halves, dev = {sum d,
 // max d} per local chain, R the matrix or NULL); pass 1 (N), pass 2 (Q and dev against the N of m groups in all), the

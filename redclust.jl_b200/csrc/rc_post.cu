@@ -5,6 +5,8 @@
 //         (Clustering.jl randindex / varinfo / mutualinfo, restated from their contingency-table definitions)
 //   Binder MPEL over pooled samples   the same argmin for binderloss (pointestimate.jl:68-76) from the counts alone:
 //         O(S n^2) compares, no S x S matrix (k_binder_w, k_binder_pairs, rc_binder_finish)
+//   Distances from given partitions to every sample   the MPEL losses with reference rows (k_pair_loss<true>), for the
+//         posterior expected loss of any partition and the credible ball of Wade & Ghahramani (2018, section 4)
 // The reference materialises S dense n x n Bool matrices; here the label matrix is transposed once
 // (point-major, samples contiguous) and co-clustering counts are byte-compare popcounts -- exact integers.
 #include <vector>
@@ -297,26 +299,35 @@ __global__ void k_nlogn(int64_t n, double* __restrict__ out) {
 __device__ __forceinline__ unsigned tab_get(const unsigned* tab, int t, int wide) {
   return wide ? tab[t] : ((tab[t >> 1] >> ((t & 1) * 16)) & 0xffffu);
 }
+// REF = false (MPEL): rows and columns are the S label vectors of L, column j > row i, output the loss matrix M.
+// REF = true (reference partitions): row r = blockIdx.y is reference r of Lref (K Kref[r]), the columns are every sample of
+// L, output dist[r * S + t] in M, and, when pairs is not NULL, the exact Binder disagreement count
+// (sum_k a_k^2 + sum_l b_l^2) / 2 - sum_kl n_kl^2 from integer sums of the same table.  The table, its loops and the
+// fp64 formulas are the same code in both modes, so dist[r][t] is bit-equal to M[0][t + 1] of MPEL on [ref_r; samples].
+template <bool REF>
 __global__ void __launch_bounds__(256) k_pair_loss(const uint8_t* __restrict__ L, const int* __restrict__ Kc, int64_t S,
                                                    int64_t n, int loss, int wide, int tabwords, int stride,
                                                    const double* __restrict__ nlogn, double* __restrict__ M, int64_t row_first,
-                                                   int64_t row_stride, int mirror) {
-  const int64_t i = row_first + (int64_t)blockIdx.y * row_stride;       // sharded: this rank's rows are row_first, + stride, ...
-  if (i >= S) return;
-  const int64_t jlo = max((long long)(i + 1), (long long)blockIdx.x * PJ), jhi = min((long long)S, (long long)(blockIdx.x + 1) * PJ);
+                                                   int64_t row_stride, int mirror, const uint8_t* __restrict__ Lref,
+                                                   const int* __restrict__ Kref, long long* __restrict__ pairs) {
+  const int64_t i = REF ? (int64_t)blockIdx.y : row_first + (int64_t)blockIdx.y * row_stride;   // MPEL sharded: row_first, + stride, ...
+  if (!REF && i >= S) return;
+  const int64_t jlo = REF ? (int64_t)blockIdx.x * PJ : max((long long)(i + 1), (long long)blockIdx.x * PJ);
+  const int64_t jhi = min((long long)S, (long long)(blockIdx.x + 1) * PJ);
   if (jlo >= jhi) return;
   extern __shared__ __align__(16) unsigned tab[];
   const int64_t nv = (n + 15) / 16;                       // 16-byte vectors per label vector
   uint8_t* la = reinterpret_cast<uint8_t*>(tab + tabwords);
   uint8_t* lb = la + nv * 16;
   __shared__ double red[6][8];
+  __shared__ unsigned long long redi[2][8];
   const bool vec = (n % 16) == 0;                          // rows of L are 16-byte aligned only then
   auto stage = [&](uint8_t* dst, const uint8_t* src) {
     if (vec) for (int64_t t = threadIdx.x; t < nv; t += blockDim.x) reinterpret_cast<uint4*>(dst)[t] = reinterpret_cast<const uint4*>(src)[t];
     else for (int64_t t = threadIdx.x; t < n; t += blockDim.x) dst[t] = src[t];
   };
-  stage(la, L + i * n);
-  const int Ki = Kc[i];
+  stage(la, REF ? Lref + i * n : L + i * n);
+  const int Ki = REF ? Kref[i] : Kc[i];
   const double dn = (double)n;
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   for (int64_t j = jlo; j < jhi; ++j) {
@@ -338,9 +349,11 @@ __global__ void __launch_bounds__(256) k_pair_loss(const uint8_t* __restrict__ L
     __syncthreads();
     // sums over the table: t2 = sum N^2, snl = sum N log N; margins via row / column passes
     double t2 = 0, snl = 0, nis = 0, njs = 0, hA = 0, hB = 0;
+    unsigned long long q2 = 0, qm = 0;                     // REF with pairs: sum N^2 and sum a^2 + sum b^2 as integers
     for (int t = threadIdx.x; t < cells; t += blockDim.x) {
       const unsigned c = tab_get(tab, t, wide);
       const double d = (double)c; t2 += d * d; snl += nlogn[c];
+      if (REF && pairs) q2 += (unsigned long long)c * c;
     }
     for (int r = threadIdx.x; r < Ki + Kj; r += blockDim.x) {
       unsigned sm = 0;
@@ -348,12 +361,17 @@ __global__ void __launch_bounds__(256) k_pair_loss(const uint8_t* __restrict__ L
       else { const int q = r - Ki; for (int pp = 0; pp < Ki; ++pp) sm += tab_get(tab, pp * Kj + q, wide); }
       const double d = (double)sm;
       if (r < Ki) { nis += d * d; hA += nlogn[sm]; } else { njs += d * d; hB += nlogn[sm]; }
+      if (REF && pairs) qm += (unsigned long long)sm * sm;
     }
   double v[6] = {t2, snl, nis, njs, hA, hB};
 #pragma unroll
   for (int q = 0; q < 6; ++q) {
     for (int off = 16; off; off >>= 1) v[q] += __shfl_xor_sync(0xffffffffu, v[q], off);
     if ((threadIdx.x & 31) == 0) red[q][threadIdx.x >> 5] = v[q];
+  }
+  if (REF && pairs) {
+    for (int off = 16; off; off >>= 1) { q2 += __shfl_xor_sync(0xffffffffu, q2, off); qm += __shfl_xor_sync(0xffffffffu, qm, off); }
+    if ((threadIdx.x & 31) == 0) { redi[0][threadIdx.x >> 5] = q2; redi[1][threadIdx.x >> 5] = qm; }
   }
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -372,7 +390,14 @@ __global__ void __launch_bounds__(256) k_pair_loss(const uint8_t* __restrict__ L
       const double I = snl / dn - hA / dn - hB / dn + log(dn);
       out = loss == 2 ? (HA + HB - 2 * I) : ((HA > HB ? HA : HB) - I);
     }
-    if (mirror) { M[i * S + j] = out; M[j * S + i] = out; }
+    if (REF) {
+      M[i * S + j] = out;
+      if (pairs) {
+        unsigned long long s2 = 0, sm = 0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) { s2 += redi[0][w]; sm += redi[1][w]; }
+        pairs[i * S + j] = (long long)(sm / 2 - s2);       // sum a^2 + sum b^2 is even: both are = n (mod 2)
+      }
+    } else if (mirror) { M[i * S + j] = out; M[j * S + i] = out; }
     else M[(int64_t)blockIdx.y * S + j] = out;                         // row block of the upper triangle
   }
   }
@@ -563,6 +588,28 @@ int32_t rc_sampler_binder_mpel(const rc_sampler* s, int64_t chain0, int64_t nch,
 
 }  // extern "C"
 
+// Launch geometry of k_pair_loss for tables of at most krow x kcol cells: packed 16-bit cells up to n = 65 535, 32-bit
+// cells beyond; the table and two staged label vectors must fit the shared memory (RC_ERR_SLOTS).  No device work.
+int pair_geometry(int64_t n, int krow, int kcol, const char* who, PairLaunch& p) {
+  p.wide = n > 65535;
+  const int cells = krow * kcol;
+  p.tabwords = ((p.wide ? cells : (cells + 1) / 2) + 3) & ~3;
+  p.smem = (size_t)p.tabwords * 4 + 2 * (size_t)((n + 15) / 16) * 16;
+  if (p.smem > 220 * 1024) { rc_set_error("%s: n = %lld with %d x %d clusters does not fit shared memory", who, (long long)n, krow, kcol); return RC_ERR_SLOTS; }
+  p.stride = (int)((n + 31) / 32);
+  while ((p.stride & 3) || !((p.stride >> 2) & 1)) ++p.stride;      // multiple of 4 with an odd quotient: lane segments start in different banks
+  p.nlogn = nullptr;
+  return RC_OK;
+}
+
+// the N log N table of k_pair_loss (n + 1 entries, a buffer of B)
+int pair_nlogn(int64_t n, Bufs& B, PairLaunch& p) {
+  TRYP(B.get(&p.nlogn, (size_t)(n + 1)));
+  k_nlogn<<<(unsigned)((n + 256) / 256), 256>>>(n, p.nlogn);
+  RC_CUDA(cudaGetLastError());
+  return RC_OK;
+}
+
 // Shared front end of the MPEL entry points: relabel, upload, size the contingency table, and launch the pair-loss
 // kernel for the rows row_first, row_first + row_stride, ... (nrows of them).  mirror = 1 writes the full symmetric
 // S x S matrix M; mirror = 0 writes the rows' strict upper triangle into an nrows x S block.
@@ -573,23 +620,126 @@ static int mpel_pairs(const int64_t* labels, int64_t S, int64_t n, int32_t loss,
   int kmax = 0;
   for (int k : K) kmax = std::max(kmax, k);
   if (kmax_out) *kmax_out = kmax;
-  const int wide = n > 65535;
-  const int tabwords = ((wide ? kmax * kmax : (kmax * kmax + 1) / 2) + 3) & ~3;
-  const size_t smem = (size_t)tabwords * 4 + 2 * (size_t)((n + 15) / 16) * 16;
-  if (smem > 220 * 1024) { rc_set_error("rc_mpel: n = %lld with %d x %d clusters does not fit shared memory", (long long)n, kmax, kmax); return RC_ERR_SLOTS; }
-  int stride = (int)((n + 31) / 32);
-  while ((stride & 3) || !((stride >> 2) & 1)) ++stride;      // multiple of 4 with an odd quotient: lane segments start in different banks
-  int* dK; double* nlogn;
-  TRYP(B.get(&dK, (size_t)S)); TRYP(B.get(&nlogn, (size_t)(n + 1)));
+  PairLaunch p;
+  TRYP(pair_geometry(n, kmax, kmax, "rc_mpel", p));
+  TRYP(pair_nlogn(n, B, p));
+  int* dK;
+  TRYP(B.get(&dK, (size_t)S));
   RC_CUDA(cudaMemcpy(dK, K.data(), sizeof(int) * S, cudaMemcpyHostToDevice));
-  k_nlogn<<<(unsigned)((n + 256) / 256), 256>>>(n, nlogn);
-  RC_CUDA(cudaFuncSetAttribute(k_pair_loss, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  RC_CUDA(cudaFuncSetAttribute(k_pair_loss<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
   if (nrows > 0)
-    k_pair_loss<<<dim3((unsigned)((S + PJ - 1) / PJ), (unsigned)nrows), 256, smem>>>(dL, dK, S, n, loss, wide, tabwords, stride, nlogn, M,
-                                                                                  row_first, row_stride, mirror);
+    k_pair_loss<false><<<dim3((unsigned)((S + PJ - 1) / PJ), (unsigned)nrows), 256, p.smem>>>(dL, dK, S, n, loss, p.wide, p.tabwords, p.stride,
+                                                                                           p.nlogn, M, row_first, row_stride, mirror,
+                                                                                           nullptr, nullptr, nullptr);
   RC_CUDA(cudaGetLastError());
   return RC_OK;
 }
+
+// ---- distances from reference partitions to the samples ----------------------------------------------------------------
+// The reference partitions of the rc_*partition_dists entry points: argument checks, then relabelled and uploaded into B.
+int partition_refs(const int64_t* refs, int64_t nref, int64_t n, int32_t loss, const void* dist_out, const char* who, Bufs& B,
+                   PartitionRefs& r) {
+  if (!refs || !dist_out || nref < 1 || n < 1 || loss < 0 || loss > 3) {
+    rc_set_error("%s: needs reference partitions (nref >= 1), a loss code 0..3 and dist_out (nref = %lld, loss = %d)", who,
+                 (long long)nref, (int)loss);
+    return RC_ERR_ARG;
+  }
+  std::vector<int> K;
+  TRYP(upload_labels(refs, nref, n, B, &r.L, K));
+  TRYP(B.get(&r.K, (size_t)nref));
+  RC_CUDA(cudaMemcpy(r.K, K.data(), sizeof(int) * nref, cudaMemcpyHostToDevice));
+  r.kmax = *std::max_element(K.begin(), K.end());
+  r.nref = nref;
+  r.loss = loss;
+  return RC_OK;
+}
+
+// the K of S device samples on the host, and their largest
+int sample_K(const int* Kd, int64_t S, std::vector<int>& Kh, int* kmax) {
+  Kh.resize((size_t)S);
+  RC_CUDA(cudaMemcpy(Kh.data(), Kd, sizeof(int) * S, cudaMemcpyDeviceToHost));
+  *kmax = S > 0 ? *std::max_element(Kh.begin(), Kh.end()) : 0;
+  return RC_OK;
+}
+
+// dist (nref x S fp64) and, when pairs is not NULL, the exact Binder counts (nref x S int64) of the references against S
+// device samples L (bytes 1..K, K on the device in Kd), into DEVICE buffers, with the geometry p (pair_geometry with the
+// samples' largest K, pair_nlogn).  One launch of k_pair_loss<true> per 65 535 references (the grid's y limit).
+int partition_dists_run(const PartitionRefs& r, const PairLaunch& p, const uint8_t* L, const int* Kd, int64_t S, int64_t n, double* dist,
+                        long long* pairs) {
+  RC_CUDA(cudaFuncSetAttribute(k_pair_loss<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
+  const bool verbose = getenv("RCB200_VERBOSE") != nullptr;
+  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  if (verbose) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, 0); }
+  for (int64_t r0 = 0; r0 < r.nref; r0 += 65535) {
+    const unsigned rows = (unsigned)std::min<int64_t>(65535, r.nref - r0);
+    k_pair_loss<true><<<dim3((unsigned)((S + PJ - 1) / PJ), rows), 256, p.smem>>>(L, Kd, S, n, r.loss, p.wide, p.tabwords, p.stride, p.nlogn,
+                                                                                 dist + r0 * S, 0, 1, 0, r.L + r0 * n, r.K + r0,
+                                                                                 pairs ? pairs + r0 * S : nullptr);
+  }
+  if (verbose) cudaEventRecord(e1, 0);
+  RC_CUDA(cudaGetLastError());
+  const cudaError_t e = cudaDeviceSynchronize();
+  if (verbose) {
+    float ms = 0; cudaEventElapsedTime(&ms, e0, e1);
+    fprintf(stderr, "[rcb200] partition dists: refs=%lld samples=%lld n=%lld refs' kmax %d loss=%d pairs=%d k_pair_loss %.3f ms (CUDA events) %.3e pairs/s\n",
+            (long long)r.nref, (long long)S, (long long)n, r.kmax, r.loss, pairs != nullptr, ms, (double)r.nref * S / (ms * 1e-3));
+    cudaEventDestroy(e0); cudaEventDestroy(e1);
+  }
+  RC_CUDA(e);
+  return RC_OK;
+}
+
+// the single-GPU entry points: distances of the references to S device samples, copied to the caller's host outputs
+static int partition_dists_host(const PartitionRefs& r, const uint8_t* L, const int* Kd, int64_t S, int64_t n, double* dist_out,
+                                int64_t* pairs_out, int32_t* K_out, const char* who, Bufs& B) {
+  if (S < 1) { rc_set_error("%s: no samples", who); return RC_ERR_ARG; }
+  std::vector<int> Kh;
+  int kmax;
+  TRYP(sample_K(Kd, S, Kh, &kmax));
+  PairLaunch p;
+  TRYP(pair_geometry(n, r.kmax, kmax, who, p));
+  TRYP(pair_nlogn(n, B, p));
+  double* dist; long long* pairs = nullptr;
+  TRYP(B.get(&dist, (size_t)r.nref * S));
+  if (pairs_out) TRYP(B.get(&pairs, (size_t)r.nref * S));
+  TRYP(partition_dists_run(r, p, L, Kd, S, n, dist, pairs));
+  RC_CUDA(cudaMemcpy(dist_out, dist, sizeof(double) * r.nref * S, cudaMemcpyDeviceToHost));
+  if (pairs_out) RC_CUDA(cudaMemcpy(pairs_out, pairs, sizeof(long long) * r.nref * S, cudaMemcpyDeviceToHost));
+  if (K_out) std::copy(Kh.begin(), Kh.end(), K_out);
+  return RC_OK;
+}
+
+extern "C" {
+
+int32_t rc_partition_dists(const int64_t* refs, int64_t nref, const int64_t* labels, int64_t S, int64_t n, int32_t loss, int32_t device,
+                           double* dist_out, int64_t* pairs_out, int32_t* K_out) {
+  const char* who = "rc_partition_dists";
+  if (!labels || S < 1) { rc_set_error("%s: needs S >= 1 sample label vectors (S = %lld)", who, (long long)S); return RC_ERR_ARG; }
+  TRYP(rc_select_device(device));
+  Bufs B;
+  PartitionRefs r;
+  TRYP(partition_refs(refs, nref, n, loss, dist_out, who, B, r));
+  uint8_t* dL; int* dK; std::vector<int> K;
+  TRYP(upload_labels(labels, S, n, B, &dL, K));
+  TRYP(B.get(&dK, (size_t)S));
+  RC_CUDA(cudaMemcpy(dK, K.data(), sizeof(int) * S, cudaMemcpyHostToDevice));
+  return partition_dists_host(r, dL, dK, S, n, dist_out, pairs_out, K_out, who, B);
+}
+
+int32_t rc_sampler_partition_dists(const rc_sampler* s, const int64_t* refs, int64_t nref, int64_t chain0, int64_t nch, int32_t loss,
+                                   double* dist_out, int64_t* pairs_out, int32_t* K_out) {
+  const char* who = "rc_sampler_partition_dists";
+  if (!s) { rc_set_error("%s: null handle", who); return RC_ERR_ARG; }
+  rc_sample_range v;
+  TRYP(rc_sampler_range(s, chain0, nch, who, v));
+  Bufs B;
+  PartitionRefs r;
+  TRYP(partition_refs(refs, nref, v.n, loss, dist_out, who, B, r));
+  return partition_dists_host(r, v.labels, v.K, v.R, v.n, dist_out, pairs_out, K_out, who, B);   // chain-major, sample-minor
+}
+
+}  // extern "C"
 
 static int mpel_argmin(const double* sums_dev, int64_t S, double* loss_sums, int64_t* best) {
   std::vector<double> hs((size_t)S);

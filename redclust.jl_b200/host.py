@@ -431,6 +431,67 @@ class Sampler:
             tr = {k: np.concatenate([p[k] for p in parts]) for k in _TRACES}
         return _rhat_dict(sm, R, md, xd, {name: _split_rhat(x) for name, x in tr.items()})
 
+    def _partition_dists(self, refs, chain0, nch, loss):
+        """partitiondistances over the device-resident samples of chains chain0 .. chain0 + nch - 1 (rc_sampler_partition_dists)."""
+        code = _loss_code(loss)
+        P = _partitions(refs, self.data.n, "the partitions")
+        out = _dists_out(P.shape[0], max(nch, 0) * int(lib().rc_sampler_numsamples(self._h)), loss)
+        check(lib().rc_sampler_partition_dists(self._h, ptr(P), P.shape[0], chain0, nch, code, ptr(out["dist"]), ptr(out["pairs"]),
+                                               ptr(out["K"])))
+        return out
+
+    def expectedloss(self, partitions, chain0=0, nch=None, loss="VI"):
+        """expectedloss over the recorded samples of chains chain0 .. chain0 + nch - 1 (chain-major), from the device-resident
+        samples: dict(expectedloss, totals)."""
+        nch = self.nchains - chain0 if nch is None else nch
+        return _expected(self._partition_dists(partitions, chain0, nch, loss), loss)
+
+    def credibleball(self, estimate, chain0=0, nch=None, loss="VI", alpha=0.05):
+        """credibleball over the recorded samples of chains chain0 .. chain0 + nch - 1 (chain-major: indices count the
+        samples of chain0 first), from the device-resident samples."""
+        _check_alpha(alpha)
+        nch = self.nchains - chain0 if nch is None else nch
+        S = int(lib().rc_sampler_numsamples(self._h))
+        out = self._partition_dists(_estimate(estimate, self.data.n), chain0, nch, loss)
+        return _ball_result(out, alpha, self._labels_of(lambda i: (chain0 + i // S, i % S)))
+
+    def credibleball_allreduce(self, estimate, loss="VI", alpha=0.05, group=None, device=None, comm=None):
+        """credibleball over the chains of every rank (rc_comm_sampler_partition_dists): each rank computes its own samples,
+        one ncclAllGather assembles the distances, equal to one GPU over the same chains.  Indices count every rank's
+        samples in rank order; a bound's clust is filled on the rank that holds its first sample, None on the others."""
+        _check_alpha(alpha)
+        code = _loss_code(loss)
+        P = np.ascontiguousarray(_estimate(estimate, self.data.n))
+        comm = comm or Comm.from_torch(group, self.data.device if device is None else device)
+        S = int(lib().rc_sampler_numsamples(self._h))
+        mine = self.nchains * S
+        if comm.world > 1:
+            import torch.distributed as dist
+            sizes = [None] * comm.world
+            dist.all_gather_object(sizes, mine, group=group)
+        else:
+            sizes = [mine]
+        out = _dists_out(1, sum(sizes), loss)
+        check(lib().rc_comm_sampler_partition_dists(comm._h, self._h, ptr(P), 1, code, ptr(out["dist"]), ptr(out["pairs"]), ptr(out["K"])))
+        first = sum(sizes[:comm.rank])
+        return _ball_result(out, alpha, self._labels_of(lambda i: ((i - first) // S, (i - first) % S) if 0 <= i - first < mine else None))
+
+    def _labels_of(self, where):
+        """clust_of for _ball_result: where(i) = (chain, sample) of pooled sample i on this sampler, or None.  Each chain's
+        labels are copied to the host once (labels only, not the traces)."""
+        S, n, chains = int(lib().rc_sampler_numsamples(self._h)), self.data.n, {}
+
+        def clust_of(i):
+            w = where(i)
+            if w is None:
+                return None
+            c, t = w
+            if c not in chains:
+                chains[c] = np.empty((S, n), np.int64)
+                check(lib().rc_sampler_copy_samples(self._h, c, ptr(chains[c]), None, None, None, None, None))
+            return chains[c][t].copy()
+        return clust_of
+
     def close(self):
         L = getattr(_lib, "_lib", None)
         if getattr(self, "_h", None) and L is not None:
@@ -783,6 +844,142 @@ def convergencediagnostics(results, device=0, matrix=False):
     out = cocl_rhat(np.stack([np.stack(r.clusts) for r in res]), device, matrix)
     out["traces"] = {k: _split_rhat(np.stack([np.asarray(getattr(r, k)) for r in res])) for k in _TRACES}
     return out
+
+
+# ---- distances from given partitions to the samples: posterior expected loss and credible balls (no reference call; Wade &
+# Ghahramani 2018, Bayesian Analysis 13(2), section 4, as mcclust.ext::credibleball) ----
+def _loss_code(loss):
+    if not (isinstance(loss, str) and loss in _LOSS):
+        raise ArgumentError('loss must be one of "binder", "omARI", "VI" and "ID" (a function-valued loss is not supported here).')
+    return _LOSS[loss]
+
+
+def _check_alpha(alpha):
+    if not 0 < alpha < 1:
+        raise ArgumentError("alpha must lie in (0, 1).")
+
+
+def _estimate(estimate, n):
+    est = np.asarray(estimate, dtype=np.int64)
+    if est.shape != (n,):
+        raise ArgumentError(f"estimate must label the {n} points of the samples.")
+    return est
+
+
+def _partitions(parts, n, what):
+    """nref x n int64 label array of one partition (length n) or several (nref x n)."""
+    P = np.asarray(parts, dtype=np.int64)
+    if P.ndim == 1:
+        P = P[None, :]
+    if P.ndim != 2 or P.shape[0] < 1 or P.shape[1] != n:
+        raise ArgumentError(f"{what} must label the {n} points of the samples.")
+    return np.ascontiguousarray(P)
+
+
+def _sample_labels(samples):
+    """S x n int64 labels of an MCMCResult, a list of them (pooled in list order) or an S x n label array."""
+    if isinstance(samples, (list, tuple)):
+        if not samples:
+            raise ArgumentError("samples must hold at least one MCMCResult.")
+        if any(r is None for r in samples):
+            raise ArgumentError("a chain stopped at the slot capacity (its result is None); drop it before pooling.")
+        clusts = [c for r in samples for c in r.clusts]
+    elif isinstance(samples, MCMCResult):
+        clusts = list(samples.clusts)
+    else:
+        L = np.asarray(samples, dtype=np.int64)
+        if L.ndim != 2 or L.shape[0] == 0:
+            raise ArgumentError("samples must be an MCMCResult, a list of them or a non-empty S × n label array.")
+        return np.ascontiguousarray(L)
+    if not clusts:
+        raise ArgumentError("samples hold no sample.")
+    if len({np.asarray(c).shape for c in clusts}) > 1:
+        raise ArgumentError("the results to pool label different numbers of points.")
+    return np.ascontiguousarray(np.stack(clusts).astype(np.int64, copy=False))
+
+
+def _dists_out(nref, S, loss):
+    """Output arrays of the partition-distance calls; the exact Binder counts only with loss="binder" (else None: the kernel
+    then skips their integer sums)."""
+    return dict(dist=np.empty((nref, S)), pairs=np.empty((nref, S), np.int64) if loss == "binder" else None, K=np.empty(S, np.int32))
+
+
+def _expected(out, loss):
+    """(sum_t d_t) / S per partition, the sum in ascending sample order from +0.0 (np.cumsum adds sequentially): bit-equal
+    to rc_mpel's loss_sums[0] / S for a partition stacked before the samples."""
+    d = out["dist"]
+    sums = np.cumsum(np.hstack([np.zeros((d.shape[0], 1)), d]), axis=1)[:, -1]
+    return dict(expectedloss=sums / d.shape[1], totals=out["pairs"].sum(axis=1) if loss == "binder" else None)
+
+
+def _credibleball(d, K, alpha):
+    """The credible ball of Wade & Ghahramani (2018, section 4) from the distances d of the S samples to the estimate and
+    their numbers of clusters K.  radius: the smallest sample distance e with #{t: d_t <= e} / S >= 1 - alpha (fp64 division
+    and comparison); the ball is every sample with d_t <= radius, ties included.  horizontal: the ball's samples at the
+    largest distance; upper: among the ball's samples with the fewest clusters, those at the largest distance; lower: the
+    same among those with the most clusters.  Each bound is dict(dist, K = the first one's, indices = every sample attaining
+    it, ascending)."""
+    d = np.asarray(d, dtype=np.float64)
+    K = np.asarray(K, dtype=np.int64)
+    ds = np.sort(d)
+    frac = np.searchsorted(ds, ds, side="right") / np.float64(d.size)
+    radius = float(ds[int(np.argmax(frac >= 1.0 - alpha))])
+    inball = d <= radius
+
+    def bound(mask):
+        far = d[mask].max()
+        idx = np.flatnonzero(mask & (d == far))
+        return dict(dist=float(far), K=int(K[idx[0]]), indices=idx)
+    return dict(radius=radius, inball=int(inball.sum()), horizontal=bound(inball), upper=bound(inball & (K == K[inball].min())),
+                lower=bound(inball & (K == K[inball].max())))
+
+
+def _ball_result(out, alpha, clust_of):
+    """credibleball's dict from the distances of one estimate (partitiondistances' dict); clust_of(i) gives the labels of
+    pooled sample i (or None where they are not held)."""
+    ball = _credibleball(out["dist"][0], out["K"], alpha)
+    for name in ("horizontal", "upper", "lower"):
+        ball[name]["clust"] = clust_of(int(ball[name]["indices"][0]))
+    ball["expectedloss"] = float(_expected(out, None)["expectedloss"][0])
+    ball["dist"] = out["dist"][0]
+    return ball
+
+
+def partitiondistances(refs, samples, loss="VI", device=0):
+    """Distances from reference partitions (one of length n, or nref x n; any positive labels, at most 255 clusters each)
+    to every sample, with the losses of getpointestimate: one contingency table per (reference, sample) on the device
+    (rc_partition_dists).  `samples` is an MCMCResult, a list of them (pooled in list order) or an S x n label array.
+    Returns dict(dist = nref x S, pairs = with loss="binder" the nref x S exact counts of disagreeing pairs, else None,
+    K = clusters per sample)."""
+    code = _loss_code(loss)
+    L = _sample_labels(samples)
+    S, n = L.shape
+    P = _partitions(refs, n, "refs")
+    out = _dists_out(P.shape[0], S, loss)
+    check(lib().rc_partition_dists(ptr(P), P.shape[0], ptr(L), S, n, code, device, ptr(out["dist"]), ptr(out["pairs"]), ptr(out["K"])))
+    return out
+
+
+def expectedloss(partitions, samples, loss="VI", device=0):
+    """Posterior expected loss of given partitions (the MAP sample, a point estimate, a k-medoids clustering, the true labels
+    of a simulation, ...) over the samples: dict(expectedloss = (sum_t d_t) / S per partition, summed in ascending pooled
+    order; totals = with loss="binder" the exact int64 total of disagreeing pairs per partition, else None).  O(S n) per
+    partition, so it scores pooled chains under any of the four losses."""
+    _loss_code(loss)
+    L = _sample_labels(samples)
+    return _expected(partitiondistances(_partitions(partitions, L.shape[1], "partitions"), L, loss, device), loss)
+
+
+def credibleball(estimate, samples, loss="VI", alpha=0.05, device=0):
+    """Credible ball around a point estimate (Wade & Ghahramani 2018, section 4; mcclust.ext::credibleball): the smallest
+    ball in the given loss around `estimate` that holds 1 - alpha of the samples, and its bounds.  Returns dict(radius,
+    inball = samples in the ball, expectedloss of the estimate, dist = the S distances, horizontal / upper / lower =
+    dict(dist, K, indices = pooled sample indices attaining the bound, clust = labels of the first))."""
+    _loss_code(loss)
+    _check_alpha(alpha)
+    L = _sample_labels(samples)
+    out = partitiondistances(_estimate(estimate, L.shape[1]), L, loss, device)
+    return _ball_result(out, alpha, lambda i: L[i].copy())
 
 
 _PAIRWISE_BYTES = 64 << 30          # the S x S fp64 loss matrix of the pairwise MPEL path must stay below this

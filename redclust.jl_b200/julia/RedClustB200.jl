@@ -443,4 +443,94 @@ function convergencediagnostics(results::Vector{MCMCResult}; device::Integer = 0
     return merge(out, (traces = traces,))
 end
 
+# ---- distances from given partitions to the samples: expected loss and credible balls (no reference call; Wade &
+# Ghahramani 2018, Bayesian Analysis 13(2), section 4, as mcclust.ext::credibleball).  Never executed, like the rest of
+# this file; host.py's partitiondistances / expectedloss / credibleball are the tested twins.
+const LOSSCODE = Dict("binder" => 0, "omARI" => 1, "VI" => 2, "ID" => 3)
+
+function _losscode(loss)
+    (loss isa String && haskey(LOSSCODE, loss)) ||
+        throw(ArgumentError("loss must be one of \"binder\", \"omARI\", \"VI\" and \"ID\" (a function-valued loss is not supported here)."))
+    return LOSSCODE[loss]
+end
+
+function _pooled(samples::Union{MCMCResult,Vector{MCMCResult}})
+    res = samples isa MCMCResult ? [samples] : samples
+    isempty(res) && throw(ArgumentError("samples must hold at least one MCMCResult."))
+    clusts = [c for r in res for c in r.clusts]
+    isempty(clusts) && throw(ArgumentError("samples hold no sample."))
+    all(length(c) == length(clusts[1]) for c in clusts) || throw(ArgumentError("the results to pool label different numbers of points."))
+    return clusts
+end
+
+"""
+    partitiondistances(refs, samples; loss = "VI", device = 0) -> (dist, pairs, K)
+
+Distances from reference partitions (a vector of label vectors, at most 255 clusters each) to every sample of an
+MCMCResult or a vector of them (pooled in vector order), with the losses of getpointestimate: one contingency table per
+(reference, sample) on the GPU (rc_partition_dists).  dist is nref x S; pairs, with loss = "binder", the nref x S exact
+counts of disagreeing pairs (else nothing); K the clusters per sample.
+"""
+function partitiondistances(refs::Vector{<:AbstractVector{<:Integer}}, samples::Union{MCMCResult,Vector{MCMCResult}};
+                            loss::String = "VI", device::Integer = 0)
+    code = _losscode(loss)
+    clusts = _pooled(samples)
+    S, n, nref = length(clusts), length(clusts[1]), length(refs)
+    (nref >= 1 && all(length(r) == n for r in refs)) || throw(ArgumentError("refs must label the $n points of the samples."))
+    L = Matrix{Int64}(undef, n, S); P = Matrix{Int64}(undef, n, nref)
+    for j in 1:S; L[:, j] .= clusts[j]; end
+    for j in 1:nref; P[:, j] .= refs[j]; end
+    dist = Matrix{Float64}(undef, S, nref); K = Vector{Int32}(undef, S)
+    pairs = loss == "binder" ? Matrix{Int64}(undef, S, nref) : nothing          # the kernel skips the counts without them
+    GC.@preserve P L dist pairs K check(ccall((:rc_partition_dists, LIB[]), Int32,
+        (Ptr{Int64}, Int64, Ptr{Int64}, Int64, Int64, Int32, Int32, Ptr{Float64}, Ptr{Int64}, Ptr{Int32}),
+        P, nref, L, S, n, code, device, dist, isnothing(pairs) ? C_NULL : pairs, K))
+    return (dist = permutedims(dist), pairs = isnothing(pairs) ? nothing : permutedims(pairs), K = K)
+end
+
+_seqmean(d) = foldl(+, d; init = 0.0) / length(d)          # ascending order from +0.0, as rc_mpel's column sums
+
+"""
+    expectedloss(partitions, samples; loss = "VI", device = 0) -> (expectedloss, totals)
+
+Posterior expected loss of given partitions over the samples: (sum_t d_t) / S per partition, summed in ascending pooled
+order; totals = with loss = "binder" the exact total of disagreeing pairs per partition, else nothing.
+"""
+function expectedloss(partitions::Vector{<:AbstractVector{<:Integer}}, samples::Union{MCMCResult,Vector{MCMCResult}};
+                      loss::String = "VI", device::Integer = 0)
+    out = partitiondistances(partitions, samples; loss = loss, device = device)
+    return (expectedloss = [_seqmean(out.dist[r, :]) for r in 1:size(out.dist, 1)],
+            totals = loss == "binder" ? vec(sum(out.pairs, dims = 2)) : nothing)
+end
+
+"""
+    credibleball(estimate, samples; loss = "VI", alpha = 0.05, device = 0)
+
+Credible ball around a point estimate (Wade & Ghahramani 2018, section 4): radius = the smallest sample distance e with
+#{t: d_t <= e} / S >= 1 - alpha; the ball is every sample with d_t <= radius.  horizontal: the ball's samples at the largest
+distance; upper / lower: among the ball's samples with the fewest / most clusters, those at the largest distance.  Each bound
+is (dist, K, indices = every pooled index attaining it, 1-based ascending, clust = labels of the first).
+"""
+function credibleball(estimate::AbstractVector{<:Integer}, samples::Union{MCMCResult,Vector{MCMCResult}};
+                      loss::String = "VI", alpha::Real = 0.05, device::Integer = 0)
+    _losscode(loss)
+    0 < alpha < 1 || throw(ArgumentError("alpha must lie in (0, 1)."))
+    clusts = _pooled(samples)
+    length(estimate) == length(clusts[1]) || throw(ArgumentError("estimate must label the $(length(clusts[1])) points of the samples."))
+    out = partitiondistances([estimate], samples; loss = loss, device = device)
+    d, K = out.dist[1, :], out.K
+    S = length(d)
+    ds = sort(d)
+    radius = ds[findfirst(e -> searchsortedlast(ds, e) / S >= 1 - alpha, ds)]   # O(S log S), as host.py's searchsorted
+    inball = d .<= radius
+    function bound(mask)
+        far = maximum(d[mask])
+        idx = findall(mask .& (d .== far))
+        return (dist = far, K = Int(K[idx[1]]), indices = idx, clust = clusts[idx[1]])
+    end
+    kin = K[inball]
+    return (radius = radius, inball = count(inball), expectedloss = _seqmean(d), dist = d, horizontal = bound(inball),
+            upper = bound(inball .& (K .== minimum(kin))), lower = bound(inball .& (K .== maximum(kin))))
+end
+
 end # module

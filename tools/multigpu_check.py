@@ -1,6 +1,6 @@
 """N-rank check of the sharded paths of SURVEY 8e over NCCL: distance build by row blocks + all_gather, chains sharded
 across GPUs with per-rank int32 PSM counts + one all_reduce of the n x n matrix, MPEL candidates sharded + all_gather,
-and the convergence diagnostics over the chains of every rank.
+the convergence diagnostics and the credible ball over the chains of every rank.
 torchrun --nproc-per-node N tools/multigpu_check.py [n] [chains_per_rank] [iters]
 Rank 0 compares each with the single-process result (all three are bit-equal) and prints timings."""
 import os, sys, time
@@ -77,6 +77,22 @@ if rank == 0:
     print(f"world={world} n={n} chains={cpr * world}: convergencediagnostics_allreduce {dt * 1e3:.1f} ms; "
           f"equal to one process over the same chains: {okc}", flush=True)
     assert okc
+# credible ball over the chains of every rank: each rank's distances to the estimate, one all_gather of {dist, pairs, K}
+for loss in ("VI", "binder"):
+    torch.cuda.synchronize(); dist.barrier()
+    t = time.perf_counter()
+    cb = smp.credibleball_allreduce(lab, loss=loss)
+    torch.cuda.synchronize(); dist.barrier()
+    dt = time.perf_counter() - t
+    if rank == 0:
+        one = make(0, cpr * world, data).credibleball(lab, loss=loss)
+        okb = (np.array_equal(cb["dist"], one["dist"]) and cb["radius"] == one["radius"] and cb["inball"] == one["inball"]
+               and cb["expectedloss"] == one["expectedloss"]
+               and all(np.array_equal(cb[k]["indices"], one[k]["indices"]) and cb[k]["dist"] == one[k]["dist"] and cb[k]["K"] == one[k]["K"]
+                       for k in ("horizontal", "upper", "lower")))
+        print(f"world={world} n={n} chains={cpr * world}: credibleball_allreduce ({loss}) over {cb['dist'].size} samples {dt * 1e3:.1f} ms; "
+              f"equal to one process over the same chains: {okb}", flush=True)
+        assert okb
 # one common set of label vectors on every rank: rank 0's samples, broadcast, then 5 % of the labels reshuffled with a
 # fixed seed so that the samples differ from each other
 S = np.ascontiguousarray(smp.samples(0)["labels"])
