@@ -270,6 +270,26 @@ int32_t rc_partition_dists(const int64_t* refs, int64_t nref, const int64_t* lab
 int32_t rc_sampler_partition_dists(const rc_sampler* s, const int64_t* refs, int64_t nref, int64_t chain0, int64_t nch,
                                    int32_t loss, double* dist_out, int64_t* pairs_out, int32_t* K_out);
 
+/* ---- allocation probabilities to the clusters of an estimate (no reference call; ECR pivot method, Papastamoulis &
+ * Iliopoulos 2010) ----------------------------------------------------------------------------------------------------
+ * The estimate (host, n labels, any positive values, <= 255 clusters) is relabelled in first-appearance order to 1..Kh.
+ * Each sample's clusters are matched to the estimate's by the assignment that maximises the number of agreeing points
+ * (the canonical Hungarian method of rc_align.cu, which fixes the optimum returned on ties); sigma_t(l) = k when sample
+ * cluster l is assigned to estimate cluster k with a non-empty overlap, else 0 (unmatched).
+ * counts_out (n x (Kh + 1) int32): counts_out[i][k - 1] = #{t : sigma_t(c_t(i)) = k}, column Kh the samples in which
+ * point i's cluster was unmatched; every row sums to S.  matched_out (NULL or S int64): the number of agreeing points,
+ * n - matched is the transfer distance.  K_out (NULL or S int32): clusters per sample.  maps_out (NULL or S x 255 bytes):
+ * sigma_t(l) at [t][l - 1], 0 beyond K_t.  S < 1 or S >= 2^31, or a NULL counts_out: RC_ERR_ARG; more than 255 clusters
+ * in the estimate or a table that does not fit shared memory: RC_ERR_SLOTS; buffers beyond the free device memory:
+ * RC_ERR_CUDA with their sizes.                                                                                         */
+int32_t rc_aligned_alloc(const int64_t* estimate, const int64_t* labels, int64_t S, int64_t n, int32_t device,
+                         int32_t* counts_out, int64_t* matched_out, int32_t* K_out, uint8_t* maps_out);
+/* The same over the device-resident samples of chains [chain0, chain0 + nch) (chain-major, sample-minor); no sample is
+ * copied to the host.  RC_ERR_STATE before a run to numiters, RC_ERR_SLOTS when a chain of the range stopped at the slot
+ * capacity, RC_ERR_ARG for a bad range.                                                                                */
+int32_t rc_sampler_aligned_alloc(const rc_sampler* s, const int64_t* estimate, int64_t chain0, int64_t nch,
+                                 int32_t* counts_out, int64_t* matched_out, int32_t* K_out, uint8_t* maps_out);
+
 /* ---- multi-GPU exchange steps (SURVEY.md 8e) -------------------------------------------------------
  * One process per GPU.  The sampler needs no collective (independent chains: chain_offset above).  The three steps
  * that exchange data run over an NCCL communicator owned by an rc_comm handle: rank 0 calls rc_comm_unique_id, the
@@ -289,6 +309,9 @@ int32_t rc_sampler_partition_dists(const rc_sampler* s, const int64_t* refs, int
  *   rc_comm_sampler_partition_dists  rc_sampler_partition_dists over the chains of every rank: the references on every
  *                             rank, ONE all-gather of the per-rank {dist, pairs, K}; the outputs cover every rank's samples
  *                             in rank order (dist_out nref x all samples)
+ *   rc_comm_sampler_aligned_alloc  rc_sampler_aligned_alloc over the chains of every rank: the estimate on every rank,
+ *                             ONE all-reduce of the counts and ONE all-gather of the per-rank {matched, K, maps}; the
+ *                             per-sample outputs cover every rank's samples in rank order
  * psm_out (host, n x n fp64) and counts_dev_out (device, n x n int32) may each be NULL.  Results are bit-equal to the
  * single-GPU entry points.                                                                              */
 typedef struct rc_comm rc_comm;
@@ -306,6 +329,8 @@ int32_t rc_comm_sampler_cocl_rhat(rc_comm* c, const rc_sampler* s, rc_rhat_summa
                                   double* maxdev);
 int32_t rc_comm_sampler_partition_dists(rc_comm* c, const rc_sampler* s, const int64_t* refs, int64_t nref, int32_t loss,
                                         double* dist_out, int64_t* pairs_out, int32_t* K_out);
+int32_t rc_comm_sampler_aligned_alloc(rc_comm* c, const rc_sampler* s, const int64_t* estimate, int32_t* counts_out,
+                                      int64_t* matched_out, int32_t* K_out, uint8_t* maps_out);
 
 #ifdef __cplusplus
 }

@@ -14,6 +14,7 @@ from .host import (Comm, MCMCOptionsList, PriorHyperparamsList, MCMCData, MCMCSt
                    getpointestimate, binderloss, infodist, adjacencymatrix, sortlabels, makematrix, uppertriangle,
                    generatemixture, example_dataset, example_datasets, prettytime, prettynumber, evaluateclustering, summarise, params_from_labels, pair_stats, psm, psm_counts_dev, psm_sharded, mpel_loss_sums, binder_loss_sums, mpel_loss_sums_sharded, cyclic_rows, assemble_cyclic_rows, init_rp, ArgumentError,
                    crossdistances, predictivecoclustering, allocationprobabilities, predictive_from_labels,
-                   convergencediagnostics, cocl_rhat, partitiondistances, expectedloss, credibleball)
+                   convergencediagnostics, cocl_rhat, partitiondistances, expectedloss, credibleball,
+                   alignedallocation)
 from ._lib import RCError, LIB_PATH
 from .prior import fitprior, fitprior2, sampledist, sampleK, kmedoids, kmedoids_device, kmeans

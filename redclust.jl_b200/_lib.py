@@ -91,6 +91,8 @@ SIGNATURES = {
     "rc_sampler_cocl_rhat": (C.c_int32, [_vp, C.c_int64, C.c_int64, _P(rc_rhat_summary), _vp, _vp, _vp]),
     "rc_partition_dists": (C.c_int32, [_vp, C.c_int64, _vp, C.c_int64, C.c_int64, C.c_int32, C.c_int32, _vp, _vp, _vp]),
     "rc_sampler_partition_dists": (C.c_int32, [_vp, _vp, C.c_int64, C.c_int64, C.c_int64, C.c_int32, _vp, _vp, _vp]),
+    "rc_aligned_alloc": (C.c_int32, [_vp, _vp, C.c_int64, C.c_int64, C.c_int32, _vp, _vp, _vp, _vp]),
+    "rc_sampler_aligned_alloc": (C.c_int32, [_vp, _vp, C.c_int64, C.c_int64, _vp, _vp, _vp, _vp]),
     "rc_comm_unique_id": (C.c_int32, [_vp]),
     "rc_comm_init": (C.c_int32, [_vp, C.c_int32, C.c_int32, C.c_int32, _P(_vp)]),
     "rc_comm_info": (C.c_int32, [_vp, _P(C.c_int32), _P(C.c_int32)]),
@@ -103,6 +105,7 @@ SIGNATURES = {
     "rc_comm_sampler_binder_mpel": (C.c_int32, [_vp, _vp, _vp, _P(C.c_int64), _vp]),
     "rc_comm_sampler_cocl_rhat": (C.c_int32, [_vp, _vp, _P(rc_rhat_summary), _vp, _vp, _vp]),
     "rc_comm_sampler_partition_dists": (C.c_int32, [_vp, _vp, _vp, C.c_int64, C.c_int32, _vp, _vp, _vp]),
+    "rc_comm_sampler_aligned_alloc": (C.c_int32, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 
 

@@ -440,6 +440,83 @@ int32_t rc_comm_sampler_partition_dists(rc_comm* c, const rc_sampler* s, const i
   return RC_OK;
 }
 
+// Allocation probabilities to the clusters of an estimate over the samples of every rank (rc_sampler_aligned_alloc over
+// chains sharded over GPUs): every rank holds the estimate and aligns its own samples; ONE all-reduce of the int32 counts
+// and ONE all-gather of the per-rank {matched, K, maps} blocks (8-byte words, padded to the largest rank) give every rank
+// the results of all samples in rank order (= global chain order).  Each sample's assignment comes from the same kernel and
+// the same table as on one GPU, and the counts are integer sums: identical to one GPU over the same chains.  The first
+// exchange carries {samples, their largest K, a hash of the estimate}: every rank then applies the same checks to the same
+// values (the same estimate on every rank, fewer than 2^31 samples in all, the table of the estimate against the largest K
+// of ALL samples fits the shared memory).  The buffers are allocated before a second exchange of the status.
+int32_t rc_comm_sampler_aligned_alloc(rc_comm* c, const rc_sampler* s, const int64_t* estimate, int32_t* counts_out,
+                                      int64_t* matched_out, int32_t* K_out, uint8_t* maps_out) {
+  if (!c || !s || !counts_out) { rc_set_error("rc_comm_sampler_aligned_alloc: needs the handles and counts_out"); return RC_ERR_ARG; }
+  RC_CUDA(cudaSetDevice(c->device));
+  const char* who = "rc_comm_sampler_aligned_alloc";
+  rc_sample_range v;
+  Bufs B;
+  AlignEstimate e;
+  std::vector<int> Kh;
+  int kmax = 0;
+  int local = rc_sampler_range(s, 0, rc_sampler_nchains(s), who, v);
+  if (!local) local = align_estimate(estimate, v.n, who, B, e);
+  if (!local) local = sample_K(v.K, v.R, Kh, &kmax);
+  unsigned long long h = 14695981039346656037ull;             // FNV-1a of the estimate as given
+  if (!local)
+    for (int64_t t = 0; t < v.n; ++t) h = (h ^ (unsigned long long)estimate[t]) * 1099511628211ull;
+  std::vector<long long> all, ok;
+  TRYP(agree_vals(c, local, {local ? 0 : (long long)v.R, kmax, (long long)h}, who, all));
+  int64_t total = 0, per = 0;
+  int kall = 0;
+  for (int q = 0; q < c->world; ++q) {
+    const long long* a = all.data() + 4 * q;
+    total += a[1];
+    per = std::max<int64_t>(per, a[1]);
+    kall = std::max<int>(kall, (int)a[2]);
+    if (a[3] != (long long)h) { rc_set_error("%s: rank %d holds another estimate", who, q); return RC_ERR_ARG; }
+  }
+  PairLaunch p;
+  TRYP(align_check(e, total, kall, who, p));
+  // one rank's block: matched (per words), K (per words), then the maps (per x 255 bytes)
+  const int64_t words = 2 * per + (per * 255 + 7) / 8;
+  AlignDev d;
+  long long* buf = nullptr;                                    // [world + 1][words]: this rank's block, then the gathered ranks
+  local = align_alloc(e, v.R, 8.0 * words * (c->world + 1), "exchange buffers", who, B, d);
+  if (!local) local = B.get(&buf, (size_t)words * (c->world + 1));
+  TRYP(agree(c, local, 0, who, ok));
+  TRYP(align_run(e, p, v.labels, v.K, v.R, d));
+  RC_CUDA(cudaMemset(buf, 0, sizeof(long long) * words));
+  if (v.R > 0) {
+    const std::vector<long long> K64(Kh.begin(), Kh.end());
+    RC_CUDA(cudaMemcpy(buf, d.matched, sizeof(long long) * v.R, cudaMemcpyDeviceToDevice));
+    RC_CUDA(cudaMemcpy(buf + per, K64.data(), sizeof(long long) * v.R, cudaMemcpyHostToDevice));
+    RC_CUDA(cudaMemcpy2D(buf + 2 * per, 255, d.maps, 256, 255, (size_t)v.R, cudaMemcpyDeviceToDevice));
+  }
+  const size_t ncount = (size_t)(e.n * (e.K + 1));
+  const long long* gathered = buf;
+  if (c->world > 1) {
+    if (nccl()->AllReduce(d.counts, d.counts, ncount, ncclInt32, ncclSum, c->comm, c->stream) != ncclSuccess ||
+        nccl()->AllGather(buf, buf + words, (size_t)words, ncclInt64, c->comm, c->stream) != ncclSuccess ||
+        cudaStreamSynchronize(c->stream) != cudaSuccess) {
+      rc_set_error("%s: all-reduce of the counts or all-gather of the per-rank alignments failed", who); return RC_ERR_CUDA;
+    }
+    gathered = buf + words;
+  }
+  RC_CUDA(cudaMemcpy(counts_out, d.counts, sizeof(int) * ncount, cudaMemcpyDeviceToHost));
+  std::vector<long long> hv((size_t)words * c->world);
+  RC_CUDA(cudaMemcpy(hv.data(), gathered, sizeof(long long) * hv.size(), cudaMemcpyDeviceToHost));
+  int64_t off = 0;                                             // rank order = global chain order
+  for (int q = 0; q < c->world; ++q) {
+    const int64_t Rq = all[4 * q + 1];
+    const long long* g = hv.data() + (size_t)words * q;
+    if (matched_out) memcpy(matched_out + off, g, sizeof(long long) * Rq);
+    if (K_out) for (int64_t t = 0; t < Rq; ++t) K_out[off + t] = (int32_t)g[per + t];
+    if (maps_out) memcpy(maps_out + off * 255, g + 2 * per, (size_t)Rq * 255);
+    off += Rq;
+  }
+  return RC_OK;
+}
+
 // MPEL search with the candidate samples dealt cyclically over the ranks (src/pointestimate.jl:49-57): every rank holds
 // all S label vectors, evaluates rows rank, rank + world, ... of the upper triangle of the loss matrix, one all-gather
 // assembles it, the column sums run in ascending row order -- bit-equal to rc_mpel on one GPU.

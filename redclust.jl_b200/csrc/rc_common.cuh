@@ -99,6 +99,28 @@ int sample_K(const int* Kd, int64_t S, std::vector<int>& Kh, int* kmax);
 int partition_dists_run(const PartitionRefs& r, const PairLaunch& p, const uint8_t* L, const int* Kd, int64_t S, int64_t n, double* dist,
                         long long* pairs);
 
+// allocation probabilities to the clusters of an estimate (rc_align.cu).  AlignEstimate: the estimate relabelled and uploaded
+// (bytes 1..K, n points), after align_estimate's checks (more than 255 clusters: RC_ERR_SLOTS).  align_check: 1 <= S < 2^31
+// pooled samples (RC_ERR_ARG) and the table of the estimate against the samples' largest K (pair_geometry).  AlignDev: the
+// device results of R samples (counts n x (K + 1) int32, maps R x 256 bytes with sigma_t(l) at [t][l - 1], matched R
+// int64); align_alloc refuses them, plus extra_bytes of the caller's own buffers (named extra_what), when they do not fit
+// the free device memory, with their sizes.  align_run: zeroes the counts, then k_align_match and k_align_count over R
+// device samples L (bytes 1..K, K on the device in Kd).
+struct AlignEstimate {
+  uint8_t* L;
+  int K;
+  int64_t n;
+};
+struct AlignDev {
+  int* counts;
+  uint8_t* maps;
+  long long* matched;
+};
+int align_estimate(const int64_t* estimate, int64_t n, const char* who, Bufs& B, AlignEstimate& e);
+int align_check(const AlignEstimate& e, int64_t S, int kmax, const char* who, PairLaunch& p);
+int align_alloc(const AlignEstimate& e, int64_t R, double extra_bytes, const char* extra_what, const char* who, Bufs& B, AlignDev& d);
+int align_run(const AlignEstimate& e, const PairLaunch& p, const uint8_t* L, const int* Kd, int64_t R, AlignDev& d);
+
 // split-R-hat of the co-clustering indicators (rc_rhat.cu).  The limits on chains, samples per chain and n; the device
 // buffers of one call (N the pooled counts, Q = sum of squared group counts, Na / Nb one chain's halves, dev = {sum d,
 // max d} per local chain, R the matrix or NULL); pass 1 (N), pass 2 (Q and dev against the N of m groups in all), the

@@ -476,6 +476,34 @@ class Sampler:
         first = sum(sizes[:comm.rank])
         return _ball_result(out, alpha, self._labels_of(lambda i: ((i - first) // S, (i - first) % S) if 0 <= i - first < mine else None))
 
+    def alignedallocation(self, estimate, chain0=0, nch=None, maps=False):
+        """alignedallocation over the recorded samples of chains chain0 .. chain0 + nch - 1 (chain-major), from the
+        device-resident samples (rc_sampler_aligned_alloc)."""
+        est = np.ascontiguousarray(_estimate(estimate, self.data.n))
+        nch = self.nchains - chain0 if nch is None else nch
+        out, clusters = _aligned_out(est, max(nch, 0) * int(lib().rc_sampler_numsamples(self._h)), maps)
+        check(lib().rc_sampler_aligned_alloc(self._h, ptr(est), chain0, nch, ptr(out["counts"]), ptr(out["matched"]),
+                                             ptr(out["K"]), ptr(out["maps"])))
+        return _aligned_result(out, clusters, est)
+
+    def alignedallocation_allreduce(self, estimate, maps=False, group=None, device=None, comm=None):
+        """alignedallocation over the chains of every rank (rc_comm_sampler_aligned_alloc): each rank aligns its own samples,
+        one ncclAllReduce sums the counts and one ncclAllGather assembles the per-sample outputs in rank order, equal to one
+        GPU over the same chains."""
+        est = np.ascontiguousarray(_estimate(estimate, self.data.n))
+        comm = comm or Comm.from_torch(group, self.data.device if device is None else device)
+        mine = self.nchains * int(lib().rc_sampler_numsamples(self._h))
+        if comm.world > 1:
+            import torch.distributed as dist
+            sizes = [None] * comm.world
+            dist.all_gather_object(sizes, mine, group=group)
+        else:
+            sizes = [mine]
+        out, clusters = _aligned_out(est, sum(sizes), maps)
+        check(lib().rc_comm_sampler_aligned_alloc(comm._h, self._h, ptr(est), ptr(out["counts"]), ptr(out["matched"]),
+                                                  ptr(out["K"]), ptr(out["maps"])))
+        return _aligned_result(out, clusters, est)
+
     def _labels_of(self, where):
         """clust_of for _ball_result: where(i) = (chain, sample) of pooled sample i on this sampler, or None.  Each chain's
         labels are copied to the host once (labels only, not the traces)."""
@@ -980,6 +1008,47 @@ def credibleball(estimate, samples, loss="VI", alpha=0.05, device=0):
     L = _sample_labels(samples)
     out = partitiondistances(_estimate(estimate, L.shape[1]), L, loss, device)
     return _ball_result(out, alpha, lambda i: L[i].copy())
+
+
+# ---- allocation probabilities to the clusters of a point estimate (no reference call; the pivot method of the ECR algorithm,
+# Papastamoulis & Iliopoulos 2010, JCGS 19(2), as label.switching::ecr) ----
+def _aligned_out(est, S, maps):
+    """Output arrays of the aligned-allocation calls, and the estimate's labels in first-appearance order (the columns).
+    With more than 255 clusters the library refuses before it writes, so the counts never need more than 256 columns."""
+    first = np.sort(np.unique(est, return_index=True)[1])
+    kh = min(first.size, 255)
+    return dict(counts=np.empty((est.size, kh + 1), np.int32), matched=np.empty(S, np.int64), K=np.empty(S, np.int32),
+                maps=np.empty((S, 255), np.uint8) if maps else None), est[first]
+
+
+def _aligned_result(out, clusters, est):
+    S = out["matched"].size
+    prob = out["counts"] / np.float64(S)
+    col = np.argsort(clusters)[np.unique(est, return_inverse=True)[1]]    # the column of each point's estimate cluster
+    res = dict(prob=prob, clusters=clusters, self=prob[np.arange(est.size), col], counts=out["counts"], matched=out["matched"],
+               K=out["K"])
+    if out["maps"] is not None:
+        res["maps"] = out["maps"]
+    return res
+
+
+def alignedallocation(estimate, samples, maps=False, device=0):
+    """Allocation probabilities of every point to the clusters of a point estimate: each sample's clusters are matched to
+    the estimate's by the assignment that maximises the number of agreeing points (the ECR pivot method, Papastamoulis &
+    Iliopoulos 2010; ties resolved by one canonical Hungarian method), then prob[i, k] = the share of samples in which point
+    i's matched cluster is estimate cluster k.  `samples` is an MCMCResult, a list of them (pooled in list order) or an S x n
+    label array; the estimate takes any positive labels (at most 255 clusters).  Returns dict(prob = n x (K + 1) fp64, the
+    last column the samples in which the point's cluster was unmatched; clusters = the estimate's labels in column order;
+    self = prob[i, column of estimate(i)]; counts = the n x (K + 1) int32 counts, rows summing to S; matched = agreeing points
+    per sample, n - matched the transfer distance; K = clusters per sample; maps = with maps=True the S x 255 uint8
+    sigma_t(l) at [t, l - 1], 0 for unmatched and beyond K_t)."""
+    L = _sample_labels(samples)
+    S, n = L.shape
+    est = np.ascontiguousarray(_estimate(estimate, n))
+    out, clusters = _aligned_out(est, S, maps)
+    check(lib().rc_aligned_alloc(ptr(est), ptr(L), S, n, device, ptr(out["counts"]), ptr(out["matched"]), ptr(out["K"]),
+                                 ptr(out["maps"])))
+    return _aligned_result(out, clusters, est)
 
 
 _PAIRWISE_BYTES = 64 << 30          # the S x S fp64 loss matrix of the pairwise MPEL path must stay below this

@@ -533,4 +533,35 @@ function credibleball(estimate::AbstractVector{<:Integer}, samples::Union{MCMCRe
             upper = bound(inball .& (K .== minimum(kin))), lower = bound(inball .& (K .== maximum(kin))))
 end
 
+"""
+    alignedallocation(estimate, samples; maps = false, device = 0)
+
+Allocation probabilities of every point to the clusters of a point estimate (the ECR pivot method, Papastamoulis &
+Iliopoulos 2010): each sample's clusters are matched to the estimate's by the assignment that maximises the number of
+agreeing points (rc_aligned_alloc; ties resolved by one canonical Hungarian method).  prob is n x (K + 1), the last column
+the samples in which the point's cluster was unmatched; clusters the estimate's labels in column order; self the
+probability of each point's own estimate cluster; counts (rows summing to S), matched (n - matched is the transfer
+distance) and K per sample; maps, with maps = true, the 255 x S sigma_t(l) (0 = unmatched and beyond K_t).
+"""
+function alignedallocation(estimate::AbstractVector{<:Integer}, samples::Union{MCMCResult,Vector{MCMCResult}};
+                           maps::Bool = false, device::Integer = 0)
+    clusts = _pooled(samples)
+    S, n = length(clusts), length(clusts[1])
+    length(estimate) == n || throw(ArgumentError("estimate must label the $n points of the samples."))
+    est = Vector{Int64}(estimate)
+    clusters = unique(est)                                   # first-appearance order: the columns
+    kh = min(length(clusters), 255)                          # more than 255: the library refuses before it writes
+    L = Matrix{Int64}(undef, n, S)
+    for j in 1:S; L[:, j] .= clusts[j]; end
+    counts = Matrix{Int32}(undef, kh + 1, n); matched = Vector{Int64}(undef, S); K = Vector{Int32}(undef, S)
+    M = maps ? Matrix{UInt8}(undef, 255, S) : nothing
+    GC.@preserve est L counts matched K M check(ccall((:rc_aligned_alloc, LIB[]), Int32,
+        (Ptr{Int64}, Ptr{Int64}, Int64, Int64, Int32, Ptr{Int32}, Ptr{Int64}, Ptr{Int32}, Ptr{UInt8}),
+        est, L, S, n, device, counts, matched, K, isnothing(M) ? C_NULL : M))
+    prob = permutedims(counts) ./ S
+    col = Dict(c => k for (k, c) in enumerate(clusters))
+    return (prob = prob, clusters = clusters, self = [prob[i, col[est[i]]] for i in 1:n], counts = permutedims(counts),
+            matched = matched, K = K, maps = M)
+end
+
 end # module

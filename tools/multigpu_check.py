@@ -1,6 +1,6 @@
 """N-rank check of the sharded paths of SURVEY 8e over NCCL: distance build by row blocks + all_gather, chains sharded
 across GPUs with per-rank int32 PSM counts + one all_reduce of the n x n matrix, MPEL candidates sharded + all_gather,
-the convergence diagnostics and the credible ball over the chains of every rank.
+the convergence diagnostics, the credible ball and the aligned allocation over the chains of every rank.
 torchrun --nproc-per-node N tools/multigpu_check.py [n] [chains_per_rank] [iters]
 Rank 0 compares each with the single-process result (all three are bit-equal) and prints timings."""
 import os, sys, time
@@ -93,6 +93,19 @@ for loss in ("VI", "binder"):
         print(f"world={world} n={n} chains={cpr * world}: credibleball_allreduce ({loss}) over {cb['dist'].size} samples {dt * 1e3:.1f} ms; "
               f"equal to one process over the same chains: {okb}", flush=True)
         assert okb
+# allocation probabilities to the estimate's clusters over the chains of every rank: one all_reduce of the counts, one
+# all_gather of {matched, K, maps}
+torch.cuda.synchronize(); dist.barrier()
+t = time.perf_counter()
+al = smp.alignedallocation_allreduce(lab, maps=True)
+torch.cuda.synchronize(); dist.barrier()
+dt = time.perf_counter() - t
+if rank == 0:
+    one = make(0, cpr * world, data).alignedallocation(lab, maps=True)
+    oka = all(np.array_equal(al[k], one[k]) for k in one) and set(al) == set(one)
+    print(f"world={world} n={n} chains={cpr * world}: alignedallocation_allreduce over {al['matched'].size} samples {dt * 1e3:.1f} ms; "
+          f"equal to one process over the same chains: {oka}", flush=True)
+    assert oka
 # one common set of label vectors on every rank: rank 0's samples, broadcast, then 5 % of the labels reshuffled with a
 # fixed seed so that the samples differ from each other
 S = np.ascontiguousarray(smp.samples(0)["labels"])
