@@ -151,6 +151,67 @@ def distm(points):
     return D
 
 
+DIST_TAU = 2.0 ** -6        # rc_dist_unresolved's threshold (rc_math.h)
+
+
+def distm_longdouble(X, Y=None):
+    """sqrt(sum_t (x_it - y_jt)^2) in np.longdouble (x86 extended: 63-bit mantissa), one row at a time: the difference
+    form, free of the Gram form's cancellation.  Y defaults to X."""
+    assert np.finfo(np.longdouble).nmant >= 63, "np.longdouble is no wider than fp64 here"
+    X = np.asarray(X, dtype=np.longdouble)
+    Y = X if Y is None else np.asarray(Y, dtype=np.longdouble)
+    R = np.empty((Y.shape[0], X.shape[0]), dtype=np.longdouble)
+    for i in range(Y.shape[0]):
+        R[i] = np.sqrt(((X - Y[i]) ** 2).sum(axis=1))
+    return R
+
+
+def distm_bound(dim):
+    """Relative error every off-diagonal distance entry must meet: (dim + 4) u / tau, u = 2^-53 (DESIGN section 4)."""
+    return (dim + 4) * 2.0 ** -53 / DIST_TAU
+
+
+def distm_within_bound(D, R, dim):
+    """Largest |D - R| / R over the entries with R > 0, over distm_bound(dim); entries with R == 0 must be exactly 0."""
+    R = np.asarray(R, dtype=np.longdouble)
+    pos = R > 0
+    assert np.all(D[~pos] == 0), "identical points with a non-zero distance"
+    assert np.all(D[pos] > 0), "distinct points with a zero distance"
+    return float((np.abs(np.asarray(D, dtype=np.longdouble)[pos] - R[pos]) / R[pos]).max(initial=0) / distm_bound(dim))
+
+
+def distance_family(name, n, dim, rng):
+    """n x dim points on which the Gram form of the Euclidean distance loses accuracy to a different degree:
+    centred        normal(0, 1);
+    offset1e2/1e4  normal(0, 1) + 1e2 / 1e4 in every coordinate;
+    utm            5e6 + normal(0, 100): projected geographic coordinates in metres (dim 2 in the tests);
+    planted        centred points, pairs at separations 1e-3 ... 1e-9 of their norm;
+    mixed          one coordinate near 1e6 (three distinct values, so many pairs share it), the others near 1e-3;
+    collinear      a + t b for one random a, b."""
+    if name == "centred":
+        return rng.normal(size=(n, dim))
+    if name in ("offset1e2", "offset1e4"):
+        return rng.normal(size=(n, dim)) + float(name[6:])
+    if name == "utm":
+        return 5e6 + 100.0 * rng.normal(size=(n, dim))
+    if name == "planted":
+        X = rng.normal(size=(n, dim))
+        for k, i in enumerate(range(0, n - 1, max(2, n // 8))):
+            u = rng.normal(size=dim)
+            X[i + 1] = X[i] + 10.0 ** -(3 + k % 7) * np.linalg.norm(X[i]) * u / np.linalg.norm(u)
+        return X
+    if name == "mixed":
+        X = 1e-3 * rng.normal(size=(n, dim))
+        X[:, 0] = 1e6 + rng.integers(0, 3, size=n)
+        return X
+    if name == "collinear":
+        return rng.normal(size=dim)[None, :] + rng.uniform(-1, 1, size=n)[:, None] * rng.normal(size=dim)[None, :]
+    raise ValueError(name)
+
+
+DISTANCE_FAMILIES = ("centred", "offset1e2", "offset1e4", "utm", "planted", "mixed", "collinear")
+
+
 def philox(ctr, key):
     c = np.asarray(ctr, np.uint32); k = np.asarray(key, np.uint32); o = np.zeros(4, np.uint32)
     lib().rco_philox(_p(c, C.c_uint32), _p(k, C.c_uint32), _p(o, C.c_uint32))

@@ -543,7 +543,8 @@ void rco_init_rp(const rc_params* P, uint64_t seed, uint64_t chain, double* r, d
 
 // pairwise(Euclidean(), X, dims=2), types.jl:160 / utils.jl:144-145 / prior.jl:51,180.
 // Restates the Gram formulation of Distances.jl 0.10 (not vendored in /root/reference):
-// D_ij = sqrt(max(|x_i|^2 + |x_j|^2 - 2 x_i.x_j, 0)), one triangle mirrored, zero diagonal.
+// D_ij = sqrt(max(|x_i|^2 + |x_j|^2 - 2 x_i.x_j, 0)), one triangle mirrored, zero diagonal; an entry the Gram form
+// cannot resolve is recomputed from the differences (rc_dist_unresolved, Distances.jl's Euclidean(thresh)).
 void rco_distm(const double* X, int64_t dim, int64_t n, double* D) {
   std::vector<double> sq(n);
   for (int64_t i = 0; i < n; ++i) { double a = 0; for (int64_t t = 0; t < dim; ++t) a += X[i * dim + t] * X[i * dim + t]; sq[i] = a; }
@@ -553,6 +554,7 @@ void rco_distm(const double* X, int64_t dim, int64_t n, double* D) {
       double dot = 0;
       for (int64_t t = 0; t < dim; ++t) dot += X[i * dim + t] * X[j * dim + t];
       double v = sq[i] + sq[j] - 2 * dot;
+      if (rc_dist_unresolved(v, sq[i] + sq[j])) v = rc_dist_direct2(X + i * dim, X + j * dim, dim);
       double r = sqrt(v > 0 ? v : 0.0);
       D[i * n + j] = r; D[j * n + i] = r;
     }

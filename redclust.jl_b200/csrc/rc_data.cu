@@ -103,11 +103,13 @@ __global__ void __launch_bounds__(256) k_distm(const double* __restrict__ X, con
 #pragma unroll
   for (int q = 0; q < 4; ++q) {
     const int64_t i = i0 + ty + 8 * q, j = j0 + tx;
-    if (i >= n || j >= n) continue;
-    if (i == j) { D[i * n + i] = 0.0; continue; }
-    if (j < i) continue;                        // diagonal tile: lower half comes from the mirror
-    const double v = sq[i] + sq[j] - 2 * acc[q];
-    const double r = sqrt(v > 0.0 ? v : 0.0);
+    if (i >= n || j >= n || j < i) continue;    // diagonal tile: lower half comes from the mirror
+    double r = 0.0;
+    if (i != j) {
+      double v = sq[i] + sq[j] - 2 * acc[q];
+      if (rc_dist_unresolved(v, sq[i] + sq[j])) v = rc_dist_direct2(X + i * dim, X + j * dim, dim);
+      r = sqrt(v > 0.0 ? v : 0.0);
+    }
     D[i * n + j] = r;
     D[j * n + i] = r;
   }
@@ -117,7 +119,7 @@ __global__ void __launch_bounds__(256) k_distm(const double* __restrict__ X, con
 // mma.sync.aligned.m8n8k4.row.col.f64 (DMMA; tcgen05 has no f64 kind).  32x32 output tile per CTA of 4 warps, warp w
 // owns rows 8w..8w+7 and the four 8-column blocks; operands are staged through shared memory in chunks of 32
 // coordinates.  The summation order differs from the sequential kernel above (k-blocks of 4, fused multiply-add inside
-// the tensor core), so this path is checked to 1e-10 relative instead of bit-exactly; symmetry and the zero diagonal
+// the tensor core), so this path is checked against the error bound instead of bit-exactly; symmetry and the zero diagonal
 // stay exact (upper triangle mirrored).
 __global__ void __launch_bounds__(128) k_distm_dmma(const double* __restrict__ X, const double* __restrict__ sq, int64_t dim,
                                                      int64_t n, double* __restrict__ D) {
@@ -156,7 +158,8 @@ __global__ void __launch_bounds__(128) k_distm_dmma(const double* __restrict__ X
       if (i >= n || j >= n) continue;
       if (i == j) { D[i * n + i] = 0.0; continue; }
       if (j < i) continue;
-      const double v = sq[i] + sq[j] - 2 * (h ? c1[nt] : c0[nt]);
+      double v = sq[i] + sq[j] - 2 * (h ? c1[nt] : c0[nt]);
+      if (rc_dist_unresolved(v, sq[i] + sq[j])) v = rc_dist_direct2(X + i * dim, X + j * dim, dim);
       const double r = sqrt(v > 0.0 ? v : 0.0);
       D[i * n + j] = r;
       D[j * n + i] = r;
@@ -227,7 +230,8 @@ __global__ void __launch_bounds__(256) k_distm_rows(const double* __restrict__ X
     if (i >= iend || j >= n) continue;
     double r = 0.0;
     if (i != j) {
-      const double v = (i < j ? sq[i] + sq[j] : sq[j] + sq[i]) - 2 * acc[q];
+      double v = sq[i] + sq[j] - 2 * acc[q];
+      if (rc_dist_unresolved(v, sq[i] + sq[j])) v = rc_dist_direct2(X + i * dim, X + j * dim, dim);
       r = sqrt(v > 0.0 ? v : 0.0);
     }
     Drows[(i - row0) * n + j] = r;
@@ -294,7 +298,8 @@ int32_t rc_data_from_points(const double* X, int64_t dim, int64_t n, int32_t dev
   cudaMemcpy(dX, X, sizeof(double) * (size_t)n * dim, cudaMemcpyHostToDevice);
   k_sqnorm<<<(unsigned)((n + 255) / 256), 256>>>(dX, dim, n, sq);
   const unsigned nb = (unsigned)((n + DT - 1) / DT);
-  // Default: the Gram blocks on the FP64 tensor cores (rc_gram.cu, <= 1e-10 relative to the reference's fixture).
+  // Default: the Gram blocks on the FP64 tensor cores (rc_gram.cu).  Every path is within (dim + 4) u / tau relative of the
+  // exact distance (rc_dist_unresolved, rc_math.h).
   // RCB200_DISTM=exact: the ascending-coordinate kernel whose operation order is the oracle's (bit-equal to it);
   // RCB200_DISTM=dmma32: round 1's 32 x 32-tile DMMA kernel (kept for comparison).
   const char* mode = getenv("RCB200_DISTM");
@@ -322,7 +327,8 @@ int32_t rc_distm_rows_dev(const double* X, int64_t dim, int64_t n, int64_t row0,
     rc_set_error("out of device memory for the points"); cudaFree(dX); cudaFree(sq); return RC_ERR_CUDA;
   }
   cudaMemcpy(dX, X, sizeof(double) * (size_t)n * dim, cudaMemcpyHostToDevice);
-  const char* mode = getenv("RCB200_DISTM");            // same choice as rc_data_from_points: the row block equals its rows bit for bit
+  const char* mode = getenv("RCB200_DISTM");            // default / exact: the row block equals the same rows of rc_data_from_points bit
+                                                        // for bit (dmma32 has no row kernel: its blocks are the exact kernel's rows)
   if (mode && (!strcmp(mode, "exact") || !strcmp(mode, "dmma32"))) {
     k_sqnorm<<<(unsigned)((n + 255) / 256), 256>>>(dX, dim, n, sq);
     k_distm_rows<<<dim3((unsigned)((n + DT - 1) / DT), (unsigned)((nrows + DT - 1) / DT)), 256>>>(dX, sq, dim, n, row0, nrows, (double*)D_rows_dev);

@@ -2,7 +2,8 @@
 // sm_100a fp64 matrix math is the warp-level mma.sync.m8n8k4 -- SASS DMMA.8x8x4; the larger PTX shapes lower to the same
 // instruction):
 //   * pairwise(Euclidean(), X, dims=2) (src/types.jl:160, src/utils.jl:144-145, src/prior.jl:51,180): the Gram block
-//     X_i X_j^T, epilogue sqrt(max(|x_i|^2 + |x_j|^2 - 2 g, 0)), exact zero diagonal, upper-triangle tiles mirrored;
+//     X_i X_j^T, epilogue sqrt(max(|x_i|^2 + |x_j|^2 - 2 g, 0)) (an entry it cannot resolve recomputed from the
+//     differences, rc_math.h), exact zero diagonal, upper-triangle tiles mirrored;
 //   * the oracle co-clustering matrix of generatemixture (src/utils.jl:130-143): sum over 5000 Dirichlet draws of P'P --
 //     a Gram matrix of the stacked posterior rows, accumulated chunk by chunk.
 // One kernel serves both: C tile 128 x 128 per CTA, 8 warps as 2 x 4 (warp tile 64 x 32 = 8 x 4 DMMA tiles, 64 fp64
@@ -120,18 +121,35 @@ __global__ void __launch_bounds__(256, 1) k_gram128(const double* __restrict__ A
 // ---- epilogues -------------------------------------------------------------------------------------------------------
 struct EpiDistImpl : EpiDist {
   int64_t row0, nrows;     // row block [row0, row0 + nrows) of the matrix held by D (row0 = 0, nrows = n for the whole matrix)
+  const double* Xp;        // the padded points (n x Kd): an entry the Gram form cannot resolve is recomputed from them
+  int64_t Kd;              // (the padding adds exact zeros to the direct sum)
   __device__ __forceinline__ void store(double* T, int64_t i0, int64_t j0, bool diag, bool sym, int tid) const {
     // rows of the tile: thread t handles column t % 128 of rows t / 128, t / 128 + 2, ...
     const int c = tid & (GT - 1);
+    bool redo = false;
 #pragma unroll 8
     for (int r = tid >> 7; r < GT; r += 2) {                                // (unrolled: the fp64 square roots of several rows overlap)
       const int64_t il = i0 + r, i = row0 + il, j = j0 + c;                 // il: row within the block
       if (il >= nrows || j >= n) continue;
       double v = 0.0;
-      if (i != j) { const double w = sq[i] + sq[j] - 2 * T[(size_t)r * GTP + c]; v = sqrt(w > 0.0 ? w : 0.0); }
+      if (i != j) {
+        const double s = sq[i] + sq[j], w = s - 2 * T[(size_t)r * GTP + c];
+        v = sqrt(w > 0.0 ? w : 0.0);
+        if (rc_dist_unresolved(w, s)) { v = -1.0; redo = true; }            // marked for the loop below
+      }
       D[il * n + j] = v;
       T[(size_t)r * GTP + c] = v;                                            // the mirror image below copies it (one square root per pair)
     }
+    // the unresolved entries, out of the unrolled loop, so that tiles without any pay only the test (with the direct sum
+    // inside it the kernel took 9 % longer on the bench points, where no entry is recomputed; B200 at 1000 W)
+    if (redo)
+      for (int r = tid >> 7; r < GT; r += 2) {
+        const int64_t il = i0 + r, i = row0 + il, j = j0 + c;
+        if (il >= nrows || j >= n || !(T[(size_t)r * GTP + c] < 0.0)) continue;
+        const double v = sqrt(rc_dist_direct2(Xp + i * Kd, Xp + j * Kd, Kd));
+        D[il * n + j] = v;
+        T[(size_t)r * GTP + c] = v;
+      }
     if (diag || !sym) return;
     __syncthreads();
     // the mirror image: row j0 + c of D, columns i0 + r (r fastest across the threads: column reads of T, pitch 129)
@@ -233,7 +251,7 @@ int rc_distm_dmma(const double* X_dev, int64_t dim, int64_t n, int64_t row0, int
   k_pad_rows<<<1024, 256>>>(X_dev, dim, Kd, n, Xp);
   k_sqnorm_pad<<<(unsigned)((n + 255) / 256), 256>>>(Xp, Kd, n, sq);
   const int nb = (int)((n + GT - 1) / GT);
-  EpiDistImpl epi; epi.sq = sq; epi.D = D_dev; epi.n = n; epi.flags = nullptr; epi.row0 = row0; epi.nrows = nrows;
+  EpiDistImpl epi; epi.sq = sq; epi.D = D_dev; epi.n = n; epi.flags = nullptr; epi.row0 = row0; epi.nrows = nrows; epi.Xp = Xp; epi.Kd = Kd;
   cudaEvent_t e0 = nullptr, e1 = nullptr;
   const bool verbose = getenv("RCB200_VERBOSE") != nullptr;
   if (verbose) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0); }

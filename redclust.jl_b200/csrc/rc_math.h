@@ -219,6 +219,21 @@ RC_HD double rc_min0(double x) {
 // between-cluster dissimilarities, abratio = (alpha, beta) and zgratio = (zeta, gamma) at /root/reference/src/mcmc.jl:17-18,186-187,293-294.
 RC_HD double rc_gamma_lognorm(double shape, double rate) { return shape * rc_log(rate) - rc_lgamma(shape); }
 
+// ---- Euclidean distance entries -------------------------------------------------------------
+// Every distance path computes v = |x_i|^2 + |x_j|^2 - 2 x_i.x_j (the Gram form of Distances.jl's pairwise).  Its
+// rounding error is up to ~dim u (|x_i|^2 + |x_j|^2), which swamps v when the two points are close relative to their
+// norms (offset data such as geographic coordinates, near-duplicates): the Gram form can then return 0 for two distinct
+// points.  An entry with v < tau (|x_i|^2 + |x_j|^2), tau = 2^-6, is recomputed from the differences, as Distances.jl's
+// Euclidean(thresh) does; a kept entry then has relative error <= (dim + 2) u / tau, a recomputed one <= (dim / 2 + 2) u.
+// s = |x_i|^2 + |x_j|^2 (commutes, so the decision does not depend on the operand order).
+RC_HD bool rc_dist_unresolved(double v, double s) { return v < 0x1p-6 * s; }
+// sum_t (x_t - y_t)^2 in ascending coordinates; (x_t - y_t)^2 == (y_t - x_t)^2 bitwise, so it is symmetric too.
+RC_HD double rc_dist_direct2(const double* x, const double* y, int64_t dim) {
+  double a = 0.0;
+  for (int64_t t = 0; t < dim; ++t) { const double d = x[t] - y[t]; a += d * d; }
+  return a;
+}
+
 // ---- fixed-point images of D and log D ------------------------------------------------------
 // Row/cluster sums of D and log D are accumulated as exact 64-bit integers of q-bit fixed-point
 // images (order-independent => identical on CPU and GPU for any tiling).  Block totals for the
