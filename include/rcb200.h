@@ -312,6 +312,11 @@ int32_t rc_sampler_aligned_alloc(const rc_sampler* s, const int64_t* estimate, i
  *   rc_comm_sampler_aligned_alloc  rc_sampler_aligned_alloc over the chains of every rank: the estimate on every rank,
  *                             ONE all-reduce of the counts and ONE all-gather of the per-rank {matched, K, maps}; the
  *                             per-sample outputs cover every rank's samples in rank order
+ * Before its first collective, every entry point exchanges status, n and the values that must agree; disagreement is
+ * RC_ERR_ARG on every rank.  A rank that refuses returns its own error and the others "rank r refused" with its status,
+ * so no rank is left waiting in a collective.  The values that must agree besides n: samples per chain
+ * (cocl_rhat); nref, whether pairs_out is given and the references (partition_dists); the estimate (aligned_alloc); S,
+ * loss and the labels (mpel); dim and the points (data_from_points).  Host arrays are compared through a hash.
  * psm_out (host, n x n fp64) and counts_dev_out (device, n x n int32) may each be NULL.  Results are bit-equal to the
  * single-GPU entry points.                                                                              */
 typedef struct rc_comm rc_comm;

@@ -95,7 +95,7 @@ class Comm:
 
     def __init__(self, unique_id, rank, world, device):
         self._h = C.c_void_p()
-        self.rank, self.world, self.device = rank, world, device
+        self.rank, self.world, self.device, self.group = rank, world, device, None
         idb = np.frombuffer(bytes(unique_id), dtype=np.uint8).copy()
         check(lib().rc_comm_init(ptr(idb), rank, world, device, C.byref(self._h)))
 
@@ -121,10 +121,21 @@ class Comm:
             src = dist.get_global_rank(group, 0) if group is not None else 0
             dist.broadcast_object_list(box, src=src, group=group)
             c = cls(box[0], rank, world, dev)
+            c.group = group
         else:
             c = cls(cls.unique_id(), 0, 1, dev)
         cls._cache[key] = c
         return c
+
+    def all_ranks(self, obj):
+        """obj of every rank in rank order, exchanged over the torch.distributed group of from_torch ([obj] in a world of
+        one)."""
+        if self.world == 1:
+            return [obj]
+        import torch.distributed as dist
+        out = [None] * self.world
+        dist.all_gather_object(out, obj, group=self.group)
+        return out
 
     def close(self):
         L = getattr(_lib, "_lib", None)
@@ -329,11 +340,15 @@ class Sampler:
         nch = self.nchains - chain0 if nch is None else nch
         check(lib().rc_sampler_psm_counts_dev(self._h, chain0, nch, C.c_void_p(counts_ptr)))
 
+    def _comm(self, group, device, comm):
+        """The communicator of an *_allreduce call: comm, else the one of the process group on this sampler's device."""
+        return comm or Comm.from_torch(group, self.data.device if device is None else device)
+
     def psm_allreduce(self, group=None, device=None, comm=None):
         """PSM over the samples of every rank (mcmc.jl:560 across chain shards): per-rank exact int32 co-clustering
         counts stay on the device, ONE ncclAllReduce(sum) of the n x n matrix combines them, then a single divide by
         the global number of samples (rc_comm_sampler_psm)."""
-        comm = comm or Comm.from_torch(group, self.data.device if device is None else device)
+        comm = self._comm(group, device, comm)
         out = np.empty((self.data.n, self.data.n))
         check(lib().rc_comm_sampler_psm(comm._h, self._h, ptr(out), None))
         return out
@@ -366,15 +381,10 @@ class Sampler:
         ncclAllGather of the per-rank totals; equal to one GPU over the same chains.  dict(best = index into the samples
         of all ranks in rank order, sums, totals, and clust / chain / index of the winner on the rank that holds it, None
         on the others)."""
-        comm = comm or Comm.from_torch(group, self.data.device if device is None else device)
+        comm = self._comm(group, device, comm)
         S = int(lib().rc_sampler_numsamples(self._h))
         mine = self.nchains * S
-        if comm.world > 1:
-            import torch.distributed as dist
-            sizes = [None] * comm.world
-            dist.all_gather_object(sizes, mine, group=group)
-        else:
-            sizes = [mine]
+        sizes = comm.all_ranks(mine)
         total = sum(sizes)
         sums, totals, best = np.empty(total), np.empty(total, np.int64), C.c_int64()
         check(lib().rc_comm_sampler_binder_mpel(comm._h, self._h, ptr(sums), C.byref(best), ptr(totals)))
@@ -413,22 +423,13 @@ class Sampler:
         """convergencediagnostics over the chains of every rank (rc_comm_sampler_cocl_rhat): the all-reduced co-clustering
         counts, one ncclAllReduce of the squared group counts and one ncclAllGather of the chain deviations; equal to one
         GPU over the same chains.  chain_meandev / chain_maxdev and the traces cover every rank's chains in rank order."""
-        comm = comm or Comm.from_torch(group, self.data.device if device is None else device)
-        if comm.world > 1:
-            import torch.distributed as dist
-            sizes = [None] * comm.world
-            dist.all_gather_object(sizes, self.nchains, group=group)
-        else:
-            sizes = [self.nchains]
-        n, total = self.data.n, sum(sizes)
+        comm = self._comm(group, device, comm)
+        n, total = self.data.n, sum(comm.all_ranks(self.nchains))
         sm, md, xd = rc_rhat_summary(), np.empty(total), np.empty(total)
         R = np.empty((n, n)) if matrix else None
         check(lib().rc_comm_sampler_cocl_rhat(comm._h, self._h, C.byref(sm), ptr(R), ptr(md), ptr(xd)))
-        tr = self._traces(0, self.nchains)
-        if comm.world > 1:
-            parts = [None] * comm.world
-            dist.all_gather_object(parts, tr, group=group)
-            tr = {k: np.concatenate([p[k] for p in parts]) for k in _TRACES}
+        parts = comm.all_ranks(self._traces(0, self.nchains))
+        tr = {k: np.concatenate([p[k] for p in parts]) for k in _TRACES}
         return _rhat_dict(sm, R, md, xd, {name: _split_rhat(x) for name, x in tr.items()})
 
     def _partition_dists(self, refs, chain0, nch, loss):
@@ -462,15 +463,10 @@ class Sampler:
         _check_alpha(alpha)
         code = _loss_code(loss)
         P = np.ascontiguousarray(_estimate(estimate, self.data.n))
-        comm = comm or Comm.from_torch(group, self.data.device if device is None else device)
+        comm = self._comm(group, device, comm)
         S = int(lib().rc_sampler_numsamples(self._h))
         mine = self.nchains * S
-        if comm.world > 1:
-            import torch.distributed as dist
-            sizes = [None] * comm.world
-            dist.all_gather_object(sizes, mine, group=group)
-        else:
-            sizes = [mine]
+        sizes = comm.all_ranks(mine)
         out = _dists_out(1, sum(sizes), loss)
         check(lib().rc_comm_sampler_partition_dists(comm._h, self._h, ptr(P), 1, code, ptr(out["dist"]), ptr(out["pairs"]), ptr(out["K"])))
         first = sum(sizes[:comm.rank])
@@ -491,15 +487,8 @@ class Sampler:
         one ncclAllReduce sums the counts and one ncclAllGather assembles the per-sample outputs in rank order, equal to one
         GPU over the same chains."""
         est = np.ascontiguousarray(_estimate(estimate, self.data.n))
-        comm = comm or Comm.from_torch(group, self.data.device if device is None else device)
-        mine = self.nchains * int(lib().rc_sampler_numsamples(self._h))
-        if comm.world > 1:
-            import torch.distributed as dist
-            sizes = [None] * comm.world
-            dist.all_gather_object(sizes, mine, group=group)
-        else:
-            sizes = [mine]
-        out, clusters = _aligned_out(est, sum(sizes), maps)
+        comm = self._comm(group, device, comm)
+        out, clusters = _aligned_out(est, sum(comm.all_ranks(self.nchains * int(lib().rc_sampler_numsamples(self._h)))), maps)
         check(lib().rc_comm_sampler_aligned_alloc(comm._h, self._h, ptr(est), ptr(out["counts"]), ptr(out["matched"]),
                                                   ptr(out["K"]), ptr(out["maps"])))
         return _aligned_result(out, clusters, est)
