@@ -81,7 +81,8 @@ int64_t rc_data_n(const rc_data* d);
 int32_t rc_data_copy_dist(const rc_data* d, double* D_out);
 int32_t rc_data_copy_logdist(const rc_data* d, double* logD_out);
 /* Fixed-point scales of the images the sampler streams: Dq = round(D * 2^qD), Lq = round(logD * 2^qL)
- * (largest q <= 50 with n * max|.| * 2^q < 2^61, so that every cluster sum is an exact 64-bit integer). */
+ * (largest q with n * max|.| * 2^q < 2^61, so that every cluster sum is an exact 64-bit integer whose resolution
+ * follows the scale of the data; clamped to [-1022, 1022], 50 for all-zero data). */
 int32_t rc_data_scales(const rc_data* d, int32_t* qD, int32_t* qL);
 /* One row of data.D (the k-medoids++ seeding of the host draws its weights from medoid rows). */
 int32_t rc_data_copy_row(const rc_data* d, int64_t i, double* row_out);

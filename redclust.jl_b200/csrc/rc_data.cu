@@ -193,7 +193,7 @@ int finish_data(rc_data* d) {
   d->mD = mD; d->mL = mL;
   d->qD = rc_choose_q(mD, n);
   d->qL = rc_choose_q(mL, n);
-  if (d->qD < 0 || d->qL < 0) { rc_set_error("dissimilarities too large for the fixed-point image."); return RC_ERR_DOMAIN; }
+  if (d->qD == RC_Q_NONE || d->qL == RC_Q_NONE) { rc_set_error("dissimilarities too large for the fixed-point image."); return RC_ERR_DOMAIN; }
   RC_CUDA(rc_dev_malloc((void**)&d->DL, sizeof(longlong2) * (size_t)n * n));
   k_build_dl<<<grid, 256>>>(d->D, n, d->qD, d->qL, d->DL);
   RC_CUDA(cudaGetLastError());

@@ -12,7 +12,8 @@
 // These replace, for the sampler hot path, the third-party functions the reference calls:
 //   Base.log / Base.exp / Base.log1p (Julia),  SpecialFunctions.loggamma (openlibm lgamma_r)
 //   at /root/reference/src/mcmc.jl:17-20,35,51,73,75,117-121,186-191,223-241,293-297,323-329,
-//   348-351,427-430,448-451 and src/utils.jl:5.  Agreement with libm is ~1 ulp (tests/test_math.py).
+//   348-351,427-430,448-451 and src/utils.jl:5.  Agreement with libm is ~1 ulp
+//   (tests/test_oracle_golden.py::test_math_accuracy).
 #pragma once
 #include <stdint.h>
 #include <math.h>
@@ -252,17 +253,21 @@ RC_HD double rc_dequant128(int64_t hi, uint64_t lo, int q) {
   return d * rc_from_bits((uint64_t)(0x3ff - q) << 52);
 }
 
-// Fixed-point scale: the largest q <= 50 with n * maxabs * 2^q < 2^61 (host side, both the
-// library and the oracle call this so the images are identical).  Returns -1 if none exists.
+// Fixed-point scale: the largest q with n * maxabs * 2^q < 2^61, so that every sum of n image
+// entries fits an int64 and its resolution follows the data's scale (host side, both the library
+// and the oracle call this so the images are identical).  q is clamped to [-1022, 1022] so that
+// 2^q and 2^-q stay normal doubles; the upper clamp binds only for n * maxabs < 2^-961.  All-zero
+// data gets 50.  Returns RC_Q_NONE when n * maxabs is not finite.
+#define RC_Q_NONE INT32_MIN
 #if defined(__CUDACC__)
 __host__
 #endif
 static inline int rc_choose_q(double maxabs, int64_t n) {
   double v = maxabs * (double)n;
-  if (!(v > 0.0)) return 50;
+  if (v == 0.0) return 50;
+  if (!(v > 0.0 && v < RC_INF)) return RC_Q_NONE;
   int e = 0;
   (void)frexp(v, &e);            // v = m * 2^e, m in [0.5, 1)  =>  v < 2^e
   int q = 61 - e;
-  if (q > 50) q = 50;
-  return q < 0 ? -1 : q;
+  return q > 1022 ? 1022 : (q < -1022 ? -1022 : q);
 }

@@ -352,7 +352,7 @@ int new_image(const rc_data* d, const double* Dnew, int64_t m, Bufs& B, longlong
   for (int64_t x = 0; x < m; ++x) {
     hq[x].x = rc_choose_q(std::max(d->mD, hm[x].x), n + 1);   // scales of the augmented data, n + 1 points
     hq[x].y = rc_choose_q(std::max(d->mL, hm[x].y), n + 1);
-    if (hq[x].x < 0 || hq[x].y < 0) { rc_set_error("dissimilarities too large for the fixed-point image."); return RC_ERR_DOMAIN; }
+    if (hq[x].x == RC_Q_NONE || hq[x].y == RC_Q_NONE) { rc_set_error("dissimilarities too large for the fixed-point image."); return RC_ERR_DOMAIN; }
   }
   RC_CUDA(cudaMemcpy(*qdev, hq.data(), sizeof(int2) * (size_t)m, cudaMemcpyHostToDevice));
   int nsm = 148;

@@ -368,7 +368,7 @@ int32_t rc_kmedoids(const rc_data* d, int64_t k, const int64_t* init_medoids, in
   for (long long v : hp) rc_add128(tot, v);
   for (int64_t i = 0; i < n; ++i) assignments[i] = (int64_t)ha[i] + 1;
   for (int64_t c = 0; c < k; ++c) medoids[c] = hmed[c];
-  if (totalcost) *totalcost = ((double)tot.hi * 18446744073709551616.0 + (double)tot.lo) / (double)(1ull << d->qD);
+  if (totalcost) *totalcost = rc_deq128(tot, d->qD);
   if (converged) *converged = conv ? 1 : 0;
   if (iterations) *iterations = it + (conv ? 1 : 0);
   return RC_OK;

@@ -232,8 +232,9 @@ function pairstats(data::MCMCData, labels::Vector{Int})
     check(ccall((:rc_data_scales, LIB[]), Int32, (Ptr{Cvoid}, Ref{Int32}, Ref{Int32}), getfield(data, :handle), qD, qL))
     t = [sum(big.(rows[c, :])) for c in 1:5]
     nA = Int(t[5]); nB = n * (n - 1) ÷ 2 - nA
-    return (nA = nA, sA = Float64(t[1] / big(2)^qD[]), lA = Float64(t[2] / big(2)^qL[]),
-            nB = nB, sB = Float64((t[3] - t[1]) / big(2)^qD[]), lB = Float64((t[4] - t[2]) / big(2)^qL[]))
+    # q may be negative (data of large scale), where big(2)^q throws: one rounding to Float64, then an exact 2^-q
+    return (nA = nA, sA = ldexp(Float64(t[1]), -qD[]), lA = ldexp(Float64(t[2]), -qL[]),
+            nB = nB, sB = ldexp(Float64(t[3] - t[1]), -qD[]), lB = ldexp(Float64(t[4] - t[2]), -qL[]))
 end
 
 "sample_rp(clustsizes, options, params) (src/mcmc.jl:592-636) on the device: the (r, p)-only chain of fitprior."
